@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Gbases/s of the batch-tokenisation hot path on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch: BASELINE.json configs[1], PROTEIN
 `pbeos` batch_tokenize (BOS+EOS+PAD), 65536 ragged sequences of 50..1022 residues, padlen 1024,
@@ -22,6 +22,13 @@ sequences; the path has no collective).  Units are input residues ("bases").
             parity check of the timed GPU batch.
 
 --impl reference times only that CPU arm and prints the same JSON shape.
+
+--dump-outputs DIR writes what the timed call returned in its last step: a fixed sample of DUMP_ROWS rows of the
+(65536, 1024) token matrix as DIR/tokens.npy (float32; token ids are exact) and their indices as DIR/rows.npy
+(float64).  The inputs are seeded, so two builds can be compared output for output.  The reference arm times the
+batch of the GPU arm's last step (rotation index (K - 1) % 4), so the two arms' files can be compared as well.  With
+N > 1 ranks every rank writes tokens_rank<r>.npy / rows_rank<r>.npy for its own shard, DUMP_ROWS // N rows each:
+at most 33.6 MB in all, whatever N.
 """
 import argparse
 import json
@@ -40,6 +47,7 @@ import numpy as np  # noqa: E402
 NSEQ, LO, HI, PADLEN = 65536, 50, 1022, 1024
 KEY, FLAGS = "PROTEIN", dict(bos=True, eos=True, padchar=True)
 ROT = 4
+DUMP_ROWS, DUMP_SEED = 8192, 2024      # 8192 x 1024 float32 = 33.6 MB over all ranks
 WORKLOAD = ("configs[1]: PROTEIN pbeos batch_tokenize (BOS+EOS+PAD), 65536 ragged seqs len 50-1022, "
             "padlen 1024, batch_first, 1-byte tokens, per GPU")
 
@@ -74,6 +82,19 @@ def bench_config(world):
             "tokenizer": "PROTEIN bos+eos+padchar", "batch_first": True, "dtype": "u8", "seed": 102,
             "l2": f"inputs+outputs rotate through {ROT} distinct 103 MB sets (> 126 MB L2)",
             "parallelism": f"{world} ranks, sequences sharded by index (byte-balanced ranges), no collective"}
+
+
+def dump_rows(nseq, world):
+    """The sorted row indices --dump-outputs keeps of one rank's batch: the same for every run with the same batch size
+    and rank count.  Each of the `world` ranks keeps DUMP_ROWS // world rows, so the whole dump stays at DUMP_ROWS rows."""
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(nseq, size=min(nseq, DUMP_ROWS // world), replace=False))
+
+
+def dump_outputs(d, rows, tokens, rank, world):
+    os.makedirs(d, exist_ok=True)
+    sfx = f"_rank{rank}" if world > 1 else ""
+    np.save(os.path.join(d, f"tokens{sfx}.npy"), np.ascontiguousarray(tokens).view(np.uint8).astype(np.float32))
+    np.save(os.path.join(d, f"rows{sfx}.npy"), rows.astype(np.float64))
 
 
 def algorithmic_bytes(nbases, nseq, padlen, itemsize=1, ncols=1):
@@ -165,7 +186,7 @@ def cpu_arm(buf, offs, steps, warmup, budget_s=20.0, opt="O3", nthreads=None):
         t0 = time.perf_counter()
         out = fn()
         times.append(time.perf_counter() - t0)
-        if time.perf_counter() - t_begin > budget_s:
+        if budget_s is not None and time.perf_counter() - t_begin > budget_s:
             break
     total = sum(times)
     return {"value": nbases * len(times) / total / 1e9, "unit": "Gbases/s", "cores": used, "kind": kind,
@@ -190,8 +211,11 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    buf, offs = make_batch(102)
-    res, _ = cpu_arm(buf, offs, args.steps, args.warmup, budget_s=120.0, opt=args.ref_opt, nthreads=args.ref_threads or None)
+    buf, offs = make_batch(102 + (args.steps - 1) % ROT)   # the batch of the GPU arm's last timed step
+    res, out = cpu_arm(buf, offs, args.steps, args.warmup, budget_s=None, opt=args.ref_opt, nthreads=args.ref_threads or None)
+    if args.dump_outputs:
+        rows = dump_rows(len(offs) - 1, 1)
+        dump_outputs(args.dump_outputs, rows, np.ascontiguousarray(out)[rows], 0, 1)
     line = {"impl": "reference", "metric": "tokenize_throughput", "value": res["value"], "unit": "Gbases/s",
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": res["ms_per_step"],
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u8", "data": "synthetic",
@@ -331,6 +355,11 @@ def run_ours(args):
     ms_total = ev[0].elapsed_time(ev[1])
     bases_timed = sum(sets[i % ROT]["nbases"] for i in range(args.steps))
     alg_bytes = sum(algorithmic_bytes(sets[i % ROT]["nbases"], sets[i % ROT]["n"], PADLEN) for i in range(args.steps))
+    dumped = None
+    if args.dump_outputs:   # copied out now, written once every timed section is over
+        final = sets[(args.steps - 1) % ROT]
+        rows = dump_rows(final["n"], world)
+        dumped = (rows, final["out"][torch.from_numpy(rows).cuda()].cpu().numpy())
 
     # ---- the same HBM traffic as a plain device-to-device copy, in the same run, rotated the same way -------------
     # (cudaMemcpyAsync of half the step's algorithmic bytes: reads n and writes n.)  What a 103 MB launch can reach at
@@ -574,6 +603,8 @@ def run_ours(args):
                                                             "h2d_GBs_all_ranks": c5f_h2d / c5f_ms_reg / 1e6},
                                    parity_sampled_chunk_every_rank=c5f_parity)
         print(json.dumps(line), flush=True)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, *dumped, rank, world)
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
@@ -1194,7 +1225,11 @@ def main():
                     help="configs[4] at full size (8 M sequences per GPU streamed from a FlatFile): auto = only at --gpus 8")
     ap.add_argument("--sections", default="value,e2e,extra,frows,cpu,c4,c5",
                     help="comma list of measurement sections to run (profiling runs use --sections value)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's tokens to DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

@@ -1,9 +1,13 @@
 """Shared helpers for the parity tests (test infrastructure; may import oracle/)."""
 import hashlib
+import json
+import os
 
 import numpy as np
 
 from bioseq_b200.synth import gen, gen_mask, as_list  # noqa: F401
+
+REFERENCE_JSON = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference.json")
 
 
 def sha(a):
@@ -36,3 +40,68 @@ def golden_inputs(rec):
     assert sha(buf) == rec["buf_sha"] and sha(offs) == rec["offs_sha"], "synthetic generator drifted"
     mask = gen_mask(rec["mask_seed"], buf.size) if "mask_seed" in rec else None
     return buf, offs, mask
+
+
+def _plain(x):
+    if isinstance(x, (bytes, bytearray, memoryview)):
+        return bytes(x)
+    if isinstance(x, (list, tuple)):
+        return [_plain(v) for v in x]
+    if isinstance(x, np.integer):
+        return int(x)
+    return x
+
+
+def digest(x):
+    """Arrays: item size, shape and SHA-256 of the raw bytes (the terms of assert_same_bits); anything else (text,
+    lists of strings or bytes, numbers, error messages): SHA-256 of its repr."""
+    if isinstance(x, np.ndarray):
+        a = np.ascontiguousarray(x)
+        return f"{a.itemsize}:{'x'.join(map(str, a.shape))}:{sha(a)}"
+    return "repr:" + hashlib.sha256(repr(_plain(x)).encode("utf-8", "surrogatepass")).hexdigest()[:16]
+
+
+class Reference:
+    """What the original project's compiled tokenizer (oracle/_ref, built by `make -C oracle ref` from its sources)
+    returned at each comparison of one test, in call order, kept as digests in tests/golden/reference.json so that the
+    comparison runs without it.  When oracle/_ref is present the live reference is compared as well.
+
+    BSQ_RECORD_REFERENCE=<file> rewrites the test's entry of that file (created from tests/golden/reference.json) from
+    the outputs the test compares instead of checking them.  It needs oracle/_ref: each recorded output must first
+    equal the live reference's, so what is recorded is the reference's output."""
+
+    def __init__(self, test, ref_module):
+        self.test, self.live = test, ref_module is not None
+        self.record_to = os.environ.get("BSQ_RECORD_REFERENCE")
+        assert self.live or not self.record_to, "BSQ_RECORD_REFERENCE needs the compiled reference (make -C oracle ref)"
+        with open(REFERENCE_JSON) as f:
+            self.want = json.load(f)["tests"].get(test, [])
+        self.got = []
+
+    def check(self, ours, reference):
+        """`ours`: this project's output; `reference`: a call that returns the reference's (made only when oracle/_ref
+        is present).  Returns the reference's output, or None."""
+        d = digest(ours)
+        where = f"{self.test}, comparison {len(self.got)}"
+        theirs = None
+        if self.live:
+            theirs = reference()
+            if isinstance(ours, np.ndarray) and isinstance(theirs, np.ndarray):
+                assert_same_bits(theirs, ours)
+            assert digest(theirs) == d, f"{where}: reference {digest(theirs)}, ours {d}"
+        if not self.record_to:
+            assert len(self.got) < len(self.want), f"{self.test}: more comparisons than recorded"
+            assert d == self.want[len(self.got)], f"{where}: recorded reference {self.want[len(self.got)]}, ours {d}"
+        self.got.append(d)
+        return theirs
+
+    def done(self):
+        if self.record_to:
+            path = self.record_to if os.path.exists(self.record_to) else REFERENCE_JSON
+            with open(path) as f:
+                rec = json.load(f)
+            rec["tests"][self.test] = self.got
+            with open(self.record_to, "w") as f:
+                json.dump(rec, f, indent=0, sort_keys=True)
+        else:
+            assert len(self.got) == len(self.want), f"{self.test}: {len(self.got)} comparisons, {len(self.want)} recorded"

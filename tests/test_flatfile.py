@@ -2,9 +2,10 @@
 
 CPU: the file writer/reader of libbsq (bsq_flatfile_*) and the `cbioseq.FlatFile` class against
 (1) tests/golden/flatfile.json -- exact bytes the reference's FlatFile wrote for each input,
-(2) the Python restatement in oracle/oracle.py, (3) the compiled reference itself when
-oracle/_ref is present.  GPU: batches taken straight from a FlatFile (mapped and pinned)
-against the oracle tokenizer on the same sequences.
+(2) the Python restatement in oracle/oracle.py, (3) on random inputs, the reference's outputs
+recorded in tests/golden/reference.json, and the compiled reference itself when oracle/_ref is
+present.  GPU: batches taken straight from a FlatFile (mapped and pinned) against the oracle
+tokenizer on the same sequences.
 """
 import gzip
 import json
@@ -17,6 +18,7 @@ import pytest
 from bioseq_b200 import cbioseq
 from oracle.oracle import parse_fastx, flatfile_image, load_ref, OracleTokenizer, pack
 from oracle.fastx_cases import cases, random_fastx
+from helpers import Reference
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -117,31 +119,36 @@ def test_access_forms(tmp_path):
 
 def test_against_compiled_reference(tmp_path):
     R = load_ref()
-    if R is None or not hasattr(R, "FlatFile"):
-        pytest.skip("oracle/_ref not built")
+    rec = Reference("test_flatfile::test_against_compiled_reference", R)
     rng = random.Random(7)
+
+    def walk(f):
+        try:
+            return [bytes(x.seq) for x in f]
+        except IndexError:   # the reference's iterator never meets its end on an empty file; mirrored
+            return "IndexError"
+
     for i in range(300):
         data = random_fastx(rng)
         gz = i % 7 == 0
         src = write_input(tmp_path, "r.fa", data, gz)
         a, b = str(tmp_path / "ref.ff"), str(tmp_path / "our.ff")
-        made = R.FlatFile(src, a)
-        del made
+
+        def ref_file():
+            R.FlatFile(src, a)   # written out when the object goes
+            return open(a, "rb").read()
+
         ours = cbioseq.FlatFile(src, b)
-        assert open(a, "rb").read() == open(b, "rb").read(), data
-        assert open(a, "rb").read() == flatfile_image(parse_fastx(data)), data
-        ref = R.FlatFile(a)
-        assert (ref.nseqs(), ref.seq_offset(), ref.maxseqlen) == (ours.nseqs(), ours.seq_offset(), ours.maxseqlen)
-        assert ref.access(0, ref.nseqs()) == ours.access(0, ours.nseqs())
-        if ref.nseqs() > 0:
-            assert [bytes(x.seq) for x in ref] == [bytes(x.seq) for x in ours]
-        else:   # the reference's iterator never meets its end on an empty file; mirrored
-            for f in (ref, ours):
-                with pytest.raises(IndexError):
-                    [x.seq for x in f]
-        assert R.getstats([src])[0].tolist() == cbioseq.getstats([src])[0].tolist()
+        rec.check(open(b, "rb").read(), ref_file)
+        assert open(b, "rb").read() == flatfile_image(parse_fastx(data)), data
+        ref = R and R.FlatFile(a)
+        rec.check((ours.nseqs(), ours.seq_offset(), ours.maxseqlen), lambda: (ref.nseqs(), ref.seq_offset(), ref.maxseqlen))
+        rec.check(ours.access(0, ours.nseqs()), lambda: ref.access(0, ref.nseqs()))
+        rec.check(walk(ours), lambda: walk(ref))
+        rec.check(cbioseq.getstats([src])[0].tolist(), lambda: R.getstats([src])[0].tolist())
         if gz:
             os.remove(src)
+    rec.done()
 
 
 # ------------------------------------------------------------------------------------------ GPU

@@ -11,7 +11,7 @@ pytestmark = pytest.mark.gpu
 import bioseq_b200  # noqa: E402
 from bioseq_b200 import capi  # noqa: E402
 from oracle.oracle import OracleTokenizer, alphabet_keys, load_ref  # noqa: E402
-from helpers import sha, sha_strs, assert_same_bits, golden_inputs, gen, gen_mask, as_list  # noqa: E402
+from helpers import sha, sha_strs, assert_same_bits, golden_inputs, gen, gen_mask, as_list, Reference  # noqa: E402
 
 TORCH_DT = {0: torch.int8, 1: torch.int16, 2: torch.int32, 3: torch.int64, 4: torch.float32, 5: torch.float64}
 MIX = b"ACDEFGHIKLMNPQRSTVWYacdefghiklmnpqrstvwyXBZOUJ*-NnUu .\x00\x7f\x80\xc3\xff"
@@ -357,10 +357,9 @@ def test_decode_errors_and_itemsizes():
 
 def test_single_sequence_onehot_encode():
     R = load_ref()
-    if R is None:
-        pytest.skip("oracle/_ref not present")
+    ref = Reference("test_gpu_parity::test_single_sequence_onehot_encode", R)
     for key, flags in (("DNA", {}), ("DNA", dict(bos=True, eos=True, padchar=True)), ("PROTEIN", dict(eos=True, padchar=True))):
-        ref_t, t = R.Tokenizer(key, **flags), bioseq_b200.Tokenizer(key, **flags)
+        ref_t, t = R and R.Tokenizer(key, **flags), bioseq_b200.Tokenizer(key, **flags)
         for seq in ("ACGT", "", "ACGTACGTAC", b"GATTACA", bytearray(b"CCGG")):
             # len + 1: with BOS + EOS + padchar the EOS row lies at `padlen` itself (ADVICE r1: it must not be zeroed)
             for padlen in (0, 3, 12, len(seq) + 1, len(seq)):
@@ -369,10 +368,9 @@ def test_single_sequence_onehot_encode():
                         t.onehot_encode(seq, padlen)
                     continue
                 for dc in ("f", "B", "H", "i", "d"):
-                    want = ref_t.onehot_encode(seq, padlen, dc)
-                    got = t.onehot_encode(seq, padlen, dc).cpu().numpy()
-                    assert_same_bits(want, got)
-                assert_same_bits(ref_t.onehot_encode(seq, padlen), t.onehot_encode(seq, padlen).cpu().numpy())
+                    ref.check(t.onehot_encode(seq, padlen, dc).cpu().numpy(), lambda: ref_t.onehot_encode(seq, padlen, dc))
+                ref.check(t.onehot_encode(seq, padlen).cpu().numpy(), lambda: ref_t.onehot_encode(seq, padlen))
+    ref.done()
 
 
 # ------------------------------------------------------------------------------------- BASELINE.json sizes
@@ -630,13 +628,11 @@ def test_concurrent_python_threads_share_pool_and_stager():
     assert not errors, errors
 
 
-# ------------------------------------------------------------------------------------- the live reference on the GPU box
+# ------------------------------------------------------------------------------------- the reference on the GPU machine
 def test_oracle_pinned_to_live_reference_on_this_box():
-    """The oracle <-> reference pin of tests/test_oracle.py, run here as well: the driver's GPU test pass selects `-m gpu`
-    only, and it is the reference itself (oracle/_ref, shipped prebuilt) that makes the oracle an oracle."""
+    """The oracle <-> reference pin of tests/test_oracle.py, run in a GPU-only test pass (`-m gpu`) as well: it is the
+    reference (recorded in tests/golden/reference.json; live when oracle/_ref is built) that makes the oracle an oracle."""
     import test_oracle as TO
-    if TO.R is None:
-        pytest.skip("oracle/_ref not present")
     for seed in range(6):
         TO.test_live_reference_tokenize_onehot_decode(seed)
     TO.test_live_reference_str_inputs_utf8()
@@ -649,8 +645,7 @@ def test_gpu_vs_live_reference_dropin_calls(seed):
     bytearray items in, arrays (tokens in both layouts and every dtype, one-hot with and without mask) and decoded
     strings out."""
     R = load_ref()
-    if R is None:
-        pytest.skip("oracle/_ref not present")
+    ref = Reference(f"test_gpu_parity::test_gpu_vs_live_reference_dropin_calls[{seed}]", R)
     rng = np.random.default_rng(4242 + seed)
     keys = [k for k in alphabet_keys() if k != "BYTES"]   # BYTES ids wrap differently by design (DESIGN.md section 5)
     for trial in range(10):
@@ -668,19 +663,18 @@ def test_gpu_vs_live_reference_dropin_calls(seed):
         padlen = hi + 2 + int(rng.integers(0, 40))
         dc = "bhilqfd"[int(rng.integers(7))]
         bf = bool(rng.integers(2))
-        ref_t, t = R.Tokenizer(key, **flags), bioseq_b200.Tokenizer(key, **flags)
-        a = ref_t.batch_tokenize(seqs, padlen=padlen, destchar=dc, batch_first=bf, nthreads=2)
+        ref_t, t = R and R.Tokenizer(key, **flags), bioseq_b200.Tokenizer(key, **flags)
         b = t.batch_tokenize(seqs, padlen=padlen, destchar=dc, batch_first=bf, nthreads=int(rng.integers(1, 9)))
-        assert_same_bits(a, b.cpu().numpy())
+        a = ref.check(b.cpu().numpy(), lambda: ref_t.batch_tokenize(seqs, padlen=padlen, destchar=dc, batch_first=bf, nthreads=2))
         if dc not in "fd":
-            assert ref_t.decode_tokens(a) == t.decode_tokens(b)
+            ref.check(t.decode_tokens(b), lambda: ref_t.decode_tokens(a))
         mask = None
         if rng.integers(2) and n:
             m = gen_mask(int(rng.integers(1 << 30)), buf.size, 0.7)
             mask = [m[offs[i]:offs[i + 1]] for i in range(n)]
-        a = ref_t.batch_onehot_encode(seqs, padlen=padlen, destchar=dc, mask=mask)
         b = t.batch_onehot_encode(seqs, padlen=padlen, destchar=dc, mask=mask)
-        assert_same_bits(a, b.cpu().numpy())
+        ref.check(b.cpu().numpy(), lambda: ref_t.batch_onehot_encode(seqs, padlen=padlen, destchar=dc, mask=mask))
+    ref.done()
 
 
 def test_streamed_items_ranges_and_growth():
