@@ -102,7 +102,8 @@ struct SpanBatches {
 struct SpanParams {
     int64_t ntiles;
     int nbatch;
-    // Tiles beyond a CTA's first (= blockIdx.x) are handed out by an atomic counter, gridDim.x + atomicAdd(ctr, 1):
+    // A CTA's first two tiles are static, blockIdx.x and blockIdx.x + gridDim.x (no atomic result is waited on before
+    // both copies are in flight); the rest are handed out by an atomic counter, 2 * gridDim.x + atomicAdd(ctr, 1):
     // whatever the placement and start time of the CTAs (a programmatically launched grid gets its SM slots as the
     // previous grid drains), the work stays balanced.  ctr[0] = tiles handed out, ctr[1] = CTAs that have seen the end;
     // the last of those resets both for the slot's next launch.  nullptr: static round-robin (tile += gridDim.x).
@@ -113,7 +114,51 @@ struct SpanParams {
     int max_rows;     // row-table entries of a stage
     uint32_t div_mul, div_shift;  // n / padlen = umulhi(n, div_mul) >> div_shift for 0 <= n < 2^31 (span_magic)
     int straddle;     // != 0: a warp's 32 vectors can lie in two rows (padlen % 512 != 0)
+#ifdef BSQ_SPAN_TRACE
+    unsigned long long *trace;  // kSpanTraceWords per CTA (bsq_span_trace_arm), nullptr: not recorded
+#endif
 };
+
+#ifdef BSQ_SPAN_TRACE
+// Timeline probe (tools/span_timeline.py builds the library with -DBSQ_SPAN_TRACE; the shipped build has none of it).
+// Per CTA: words 0-5 %globaltimer at the events below, word 6 %smid, word 7 tiles the CTA took, words 8-13 clock64 at
+// the same events (SM-local: intervals inside one CTA only).  The exit words are maxima over the consumer warps.
+constexpr int kSpanTraceWords = 16;
+enum SpanTraceEvent { kTrEntry = 0, kTrWait = 1, kTrCopy0 = 2, kTrFull0 = 3, kTrStore0 = 4, kTrExit = 5 };
+__device__ __forceinline__ unsigned long long span_globaltimer() {
+    unsigned long long g;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
+    return g;
+}
+__device__ __forceinline__ unsigned span_smid() {
+    unsigned v;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(v));
+    return v;
+}
+__device__ __forceinline__ void span_trace(const SpanParams &q, int ev) {
+    if (q.trace == nullptr) return;
+    unsigned long long *r = q.trace + kSpanTraceWords * blockIdx.x;
+    const unsigned long long g = span_globaltimer(), c = clock64();
+    if (ev == kTrExit) {
+        atomicMax(r + ev, g);
+        atomicMax(r + 8 + ev, c);
+    } else {
+        r[ev] = g;
+        r[8 + ev] = c;
+    }
+}
+__device__ __forceinline__ void span_trace_word(const SpanParams &q, int w, unsigned long long v) {
+    if (q.trace != nullptr) q.trace[kSpanTraceWords * blockIdx.x + w] = v;
+}
+#define BSQ_SPAN_MARK(cond, ev) \
+    do {                        \
+        if (cond) span_trace(q, ev); \
+    } while (0)
+#else
+#define BSQ_SPAN_MARK(cond, ev) \
+    do {                        \
+    } while (0)
+#endif
 
 // Shared-memory loads by 32-bit shared address (the addresses are formed once per tile, outside the vector loop).
 __device__ __forceinline__ uint4 lds128(uint32_t a) {
@@ -281,6 +326,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
 
     // Programmatic dependent launch: the next kernel of the stream may start its prologue now; ours (LUT, mask
     // tables, barriers: no global memory) runs before the previous kernel of the stream has finished.
+    BSQ_SPAN_MARK(threadIdx.x == kSpanConsumers, kTrEntry);
     asm volatile("griddepcontrol.launch_dependents;");
     load_lut(lut, lutp);
     init_tailtab(tab, sp);
@@ -344,51 +390,39 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
             e.b0 = __ldg(offs + c.r1); e.b1 = __ldg(offs + c.r1 + 1);
             return e;
         };
-        // next tile index of this CTA, requested one tile ahead of its use (lane 0 asks, everybody gets the answer)
-        auto next_tile = [&](int64_t tt) -> int64_t {
-            if (q.ctr == nullptr) return tt + gridDim.x;
-            unsigned int v = 0;
-            if (lane == 0) v = atomicAdd(q.ctr, 1u);
-            return static_cast<int64_t>(gridDim.x) + __shfl_sync(0xffffffffu, v, 0);
-        };
         int64_t t = blockIdx.x;  // < ntiles (the grid is never larger)
         Coord cc = coord_of(t);
-        // offsets of this CTA's first tile: into L2 while the previous kernel drains (a prefetch is only a hint,
-        // the real loads come after the wait)
-        const int64_t *offs0 = mb.b[cc.batch].offs;
-        if (16 * lane <= tile_bytes / q.padlen + 2 && cc.r0 + 16 * lane <= mb.b[cc.batch].nseq) asm volatile("prefetch.global.L2 [%0];" ::"l"(offs0 + cc.r0 + 16 * lane));
         const int maxlen = max(q.padlen - sp.bos - sp.eos, 0);
         {
-            // ... and the tile's residues too, from the offsets as they read NOW.  The previous kernel of the stream may
-            // still be producing them, so these values are hints only: they go through L2 (ld.global.cg: nothing stale
-            // can stay in L1), address nothing but an L2 prefetch -- which is dropped when its address is not mapped
-            // (tools/probes/prefetch_probe.cu) -- and are read again for real after the wait.
-            int64_t sa0, sb0, sb1;
-            asm volatile("ld.global.cg.s64 %0, [%1];" : "=l"(sa0) : "l"(offs0 + cc.r0));
-            asm volatile("ld.global.cg.s64 %0, [%1];" : "=l"(sb0) : "l"(offs0 + cc.r1));
-            asm volatile("ld.global.cg.s64 %0, [%1];" : "=l"(sb1) : "l"(offs0 + cc.r1 + 1));
-            const int64_t span = min(max(sb1 - sa0, int64_t(0)), static_cast<int64_t>(q.stage_bytes));
-            (void)sb0;
-            const uintptr_t pa = reinterpret_cast<uintptr_t>(mb.b[cc.batch].bytes + sa0) & ~uintptr_t(15);
-            const uint32_t pn = static_cast<uint32_t>((span + 31) & ~int64_t(15));
-            if (lane == 0 && pn > 0) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pa), "r"(pn) : "memory");
+            // Both static tiles go into L2 while the previous kernel drains (a prefetch is only a hint, the real loads
+            // come after the wait): their offsets, and their residues from the offsets as they read NOW.  The previous
+            // kernel of the stream may still be producing them, so these values are hints only: they go through L2
+            // (ld.global.cg: nothing stale can stay in L1), address nothing but an L2 prefetch -- which is dropped when
+            // its address is not mapped (tools/probes/prefetch_probe.cu) -- and are read again for real after the wait.
+            const int64_t t1 = t + gridDim.x;
+            const Coord pc[2] = {cc, t1 < q.ntiles ? coord_of(t1) : cc};
+            const int npf = t1 < q.ntiles ? 2 : 1;
+            int64_t sa[2] = {0, 0}, sb[2] = {0, 0};
+            for (int k = 0; k < npf; ++k) {
+                const int64_t *o = mb.b[pc[k].batch].offs;
+                if (16 * lane <= pc[k].len / q.padlen + 2 && pc[k].r0 + 16 * lane <= mb.b[pc[k].batch].nseq)
+                    asm volatile("prefetch.global.L2 [%0];" ::"l"(o + pc[k].r0 + 16 * lane));
+                asm volatile("ld.global.cg.s64 %0, [%1];" : "=l"(sa[k]) : "l"(o + pc[k].r0));
+                asm volatile("ld.global.cg.s64 %0, [%1];" : "=l"(sb[k]) : "l"(o + pc[k].r1 + 1));
+            }
+            for (int k = 0; k < npf; ++k) {
+                const int64_t span = min(max(sb[k] - sa[k], int64_t(0)), static_cast<int64_t>(q.stage_bytes));
+                const uintptr_t pa = reinterpret_cast<uintptr_t>(mb.b[pc[k].batch].bytes + sa[k]) & ~uintptr_t(15);
+                const uint32_t pn = static_cast<uint32_t>((span + 31) & ~int64_t(15));
+                if (lane == 0 && pn > 0) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pa), "r"(pn) : "memory");
+            }
         }
         asm volatile("griddepcontrol.wait;" ::: "memory");
+        BSQ_SPAN_MARK(lane == 0, kTrWait);
         SpanEdges cur = load_edges(cc);
-        int64_t tn = next_tile(t);
+        unsigned int ask = 0;  // lane 0: the counter's answer for the tile after the next one, read one iteration later
         uint32_t it = 0;
         for (;; ++it) {
-            // the next tile's edge offsets (and the index of the tile after it) are requested now and consumed one
-            // iteration later: their latency hides behind this tile's barrier wait, copy issue and row table
-            const bool more = tn < q.ntiles;
-            Coord cn = cc;
-            SpanEdges nxt = cur;
-            int64_t tnn = tn;
-            if (more) {
-                cn = coord_of(tn);
-                nxt = load_edges(cn);
-                tnn = next_tile(tn);
-            }
             const int s = static_cast<int>(it % NSTAGE);
             const uint32_t ph = (it / NSTAGE) & 1u;
             const uint8_t *bytes = mb.b[cc.batch].bytes;
@@ -425,6 +459,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
                     bar_expect_tx(s_u32(full + s), nbytes);
                     bulk_load(s_u32(stage + kSpanSlack), reinterpret_cast<const void *>(A_lo), nbytes, s_u32(full + s));
                 }
+                BSQ_SPAN_MARK(it == 0, kTrCopy0);
                 // {first column, bytes to keep of a final partial vector (0: none), vectors, staged bytes}
                 hdr[s] = make_int4(cc.c_first, cc.len & 15, (cc.len + 15) >> 4, static_cast<int>(nbytes));
                 tile_out[s] = mb.b[cc.batch].out + cc.f0;
@@ -433,8 +468,16 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
             for (int i = lane + 32; i < nrows; i += 32) rows[i] = row_entry(i);
             __syncwarp();
             if (lane == 0) bar_arrive(s_u32(full + s));  // release: row table + header visible to whoever sees the phase flip
-            if (!more) break;
-            t = tn; tn = tnn; cc = cn; cur = nxt;
+            // The next tile: static for the first two, then the counter's answer to the request made one iteration ago,
+            // so no atomic result is waited on before both static copies are in flight.  The counter is asked for the
+            // tile after it now, and its edge offsets are loaded for the next iteration.
+            const int64_t tn = (q.ctr == nullptr || it == 0) ? t + gridDim.x
+                                                             : 2 * static_cast<int64_t>(gridDim.x) + __shfl_sync(0xffffffffu, ask, 0);
+            if (tn >= q.ntiles) break;
+            if (q.ctr != nullptr && lane == 0) ask = atomicAdd(q.ctr, 1u);
+            t = tn;
+            cc = coord_of(t);
+            cur = load_edges(cc);
         }
         // end of work for this CTA: a stage whose header says so
         {
@@ -446,6 +489,9 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
                 hdr[s] = make_int4(0, 0, -1, 0);
                 bar_arrive(s_u32(full + s));
             }
+#ifdef BSQ_SPAN_TRACE
+            if (lane == 0) span_trace_word(q, 6, span_smid()), span_trace_word(q, 7, it);
+#endif
         }
         // the last CTA to see the end of the tiles re-arms the counter for the next launch that uses this slot
         if (q.ctr != nullptr && lane == 0) {
@@ -482,6 +528,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
         const uint32_t ph = (it / NSTAGE) & 1u;
         const uint32_t rows_a = dyn_a + static_cast<uint32_t>(s * stage_stride + q.stage_bytes);
         bar_wait(s_u32(full + s), ph);
+        BSQ_SPAN_MARK(it == 0 && ctid == 0, kTrFull0);
         const int4 h = hdr[s];
         if (h.z < 0) break;  // no more tiles for this CTA
         uint8_t *const otile = tile_out[s];
@@ -508,6 +555,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
                 const int4 ri = lds128i(rows_a + 16u * rl);  // {shared address of column 0's source byte, bos + len, bos + len + eos, -}
                 if (col >= ri.z) __stcs(reinterpret_cast<uint4 *>(dst), g.padq);
                 else __stcs(reinterpret_cast<uint4 *>(dst), span_row_codes<PRE>(static_cast<uint32_t>(ri.x), ri.y, col, g));
+                BSQ_SPAN_MARK(it == 0 && ctid == 0 && dst == otile, kTrStore0);
             }
         } else {
             // padlen % 16 != 0: vectors stay 16-byte aligned in the flat output, so one vector per row straddles two rows.
@@ -527,6 +575,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
                 } else {
                     __stcs(reinterpret_cast<uint4 *>(dst), span_straddle_general<PRE>(rows_a, rl, col, g));
                 }
+                BSQ_SPAN_MARK(it == 0 && ctid == 0 && dst == otile, kTrStore0);
             }
             if (partial_tail && F == Fsafe) {  // exactly one lane of the CTA: the final vector, bytewise
                 const uint32_t rl = __umulhi(F, g.mul) >> g.shift;  // the row of its first byte (the batch's last row)
@@ -546,6 +595,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
         __syncwarp();
         if (lane == 0) bar_arrive(s_u32(empty + s));
     }
+    BSQ_SPAN_MARK(lane == 0, kTrExit);
 }
 
 
@@ -566,6 +616,10 @@ struct DevInfo {
     std::unordered_map<cudaStream_t, int> pair_of;  // stream -> 2 * pair index + flip
 };
 constexpr int kCtrPairs = 1024;
+
+#ifdef BSQ_SPAN_TRACE
+unsigned long long *g_span_trace = nullptr;  // where the next launches record their timeline (bsq_span_trace_arm)
+#endif
 
 std::mutex g_dev_mu;
 DevInfo &dev_info(int dev) {
@@ -698,6 +752,9 @@ int launch_tokenize_span_many(int device, cudaStream_t st, int nbatch, const uin
     q.stage_bytes = (kSpanSlack + static_cast<int>(vt) * 16 + 32 + kSpanTail + 127) / 128 * 128;
     q.max_rows = (static_cast<int>(std::min<int64_t>(vt * 16 / padlen + 3, max_nseq + 1)) + 7) / 8 * 8;
     span_magic(static_cast<uint32_t>(padlen), &q.div_mul, &q.div_shift);
+#ifdef BSQ_SPAN_TRACE
+    q.trace = g_span_trace;
+#endif
     {
         static int sel_body = span_env("BSQ_SPAN_SEL", 1);
         if (tune) sel_body = span_env("BSQ_SPAN_SEL", 1);
@@ -761,3 +818,12 @@ int launch_tokenize_span(int device, cudaStream_t st, const SeqView &v, int64_t 
 }
 
 }  // namespace bsq
+
+#ifdef BSQ_SPAN_TRACE
+// Traced builds only (not part of include/bsq.h): K1s launches from now on record their per-CTA timeline into `buf`
+// (kSpanTraceWords 64-bit words per CTA, zeroed by the caller); nullptr stops recording.
+extern "C" void bsq_span_trace_arm(void *buf) {
+    std::lock_guard<std::mutex> g(bsq::g_dev_mu);
+    bsq::g_span_trace = static_cast<unsigned long long *>(buf);
+}
+#endif
