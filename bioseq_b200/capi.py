@@ -94,6 +94,8 @@ def lib():
         "bsq_tokenize_host_sharded": (i32, [vp, vp, i32, vp, vp, i64, i64, tokp, i32, i32, i32, vp, vp]),
         "bsq_memcpy_d2d": (i32, [i32, vp, vp, vp, C.c_size_t]),
         "bsq_tokenize_many": (i32, [i32, vp, i32, vp, vp, vp, i64, tokp, i32, i32, vp]),
+        "bsq_tokenize_varlen": (i32, [i32, vp, vp, vp, i64, tokp, i32, vp, vp]),
+        "bsq_varlen_extent_device": (i32, [i32, vp, vp, i64, i64, tokp, C.POINTER(i64), C.POINTER(i64)]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(L, name)
@@ -111,7 +113,8 @@ EXPORTS = ("bsq_abi_version bsq_last_error bsq_launch_count bsq_launch_count_res
            "bsq_flatfile_max_seq_len bsq_flatfile_offsets bsq_flatfile_bytes bsq_flatfile_is_pinned bsq_fastx_lengths "
            "bsq_free bsq_stage_host bsq_stage_release bsq_stager_set_augment bsq_onehot_bcl bsq_embed bsq_augment_blosum62 "
            "bsq_blosum62_thresholds bsq_tokenize_items bsq_onehot_items bsq_fetch_rows bsq_parallel_for "
-           "bsq_tokenize_stream_items bsq_onehot_stream_items bsq_shard_bounds bsq_tokenize_host_sharded bsq_memcpy_d2d bsq_tokenize_many").split()
+           "bsq_tokenize_stream_items bsq_onehot_stream_items bsq_shard_bounds bsq_tokenize_host_sharded bsq_memcpy_d2d bsq_tokenize_many "
+           "bsq_tokenize_varlen bsq_varlen_extent_device").split()
 
 
 def last_error():
@@ -165,6 +168,20 @@ def tokenize_many(device, stream, batches, padlen, tok, batch_first, kind):
     ns = (C.c_int64 * n)(*[int(b[2]) for b in batches])
     pd = (C.c_void_p * n)(*[_ptr(b[3]) for b in batches])
     check(lib().bsq_tokenize_many(device, stream, n, pb, po, ns, padlen, C.byref(tok), int(batch_first), kind, pd))
+
+
+def tokenize_varlen(device, stream, d_bytes, d_offsets, nseq, tok, kind, d_out, d_cu_seqlens):
+    """Packed tokens + int32 cu_seqlens (bsq_tokenize_varlen); d_out holds exactly T elements."""
+    check(lib().bsq_tokenize_varlen(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, C.byref(tok), kind, _ptr(d_out),
+                                    _ptr(d_cu_seqlens)))
+
+
+def varlen_extent_device(device, stream, d_offsets, nseq, tok, nbytes=-1):
+    """-> (T, max_seqlen) of device-resident offsets (bsq_varlen_extent_device: validates them; synchronises)."""
+    total, maxlen = C.c_int64(), C.c_int64()
+    check(lib().bsq_varlen_extent_device(device, stream, _ptr(d_offsets), nseq, nbytes, C.byref(tok), C.byref(total),
+                                         C.byref(maxlen)))
+    return total.value, maxlen.value
 
 
 def onehot(device, stream, d_bytes, d_offsets, d_mask, nseq, padlen, tok, kind, d_out):

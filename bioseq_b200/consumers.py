@@ -10,6 +10,9 @@ Reference counterparts:
   materialised, the kernel writes embedding rows.
 * ``augment_packed`` -- ``bioseq.blosum.augment_seq`` (bioseq/blosum.py:63-87) applied to each sequence of a packed
   batch on the device (the reference mutates Python strings one by one, bioseq/loaders.py:71-73).
+* ``batch_tokenize_varlen`` -- the tokens of ``batch_tokenize(..., batch_first=True)`` without their padding, as one
+  packed stream plus int32 ``cu_seqlens`` (what varlen attention takes), written by one kernel instead of padded
+  tokenize + mask + ``out[mask]``.
 
 All of these call the C ABI (``include/bsq.h``) through ``capi``; torch supplies memory and the stream.
 A *batch* is one of
@@ -19,6 +22,7 @@ A *batch* is one of
 * ``(flatfile, start, stop)`` -- a range of a ``cbioseq.FlatFile`` (its packed form goes to the device as is),
 * a list/tuple of ``str`` / ``bytes`` / ``bytearray`` (packed into pinned memory first, like ``batch_tokenize``).
 """
+import collections
 import threading
 
 import numpy as np
@@ -97,9 +101,10 @@ class _Resolved:
             self.ctx = None
 
 
-def _resolve(batch, device, augment=None):
+def _resolve(batch, device, augment=None, before_stage=None):
     """-> _Resolved.  Host batches are staged (and, with ``augment``, mutated on the device after the copy);
-    device batches are used in place (with ``augment``: a mutated clone)."""
+    device batches are used in place (with ``augment``: a mutated clone).  ``before_stage(host_offsets, n)`` checks a
+    host batch before anything is copied to the device."""
     torch = _torch()
     r = _Resolved()
     r.ctx, r.keep, r.h_offs, r.base = None, [], None, 0
@@ -160,6 +165,8 @@ def _resolve(batch, device, augment=None):
                 raise ValueError("offsets run past the end of bytes")
             hb_ptr = host_b.ctypes.data
             r.keep += [host_b, host_o]
+        if before_stage is not None:
+            before_stage(host_o, n)
         if augment:
             ctx.stager.set_augment(*augment)
         try:
@@ -293,5 +300,69 @@ def batch_tokenize_augmented(tokenizer, batch, padlen=-1, destchar="B", batch_fi
         out = torch.empty(shape, dtype=dtype, device=torch.device("cuda", r.device))
         capi.tokenize(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, padlen, tok, batch_first, kind, out)
         return out
+    finally:
+        r.release()
+
+
+VarlenBatch = collections.namedtuple("VarlenBatch", ["tokens", "cu_seqlens", "max_seqlen"])
+VarlenBatch.__doc__ = """A padding-free token batch: ``tokens`` (1-D, all rows back to back), ``cu_seqlens`` (int32, ``n + 1``
+entries: row ``i`` is ``tokens[cu_seqlens[i]:cu_seqlens[i + 1]]``) and ``max_seqlen`` (int) -- the arguments of varlen
+attention (``flash_attn_varlen_func(q, k, v, cu_seqlens, cu_seqlens, max_seqlen, max_seqlen)``)."""
+
+_INT32_MAX = 2 ** 31 - 1
+
+
+def _varlen_extent_host(h_offs, n, k):
+    """(T, max_seqlen) of host offsets; ValueError on offsets the kernels must not index with, or T > 2^31 - 1."""
+    if n == 0:
+        return 0, 0
+    o = np.asarray(h_offs[:n + 1], dtype=np.int64)
+    lens = np.diff(o)
+    if int(o[0]) < 0:
+        raise ValueError("offsets must start at or after 0")
+    if lens.size and int(lens.min()) < 0:
+        raise ValueError("offsets must be non-decreasing")
+    total = int(o[n]) - int(o[0]) + n * k
+    if total > _INT32_MAX:
+        raise ValueError(f"varlen batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one batch; "
+                         "split the batch")
+    return total, int(lens.max()) + k
+
+
+def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None):
+    """Tokens of every sequence of ``batch`` back to back, without padding: a :class:`VarlenBatch`.
+
+    Row ``i`` (``tokens[cu_seqlens[i]:cu_seqlens[i + 1]]``) equals ``batch_tokenize(batch, padlen=P, batch_first=True,
+    destchar=destchar)[i, :len_i + bos + eos]`` for any large enough ``P``: ``[BOS] residues [EOS]``, no PAD token
+    whatever ``padchar`` is.  ``cu_seqlens[i] = (offsets[i] - offsets[0]) + i * (bos + eos)`` as int32; a batch of more
+    than 2^31 - 1 tokens raises ``ValueError``.  Host batches are sized from their host offsets without synchronising;
+    CUDA batches pay one synchronisation (the extent is read back)."""
+    return _tokenize_varlen(tokenizer, batch, destchar, device)
+
+
+def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None):
+    """batch_tokenize_varlen; ``augment``: BLOSUM62 arguments as ``_augment_args`` makes them (FlatFileDataset)."""
+    torch = _torch()
+    tok = descriptor(tokenizer)
+    kind, dtype = _dtype_of(destchar)
+    k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
+    extent = []
+    r = _resolve(batch, device, augment, before_stage=lambda h_offs, n: extent.extend(_varlen_extent_host(h_offs, n, k)))
+    try:
+        if r.h_offs is None:
+            nbytes = -1
+            if isinstance(batch, tuple) and len(batch) == 2:
+                nbytes = batch[0].numel()
+            total, max_seqlen = capi.varlen_extent_device(r.device, r.stream, r.d_offs, r.nseq, tok, nbytes=nbytes)
+            if total > _INT32_MAX:
+                raise ValueError(f"varlen batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one "
+                                 "batch; split the batch")
+        else:
+            total, max_seqlen = extent
+        dev = torch.device("cuda", r.device)
+        tokens = torch.empty(total, dtype=dtype, device=dev)
+        cu_seqlens = torch.empty(r.nseq + 1, dtype=torch.int32, device=dev)
+        capi.tokenize_varlen(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, tok, kind, tokens, cu_seqlens)
+        return VarlenBatch(tokens, cu_seqlens, max_seqlen)
     finally:
         r.release()

@@ -910,8 +910,10 @@ seqfirst_tok8_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, FastDiv di
 // ------------------------------------------------------------------------------------------
 // out[0] = longest sequence; out[1] = what is wrong with the offsets, if anything: 1 a negative length, 2 offsets[0] < 0,
 // 4 offsets[nseq] > nbytes (nbytes < 0: the size of the byte buffer is not known) -- the kernels index the byte buffer
-// with these offsets, so a bad array must fail here and not read out of bounds.
-__global__ void maxlen_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, unsigned long long *out) {
+// with these offsets, so a bad array must fail here and not read out of bounds.  span (optional): offsets[nseq] -
+// offsets[0], the residue count of a packed token stream (bsq_varlen_extent_device).
+__global__ void maxlen_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, unsigned long long *out,
+                              long long *span) {
     long long best = 0;
     unsigned bad = 0;
     for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq;
@@ -921,6 +923,7 @@ __global__ void maxlen_kernel(const int64_t *__restrict__ offs, int64_t nseq, in
         if (len < 0) bad |= 1u;
         if (i == 0 && offs[0] < 0) bad |= 2u;
         if (i == nseq - 1 && nbytes >= 0 && offs[nseq] > nbytes) bad |= 4u;
+        if (i == nseq - 1 && span != nullptr) *span = static_cast<long long>(offs[nseq] - offs[0]);
     }
     for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
     bad = __reduce_or_sync(0xffffffffu, bad);
@@ -2229,6 +2232,24 @@ int scratch_alloc(int device, void **p, size_t bytes, cudaStream_t st) {
     BSQ_CUDA_TRY(cudaMallocFromPoolAsync(p, bytes, pool, st));
     return BSQ_OK;
 }
+
+// K0 and its read-back: h_res = {longest sequence, error bits, offsets[nseq] - offsets[0]}; fails on bad offsets.
+int reduce_offsets(int device, cudaStream_t st, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, unsigned long long h_res[3]) {
+    BSQ_CUDA_TRY(cudaSetDevice(device));
+    unsigned long long *d_res = nullptr;
+    if (int rc = scratch_alloc(device, reinterpret_cast<void **>(&d_res), 3 * sizeof(*d_res), st)) return rc;
+    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, 3 * sizeof(*d_res), st));
+    const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
+    maxlen_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, d_res, reinterpret_cast<long long *>(d_res + 2));
+    count_launch();
+    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, 3 * sizeof(*d_res), cudaMemcpyDeviceToHost, st));
+    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
+    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
+    if (h_res[1] & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
+    if (h_res[1] & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
+    if (h_res[1] & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
+    return BSQ_OK;
+}
 }  // namespace
 
 int bsq_check_offsets_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, int64_t padlen,
@@ -2237,24 +2258,26 @@ int bsq_check_offsets_device(int device, void *stream, const int64_t *d_offsets,
     if (tok == nullptr) return fail(BSQ_ERR_ARG, "null tokenizer");
     if (padlen <= 0) return fail(BSQ_ERR_ARG, "batch tokenize requires padlen is provded.");
     if (nseq <= 0) return BSQ_OK;
-    BSQ_CUDA_TRY(cudaSetDevice(device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    unsigned long long *d_res = nullptr;
-    if (int rc = scratch_alloc(device, reinterpret_cast<void **>(&d_res), 2 * sizeof(*d_res), st)) return rc;
-    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, 2 * sizeof(*d_res), st));
-    const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
-    maxlen_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, d_res);
-    count_launch();
-    unsigned long long h_res[2] = {0, 0};
-    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, sizeof(h_res), cudaMemcpyDeviceToHost, st));
-    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
-    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
-    if (h_res[1] & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
-    if (h_res[1] & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
-    if (h_res[1] & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
+    unsigned long long h_res[3] = {0, 0, 0};
+    if (int rc = reduce_offsets(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, h_res)) return rc;
     const int64_t tl = static_cast<int64_t>(h_res[0]) + (tok->bos_id >= 0) + (tok->eos_id >= 0);
     if (tl > padlen)
         return fail(BSQ_ERR_TOO_LONG, "seq len + bos + eos > padlen: " + std::to_string(tl) + ", vs padlen " + std::to_string(padlen));
+    return BSQ_OK;
+}
+
+int bsq_varlen_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes,
+                             const bsq_tokenizer *tok, int64_t *total, int64_t *max_seqlen) {
+    bsq::DeviceRestore restore_device;
+    if (tok == nullptr || total == nullptr || max_seqlen == nullptr) return fail(BSQ_ERR_ARG, "null argument");
+    if (nseq < 0 || (nseq > 0 && d_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
+    *total = *max_seqlen = 0;
+    if (nseq == 0) return BSQ_OK;
+    unsigned long long h_res[3] = {0, 0, 0};
+    if (int rc = reduce_offsets(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, h_res)) return rc;
+    const int64_t k = (tok->bos_id >= 0) + (tok->eos_id >= 0);
+    *total = static_cast<int64_t>(h_res[2]) + nseq * k;
+    *max_seqlen = static_cast<int64_t>(h_res[0]) + k;
     return BSQ_OK;
 }
 

@@ -52,15 +52,23 @@ class FlatFileDataset(_dataset_base()):
     (src/tokenize.h:195), so with a BOS/EOS tokenizer a single item is longer than a slice's rows, as in the reference.
     Tensors live on ``device``.
 
+    With ``varlen=True`` a slice is a ``consumers.VarlenBatch`` -- the ``long`` tokens of its sequences back to back,
+    without padding, plus ``cu_seqlens`` and ``max_seqlen`` (what varlen attention takes) -- and a single index is that
+    sequence's unpadded 1-D ``long`` tokens.
+
     ``fetch(index, return_items=True)`` also hands back the raw sequence(s) (bioseq/loaders.py:60-84).  Two quirks of
     the reference's ``fetch`` are NOT reproduced: with ``cnn=True`` and ``return_items=False`` it falls off the end and
     returns ``None``, and without ``cnn`` it ignores ``return_items``; here both modes honour the flag.
     """
 
-    def __init__(self, ff, tokenizer, *, augment=0, augment_frac=0.5, cnn=False, device=None, maskfrac=0.15, seed=13):
+    def __init__(self, ff, tokenizer, *, augment=0, augment_frac=0.5, cnn=False, device=None, maskfrac=0.15, seed=13,
+                 varlen=False):
         super().__init__()
         assert isinstance(ff, cbioseq.FlatFile)
         assert isinstance(tokenizer, cbioseq.Tokenizer)
+        if varlen and cnn:
+            raise ValueError("FlatFileDataset: varlen=True yields tokens, cnn=True one-hot; choose one")
+        self.varlen = bool(varlen)
         self.ff, self.tokenizer = ff, tokenizer
         self.seed, self._draw = int(seed), 0  # the reference seeds its generator with 13 (bioseq/loaders.py:49-50)
         self.maskfrac, self.augment, self.augment_frac, self.cnn, self.device = maskfrac, augment, augment_frac, cnn, device
@@ -102,6 +110,10 @@ class FlatFileDataset(_dataset_base()):
                 return consumers.batch_onehot_encode_bcl(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
                                                          destchar='f', device=self.device, **aug)[0].t()
             return self.tokenizer.onehot_encode(bytes(self.ff[start]), padlen=self.max_seq_len, destchar='f', device=self.device)
+        if self.varlen:
+            vb = consumers._tokenize_varlen(self.tokenizer, (self.ff, start, stop), "l", self.device,
+                                            consumers._augment_args(**aug) if aug else None)
+            return vb if many else vb.tokens
         if aug:
             toks = consumers.batch_tokenize_augmented(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
                                                       batch_first=True, destchar='B', device=self.device, **aug).to(torch.long)
@@ -126,7 +138,7 @@ class FlatFileDataset(_dataset_base()):
         return self[slc]
 
     def batches(self, batch_size, prefetch=0):
-        """Consecutive ``(batch, max_seq_len)`` token batches covering the file.
+        """Consecutive ``(batch, max_seq_len)`` token batches (``VarlenBatch``es with ``varlen=True``) covering the file.
 
         ``prefetch=k`` (k > 0) keeps k batches ahead of the consumer on a side stream: the host-to-device copy and the
         tokeniser of batch i+1 .. i+k run while the caller's stream is still busy with batch i (the reference's
@@ -148,7 +160,9 @@ class FlatFileDataset(_dataset_base()):
             t, ev = item
             cur = torch.cuda.current_stream(dev)
             cur.wait_event(ev)
-            t.record_stream(cur)  # (allocated on the side stream, used on the caller's)
+            for x in (t if isinstance(t, tuple) else (t,)):
+                if isinstance(x, torch.Tensor):
+                    x.record_stream(cur)  # (allocated on the side stream, used on the caller's)
             return t
 
         for start in range(0, len(self), batch_size):

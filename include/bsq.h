@@ -137,6 +137,23 @@ int bsq_tokenize(int device, void *stream, const uint8_t *d_bytes, const int64_t
                  int64_t nseq, int64_t padlen, const bsq_tokenizer *tok, int batch_first,
                  int kind, void *d_out);
 
+/* Padding-free tokens: one packed token stream plus int32 cu_seqlens -- the input of varlen attention
+ * (FlashAttention's *_varlen_func), nested / jagged tensors and sequence-packing loaders.  With k = bos + eos:
+ *   d_cu_seqlens[i] = (d_offsets[i] - d_offsets[0]) + i * k for i = 0 .. nseq  (nseq + 1 int32 entries), T = d_cu_seqlens[nseq];
+ *   d_out[cu[i] .. cu[i+1]) = row i of bsq_tokenize (batch-first, any padlen >= its length) without its padding:
+ *   [bos?] lut[residues] (invalid -> 0) [eos?].  No pad id is emitted, whatever tok->padchar says.
+ * d_out holds exactly T `kind` elements and is 16-byte aligned (it may be NULL when T == 0); every element is written
+ * once.  The caller sizes d_out from T, which it knows from host offsets or from bsq_varlen_extent_device, and has
+ * checked that T <= 2^31 - 1 and that the offsets are valid.  Enqueues only (one kernel; nseq == 0: a 4-byte memset).
+ * Capturable into a CUDA graph: the kernel keeps a static tile order and no state between launches. */
+int bsq_tokenize_varlen(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq,
+                        const bsq_tokenizer *tok, int kind, void *d_out, int32_t *d_cu_seqlens);
+/* The extent of that output for device-resident offsets: *total = T and *max_seqlen = longest sequence + k (0 for
+ * nseq == 0), from one reduction kernel and one read-back (synchronises `stream`).  Validates the offsets like
+ * bsq_check_offsets_device (BSQ_ERR_ARG: negative length, offsets[0] < 0, offsets[nseq] > nbytes when nbytes >= 0). */
+int bsq_varlen_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes,
+                             const bsq_tokenizer *tok, int64_t *total, int64_t *max_seqlen);
+
 /* Several batches that share padlen and tokenizer in one launch (batch-first one-byte tokens; other layouts / element
  * types fall back to one launch per batch): batch k = (d_bytes[k], d_offsets[k], nseq[k]) -> d_out[k].  The reference's
  * per-step callers tokenise small batches (training/cnnpretrain.py:123-125,145, bioseq/decoders.py:505): a 4096 x 1000
