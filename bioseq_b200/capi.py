@@ -15,6 +15,12 @@ OK, ERR_ARG, ERR_TOO_LONG, ERR_BAD_TOKEN, ERR_KEY, ERR_CUDA, ERR_NOMEM, ERR_IO, 
 I8, I16, I32, I64, F32, F64 = range(6)
 
 
+class MLMDesc(C.Structure):
+    """struct bsq_mlm"""
+    _fields_ = [("seed", C.c_uint64), ("seq_index_base", C.c_int64), ("t_select", C.c_uint64), ("t_mask", C.c_uint64),
+                ("t_random", C.c_uint64), ("mask_id", C.c_int64), ("ignore_index", C.c_int64)]
+
+
 class TokenizerDesc(C.Structure):
     """struct bsq_tokenizer"""
     _fields_ = [("lut", C.c_int8 * 256), ("nchars", C.c_int32), ("bos_id", C.c_int32), ("eos_id", C.c_int32),
@@ -96,6 +102,8 @@ def lib():
         "bsq_tokenize_many": (i32, [i32, vp, i32, vp, vp, vp, i64, tokp, i32, i32, vp]),
         "bsq_tokenize_varlen": (i32, [i32, vp, vp, vp, i64, tokp, i32, vp, vp]),
         "bsq_varlen_extent_device": (i32, [i32, vp, vp, i64, i64, tokp, C.POINTER(i64), C.POINTER(i64)]),
+        "bsq_tokenize_mlm": (i32, [i32, vp, vp, vp, i64, i64, tokp, i32, C.POINTER(MLMDesc), vp, vp]),
+        "bsq_tokenize_varlen_mlm": (i32, [i32, vp, vp, vp, i64, tokp, i32, C.POINTER(MLMDesc), vp, vp, vp]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(L, name)
@@ -114,7 +122,7 @@ EXPORTS = ("bsq_abi_version bsq_last_error bsq_launch_count bsq_launch_count_res
            "bsq_free bsq_stage_host bsq_stage_release bsq_stager_set_augment bsq_onehot_bcl bsq_embed bsq_augment_blosum62 "
            "bsq_blosum62_thresholds bsq_tokenize_items bsq_onehot_items bsq_fetch_rows bsq_parallel_for "
            "bsq_tokenize_stream_items bsq_onehot_stream_items bsq_shard_bounds bsq_tokenize_host_sharded bsq_memcpy_d2d bsq_tokenize_many "
-           "bsq_tokenize_varlen bsq_varlen_extent_device").split()
+           "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm").split()
 
 
 def last_error():
@@ -174,6 +182,24 @@ def tokenize_varlen(device, stream, d_bytes, d_offsets, nseq, tok, kind, d_out, 
     """Packed tokens + int32 cu_seqlens (bsq_tokenize_varlen); d_out holds exactly T elements."""
     check(lib().bsq_tokenize_varlen(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, C.byref(tok), kind, _ptr(d_out),
                                     _ptr(d_cu_seqlens)))
+
+
+def mlm_desc(seed, seq_index_base, thresholds, mask_id, ignore_index):
+    """struct bsq_mlm from the integer thresholds (t_select, t_mask, t_random)."""
+    ts, tm, tr = thresholds
+    return MLMDesc(seed & 0xFFFFFFFFFFFFFFFF, seq_index_base, ts, tm, tr, mask_id, ignore_index)
+
+
+def tokenize_mlm(device, stream, d_bytes, d_offsets, nseq, padlen, tok, kind, mlm, d_inputs, d_labels):
+    """Masked inputs + int64 labels, padded batch-first (bsq_tokenize_mlm); ``mlm``: an MLMDesc."""
+    check(lib().bsq_tokenize_mlm(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, padlen, C.byref(tok), kind, C.byref(mlm),
+                                 _ptr(d_inputs), _ptr(d_labels)))
+
+
+def tokenize_varlen_mlm(device, stream, d_bytes, d_offsets, nseq, tok, kind, mlm, d_inputs, d_labels, d_cu_seqlens):
+    """Masked inputs + int64 labels, padding-free, + int32 cu_seqlens (bsq_tokenize_varlen_mlm)."""
+    check(lib().bsq_tokenize_varlen_mlm(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, C.byref(tok), kind, C.byref(mlm),
+                                        _ptr(d_inputs), _ptr(d_labels), _ptr(d_cu_seqlens)))
 
 
 def varlen_extent_device(device, stream, d_offsets, nseq, tok, nbytes=-1):

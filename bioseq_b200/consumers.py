@@ -13,6 +13,9 @@ Reference counterparts:
 * ``batch_tokenize_varlen`` -- the tokens of ``batch_tokenize(..., batch_first=True)`` without their padding, as one
   packed stream plus int32 ``cu_seqlens`` (what varlen attention takes), written by one kernel instead of padded
   tokenize + mask + ``out[mask]``.
+* ``batch_tokenize_mlm`` -- a masked-language-model batch (the objective of ``training/cnnpretrain.py:119-125``; BERT /
+  ESM pretraining): masked input tokens and ``cross_entropy``-ready int64 labels, padded or padding-free, written by
+  one kernel instead of tokenize + the HuggingFace-collator recipe in torch (rand, where, index_put, casts).
 
 All of these call the C ABI (``include/bsq.h``) through ``capi``; torch supplies memory and the stream.
 A *batch* is one of
@@ -23,6 +26,8 @@ A *batch* is one of
 * a list/tuple of ``str`` / ``bytes`` / ``bytearray`` (packed into pinned memory first, like ``batch_tokenize``).
 """
 import collections
+import math
+import operator
 import threading
 
 import numpy as np
@@ -340,8 +345,9 @@ def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None):
     return _tokenize_varlen(tokenizer, batch, destchar, device)
 
 
-def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None):
-    """batch_tokenize_varlen; ``augment``: BLOSUM62 arguments as ``_augment_args`` makes them (FlatFileDataset)."""
+def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None, mlm=None):
+    """batch_tokenize_varlen; ``augment``: BLOSUM62 arguments as ``_augment_args`` makes them (FlatFileDataset);
+    ``mlm``: a ``capi.MLMDesc`` -- then ``(VarlenBatch, labels)`` is returned."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
@@ -362,7 +368,103 @@ def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None):
         dev = torch.device("cuda", r.device)
         tokens = torch.empty(total, dtype=dtype, device=dev)
         cu_seqlens = torch.empty(r.nseq + 1, dtype=torch.int32, device=dev)
+        if mlm is not None:
+            labels = torch.empty(total, dtype=torch.int64, device=dev)
+            capi.tokenize_varlen_mlm(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, tok, kind, mlm, tokens, labels, cu_seqlens)
+            return VarlenBatch(tokens, cu_seqlens, max_seqlen), labels
         capi.tokenize_varlen(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, tok, kind, tokens, cu_seqlens)
         return VarlenBatch(tokens, cu_seqlens, max_seqlen)
+    finally:
+        r.release()
+
+
+MLMBatch = collections.namedtuple("MLMBatch", ["inputs", "labels"])
+MLMBatch.__doc__ = """A masked-language-model batch: ``inputs`` (the model's input tokens: a padded ``(n, padlen)`` tensor or a
+:class:`VarlenBatch`) and ``labels`` (int64, the same shape as the tokens: the original token where a position was
+selected, ``ignore_index`` elsewhere) -- ``F.cross_entropy(logits.view(-1, V), labels.view(-1), ignore_index=...)``."""
+
+_TWO32 = 1 << 32
+_INT64_MIN, _INT64_MAX = -(1 << 63), (1 << 63) - 1
+
+
+def _mlm_thresholds(maskfrac=0.15, mask_prob=0.8, random_prob=0.1):
+    """The integer thresholds ``(t_select, t_mask, t_random)`` the kernel compares 32-bit draws with (include/bsq.h,
+    bsq_mlm), computed once in float64.  ValueError unless 0 <= maskfrac <= 1, mask_prob, random_prob >= 0 and
+    mask_prob + random_prob <= 1."""
+    maskfrac, mask_prob, random_prob = float(maskfrac), float(mask_prob), float(random_prob)
+    if not 0.0 <= maskfrac <= 1.0:
+        raise ValueError(f"maskfrac must lie in [0, 1], got {maskfrac}")
+    if not (mask_prob >= 0.0 and random_prob >= 0.0):
+        raise ValueError(f"mask_prob and random_prob must be >= 0, got {mask_prob} and {random_prob}")
+    if not mask_prob + random_prob <= 1.0:
+        raise ValueError(f"mask_prob + random_prob must be <= 1, got {mask_prob + random_prob}")
+    t_select = _TWO32 if maskfrac >= 1.0 else math.floor(maskfrac * _TWO32)
+    t_mask = math.floor(t_select * mask_prob)
+    t_random = min(t_select, math.floor(t_select * (mask_prob + random_prob)))
+    return t_select, t_mask, t_random
+
+
+def _mask_token_limit(destchar):
+    c = destchar[0]
+    if c == "B":
+        return 255
+    return {"b": 127, "h": 32767, "f": 1 << 24}.get(c.lower(), (1 << 31) - 1)
+
+
+def _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignore_index, seed, seq_index_base):
+    """Validate everything and build the capi.MLMDesc (ValueError before anything is staged or launched)."""
+    thresholds = _mlm_thresholds(maskfrac, mask_prob, random_prob)
+    if mask_token is None:
+        mask_token = int(tok.alphabet_size)
+    try:
+        mask_token = operator.index(mask_token)
+        ignore_index = operator.index(ignore_index)
+    except TypeError:
+        raise ValueError("mask_token and ignore_index must be integers") from None
+    limit = _mask_token_limit(destchar)
+    if not 0 <= mask_token <= limit:
+        raise ValueError(f"mask_token {mask_token} is not representable in destchar {destchar!r} (0..{limit}); "
+                         "pass mask_token= explicitly")
+    if not _INT64_MIN <= ignore_index <= _INT64_MAX:
+        raise ValueError(f"ignore_index {ignore_index} does not fit int64")
+    return capi.mlm_desc(int(seed), int(seq_index_base), thresholds, mask_token, ignore_index)
+
+
+def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *, varlen=False, maskfrac=0.15, mask_prob=0.8,
+                       random_prob=0.1, mask_token=None, ignore_index=-100, seed=0, seq_index_base=0, augment=0,
+                       augment_frac=1.0):
+    """A masked-language-model batch in one launch: :class:`MLMBatch` ``(inputs, labels)``.
+
+    ``inputs`` start from ``batch_tokenize(batch, padlen, batch_first=True, destchar=destchar)`` (``varlen=False``:
+    ``(n, padlen)``) or ``batch_tokenize_varlen(batch, destchar)`` (``varlen=True``: a :class:`VarlenBatch`; passing
+    ``padlen`` is then an error).  ``labels`` are int64, shaped like the tokens.  Only residue positions are eligible
+    (never BOS / EOS / PAD).  A residue is selected with probability ``maskfrac``; a selected residue's label is its
+    token, and its input becomes ``mask_token`` (default ``alphabet_size()``, the first id the tokenizer does not
+    use) with probability ``mask_prob``, a uniformly random residue id with probability ``random_prob``, and stays
+    otherwise.  Every other label is ``ignore_index``.
+
+    The draw is Philox4x32-10 keyed by ``seed`` at (``seq_index_base + i``, residue position): the same sequence gets
+    the same mask padded or padding-free, in any slice (the exact rule is documented with ``bsq_tokenize_mlm`` in
+    include/bsq.h).  ``augment``: BLOSUM62 point mutations first (as ``batch_tokenize_augmented``, same seed), then the
+    mask."""
+    torch = _torch()
+    tok = descriptor(tokenizer)
+    kind, dtype = _dtype_of(destchar)
+    mlm = _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignore_index, seed, seq_index_base)
+    augment = _augment_args(augment, augment_frac, seed, seq_index_base)
+    if varlen:
+        if padlen is not None and padlen != -1:
+            raise ValueError("batch_tokenize_mlm(varlen=True) writes no padding: padlen must not be given")
+        vb, labels = _tokenize_varlen(tokenizer, batch, destchar, device, augment, mlm)
+        return MLMBatch(vb, labels)
+    padlen = _default_padlen(batch, tokenizer, padlen)
+    r = _resolve(batch, device, augment)
+    try:
+        _check_lengths(r, padlen, tok, onehot=False)
+        dev = torch.device("cuda", r.device)
+        inputs = torch.empty((r.nseq, padlen), dtype=dtype, device=dev)
+        labels = torch.empty((r.nseq, padlen), dtype=torch.int64, device=dev)
+        capi.tokenize_mlm(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, padlen, tok, kind, mlm, inputs, labels)
+        return MLMBatch(inputs, labels)
     finally:
         r.release()

@@ -304,26 +304,6 @@ const BlosumTab &blosum_tab() {
     return t;
 }
 
-struct Philox {
-    uint32_t c[4];
-};
-__device__ __forceinline__ Philox philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        c0 = hi1 ^ c1 ^ k0;
-        c1 = lo1;
-        c2 = hi0 ^ c3 ^ k1;
-        c3 = lo0;
-        k0 += 0x9E3779B9u;
-        k1 += 0xBB67AE85u;
-    }
-    Philox p;
-    p.c[0] = c0; p.c[1] = c1; p.c[2] = c2; p.c[3] = c3;
-    return p;
-}
-
 constexpr int kMaxTries = 4096;  // the reference retries until the substitution differs (blosum.py:79-82)
 
 // One thread per sequence.  Counter = (sequence index lo, hi, block number, 0), key = seed.

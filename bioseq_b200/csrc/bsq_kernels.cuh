@@ -294,6 +294,28 @@ __device__ __forceinline__ int32_t expand_code(uint32_t code, const Expand &ex) 
     return code < 0x80u ? static_cast<int32_t>(code) : ex.map[code & 3u];
 }
 
+// Philox4x32-10 (Salmon et al., SC'11), the counter-based generator of K7 (BLOSUM62 augmentation, counter word 3 = 0)
+// and K8 (masked-language-model batches, counter word 3 = 1 and 2): one block of four 32-bit words per counter.
+struct Philox {
+    uint32_t c[4];
+};
+__device__ __forceinline__ Philox philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+        c0 = hi1 ^ c1 ^ k0;
+        c1 = lo1;
+        c2 = hi0 ^ c3 ^ k1;
+        c3 = lo0;
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    Philox p;
+    p.c[0] = c0; p.c[1] = c1; p.c[2] = c2; p.c[3] = c3;
+    return p;
+}
+
 #endif  // __CUDACC__
 
 }  // namespace bsq

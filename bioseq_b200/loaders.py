@@ -56,19 +56,27 @@ class FlatFileDataset(_dataset_base()):
     without padding, plus ``cu_seqlens`` and ``max_seqlen`` (what varlen attention takes) -- and a single index is that
     sequence's unpadded 1-D ``long`` tokens.
 
+    With ``mlm=True`` items are masked-language-model batches (``consumers.MLMBatch(inputs, labels)``, one kernel per
+    fetch): a slice gives ``long`` inputs padded to ``max_seq_len`` (or a ``VarlenBatch`` with ``varlen=True``) and int64
+    labels of the same shape, a single index the 1-D pair.  ``maskfrac`` of the residues are selected, 80 / 10 / 10
+    masked (id ``alphabet_size()``) / randomised / kept, labels ``-100`` elsewhere.  Like augmentation, every fetch is a
+    new draw: the mask is keyed by the dataset seed, the draw number and the sequence's index in the file.
+
     ``fetch(index, return_items=True)`` also hands back the raw sequence(s) (bioseq/loaders.py:60-84).  Two quirks of
     the reference's ``fetch`` are NOT reproduced: with ``cnn=True`` and ``return_items=False`` it falls off the end and
     returns ``None``, and without ``cnn`` it ignores ``return_items``; here both modes honour the flag.
     """
 
     def __init__(self, ff, tokenizer, *, augment=0, augment_frac=0.5, cnn=False, device=None, maskfrac=0.15, seed=13,
-                 varlen=False):
+                 varlen=False, mlm=False):
         super().__init__()
         assert isinstance(ff, cbioseq.FlatFile)
         assert isinstance(tokenizer, cbioseq.Tokenizer)
         if varlen and cnn:
             raise ValueError("FlatFileDataset: varlen=True yields tokens, cnn=True one-hot; choose one")
-        self.varlen = bool(varlen)
+        if mlm and cnn:
+            raise ValueError("FlatFileDataset: mlm=True yields masked tokens and labels, cnn=True one-hot; choose one")
+        self.varlen, self.mlm = bool(varlen), bool(mlm)
         self.ff, self.tokenizer = ff, tokenizer
         self.seed, self._draw = int(seed), 0  # the reference seeds its generator with 13 (bioseq/loaders.py:49-50)
         self.maskfrac, self.augment, self.augment_frac, self.cnn, self.device = maskfrac, augment, augment_frac, cnn, device
@@ -99,6 +107,16 @@ class FlatFileDataset(_dataset_base()):
     def __getitem__(self, index):
         import torch
         start, stop, many = self._range(index)
+        if self.mlm:
+            # one draw per fetch, shared by the augmentation (counter word 3 = 0) and the mask (words 1, 2)
+            kw = self._augment_kwargs(start)
+            mb = consumers.batch_tokenize_mlm(self.tokenizer, (self.ff, start, stop),
+                                              padlen=-1 if self.varlen else self.max_seq_len, destchar="l",
+                                              device=self.device, varlen=self.varlen, maskfrac=self.maskfrac,
+                                              mask_token=self.tokenizer.alphabet_size(), **kw)
+            if many:
+                return mb
+            return consumers.MLMBatch(mb.inputs.tokens if self.varlen else mb.inputs[0], mb.labels if self.varlen else mb.labels[0])
         aug = self._augment_kwargs(start) if self.augment else {}
         if self.cnn:
             if many:  # (batch, emb, length) float, written in that layout by one kernel
@@ -138,7 +156,8 @@ class FlatFileDataset(_dataset_base()):
         return self[slc]
 
     def batches(self, batch_size, prefetch=0):
-        """Consecutive ``(batch, max_seq_len)`` token batches (``VarlenBatch``es with ``varlen=True``) covering the file.
+        """Consecutive ``(batch, max_seq_len)`` token batches (``VarlenBatch``es with ``varlen=True``, ``MLMBatch``es with
+        ``mlm=True``) covering the file.
 
         ``prefetch=k`` (k > 0) keeps k batches ahead of the consumer on a side stream: the host-to-device copy and the
         tokeniser of batch i+1 .. i+k run while the caller's stream is still busy with batch i (the reference's
@@ -156,13 +175,18 @@ class FlatFileDataset(_dataset_base()):
         side = torch.cuda.Stream(device=dev)
         ahead = collections.deque()
 
+        def record(x, cur):
+            if isinstance(x, torch.Tensor):
+                x.record_stream(cur)  # (allocated on the side stream, used on the caller's)
+            elif isinstance(x, tuple):  # VarlenBatch, MLMBatch(VarlenBatch, labels), ...
+                for y in x:
+                    record(y, cur)
+
         def hand_over(item):
             t, ev = item
             cur = torch.cuda.current_stream(dev)
             cur.wait_event(ev)
-            for x in (t if isinstance(t, tuple) else (t,)):
-                if isinstance(x, torch.Tensor):
-                    x.record_stream(cur)  # (allocated on the side stream, used on the caller's)
+            record(t, cur)
             return t
 
         for start in range(0, len(self), batch_size):

@@ -154,6 +154,44 @@ int bsq_tokenize_varlen(int device, void *stream, const uint8_t *d_bytes, const 
 int bsq_varlen_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes,
                              const bsq_tokenizer *tok, int64_t *total, int64_t *max_seqlen);
 
+/* Masked-language-model batches (BERT / ESM pretraining): the tokens of bsq_tokenize (batch-first) or
+ * bsq_tokenize_varlen with BERT-style corruption, plus int64 labels, written by one kernel.  Call the unmasked
+ * tokens `tok`.  Only residue positions are eligible -- residue j (0 <= j < len_i) of row i, at column bos + j; BOS, EOS
+ * and PAD are never selected -- and eligibility depends on the position only (an invalid byte is a residue whose token
+ * and label are 0).  With g = seq_index_base + i and u = word (j & 3) of Philox4x32-10 with counter
+ * (g_lo, g_hi, j >> 2, 1) and key (seed_lo, seed_hi):
+ *   u >= t_select              input = tok        label = ignore_index
+ *   u <  t_mask                input = mask_id    label = tok
+ *   t_mask <= u < t_random     input = (w * nchars) >> 32, w = word (j & 3) of the block with counter (g_lo, g_hi,
+ *                              j >> 2, 2)         label = tok
+ *   otherwise                  input = tok        label = tok
+ * Non-residue positions: input = tok, label = ignore_index.  The counters' word 3 (1 and 2) keeps these draws disjoint
+ * from bsq_augment_blosum62's (word 3 = 0) under the same seed, and the mask depends only on (seed, global sequence
+ * index, residue position): not on padlen, the padded or padding-free form, or how the data is sliced.
+ * The thresholds are integers in [0, 2^32] with t_mask <= t_random <= t_select; a caller with fractions computes
+ *   t_select = maskfrac >= 1 ? 2^32 : floor(maskfrac * 2^32),  t_mask = floor(t_select * mask_prob),
+ *   t_random = min(t_select, floor(t_select * (mask_prob + random_prob)))     (in double precision)
+ * so that the rule never depends on floating-point arithmetic on the device.  mask_id must be >= 0 and representable in
+ * `kind`: <= 255 for BSQ_I8 (the byte is written as is), <= 32767 for BSQ_I16, <= 2^24 for BSQ_F32, <= 2^31 - 1
+ * otherwise.  BSQ_ERR_ARG otherwise, or for thresholds out of order. */
+typedef struct bsq_mlm {
+    uint64_t seed;
+    int64_t seq_index_base;
+    uint64_t t_select, t_mask, t_random;
+    int64_t mask_id, ignore_index;
+} bsq_mlm;
+/* Padded: d_inputs is (nseq, padlen) `kind` elements and d_labels (nseq, padlen) int64, batch-first, both 16-byte
+ * aligned; every element is written once.  Lengths must already have been checked, as for bsq_tokenize. */
+int bsq_tokenize_mlm(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq, int64_t padlen,
+                     const bsq_tokenizer *tok, int kind, const bsq_mlm *mlm, void *d_inputs, int64_t *d_labels);
+/* Padding-free: d_inputs and d_labels hold exactly T elements each (T and the caller's checks as for
+ * bsq_tokenize_varlen), aligned element for element; d_cu_seqlens as there.  Both entry points only enqueue work (one
+ * kernel; nseq == 0: nothing, or a 4-byte memset of cu_seqlens), keep no state between launches and are capturable
+ * into a CUDA graph. */
+int bsq_tokenize_varlen_mlm(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq,
+                            const bsq_tokenizer *tok, int kind, const bsq_mlm *mlm, void *d_inputs, int64_t *d_labels,
+                            int32_t *d_cu_seqlens);
+
 /* Several batches that share padlen and tokenizer in one launch (batch-first one-byte tokens; other layouts / element
  * types fall back to one launch per batch): batch k = (d_bytes[k], d_offsets[k], nseq[k]) -> d_out[k].  The reference's
  * per-step callers tokenise small batches (training/cnnpretrain.py:123-125,145, bioseq/decoders.py:505): a 4096 x 1000
