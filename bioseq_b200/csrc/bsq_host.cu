@@ -179,7 +179,7 @@ inline bool have_clwb() {
     static const bool ok = [] {
         unsigned a, b, c, d;
         if (!__get_cpuid_count(7, 0, &a, &b, &c, &d)) return false;
-        return ((b >> 24) & 1u) != 0 && std::getenv("BSQ_NO_CLWB") == nullptr;
+        return ((b >> 24) & 1u) != 0;
     }();
     return ok;
 #else
@@ -706,10 +706,8 @@ int staged_run(bsq_stager *s, cudaStream_t st, const uint8_t *h_bytes, const int
     // Range size.  The call costs copy time + the kernel of the last range + a few microseconds per copy: small
     // outputs (narrow tokens: the whole batch's kernel is a few % of its copy) do best with few large ranges from a
     // pinned source, expanding outputs (one-hot, wide types) and bounced pageable sources with 4 MiB ones.
-    static const long env_mib = std::getenv("BSQ_CHUNK_MIB") ? std::atol(std::getenv("BSQ_CHUNK_MIB")) : 0;
     size_t chunk = kChunkBytes;
     if (a.pin_b && !h_mask && !onehot && bsq_kind_size(kind) <= 2) chunk = size_t(32) << 20;  // 35 MB batch, pipelined calls: 4 MiB 0.707 ms, 16 MiB 0.689, 32 MiB 0.674, one range 0.681 (raw copy 0.650)
-    if (env_mib > 0) chunk = static_cast<size_t>(env_mib) << 20;
     size_t nchunk = 0;
     int rc = BSQ_OK;
     for (int64_t i0 = 0; i0 < nseq && rc == BSQ_OK;) {

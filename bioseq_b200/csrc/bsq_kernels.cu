@@ -3,9 +3,9 @@
 //   K1 tokenize_rows_kernel (nseq, padlen) batch-first tokens.  One warp per row, one lane =
 //                           16 output bytes = one st.global.v4 per iteration; BOS/EOS/PAD fused;
 //                           ragged tails skip all loads.
-//   K2 seqfirst_kernel<..,kTok*>  (padlen, nseq) tokens: 128 seq x 128 pos shared-memory tile,
-//                           coalesced reads along each sequence; one-byte tokens leave through
-//                           register 4x4 byte transposes and 16-byte stores along the batch.
+//   K2 seqfirst_kernel<..,kTokGeneric>  (padlen, nseq) tokens of any element type: 128 seq x 128 pos
+//                           shared-memory tile, coalesced reads along each sequence, one element per
+//                           lane along the batch.
 //   K3 seqfirst_kernel<..,kOneHot> (padlen, nseq, C) one-hot: same tile, then every (pos, seq)
 //                           row is written with one 4/8/16-byte store when C*sizeof(T) allows,
 //                           else the run is zero-filled with 16-byte stores and the ones are
@@ -15,14 +15,12 @@
 //                           trailing <PAD> run starts) + scan, pass 2 decode_chars_kernel (text); bsq_decode_text
 //                           enqueues both behind one another.
 //   K0 maxlen_kernel        length and offsets validation for device-resident packed input.
-//   (K1s, the batch-first one-byte kernel for padlen >= 257 -- the headline path -- lives in bsq_span.cu;
-//    K1r tokenize_rows_ring_kernel below is its predecessor, kept behind BSQ_SPAN=0 for A/B runs.)
+//   (K1s, the batch-first one-byte kernel for padlen >= 257 -- the headline path -- lives in bsq_span.cu.)
 //
 // Reference semantics: src/tokenize.h:381-485 (K1/K2), :283-371 (K3), :131-179 (K4).
 #include <cuda_runtime.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <string>
@@ -195,33 +193,6 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
                  "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
 }
-
-// ------------------------------------------------------------------------------------------
-// K1r: batch-first one-byte tokens, persistent, bulk-copy fed, realignment specialised per row.
-//
-// Every warp owns a ring of NB shared-memory row buffers with one mbarrier each.  The lane that
-// resolved a row issues a 1-D bulk asynchronous copy (cp.async.bulk global -> shared, completion
-// counted on the mbarrier) of the 16-byte-aligned window that holds the row's residues, NB-1 rows
-// ahead of the row being translated, so a row's HBM latency is hidden behind the LUT work of the
-// previous rows.  Rows are dealt round-robin to the warps of the persistent grid (consecutive
-// warps read consecutive rows: the packed residues are consumed as one contiguous stream).
-// Per 16-byte output vector the work is the 16 LUT look-ups plus a handful of instructions:
-//   * the row's shared-memory window is addressed so that the two LDS.128 of a vector need no
-//     clamping (32 bytes of slack in front, 16 behind; whatever lies there is masked out by the
-//     BOS / tail fix-ups),
-//   * the byte shift between the packed source and the 16-byte aligned output vectors is constant
-//     along a row and uniform across the warp, so the row loop is instantiated four times (word
-//     shift Q = 0..3) and entered through one uniform branch per row: realignment is four funnel
-//     shifts with compile-time word selection instead of a data-dependent select tree,
-//   * rows whose padlen is not a multiple of 16 use the same code: vectors are aligned in the
-//     *flat* output (index i = r + column, r = misalignment of the row's first byte), the shift
-//     absorbs r, and only the (at most two) vectors a row shares with its neighbours are stored
-//     piecewise.
-// (A tensor-map TMA copy cannot do the realignment: cp.async.bulk.tensor needs the box start to be
-// 16-byte aligned in global memory -- tools/probes/tma1d_probe.cu -- exactly like the 1-D bulk copy.)
-// ------------------------------------------------------------------------------------------
-constexpr int kSlack = 32;
-
 __device__ __forceinline__ void mbar_wait_u32(uint32_t bar_smem, uint32_t parity) {
     asm volatile(
         "{\n"
@@ -232,193 +203,6 @@ __device__ __forceinline__ void mbar_wait_u32(uint32_t bar_smem, uint32_t parity
         "}\n" ::"r"(bar_smem),
         "r"(parity)
         : "memory");
-}
-
-// Store bytes [lo, hi) of a 16-byte vector (staged in this lane's 16 bytes of shared memory) with
-// at most four naturally aligned stores per side.  dst is 16-byte aligned.
-__device__ __forceinline__ void store_partial16(uint8_t *dst, const uint8_t *stg, int lo, int hi) {
-    int p = lo;
-    if (hi - p >= 1 && (p & 1)) { dst[p] = stg[p]; p += 1; }
-    if (hi - p >= 2 && (p & 2)) { *reinterpret_cast<uint16_t *>(dst + p) = *reinterpret_cast<const uint16_t *>(stg + p); p += 2; }
-    if (hi - p >= 4 && (p & 4)) { *reinterpret_cast<uint32_t *>(dst + p) = *reinterpret_cast<const uint32_t *>(stg + p); p += 4; }
-    if (hi - p >= 8 && (p & 8)) { *reinterpret_cast<uint2 *>(dst + p) = *reinterpret_cast<const uint2 *>(stg + p); p += 8; }
-    if (hi - p >= 8) { *reinterpret_cast<uint2 *>(dst + p) = *reinterpret_cast<const uint2 *>(stg + p); p += 8; }
-    if (hi - p >= 4) { *reinterpret_cast<uint32_t *>(dst + p) = *reinterpret_cast<const uint32_t *>(stg + p); p += 4; }
-    if (hi - p >= 2) { *reinterpret_cast<uint16_t *>(dst + p) = *reinterpret_cast<const uint16_t *>(stg + p); p += 2; }
-    if (hi - p >= 1) { dst[p] = stg[p]; }
-}
-
-// All vectors of one row.  Index space: i = r + column (i0 a multiple of 16 <=> the vector is 16-byte
-// aligned in the flat output at oal + i0).  rowbase + i is the shared-memory address of the aligned
-// 16-byte source word that holds the byte of index i0's first column; Q/sh = word/bit part of the
-// source-to-output byte shift.
-// ptail: (unaligned rows only) the codes of the previous row's last r columns, i.e. bytes [0, r) of
-// this row's first vector -- a row owns every aligned vector that ENDS inside it, so all stores are
-// whole vectors; `lim` is where this row's ownership ends (total rounded down to 16, except for the
-// last row of the launch, which also stores its final partial vector).
-template <int Q, bool ALIGNED>
-__device__ __forceinline__ void row_vectors(const uint8_t *rowbase, uint32_t sh, int r, int n, int npos, int lim, int total,
-                                            uint8_t *oal, int lane, const Specials &sp, const uint8_t *lut, const TailTab &tab,
-                                            const uint4 &ptail, uint8_t *pstage) {
-    const uint4 padv = make_uint4(sp.pad_w, sp.pad_w, sp.pad_w, sp.pad_w);
-    for (int i0 = 16 * lane; i0 < lim; i0 += 512) {
-        uint4 codes = padv;
-        if (i0 < npos) {
-            uint32_t t[4] = {0u, 0u, 0u, 0u};
-            if (i0 < n) {
-                const uint4 v0 = *reinterpret_cast<const uint4 *>(rowbase + i0);
-                const uint4 v1 = *reinterpret_cast<const uint4 *>(rowbase + i0 + 16);
-                const uint32_t w[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
-#pragma unroll
-                for (int k = 0; k < 4; ++k) t[k] = translate4(__funnelshift_r(w[Q + k], w[Q + k + 1], sh), lut);
-            }
-            if (ALIGNED) {
-                if (sp.bos && i0 == 0) t[0] = __byte_perm(t[0], sp.bos_w, 0x3214);
-            } else if (i0 == 0) {  // bytes [0, r): the previous row's tail; byte r: BOS
-                const uint4 ma = tab.m[r], mb = tab.m[r + sp.bos];
-                t[0] = (t[0] & ~mb.x) | (sp.bos_w & mb.x & ~ma.x) | (ptail.x & ma.x);
-                t[1] = (t[1] & ~mb.y) | (sp.bos_w & mb.y & ~ma.y) | (ptail.y & ma.y);
-                t[2] = (t[2] & ~mb.z) | (sp.bos_w & mb.z & ~ma.z) | (ptail.z & ma.z);
-                t[3] = (t[3] & ~mb.w) | (sp.bos_w & mb.w & ~ma.w) | (ptail.w & ma.w);
-            }
-            if (i0 + 16 > n) {  // the row ends inside this vector: keep n - i0 bytes, then EOS / pad
-                const uint4 m = tab.m[n - i0], f = tab.f[n - i0];
-                t[0] = (t[0] & m.x) | f.x; t[1] = (t[1] & m.y) | f.y;
-                t[2] = (t[2] & m.z) | f.z; t[3] = (t[3] & m.w) | f.w;
-            }
-            codes = make_uint4(t[0], t[1], t[2], t[3]);
-        }
-        if (ALIGNED || i0 + 16 <= total) {
-            __stcs(reinterpret_cast<uint4 *>(oal + i0), codes);
-        } else {  // final partial vector of the launch's last row
-            uint8_t *stg = pstage + 16 * lane;
-            *reinterpret_cast<uint4 *>(stg) = codes;
-            store_partial16(oal + i0, stg, 0, total - i0);
-        }
-    }
-}
-
-template <int NB, bool ALIGNED>
-__global__ void __launch_bounds__(kThreads)
-tokenize_rows_ring_kernel(SeqView v, int64_t nseq, int padlen, int bufsz, LutParam lutp, Specials sp, uint8_t *__restrict__ out) {
-    constexpr int WARPS = kThreads / 32;
-    extern __shared__ __align__(128) uint8_t ring[];  // WARPS * NB * bufsz
-    __shared__ __align__(16) uint8_t lut[256];
-    __shared__ TailTab tab;
-    __shared__ __align__(8) uint64_t bars[WARPS * NB];
-    __shared__ __align__(16) int4 rinfo[WARPS][32];  // per row: len, rowbase offset in the slot, shift | slot | parity | copy flag, r | flags
-    __shared__ __align__(16) uint8_t pstage[ALIGNED ? 16 : WARPS * 512];
-    __shared__ int64_t rstart[ALIGNED ? 1 : WARPS][32];  // unaligned rows: first residue and the previous row's length,
-    __shared__ int rprev[ALIGNED ? 1 : WARPS][32];       // read only when that row reaches into this row's first vector
-    // Programmatic dependent launch: let the next kernel of the stream start its own prologue now,
-    // and do ours (LUT, tail tables, barriers: no global memory) before waiting for the previous
-    // kernel of the stream to finish.  Both are no-ops for launches without the PDL attribute.
-    asm volatile("griddepcontrol.launch_dependents;");
-    load_lut(lut, lutp);
-    init_tailtab(tab, sp);
-    const int lane = threadIdx.x & 31;
-    const int warp = __shfl_sync(0xffffffffu, static_cast<int>(threadIdx.x >> 5), 0);
-    uint64_t *mybar = bars + warp * NB;
-    const uint32_t bar0 = smem_u32(mybar);
-    uint8_t *mybuf = ring + static_cast<size_t>(warp) * NB * bufsz;
-    if (lane < NB) mbar_init(mybar + lane, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncthreads();
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-
-    const int64_t gw = static_cast<int64_t>(blockIdx.x) * WARPS + warp;
-    const int64_t GW = static_cast<int64_t>(gridDim.x) * WARPS;
-    const int64_t row_pitch = GW * padlen;  // output distance between two consecutive rows of this warp
-    uint32_t seq_base = 0;                  // rows with residues handled so far (ring position)
-
-    for (int64_t batch0 = gw; batch0 < nseq; batch0 += 32 * GW) {
-        // lane j resolves row batch0 + j*GW of this warp's next 32 rows: the aligned window that has
-        // to be copied, the ring slot it will use, and the row's source-to-output byte shift
-        const int64_t myrow = batch0 + lane * GW;
-        int mylen = 0, myr = 0, myrb = 0, myshift = 0;
-        uint32_t mybytes = 0;
-        const uint8_t *mysrc = nullptr;
-        if (myrow < nseq) {
-            const int64_t start = __ldg(v.offs + myrow);
-            mylen = static_cast<int>(__ldg(v.offs + myrow + 1) - start);
-            if (!ALIGNED) {
-                myr = static_cast<int>((myrow * padlen) & 15);
-                if (myrow == nseq - 1) myr |= 0x200;  // last row of the launch: also stores its final partial vector
-                if ((myr & 15) != 0) {                // (row 0 starts a vector, so there is a previous row)
-                    const int plen = static_cast<int>(start - __ldg(v.offs + myrow - 1));
-                    if (sp.bos + plen + sp.eos > padlen - (myr & 15)) myr |= 0x100;  // its EOS / residues reach into our first vector
-                    rstart[warp][lane] = start;
-                    rprev[warp][lane] = plen;
-                }
-            }
-            const uint8_t *src = v.bytes + start - sp.bos;  // source of column 0
-            const int off = static_cast<int>(reinterpret_cast<uintptr_t>(src) & 15u);
-            const int fw = (off + sp.bos) & ~15;            // first aligned word that holds a residue (0 or 16)
-            const int d = off - (myr & 15);                 // source position (relative to src - off) of index 0
-            myshift = d & 15;
-            myrb = kSlack + (d < 0 ? -16 : 0) - fw;         // slot offset of the aligned word holding index 0
-            if (mylen > 0) {
-                mybytes = static_cast<uint32_t>(((off + sp.bos + mylen - 1) & ~15) - fw + 16);
-                mysrc = src - off + fw;
-            }
-        }
-        const uint32_t has = __ballot_sync(0xffffffffu, mybytes != 0u);
-        const uint32_t myseq = seq_base + __popc(has & ((1u << lane) - 1u));
-        const uint32_t myslot = myseq % NB;
-        const uint32_t my_dst = smem_u32(mybuf + myslot * bufsz + kSlack), my_bar = bar0 + 8u * myslot;
-        __syncwarp();
-        rinfo[warp][lane] = make_int4(mylen, myrb + static_cast<int>(myslot) * bufsz,
-                                      myshift | static_cast<int>(myslot << 8) | static_cast<int>(((myseq / NB) & 1u) << 12) | (mybytes ? 0x10000 : 0), myr);
-        __syncwarp();
-        seq_base += __popc(has);
-        const int nrows = static_cast<int>(min(static_cast<int64_t>(32), (nseq - batch0 + GW - 1) / GW));
-        // the lane that resolved a row also issues its copy (everything it needs is in its registers)
-        auto issue = [&](int j) {
-            if (lane == j && mybytes != 0u) {
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(my_bar), "r"(mybytes) : "memory");
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(my_dst),
-                             "l"(mysrc), "r"(mybytes), "r"(my_bar)
-                             : "memory");
-            }
-        };
-        for (int j = 0; j < min(NB - 1, nrows); ++j) issue(j);
-        uint8_t *orow = out + batch0 * padlen;
-        for (int j = 0; j < nrows; ++j, orow += row_pitch) {
-            if (j + NB - 1 < nrows) issue(j + NB - 1);
-            const int4 q = rinfo[warp][j];
-            const int len = q.x, r = ALIGNED ? 0 : (q.w & 15);
-            const int n = r + sp.bos + len, npos = n + sp.eos, total = r + padlen;
-            const int lim = (ALIGNED || (q.w & 0x200)) ? total : (total & ~15);
-            const uint8_t *rowbase = mybuf + q.y;
-            const uint32_t sh = (static_cast<uint32_t>(q.z) & 3u) * 8u;
-            uint8_t *ps = pstage + (ALIGNED ? 0 : warp * 512);
-            uint4 ptail = make_uint4(sp.pad_w, sp.pad_w, sp.pad_w, sp.pad_w);
-            if (!ALIGNED && (q.w & 0x100)) {
-                // rare: the previous row is so long that its residues / EOS reach into this row's first vector;
-                // rebuild those (at most 15) codes one by one from global memory (src/tokenize.h:464-478)
-                if (lane < r) {
-                    const int plen = rprev[warp][j];
-                    const int jres = padlen - r + lane - sp.bos;  // residue index of that column in the previous row
-                    uint32_t code = sp.pad_w & 0xffu;
-                    if (jres < plen) code = lut[__ldg(v.bytes + rstart[warp][j] - plen + jres)];
-                    else if (jres == plen && sp.eos) code = sp.eos_w & 0xffu;
-                    ps[lane] = static_cast<uint8_t>(code);
-                }
-                __syncwarp();
-                ptail = *reinterpret_cast<const uint4 *>(ps);
-                __syncwarp();
-            }
-            if (q.z & 0x10000) mbar_wait_u32(bar0 + 8u * ((static_cast<uint32_t>(q.z) >> 8) & 0xfu), (static_cast<uint32_t>(q.z) >> 12) & 1u);
-            uint8_t *oal = orow - r;
-            switch ((q.z >> 2) & 3) {  // warp-uniform
-                case 0: row_vectors<0, ALIGNED>(rowbase, sh, r, n, npos, lim, total, oal, lane, sp, lut, tab, ptail, ps); break;
-                case 1: row_vectors<1, ALIGNED>(rowbase, sh, r, n, npos, lim, total, oal, lane, sp, lut, tab, ptail, ps); break;
-                case 2: row_vectors<2, ALIGNED>(rowbase, sh, r, n, npos, lim, total, oal, lane, sp, lut, tab, ptail, ps); break;
-                default: row_vectors<3, ALIGNED>(rowbase, sh, r, n, npos, lim, total, oal, lane, sp, lut, tab, ptail, ps); break;
-            }
-            __syncwarp();  // every lane is done with this buffer before it is refilled
-        }
-    }
 }
 
 // Fallback for wide element types whose rows are not 16-byte aligned (padlen * sizeof(T) % 16
@@ -518,8 +302,8 @@ __device__ __forceinline__ void transpose4x4(const uint32_t x[4], uint32_t y[4])
     y[3] = __byte_perm(t2, t3, 0x7632);
 }
 
-// MODE: how phase 2 leaves the tile (a template parameter, so every variant gets its own register budget).
-constexpr int kTokFast = 0;     // one-byte tokens, batch extent a multiple of 16: register 4x4 transposes + st.v4
+// MODE: how phase 2 leaves the tile (a template parameter, so every variant gets its own register budget).  The
+// values appear in the kernels' names, which the profiles under profiles/ quote.
 constexpr int kTokGeneric = 1;  // any element type / alignment: one element per lane, coalesced along the batch
 constexpr int kOhRow = 2;       // one-hot, C*sizeof(T) is 4, 8 or 16: one store writes the whole one-hot row of a (pos, seq)
 constexpr int kOhVec = 3;       // one-hot, aligned runs, any C*sizeof(T): 16-byte vectors assembled in registers (zeros included)
@@ -550,10 +334,9 @@ seqfirst_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, LutParam lutp, 
     // nseq sequences are processed; ld (>= nseq) is the batch extent of the output array, so a
     // sub-range of a larger batch can be written in place (out already points at its first column).
     constexpr bool ONEHOT = MODE >= kOhRow;
-    constexpr int PITCH = MODE == kTokFast ? kTilePos : kTilePitch;
     extern __shared__ __align__(128) uint8_t stage[];  // kTileSeqs * kStagePitch residues (+ as much again for a mask)
     __shared__ __align__(16) uint8_t lut[256];
-    __shared__ __align__(16) uint8_t tile[kTileSeqs * PITCH];
+    __shared__ __align__(16) uint8_t tile[kTileSeqs * kTilePitch];
     __shared__ TailTab tab;
     __shared__ uint4 ohtab[MODE == kOhVec ? 17 : 1];  // [b] = 16-byte vector with T(1) at byte b (b % sizeof(T) == 0); [16] = zero
     __shared__ __align__(16) int4 rinfo[kTileSeqs];   // per sequence: len, (A & 15) of the residues, of the mask
@@ -639,56 +422,22 @@ seqfirst_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, LutParam lutp, 
                 }
                 codes = tokens16_finish<false>(t, len, c0, sp, tab);
             }
-            if (MODE == kTokFast) {
-                // 16-byte chunks XOR-swizzled by the sequence group, so that phase 2's column-of-words
-                // reads (16 sequences apart) hit 32 distinct banks
-                *reinterpret_cast<uint4 *>(tile + il * PITCH + 16 * (q ^ ((il >> 4) & 7))) = codes;
-            } else {
-                uint32_t *dst = reinterpret_cast<uint32_t *>(tile + il * PITCH + 16 * q);
-                dst[0] = codes.x; dst[1] = codes.y; dst[2] = codes.z; dst[3] = codes.w;
-            }
+            uint32_t *dst = reinterpret_cast<uint32_t *>(tile + il * kTilePitch + 16 * q);
+            dst[0] = codes.x; dst[1] = codes.y; dst[2] = codes.z; dst[3] = codes.w;
         }
     }
     __syncthreads();
 
     // ---- phase 2 ----
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (MODE == kTokFast) {
-        // thread = 16 sequences (group A) x 4 positions (word pw): 16 LDS.32, four 4x4 transposes,
-        // then one 16-byte store per position; lanes A = 0..7 make 128 contiguous bytes per row.
-        const int A = lane & 7, pw = 4 * warp + (lane >> 3);
-        const uint32_t *t32 = reinterpret_cast<const uint32_t *>(tile);
-        uint32_t y[4][4];
-#pragma unroll
-        for (int a = 0; a < 4; ++a) {
-            uint32_t x[4];
-#pragma unroll
-            for (int k = 0; k < 4; ++k) x[k] = t32[(16 * A + 4 * a + k) * (PITCH / 4) + (pw ^ (4 * A))];
-            transpose4x4(x, y[a]);
-        }
-        const int nvalid = nseq_tile - 16 * A;  // sequences of this group that exist
-        uint8_t *obase = reinterpret_cast<uint8_t *>(out) + i0 + 16 * A;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int pos = p0 + 4 * pw + j;
-            if (pos >= padlen || nvalid <= 0) continue;
-            uint8_t *o = obase + static_cast<int64_t>(pos) * ld;
-            if (nvalid >= 16) {
-                __stcs(reinterpret_cast<uint4 *>(o), make_uint4(y[0][j], y[1][j], y[2][j], y[3][j]));
-            } else {
-#pragma unroll
-                for (int k = 0; k < 16; ++k)
-                    if (k < nvalid) o[k] = static_cast<uint8_t>(y[k >> 2][j] >> (8 * (k & 3)));
-            }
-        }
-    } else if (MODE == kTokGeneric) {
+    if (MODE == kTokGeneric) {
         for (int pp = warp; pp < npos_tile; pp += kThreads / 32) {
             T *orow = out + (static_cast<int64_t>(p0 + pp) * ld + i0);
 #pragma unroll
             for (int m = 0; m < kTileSeqs / 32; ++m) {
                 const int il = lane + 32 * m;
                 if (il < nseq_tile) {
-                    const uint32_t code = tile[il * PITCH + pp];
+                    const uint32_t code = tile[il * kTilePitch + pp];
                     __stcs(orow + il, cast_id<T>(expand_code(code, ex)));
                 }
             }
@@ -701,7 +450,7 @@ seqfirst_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, LutParam lutp, 
             for (int m = 0; m < kTileSeqs / 32; ++m) {
                 const int il = lane + 32 * m;
                 if (il < nseq_tile) {
-                    const int col = expand_code(tile[il * PITCH + pp], ex);
+                    const int col = expand_code(tile[il * kTilePitch + pp], ex);
                     uint32_t w[4] = {0u, 0u, 0u, 0u};
                     if (col >= 0) set_one<T>(w, col);
                     uint8_t *o = orow + il * row_bytes;
@@ -729,7 +478,7 @@ seqfirst_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, LutParam lutp, 
                 int rel = il * row_bytes - b0;  // byte offset of sequence il's row inside this vector (<= 0)
                 uint4 w = make_uint4(0u, 0u, 0u, 0u);
                 for (int k = 0; k < nover; ++k, ++il, rel += row_bytes) {
-                    const uint32_t code = il < nseq_tile ? tcol[il * PITCH] : 0xffu;
+                    const uint32_t code = il < nseq_tile ? tcol[il * kTilePitch] : 0xffu;
                     const uint32_t b = min(static_cast<uint32_t>(rel + static_cast<int>(code) * S), 16u);  // 16 = not in this vector
                     const uint4 o = ohtab[b];
                     w.x |= o.x; w.y |= o.y; w.z |= o.z; w.w |= o.w;
@@ -740,7 +489,7 @@ seqfirst_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, LutParam lutp, 
             T *erow = reinterpret_cast<T *>(orow);
             for (int e = (nvec << 4) / S + lane; e < nseq_tile * ncols; e += 32) {
                 const int il = static_cast<int>(fd_div(static_cast<uint32_t>(e), div_ncols));
-                erow[e] = static_cast<int>(tcol[il * PITCH]) == e - il * ncols ? cast_id<T>(1) : cast_id<T>(0);
+                erow[e] = static_cast<int>(tcol[il * kTilePitch]) == e - il * ncols ? cast_id<T>(1) : cast_id<T>(0);
             }
         }
     } else {
@@ -750,7 +499,7 @@ seqfirst_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, LutParam lutp, 
             for (int e = lane; e < run_elems; e += 32) {
                 const int il = static_cast<int>(fd_div(static_cast<uint32_t>(e), div_ncols));
                 const int col = e - il * ncols;
-                const int hot = expand_code(tile[il * PITCH + pp], ex);
+                const int hot = expand_code(tile[il * kTilePitch + pp], ex);
                 orow[e] = hot == col ? cast_id<T>(1) : cast_id<T>(0);
             }
         }
@@ -759,8 +508,9 @@ seqfirst_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, LutParam lutp, 
 
 // ------------------------------------------------------------------------------------------
 // K2t: (padlen, nseq) one-byte tokens -- the reference's default layout (batch_first=False) -- as a
-// dedicated, instruction-lean kernel (the tile kernel above was issue-bound: 700 instructions per
-// warp per 16 KB tile, profiles/r01d_seqfirst_*).  Same 128 x 128 tile, but
+// dedicated, instruction-lean kernel (the tile kernel above, with register 4x4 transposes for one-byte
+// tokens, was issue-bound: 700 instructions per warp per 16 KB tile, profiles/r01d_seqfirst_*).  Same
+// 128 x 128 tile, but
 //   * the sequences' windows are staged with per-lane 16-byte cp.async (LDGSTS): the eight lanes that
 //     will translate a sequence's eight chunks copy them, so the hand-over needs cp.async.wait_all +
 //     __syncwarp only -- no mbarrier, no block barrier, no per-copy uniform-datapath loop;
@@ -1885,27 +1635,6 @@ namespace {
 
 inline uint32_t rep4(uint32_t b) { return (b & 0xffu) * 0x01010101u; }
 
-// Debug / A-B knobs: BSQ_RING=0 falls back to the plain warp-per-row kernel (K1), BSQ_RING_CTAS caps the
-// persistent grid (CTAs per SM, default 4), BSQ_PDL=0 disables programmatic dependent launch.
-int env_int(const char *name, int dflt) {
-    const char *e = std::getenv(name);
-    return e ? std::atoi(e) : dflt;
-}
-bool ring_enabled() {
-    static const bool on = env_int("BSQ_RING", 1) != 0;
-    return on;
-}
-bool pdl_enabled() {
-    static const bool tune = env_int("BSQ_TUNE", 0) != 0;
-    static bool on = env_int("BSQ_PDL", 1) != 0;
-    if (tune) on = env_int("BSQ_PDL", 1) != 0;
-    return on;
-}
-int ring_ctas_per_sm() {
-    static const int n = std::max(1, env_int("BSQ_RING_CTAS", 4));
-    return n;
-}
-
 }  // namespace
 
 // mode 0: batch-first one-byte tokens (codes are the output bytes: ids wrap to 8 bits like
@@ -1968,46 +1697,7 @@ int launch_bf(cudaStream_t st, const SeqView &v, int64_t nseq, int64_t /*ld*/, i
     if (sizeof(T) == 1 && span_kernel_applicable(padlen)) {
         int dev = 0;
         BSQ_CUDA_TRY(cudaGetDevice(&dev));
-        return launch_tokenize_span(dev, st, v, nseq, padlen, p, static_cast<uint8_t *>(d_out), pdl_enabled());
-    }
-    if (sizeof(T) == 1 && padlen > 256 && ring_enabled()) {
-        // K1r: persistent, bulk-copy fed, per-row specialised realignment; any padlen that fits the ring
-        constexpr int WARPS = kThreads / 32, NB = 2;
-        const bool aligned = padlen % 16 == 0;
-        const int bufsz = static_cast<int>((padlen + 80 + 15) / 16 * 16);
-        const size_t smem = static_cast<size_t>(WARPS) * NB * bufsz;
-        if (smem <= 200 * 1024) {
-            int dev = 0, sms = 0;
-            BSQ_CUDA_TRY(cudaGetDevice(&dev));
-            BSQ_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-            const size_t per_cta = smem + 8192;  // + static shared memory and allocation granularity
-            const int fit = static_cast<int>((220 * 1024) / per_cta);
-            const int per_sm = std::max(1, std::min(std::min(8, fit), ring_ctas_per_sm()));
-            const int64_t want = (nseq + WARPS - 1) / WARPS;
-            const unsigned blocks = static_cast<unsigned>(std::min<int64_t>(want, static_cast<int64_t>(sms) * per_sm));
-            // Programmatic dependent launch hides this launch's ramp behind the previous kernel's tail.  The
-            // early CTAs sit next to the previous kernel's, so it is only used when two whole persistent grids
-            // fit on the SMs at once -- otherwise the late CTAs pile up on the first SMs to drain and the
-            // static row partition becomes unbalanced (measured: 2x slower).
-            const bool pdl = pdl_enabled() && 2 * per_sm * per_cta <= 220 * 1024 && 2 * per_sm * kThreads <= 2048;
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(blocks);
-            cfg.blockDim = dim3(kThreads);
-            cfg.dynamicSmemBytes = smem;
-            cfg.stream = st;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            at[0].val.programmaticStreamSerializationAllowed = 1;
-            cfg.attrs = at;
-            cfg.numAttrs = pdl ? 1 : 0;
-            const int pl = static_cast<int>(padlen);
-            uint8_t *o = static_cast<uint8_t *>(d_out);
-            auto kern = aligned ? tokenize_rows_ring_kernel<NB, true> : tokenize_rows_ring_kernel<NB, false>;
-            BSQ_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            BSQ_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, v, nseq, pl, bufsz, p.lut, p.sp, o));
-            count_launch();
-            return BSQ_OK;
-        }
+        return launch_tokenize_span(dev, st, v, nseq, padlen, p, static_cast<uint8_t *>(d_out));
     }
     if (sizeof(T) == 1 || (padlen * sizeof(T)) % 16 == 0) {
         int lanes_log2 = 0;  // lanes per row: smallest power of two covering the row, at most a warp
@@ -2069,9 +1759,8 @@ int launch_sf(cudaStream_t st, const SeqView &v, int64_t nseq, int64_t ld, int64
         // the register-transpose path needs one-byte elements whose rows start 16-byte aligned and
         // codes that are the output bytes (every alphabet but BYTES, whose special ids exceed 8 bits)
         if (sizeof(T) == 1 && aligned && ld % 16 == 0 && tok.pad_id < 0x80) {
-            if (env_int("BSQ_SF_OLD", 0)) BSQ_SF(kTokFast);
-            else if (gx * gy > 0x7fffffffll) return fail(BSQ_ERR_ARG, "batch too large for one launch");
-            else if (env_int("BSQ_SF_TPC", 2) == 2 && gy % 2 == 0 && gx * gy / 2 >= 8ll * cur_sms() * 6)  // enough CTAs left to balance the resident slots (6 per SM)
+            if (gx * gy > 0x7fffffffll) return fail(BSQ_ERR_ARG, "batch too large for one launch");
+            else if (gy % 2 == 0 && gx * gy / 2 >= 8ll * cur_sms() * 6)  // enough CTAs left to balance the resident slots (6 per SM)
                 seqfirst_tok8_kernel<2><<<static_cast<unsigned>(gx * gy / 2), kThreads, 0, st>>>(
                     v, nseq, ld, pl, make_fastdiv(static_cast<uint32_t>(gy / 2)), p.lut, p.sp, reinterpret_cast<uint8_t *>(o));
             else seqfirst_tok8_kernel<1><<<static_cast<unsigned>(gx * gy), kThreads, 0, st>>>(
@@ -2185,7 +1874,7 @@ int bsq_tokenize_many(int device, void *stream, int nbatch, const uint8_t *const
         for (int k0 = 0; k0 < nbatch; k0 += kSpanManyMax) {  // one launch per group of up to 32 batches
             const int nb = std::min(kSpanManyMax, nbatch - k0);
             if (int rc = launch_tokenize_span_many(device, st, nb, d_bytes + k0, d_offsets + k0, nseq + k0, padlen, p,
-                                                   reinterpret_cast<uint8_t *const *>(d_out + k0), pdl_enabled()))
+                                                   reinterpret_cast<uint8_t *const *>(d_out + k0)))
                 return rc;
         }
         return BSQ_OK;
@@ -2303,7 +1992,6 @@ int decode_lengths_enqueue(int device, cudaStream_t st, const void *d_tokens, in
     const InvParam inv = make_inv(*tok);
     const int fast = decode_fast_path(d_tokens, itemsize, row_stride, col_stride);
     const bool rows16 = (reinterpret_cast<uintptr_t>(d_tokens) & 15u) == 0 && row_stride % 16 == 0;
-    static const bool len_piped = env_int("BSQ_DEC_LENPIPE", 1) != 0;
     const bool al = rows16 && cols % 16 == 0;
     const int64_t maxvec = al ? cols / 16 : (15 + cols + 15) / 16;  // vectors that cover a row, at the worst alignment
     if (fast && cols > 0) {
@@ -2315,7 +2003,7 @@ int decode_lengths_enqueue(int device, cudaStream_t st, const void *d_tokens, in
         while (a < 256 && inv.e[a + 128] != kInvNone && !(inv.e[a + 128] & 0x100u)) ++a;
         b = a;
         while (b < 256 && inv.e[b + 128] != kInvNone && (inv.e[b + 128] & 0x100u)) ++b;
-        bool thr = b >= 1 && b <= 128 && env_int("BSQ_DEC_LENTHR", 1) != 0;
+        bool thr = b >= 1 && b <= 128;
         for (int t = b; t < 256 && thr; ++t) thr = inv.e[t + 128] == kInvNone;
         const uint32_t lo4 = static_cast<uint32_t>(a) * 0x01010101u, hi4 = static_cast<uint32_t>(b) * 0x01010101u;
 #define BSQ_LEN16P(AL, V)                                                                                                                      \
@@ -2323,13 +2011,13 @@ int decode_lengths_enqueue(int device, cudaStream_t st, const void *d_tokens, in
         if (thr) decode_len16p_kernel<AL, V, true><<<grid, kDecWarps * 32, 0, st>>>(tk, rows, cols, row_stride, inv, d_row_offsets, d_row_tail, fb, lo4, hi4);  \
         else decode_len16p_kernel<AL, V, false><<<grid, kDecWarps * 32, 0, st>>>(tk, rows, cols, row_stride, inv, d_row_offsets, d_row_tail, fb, lo4, hi4); \
     } while (0)
-        if (len_piped && maxvec <= 64) {
+        if (maxvec <= 64) {
             if (al) BSQ_LEN16P(false, 2);
             else BSQ_LEN16P(true, 2);
-        } else if (len_piped && maxvec <= 96) {  // (padlen 1026, rows at any alignment: 66 vectors)
+        } else if (maxvec <= 96) {  // (padlen 1026, rows at any alignment: 66 vectors)
             if (al) BSQ_LEN16P(false, 3);
             else BSQ_LEN16P(true, 3);
-        } else if (len_piped && maxvec <= 128) {
+        } else if (maxvec <= 128) {
             if (al) BSQ_LEN16P(false, 4);
             else BSQ_LEN16P(true, 4);
 #undef BSQ_LEN16P
@@ -2397,8 +2085,7 @@ int decode_chars_enqueue(cudaStream_t st, const void *d_tokens, int itemsize, in
     const int32_t *tail = (fast && cols <= (1 << 28)) ? d_row_tail : nullptr;  // (the run's byte count is an int in the kernel)
     const uint8_t *tk = static_cast<const uint8_t *>(d_tokens);
     const size_t ring = static_cast<size_t>(kDecWarps) * 2 * ((cols + 15 + 16) / 16 * 16 + 16);
-    static const bool staged_on = env_int("BSQ_DEC_STAGED", 1) != 0;
-    if (fast && staged_on && ring <= 96 * 1024) {  // rows up to ~6 K tokens ride the ring
+    if (fast && ring <= 96 * 1024) {  // rows up to ~6 K tokens ride the ring
         auto kern = rows16 ? decode_chars_kernel<false, true> : decode_chars_kernel<true, true>;
         if (ring > 24 * 1024) BSQ_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
         kern<<<decode_grid(rows), kDecWarps * 32, ring, st>>>(tk, itemsize, rows, cols, row_stride, col_stride, fast, inv, d_row_offsets, tail, d_chars, capacity, d_first_bad);

@@ -70,8 +70,10 @@ struct Prepared {
 };
 Prepared prepare(const bsq_tokenizer &tok, int mode);
 
-// K1s (bsq_span.cu): batch-first one-byte tokens, tile-staged and warp-specialised.
-bool span_kernel_applicable(int64_t padlen);
+// K1s (bsq_span.cu): batch-first one-byte tokens, tile-staged and warp-specialised.  It runs every padlen above
+// kSpanMinPadlen (up to the 2^30 every entry point allows); shorter rows share warps in K1.
+constexpr int64_t kSpanMinPadlen = 256;
+inline bool span_kernel_applicable(int64_t padlen) { return padlen > kSpanMinPadlen; }
 int sm_count(int device);  // SMs of the device (cached per device)
 inline int cur_sms() {     // ... of the current device (the entry points have made the call's device current)
     int d = 0;
@@ -79,7 +81,7 @@ inline int cur_sms() {     // ... of the current device (the entry points have m
     return sm_count(d);
 }
 int launch_tokenize_span(int device, cudaStream_t st, const SeqView &v, int64_t nseq, int64_t padlen, const Prepared &p,
-                         uint8_t *out, bool pdl_allowed);
+                         uint8_t *out);
 // A slot of the per-stream tile counters of the dynamic schedulers (bsq_span.cu), or nullptr when none can be used
 // (stream capture in progress, out of memory): the kernels then keep their static tile order.
 unsigned int *tile_counter_slot(int device, cudaStream_t st);
@@ -87,7 +89,7 @@ unsigned int *tile_counter_slot(int device, cudaStream_t st);
 void span_magic(uint32_t d, uint32_t *mul, uint32_t *shift);
 constexpr int kSpanManyMax = 32;  // batches per launch of launch_tokenize_span_many
 int launch_tokenize_span_many(int device, cudaStream_t st, int nbatch, const uint8_t *const *d_bytes, const int64_t *const *d_offs,
-                              const int64_t *nseqs, int64_t padlen, const Prepared &p, uint8_t *const *outs, bool pdl_allowed);
+                              const int64_t *nseqs, int64_t padlen, const Prepared &p, uint8_t *const *outs);
 
 #ifdef __CUDACC__
 

@@ -9,7 +9,7 @@
 // instead of one copy, one barrier wait and one slot computation per row:
 //
 //   producer warp   per tile: divides the tile's flat range into rows, loads the rows' offsets
-//                   (coalesced), issues the span copy into the next free stage of a ring of NSTAGE
+//                   (coalesced), issues the span copy into the next free stage of a ring of kSpanStages
 //                   shared-memory buffers (completion counted on the stage's `full` mbarrier) and
 //                   writes the per-row table {source position in the stage, length} next to it;
 //   8 consumer warps per tile: one 16-byte output vector per lane and step, vectors dealt flat
@@ -25,13 +25,12 @@
 // batch's final partial vector (nseq * padlen % 16 != 0) is stored bytewise.
 //
 // Nothing per row is left in the instruction stream of the consumers except the row-table load: the
-// ring kernel it replaces (K1r, bsq_kernels.cu) spent 236 warp-instructions per 1 KiB row, 128 of them
-// on per-row bookkeeping (slot arithmetic, elect loops around each row's bulk copy, barrier waits,
+// warp-per-row ring kernel it replaced (K1r, since removed) spent 236 warp-instructions per 1 KiB row, 128 of
+// them on per-row bookkeeping (slot arithmetic, elect loops around each row's bulk copy, barrier waits,
 // uniform-datapath shuffling); see profiles/ r01x vs r02.
 #include <cuda_runtime.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
 
@@ -49,7 +48,11 @@ constexpr int kSpanConsumers = kSpanConsumerWarps * 32;
 constexpr int kSpanThreads = kSpanConsumers + 32;
 constexpr int kSpanSlack = 32;  // bytes in front of the staged span (two LDS.128 never leave the stage)
 constexpr int kSpanTail = 64;   // and behind it
-// MINB (launch bound, CTAs per SM) sets the register budget: 4 -> 56, 5 -> 40, 6 -> 32 registers per thread.
+// Stages of the ring: 3 and 4 were measured no faster than 2 (profiles/r02_sweep_span.txt).
+constexpr int kSpanStages = 2;
+// Tile size in 16-byte output vectors (24 KB), and resident CTAs per SM; both from the r02 sweep (DESIGN §3).
+constexpr int kSpanTileVecs = 1536;
+constexpr int kSpanCtasPerSm = 4;
 
 __device__ __forceinline__ uint32_t s_u32(const void *p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
 __device__ __forceinline__ void bar_init(uint64_t *bar, uint32_t count) {
@@ -86,7 +89,6 @@ __device__ __forceinline__ void bulk_load(uint32_t dst, const void *src, uint32_
 
 // One launch can serve several batches that share padlen and tokenizer (bsq_tokenize_many: the small per-step batches of
 // the reference's training loops, training/cnnpretrain.py:123-125,145): their tiles are numbered one batch after the other.
-constexpr int kSpanMaxBatches = 32;
 struct SpanBatch {
     const uint8_t *bytes;
     const int64_t *offs;
@@ -96,7 +98,7 @@ struct SpanBatch {
     int64_t first_tile;  // index of the batch's first tile
 };
 struct SpanBatches {
-    SpanBatch b[kSpanMaxBatches];
+    SpanBatch b[kSpanManyMax];
 };
 
 struct SpanParams {
@@ -194,17 +196,15 @@ __device__ __forceinline__ uint32_t span_translate4(uint32_t x, uint32_t lutb) {
 }
 
 // 16 codes from the 32-byte window {v0, v1}: word shift Q (compile time), bit shift sh (taken mod 32).
-// PRE: the stage already holds codes (two-phase form: translated in place before the vectors are placed).
-template <int Q, bool PRE>
+template <int Q>
 __device__ __forceinline__ void span_translate16(const uint4 &v0, const uint4 &v1, uint32_t sh, uint32_t lutb, uint32_t t[4]) {
     const uint32_t w[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         const uint32_t x = __funnelshift_r(w[Q + k], w[Q + k + 1], sh);
-        t[k] = PRE ? x : span_translate4(x, lutb);
+        t[k] = span_translate4(x, lutb);
     }
 }
-template <bool PRE>
 __device__ __forceinline__ void span_window16(uint32_t S, uint32_t lutb, int straddle, uint32_t t[4]) {
     const uint4 v0 = lds128(S & ~15u), v1 = lds128((S & ~15u) + 16u);
     const uint32_t sh = S << 3;
@@ -218,10 +218,10 @@ __device__ __forceinline__ void span_window16(uint32_t S, uint32_t lutb, int str
     if (straddle) __match_all_sync(__activemask(), q, &uni);
     if (uni) {
         switch (q) {
-            case 0: span_translate16<0, PRE>(v0, v1, sh, lutb, t); break;
-            case 4: span_translate16<1, PRE>(v0, v1, sh, lutb, t); break;
-            case 8: span_translate16<2, PRE>(v0, v1, sh, lutb, t); break;
-            default: span_translate16<3, PRE>(v0, v1, sh, lutb, t); break;
+            case 0: span_translate16<0>(v0, v1, sh, lutb, t); break;
+            case 4: span_translate16<1>(v0, v1, sh, lutb, t); break;
+            case 8: span_translate16<2>(v0, v1, sh, lutb, t); break;
+            default: span_translate16<3>(v0, v1, sh, lutb, t); break;
         }
     } else {
         const bool q2 = (S & 8u) != 0, q1 = (S & 4u) != 0;
@@ -231,7 +231,7 @@ __device__ __forceinline__ void span_window16(uint32_t S, uint32_t lutb, int str
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
             const uint32_t y = __funnelshift_r(x[k], x[k + 1], sh);
-            t[k] = PRE ? y : span_translate4(y, lutb);
+            t[k] = span_translate4(y, lutb);
         }
     }
 }
@@ -256,10 +256,9 @@ constexpr int kCstWords = 16;
 // address of the byte that column 0 would come from (first residue - bos), n = bos + len.  Columns >= padlen are
 // don't-care.  The residue window is loaded and translated unconditionally: whatever lies left of the first
 // residue or right of the last is replaced by the BOS / tail fix-ups (for c0 == n the whole vector is).
-template <bool PRE>
 __device__ __forceinline__ uint4 span_row_codes(uint32_t srow, int n, int c0, const SpanRegs &g) {
     uint32_t t[4];
-    span_window16<PRE>(srow + static_cast<uint32_t>(c0), g.lutb, g.straddle, t);
+    span_window16(srow + static_cast<uint32_t>(c0), g.lutb, g.straddle, t);
     if (c0 == 0) t[0] = __byte_perm(t[0], g.bos_w, g.bos_sel);
     if (c0 + 16 > n) {  // the row's residues end inside this vector: keep n - c0 bytes, then EOS / pad
         const uint32_t a = g.tab_m + 16u * static_cast<uint32_t>(n - c0);
@@ -272,10 +271,9 @@ __device__ __forceinline__ uint4 span_row_codes(uint32_t srow, int n, int c0, co
 
 // Unaligned rows: columns c0 .. c0+15 with -16 < c0 <= padlen - 16; for c0 < 0 the bytes left of column 0 are the
 // previous row's tail and are set to the pad code (the caller has checked that the previous row ends before them).
-template <bool PRE>
 __device__ __forceinline__ uint4 span_row_codes_u(uint32_t srow, int n, int c0, const SpanRegs &g) {
     uint32_t t[4];
-    span_window16<PRE>(srow + static_cast<uint32_t>(c0), g.lutb, g.straddle, t);
+    span_window16(srow + static_cast<uint32_t>(c0), g.lutb, g.straddle, t);
     if (c0 <= 0) {  // bytes [0, -c0): pad; byte -c0: BOS when the tokenizer has one -- a ready-made vector per -c0
         const uint32_t j16 = 16u * static_cast<uint32_t>(-c0);
         const uint4 mb = lds128(g.tab_m + j16 + 16u * static_cast<uint32_t>(g.bos)), hh = lds128(g.tab_h + j16);
@@ -295,13 +293,12 @@ __device__ __forceinline__ uint4 span_row_codes_u(uint32_t srow, int n, int c0, 
 
 // The rare straddling vector whose first bytes are NOT pad: the previous row (rl - 1) is so long that its residues /
 // EOS reach into them.  Both rows' codes are built and merged.  Kept out of line: it must not cost the hot loop registers.
-template <bool PRE>
 __device__ __noinline__ uint4 span_straddle_general(uint32_t rows_a, uint32_t rl, int col, const SpanRegs &g) {
     const int4 rp = lds128i(rows_a + 16u * rl - 16u), ri = lds128i(rows_a + 16u * rl);
     const int cp = col + g.padlen;  // the vector's first column in the previous row (> padlen - 16)
     uint4 prev = g.padq;
-    if (cp < rp.z) prev = span_row_codes_u<PRE>(static_cast<uint32_t>(rp.x), rp.y, cp, g);
-    const uint4 cur = span_row_codes_u<PRE>(static_cast<uint32_t>(ri.x), ri.y, col, g);
+    if (cp < rp.z) prev = span_row_codes_u(static_cast<uint32_t>(rp.x), rp.y, cp, g);
+    const uint4 cur = span_row_codes_u(static_cast<uint32_t>(ri.x), ri.y, col, g);
     const uint4 m = lds128(g.tab_m - 16u * static_cast<uint32_t>(col));  // bytes [0, -col) come from the previous row
     return make_uint4((prev.x & m.x) | (cur.x & ~m.x), (prev.y & m.y) | (cur.y & ~m.y), (prev.z & m.z) | (cur.z & ~m.z),
                       (prev.w & m.w) | (cur.w & ~m.w));
@@ -312,17 +309,18 @@ struct SpanEdges {
     int64_t a0, a1, b0, b1;
 };
 
-template <int NSTAGE, bool ALIGNED, bool PRE, int MINB>
-__global__ void __launch_bounds__(kSpanThreads, MINB)
+// 4 CTAs per SM leave 56 registers per thread; 5 and 6 (40 and 32 registers) were measured slower (r02 sweep, DESIGN §3).
+template <bool ALIGNED>
+__global__ void __launch_bounds__(kSpanThreads, kSpanCtasPerSm)
 tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb, const LutParam lutp, const Specials sp) {
-    extern __shared__ __align__(128) uint8_t dyn[];  // NSTAGE x { data[stage_bytes], rows[max_rows] x 16 B }
+    extern __shared__ __align__(128) uint8_t dyn[];  // kSpanStages x { data[stage_bytes], rows[max_rows] x 16 B }
     __shared__ __align__(256) uint8_t lut[256];
     __shared__ TailTab tab;
     __shared__ uint4 headtab[16];
-    __shared__ __align__(8) uint64_t full[NSTAGE], empty[NSTAGE];
-    __shared__ __align__(16) int4 hdr[NSTAGE];           // c_first, nrows, nvec, -
+    __shared__ __align__(8) uint64_t full[kSpanStages], empty[kSpanStages];
+    __shared__ __align__(16) int4 hdr[kSpanStages];      // c_first, nrows, nvec, -
     __shared__ __align__(16) uint32_t cst[kCstWords];    // loop invariants of the consumers (see SpanRegs)
-    __shared__ uint8_t *tile_out[NSTAGE];                // where the stage's tile starts in its batch's output
+    __shared__ uint8_t *tile_out[kSpanStages];           // where the stage's tile starts in its batch's output
 
     // Programmatic dependent launch: the next kernel of the stream may start its prologue now; ours (LUT, mask
     // tables, barriers: no global memory) runs before the previous kernel of the stream has finished.
@@ -349,7 +347,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
     }
     if (threadIdx.x == 128) {
 #pragma unroll
-        for (int s = 0; s < NSTAGE; ++s) {
+        for (int s = 0; s < kSpanStages; ++s) {
             bar_init(full + s, 1);
             bar_init(empty + s, kSpanConsumerWarps);
         }
@@ -423,8 +421,8 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
         unsigned int ask = 0;  // lane 0: the counter's answer for the tile after the next one, read one iteration later
         uint32_t it = 0;
         for (;; ++it) {
-            const int s = static_cast<int>(it % NSTAGE);
-            const uint32_t ph = (it / NSTAGE) & 1u;
+            const int s = static_cast<int>(it % kSpanStages);
+            const uint32_t ph = (it / kSpanStages) & 1u;
             const uint8_t *bytes = mb.b[cc.batch].bytes;
             const int64_t *offs = mb.b[cc.batch].offs;
             const int nrows = static_cast<int>(cc.r1 - cc.r0) + 1;
@@ -453,7 +451,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
             // the first 32 rows' entries are formed before the barrier wait (their offsets are in flight meanwhile)
             int4 e0 = make_int4(0, 0, 0, 0);
             if (lane < nrows) e0 = row_entry(lane);
-            if (it >= NSTAGE) bar_wait(s_u32(empty + s), ph ^ 1u);  // the consumers are done with this stage
+            if (it >= kSpanStages) bar_wait(s_u32(empty + s), ph ^ 1u);  // the consumers are done with this stage
             if (lane == 0) {
                 if (nbytes) {
                     bar_expect_tx(s_u32(full + s), nbytes);
@@ -482,9 +480,9 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
         // end of work for this CTA: a stage whose header says so
         {
             ++it;
-            const int s = static_cast<int>(it % NSTAGE);
-            const uint32_t ph = (it / NSTAGE) & 1u;
-            if (it >= NSTAGE) bar_wait(s_u32(empty + s), ph ^ 1u);
+            const int s = static_cast<int>(it % kSpanStages);
+            const uint32_t ph = (it / kSpanStages) & 1u;
+            if (it >= kSpanStages) bar_wait(s_u32(empty + s), ph ^ 1u);
             if (lane == 0) {
                 hdr[s] = make_int4(0, 0, -1, 0);
                 bar_arrive(s_u32(full + s));
@@ -524,26 +522,14 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
     g.padq = lds128(cst_a + 48u);
     const uint32_t dyn_a = s_u32(dyn);
     for (uint32_t it = 0;; ++it) {
-        const int s = static_cast<int>(it % NSTAGE);
-        const uint32_t ph = (it / NSTAGE) & 1u;
+        const int s = static_cast<int>(it % kSpanStages);
+        const uint32_t ph = (it / kSpanStages) & 1u;
         const uint32_t rows_a = dyn_a + static_cast<uint32_t>(s * stage_stride + q.stage_bytes);
         bar_wait(s_u32(full + s), ph);
         BSQ_SPAN_MARK(it == 0 && ctid == 0, kTrFull0);
         const int4 h = hdr[s];
         if (h.z < 0) break;  // no more tiles for this CTA
         uint8_t *const otile = tile_out[s];
-        if (PRE) {
-            // phase 1: the staged residues become codes in place -- dense (every lane busy, no row logic, no
-            // realignment): LDS.128, 16 look-ups, STS.128 per 16 bytes of the span
-            const uint32_t d0 = dyn_a + static_cast<uint32_t>(s * stage_stride + kSpanSlack);
-            for (uint32_t b = 16u * static_cast<uint32_t>(ctid); b < static_cast<uint32_t>(h.w); b += 16u * kSpanConsumers) {
-                const uint4 v = lds128(d0 + b);
-                const uint32_t c0 = span_translate4(v.x, g.lutb), c1 = span_translate4(v.y, g.lutb);
-                const uint32_t c2 = span_translate4(v.z, g.lutb), c3 = span_translate4(v.w, g.lutb);
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(d0 + b), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-            }
-            asm volatile("bar.sync 1, %0;" ::"n"(kSpanConsumers) : "memory");  // consumers only
-        }
         // F: column-space offset of the lane's vector from column 0 of the tile's first row
         uint32_t F = static_cast<uint32_t>(h.x) + 16u * static_cast<uint32_t>(ctid);
         const uint32_t Fend = static_cast<uint32_t>(h.x) + 16u * static_cast<uint32_t>(h.z);
@@ -554,7 +540,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
                 const int col = static_cast<int>(rl * static_cast<uint32_t>(g.neg_padlen) + F);
                 const int4 ri = lds128i(rows_a + 16u * rl);  // {shared address of column 0's source byte, bos + len, bos + len + eos, -}
                 if (col >= ri.z) __stcs(reinterpret_cast<uint4 *>(dst), g.padq);
-                else __stcs(reinterpret_cast<uint4 *>(dst), span_row_codes<PRE>(static_cast<uint32_t>(ri.x), ri.y, col, g));
+                else __stcs(reinterpret_cast<uint4 *>(dst), span_row_codes(static_cast<uint32_t>(ri.x), ri.y, col, g));
                 BSQ_SPAN_MARK(it == 0 && ctid == 0 && dst == otile, kTrStore0);
             }
         } else {
@@ -571,9 +557,9 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
                 if (col >= ri.z) {
                     __stcs(reinterpret_cast<uint4 *>(dst), g.padq);
                 } else if (col >= 0 || ri.w <= g.padlen + col) {
-                    __stcs(reinterpret_cast<uint4 *>(dst), span_row_codes_u<PRE>(static_cast<uint32_t>(ri.x), ri.y, col, g));
+                    __stcs(reinterpret_cast<uint4 *>(dst), span_row_codes_u(static_cast<uint32_t>(ri.x), ri.y, col, g));
                 } else {
-                    __stcs(reinterpret_cast<uint4 *>(dst), span_straddle_general<PRE>(rows_a, rl, col, g));
+                    __stcs(reinterpret_cast<uint4 *>(dst), span_straddle_general(rows_a, rl, col, g));
                 }
                 BSQ_SPAN_MARK(it == 0 && ctid == 0 && dst == otile, kTrStore0);
             }
@@ -582,7 +568,7 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
                 const int col = static_cast<int>(rl * static_cast<uint32_t>(g.neg_padlen) + F);
                 const int4 ri = lds128i(rows_a + 16u * rl);
                 uint4 codes = g.padq;
-                if (col < ri.z) codes = span_row_codes_u<PRE>(static_cast<uint32_t>(ri.x), ri.y, col, g);
+                if (col < ri.z) codes = span_row_codes_u(static_cast<uint32_t>(ri.x), ri.y, col, g);
                 const int keep = h.y;
                 const uint32_t w[4] = {codes.x, codes.y, codes.z, codes.w};
 #pragma unroll
@@ -590,23 +576,15 @@ tokenize_span_kernel(const SpanParams q, const __grid_constant__ SpanBatches mb,
                     if (j < keep) dst[j] = static_cast<uint8_t>(w[j >> 2] >> (8 * (j & 3)));
             }
         }
-        // the stage was written through the generic proxy (phase 1); the next thing to touch it is the async proxy
-        if (PRE) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();
         if (lane == 0) bar_arrive(s_u32(empty + s));
     }
     BSQ_SPAN_MARK(lane == 0, kTrExit);
 }
 
-
-int span_env(const char *name, int dflt) {
-    const char *e = std::getenv(name);
-    return e ? std::atoi(e) : dflt;
-}
-
 struct DevInfo {
     int sms = 0;
-    bool attr_set[4][2][2][3] = {};
+    bool attr_set[2] = {};  // per ALIGNED: the kernel's shared-memory limit has been raised
     // tile counters of the dynamic scheduler: kCtrPairs x 2 slots x {handed out, CTAs done}, zero when idle (the
     // kernel re-arms its slot itself).  A stream owns a pair of slots and alternates between them: kernels of one
     // stream touch their counter only after the previous kernel of the stream has completed (griddepcontrol.wait /
@@ -680,32 +658,10 @@ unsigned int *tile_counter_slot(int device, cudaStream_t st) {
     return span_counter(dev_info(device), st);
 }
 
-bool span_kernel_applicable(int64_t padlen) {
-    static const bool tune = span_env("BSQ_TUNE", 0) != 0;
-    static bool on = span_env("BSQ_SPAN", 1) != 0;
-    static int minp = span_env("BSQ_SPAN_MINPAD", 257);
-    if (tune) {
-        on = span_env("BSQ_SPAN", 1) != 0;
-        minp = span_env("BSQ_SPAN_MINPAD", 257);
-    }
-    return on && padlen >= minp && padlen <= (1ll << 30);
-}
-
-// Launches K1s over `nbatch` (<= kSpanMaxBatches) batches that share padlen and tokenizer; `device` is the current device.
+// Launches K1s over `nbatch` (<= kSpanManyMax) batches that share padlen and tokenizer; `device` is the current device.
 int launch_tokenize_span_many(int device, cudaStream_t st, int nbatch, const uint8_t *const *d_bytes, const int64_t *const *d_offs,
-                              const int64_t *nseqs, int64_t padlen, const Prepared &p, uint8_t *const *outs, bool pdl_allowed) {
-    // A/B knobs (read once; BSQ_TUNE=1 re-reads them at every launch for in-process sweeps)
-    static const bool tune = span_env("BSQ_TUNE", 0) != 0;
-    static int vt_max = 0, nstage = 0, ctas_env = 0, two_phase = 0, minb = 4, dynamic = 1;
-    if (vt_max == 0 || tune) {
-        vt_max = std::max(256, span_env("BSQ_SPAN_VT", 1536) / 256 * 256);
-        nstage = std::min(4, std::max(2, span_env("BSQ_SPAN_STAGES", 2)));
-        ctas_env = span_env("BSQ_SPAN_CTAS", 0);
-        two_phase = span_env("BSQ_SPAN_2P", 0);
-        minb = std::min(6, std::max(4, span_env("BSQ_SPAN_MINB", 4)));
-        dynamic = span_env("BSQ_SPAN_DYN", 1);
-    }
-    if (nbatch <= 0 || nbatch > kSpanMaxBatches) return fail(BSQ_ERR_ARG, "bad batch count");
+                              const int64_t *nseqs, int64_t padlen, const Prepared &p, uint8_t *const *outs) {
+    if (nbatch <= 0 || nbatch > kSpanManyMax) return fail(BSQ_ERR_ARG, "bad batch count");
     std::lock_guard<std::mutex> dev_lock(g_dev_mu);
     DevInfo &di = dev_info(device);
     const int sms = di.sms > 0 ? di.sms : 148;
@@ -719,17 +675,16 @@ int launch_tokenize_span_many(int device, cudaStream_t st, int nbatch, const uin
     auto smem_for = [&](int vt) {
         const int stage_bytes = (kSpanSlack + vt * 16 + 32 + kSpanTail + 127) / 128 * 128;
         const int max_rows = static_cast<int>(std::min<int64_t>(vt * 16 / padlen + 3, max_nseq + 1));
-        return static_cast<size_t>(nstage) * (stage_bytes + 16 * ((max_rows + 7) / 8 * 8));
+        return static_cast<size_t>(kSpanStages) * (stage_bytes + 16 * ((max_rows + 7) / 8 * 8));
     };
-    const size_t static_smem = 256 + sizeof(TailTab) + 16 * nstage * 2 + 1024;
-    int per_sm = static_cast<int>((227 * 1024) / (smem_for(vt_max) + static_smem));
-    per_sm = std::max(1, std::min(std::min(per_sm, 2048 / kSpanThreads), minb));
-    if (ctas_env > 0) per_sm = std::min(per_sm, ctas_env);
+    const size_t static_smem = 256 + sizeof(TailTab) + 16 * kSpanStages * 2 + 1024;
+    int per_sm = static_cast<int>((227 * 1024) / (smem_for(kSpanTileVecs) + static_smem));
+    per_sm = std::max(1, std::min(std::min(per_sm, 2048 / kSpanThreads), kSpanCtasPerSm));
     const int64_t grid_full = static_cast<int64_t>(sms) * per_sm;
-    // tiles: as large as vt_max allows, and a count that fills whole rounds of the persistent grid
-    const int64_t rounds = std::max<int64_t>(1, (V + grid_full * vt_max - 1) / (grid_full * vt_max));
+    // tiles: at most kSpanTileVecs vectors, and a count that fills whole rounds of the persistent grid
+    const int64_t rounds = std::max<int64_t>(1, (V + grid_full * kSpanTileVecs - 1) / (grid_full * kSpanTileVecs));
     int64_t vt = (V + grid_full * rounds - 1) / (grid_full * rounds);
-    vt = std::min<int64_t>(vt_max, (vt + kSpanConsumers - 1) / kSpanConsumers * kSpanConsumers);
+    vt = std::min<int64_t>(kSpanTileVecs, (vt + kSpanConsumers - 1) / kSpanConsumers * kSpanConsumers);
     SpanBatches mb = {};
     int64_t ntiles = 0;
     int nb = 0;
@@ -755,16 +710,12 @@ int launch_tokenize_span_many(int device, cudaStream_t st, int nbatch, const uin
 #ifdef BSQ_SPAN_TRACE
     q.trace = g_span_trace;
 #endif
-    {
-        static int sel_body = span_env("BSQ_SPAN_SEL", 1);
-        if (tune) sel_body = span_env("BSQ_SPAN_SEL", 1);
-        q.straddle = (sel_body != 0 && padlen % 512 != 0) ? 1 : 0;
-    }
-    const size_t smem = static_cast<size_t>(nstage) * (q.stage_bytes + 16 * q.max_rows);
+    q.straddle = padlen % 512 != 0;
+    const size_t smem = static_cast<size_t>(kSpanStages) * (q.stage_bytes + 16 * q.max_rows);
     const bool aligned = padlen % 16 == 0;
 
     const int64_t blocks = std::min<int64_t>(ntiles, grid_full);
-    q.ctr = (dynamic && ntiles < 0x7fffffffll) ? span_counter(di, st) : nullptr;
+    q.ctr = ntiles < 0x7fffffffll ? span_counter(di, st) : nullptr;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(static_cast<unsigned>(blocks));
     cfg.blockDim = dim3(kSpanThreads);
@@ -777,44 +728,21 @@ int launch_tokenize_span_many(int device, cudaStream_t st, int nbatch, const uin
     // Programmatic dependent launch hides this launch's ramp behind the previous kernel's tail.  With the dynamic tile
     // order any co-residency is fine; with the static order two whole persistent grids must fit on the SMs at once
     // (otherwise the late CTAs pile up on the first SMs to drain and the fixed partition becomes unbalanced).
-    const bool pdl = pdl_allowed && (q.ctr != nullptr || (2 * per_sm * (smem + static_smem) <= 227 * 1024 && 2 * per_sm * kSpanThreads <= 2048));
+    const bool pdl = q.ctr != nullptr || (2 * per_sm * (smem + static_smem) <= 227 * 1024 && 2 * per_sm * kSpanThreads <= 2048);
     cfg.numAttrs = pdl ? 1 : 0;
 
-#define BSQ_SPAN_LAUNCH(NS, AL, PR, MB)                                                                                           \
-    do {                                                                                                                          \
-        auto kern = tokenize_span_kernel<NS, AL, PR, MB>;                                                                         \
-        if (!di.attr_set[NS - 1][AL][PR][MB - 4]) {                                                                               \
-            BSQ_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));                    \
-            di.attr_set[NS - 1][AL][PR][MB - 4] = true;                                                                           \
-        }                                                                                                                         \
-        BSQ_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, q, mb, p.lut, p.sp));                                                         \
-    } while (0)
-#define BSQ_SPAN_LAUNCH3(NS, MB)                                                                                                  \
-    do {                                                                                                                          \
-        if (aligned && two_phase) BSQ_SPAN_LAUNCH(NS, true, true, MB);                                                            \
-        else if (aligned) BSQ_SPAN_LAUNCH(NS, true, false, MB);                                                                   \
-        else if (two_phase) BSQ_SPAN_LAUNCH(NS, false, true, MB);                                                                 \
-        else BSQ_SPAN_LAUNCH(NS, false, false, MB);                                                                               \
-    } while (0)
-#define BSQ_SPAN_LAUNCH2(NS)                                                                                                      \
-    do {                                                                                                                          \
-        if (minb == 4) BSQ_SPAN_LAUNCH3(NS, 4);                                                                                   \
-        else if (minb == 5) BSQ_SPAN_LAUNCH3(NS, 5);                                                                              \
-        else BSQ_SPAN_LAUNCH3(NS, 6);                                                                                             \
-    } while (0)
-    if (nstage == 2) BSQ_SPAN_LAUNCH2(2);
-    else if (nstage == 3) BSQ_SPAN_LAUNCH2(3);
-    else BSQ_SPAN_LAUNCH2(4);
-#undef BSQ_SPAN_LAUNCH3
-#undef BSQ_SPAN_LAUNCH2
-#undef BSQ_SPAN_LAUNCH
+    const auto kern = aligned ? tokenize_span_kernel<true> : tokenize_span_kernel<false>;
+    if (!di.attr_set[aligned]) {
+        BSQ_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+        di.attr_set[aligned] = true;
+    }
+    BSQ_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, q, mb, p.lut, p.sp));
     count_launch();
     return BSQ_OK;
 }
 
-int launch_tokenize_span(int device, cudaStream_t st, const SeqView &v, int64_t nseq, int64_t padlen, const Prepared &p, uint8_t *out,
-                         bool pdl_allowed) {
-    return launch_tokenize_span_many(device, st, 1, &v.bytes, &v.offs, &nseq, padlen, p, &out, pdl_allowed);
+int launch_tokenize_span(int device, cudaStream_t st, const SeqView &v, int64_t nseq, int64_t padlen, const Prepared &p, uint8_t *out) {
+    return launch_tokenize_span_many(device, st, 1, &v.bytes, &v.offs, &nseq, padlen, p, &out);
 }
 
 }  // namespace bsq

@@ -180,6 +180,17 @@ def test_product_does_not_import_oracle():
                 assert "oracle" not in text.lower() or f == "synth.py", f"{f} mentions the oracle"
 
 
+def test_library_reads_only_the_documented_environment_variable():
+    # The shipped kernels run one measured configuration each; no environment variable may select another.
+    # BSQ_POOL_CAP (INTEGRATION.md) sizes the host worker pool and is the one variable the library reads.
+    csrc = os.path.join(ROOT, "bioseq_b200", "csrc")
+    calls = []
+    for f in sorted(os.listdir(csrc)):
+        text = open(os.path.join(csrc, f), errors="ignore").read()
+        calls += [(f, arg.strip()) for arg in re.findall(r"\b\w*getenv\s*\(([^)]*)\)", text)]
+    assert [arg for _, arg in calls] == ['"BSQ_POOL_CAP"'], calls
+
+
 def test_parallel_for_runs_every_share_once():
     # the persistent host worker pool behind the gather / scatter loops (no GPU involved)
     L = capi.lib()

@@ -1,7 +1,7 @@
 """The span kernel's tile schedule at its edges, bit for bit against the oracle.
 
 Every CTA of the span kernel (tokenize_span_kernel, padlen >= 257) takes two static tiles, blockIdx.x and
-blockIdx.x + G (G = gridDim.x = SMs x 4 CTAs at the default tile size of 1536 16-byte vectors), before it asks the
+blockIdx.x + G (G = gridDim.x = SMs x 4 CTAs of tiles of at most 1536 16-byte vectors), before it asks the
 per-stream atomic counter for more; the host sizes the tiles so that the tile count fills whole rounds of G.  The cases
 below sit on the boundaries of that schedule: fewer tiles than CTAs, exactly one round, between one and two rounds, just
 past two, several batches in one launch, launches that overwrite one buffer back to back (also inside a CUDA graph, where
@@ -16,7 +16,7 @@ from oracle.oracle import OracleTokenizer  # noqa: E402
 from helpers import assert_same_bits, gen  # noqa: E402
 
 MIX = b"ACDEFGHIKLMNPQRSTVWYacdefghiklmnpqrstvwyXBZOUJ*-NnUu .\x00\x7f\x80\xc3\xff"
-VT = 1536             # vectors of a full tile (BSQ_SPAN_VT's default)
+VT = 1536             # vectors of a full tile (kSpanTileVecs in bsq_span.cu)
 CTAS_PER_SM = 4      # span kernel CTAs per SM at that tile size
 
 

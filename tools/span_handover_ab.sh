@@ -48,7 +48,7 @@ echo "== C2, C2x4, P = 1026, P = 652 in one process per build (median of 5 windo
 for r in 1 2; do
     for side in old new; do
         d=$OLD; [ $side = new ] && d=$NEW
-        echo "$side:"; timeout 600 python "$NEW/tools/sweep_span_head.py" --root "$d" --rounds 5 "" 2>&1 | tee -a "$O/sweep_$side.txt"
+        echo "$side:"; timeout 600 python "$NEW/tools/sweep_span_head.py" --root "$d" --rounds 5 2>&1 | tee -a "$O/sweep_$side.txt"
     done
 done
 echo "== outputs of the last timed step"
