@@ -124,6 +124,7 @@ from .loaders import PyViewFF  # noqa: E402
 from .consumers import batch_onehot_encode_bcl, batch_embed, augment_packed, batch_tokenize_augmented  # noqa: E402
 from .consumers import batch_tokenize_varlen, VarlenBatch  # noqa: E402
 from .consumers import batch_tokenize_mlm, MLMBatch  # noqa: E402
+from .consumers import crop_packed, batch_tokenize_cropped, CroppedBatch  # noqa: E402
 
 
 def __getattr__(name):
@@ -142,4 +143,5 @@ __all__ = ["onehot_encode", "cbioseq", "f_encode", "Tokenizer", "make_embedding"
            "Reduced14Tokenizer", "DayhoffTokenizer", "LIATokenizer", "LIBTokenizer", "torchify",
            "set_num_threads", "get_num_threads", "Threading", "keys", "bkeys", "FlatFile", "FlatFileIterator", "getstats",
            "PyViewFF", "loaders", "consumers", "batch_onehot_encode_bcl", "batch_embed", "augment_packed",
-           "batch_tokenize_augmented", "batch_tokenize_varlen", "VarlenBatch", "batch_tokenize_mlm", "MLMBatch", "TokenizerLayer", "EmbeddingTokenizerLayer"]
+           "batch_tokenize_augmented", "batch_tokenize_varlen", "VarlenBatch", "batch_tokenize_mlm", "MLMBatch", "crop_packed",
+           "batch_tokenize_cropped", "CroppedBatch", "TokenizerLayer", "EmbeddingTokenizerLayer"]

@@ -104,6 +104,8 @@ def lib():
         "bsq_varlen_extent_device": (i32, [i32, vp, vp, i64, i64, tokp, C.POINTER(i64), C.POINTER(i64)]),
         "bsq_tokenize_mlm": (i32, [i32, vp, vp, vp, i64, i64, tokp, i32, C.POINTER(MLMDesc), vp, vp]),
         "bsq_tokenize_varlen_mlm": (i32, [i32, vp, vp, vp, i64, tokp, i32, C.POINTER(MLMDesc), vp, vp, vp]),
+        "bsq_crop": (i32, [i32, vp, vp, vp, i64, i64, i32, C.c_uint64, i64, vp, vp, vp]),
+        "bsq_crop_extent_device": (i32, [i32, vp, vp, i64, i64, i64, C.POINTER(i64), C.POINTER(i64)]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(L, name)
@@ -122,7 +124,7 @@ EXPORTS = ("bsq_abi_version bsq_last_error bsq_launch_count bsq_launch_count_res
            "bsq_free bsq_stage_host bsq_stage_release bsq_stager_set_augment bsq_onehot_bcl bsq_embed bsq_augment_blosum62 "
            "bsq_blosum62_thresholds bsq_tokenize_items bsq_onehot_items bsq_fetch_rows bsq_parallel_for "
            "bsq_tokenize_stream_items bsq_onehot_stream_items bsq_shard_bounds bsq_tokenize_host_sharded bsq_memcpy_d2d bsq_tokenize_many "
-           "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm").split()
+           "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm bsq_crop bsq_crop_extent_device").split()
 
 
 def last_error():
@@ -207,6 +209,22 @@ def varlen_extent_device(device, stream, d_offsets, nseq, tok, nbytes=-1):
     total, maxlen = C.c_int64(), C.c_int64()
     check(lib().bsq_varlen_extent_device(device, stream, _ptr(d_offsets), nseq, nbytes, C.byref(tok), C.byref(total),
                                          C.byref(maxlen)))
+    return total.value, maxlen.value
+
+
+def crop(device, stream, d_bytes, d_offsets, nseq, crop_len, random, seed, seq_index_base, d_out_bytes, d_out_offsets,
+         d_starts=None):
+    """Windows of at most crop_len residues per sequence (bsq_crop); ``random``: seeded windows, else the heads."""
+    check(lib().bsq_crop(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, crop_len, int(bool(random)),
+                         seed & 0xFFFFFFFFFFFFFFFF, seq_index_base, _ptr(d_out_bytes), _ptr(d_out_offsets), _ptr(d_starts)))
+
+
+def crop_extent_device(device, stream, d_offsets, nseq, crop_len, nbytes=-1):
+    """-> (sum, max) of min(len_i, crop_len) over device-resident offsets (bsq_crop_extent_device: validates them;
+    synchronises)."""
+    total, maxlen = C.c_int64(), C.c_int64()
+    check(lib().bsq_crop_extent_device(device, stream, _ptr(d_offsets), nseq, nbytes, crop_len, C.byref(total),
+                                       C.byref(maxlen)))
     return total.value, maxlen.value
 
 

@@ -16,6 +16,9 @@ Reference counterparts:
 * ``batch_tokenize_mlm`` -- a masked-language-model batch (the objective of ``training/cnnpretrain.py:119-125``; BERT /
   ESM pretraining): masked input tokens and ``cross_entropy``-ready int64 labels, padded or padding-free, written by
   one kernel instead of tokenize + the HuggingFace-collator recipe in torch (rand, where, index_put, casts).
+* ``crop_packed`` / ``crop=`` -- every sequence cropped to a window of the model's context on the device (ESM-style
+  seeded random windows, or the heads as HF ``truncation=True`` does) instead of slicing Python strings or gathering
+  in torch; the consumers above take ``crop=`` and ``crop_len=`` and run unchanged on the cropped batch.
 
 All of these call the C ABI (``include/bsq.h``) through ``capi``; torch supplies memory and the stream.
 A *batch* is one of
@@ -97,7 +100,7 @@ def _resolve_device(device):
 
 class _Resolved:
     """Device pointers of a batch plus what is needed to validate and release it."""
-    __slots__ = ("device", "stream", "d_bytes", "d_offs", "nseq", "h_offs", "keep", "ctx", "base")
+    __slots__ = ("device", "stream", "d_bytes", "d_offs", "nseq", "h_offs", "keep", "ctx", "base", "extent")
 
     def release(self):
         if self.ctx is not None:
@@ -106,13 +109,18 @@ class _Resolved:
             self.ctx = None
 
 
-def _resolve(batch, device, augment=None, before_stage=None):
+def _resolve(batch, device, augment=None, before_stage=None, crop=None):
     """-> _Resolved.  Host batches are staged (and, with ``augment``, mutated on the device after the copy);
     device batches are used in place (with ``augment``: a mutated clone).  ``before_stage(host_offsets, n)`` checks a
-    host batch before anything is copied to the device."""
+    host batch before anything is copied to the device.
+
+    ``crop`` (from ``_crop_spec``): the batch is cropped on the device after staging and the result describes the
+    cropped batch, with ``extent = (sum, max)`` of its lengths; ``augment`` then mutates the crop's fresh buffer in
+    place.  Host batches are sized from their host offsets (``before_stage`` sees the cropped offsets); device
+    batches pay one ``bsq_crop_extent_device`` (which also validates their offsets)."""
     torch = _torch()
     r = _Resolved()
-    r.ctx, r.keep, r.h_offs, r.base = None, [], None, 0
+    r.ctx, r.keep, r.h_offs, r.base, r.extent = None, [], None, 0, None
     host_b = host_o = None
     if isinstance(batch, tuple) and len(batch) == 3 and isinstance(batch[0], cbioseq.FlatFile):
         ff, start, stop = batch
@@ -127,6 +135,12 @@ def _resolve(batch, device, augment=None, before_stage=None):
                 raise ValueError("packed batch: contiguous uint8 bytes and int64 offsets expected")
             r.device = b.device.index
             r.stream = torch.cuda.current_stream(r.device).cuda_stream
+            if crop is not None:
+                r.d_bytes, r.d_offs, r.nseq = b.data_ptr(), o.data_ptr(), o.numel() - 1
+                r.keep += [b, o]
+                r.extent = capi.crop_extent_device(r.device, r.stream, o, r.nseq, crop[1], nbytes=b.numel())
+                _apply_crop(r, crop, augment)
+                return r
             if augment:
                 with torch.cuda.device(r.device):
                     b = b.clone()  # never mutate the caller's residues
@@ -170,6 +184,15 @@ def _resolve(batch, device, augment=None, before_stage=None):
                 raise ValueError("offsets run past the end of bytes")
             hb_ptr = host_b.ctypes.data
             r.keep += [host_b, host_o]
+        if crop is not None:
+            cropped_o, r.extent = _crop_host_extent(host_o, n, crop[1])
+            if before_stage is not None:
+                before_stage(cropped_o, n)
+            r.d_bytes, r.d_offs = ctx.stager.stage(r.stream, hb_ptr, host_o.ctypes.data, n)
+            r.nseq, r.ctx = n, ctx
+            _apply_crop(r, crop, augment)
+            r.h_offs = cropped_o
+            return r
         if before_stage is not None:
             before_stage(host_o, n)
         if augment:
@@ -187,6 +210,8 @@ def _resolve(batch, device, augment=None, before_stage=None):
 
 
 def _check_lengths(r, padlen, tok, onehot):
+    if r.extent is not None:  # cropped: _crop_spec capped crop_len at padlen - bos - eos, and the crop validated the offsets
+        return
     if r.h_offs is not None:
         capi.check_lengths_host(r.h_offs, r.nseq, padlen, tok, onehot=onehot)
     else:
@@ -207,18 +232,82 @@ def _augment_args(augment, augment_frac, seed, seq_index_base):
     return (int(augment), float(augment_frac), int(seed), int(seq_index_base))
 
 
+_CROP_MODES = (None, "head", "random")
+
+
+def _crop_spec(crop, crop_len, seed, seq_index_base, max_len=None):
+    """Validate the crop arguments (ValueError before anything is staged) -> None (no crop) or
+    ``(random, crop_len, seed, seq_index_base)``.  ``max_len``: the residues a padded row holds (``padlen - bos -
+    eos``), which is also the default ``crop_len``; None for padding-free output, where ``crop_len`` is required."""
+    if crop not in _CROP_MODES:
+        raise ValueError(f"crop must be one of None, 'head', 'random', got {crop!r}")
+    if crop is None:
+        if crop_len is not None:
+            raise ValueError("crop_len is given without crop: pass crop='head' or crop='random'")
+        return None
+    if crop_len is None:
+        if max_len is None:
+            raise ValueError("padding-free output needs an explicit crop_len")
+        crop_len = max_len
+    try:
+        crop_len = operator.index(crop_len)
+    except TypeError:
+        raise ValueError("crop_len must be an integer") from None
+    if crop_len < 1:
+        raise ValueError(f"crop_len must be >= 1, got {crop_len}")
+    if max_len is not None and crop_len > max_len:
+        raise ValueError(f"crop_len {crop_len} does not fit a row: padlen - bos - eos = {max_len}")
+    return (crop == "random", int(crop_len), int(seed), int(seq_index_base))
+
+
+def _crop_host_extent(h_offs, n, crop_len):
+    """-> (cropped offsets from 0, (sum, max) of the cropped lengths) of host offsets, in numpy; ValueError on offsets
+    the crop must not index with."""
+    o = np.asarray(h_offs[:n + 1], dtype=np.int64)
+    lens = np.diff(o)
+    if n > 0 and (int(o[0]) < 0 or int(lens.min()) < 0):
+        raise ValueError("offsets must start at or after 0 and be non-decreasing")
+    kept = np.minimum(lens, crop_len)
+    out = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(kept, out=out[1:])
+    return out, (int(out[n]), int(kept.max()) if n > 0 else 0)
+
+
+def _apply_crop(r, crop, augment):
+    """Crop the resolved batch into fresh device buffers (r.extent already holds their size), then augment them in
+    place; r then describes the cropped batch."""
+    torch = _torch()
+    random, crop_len, seed, base = crop
+    dev = torch.device("cuda", r.device)
+    out_b = torch.empty(max(r.extent[0], 1), dtype=torch.uint8, device=dev)  # (never a null pointer)
+    out_o = torch.empty(r.nseq + 1, dtype=torch.int64, device=dev)
+    # an all-empty batch may have no residue buffer at all; nothing is read from it then
+    capi.crop(r.device, r.stream, r.d_bytes or out_b, r.d_offs, r.nseq, crop_len, random, seed, base, out_b, out_o)
+    r.keep += [out_b, out_o]
+    r.d_bytes, r.d_offs, r.base = out_b.data_ptr(), out_o.data_ptr(), 0
+    if augment:
+        capi.augment_blosum62(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, *augment)
+
+
+def _row_residues(tokenizer, padlen):
+    return padlen - int(tokenizer.includes_bos()) - int(tokenizer.includes_eos())
+
+
 def batch_onehot_encode_bcl(tokenizer, batch, padlen=-1, destchar="f", mask=None, device=None, *, augment=0, augment_frac=1.0,
-                            seed=0, seq_index_base=0):
+                            seed=0, seq_index_base=0, crop=None, crop_len=None):
     """One-hot ``(batch, alphabet_size, padlen)`` tensor (CNN layout), default float32.
 
     Element ``[i, c, p]`` equals ``batch_onehot_encode(...)[p, i, c]`` (src/tokenize.h:345-368), i.e. the result of the
     reference's rearrange + float (bioseq/loaders.py:74-75).  ``mask``: uint8, one entry per residue of ``bytes``
-    (packed batches only)."""
+    (packed batches only, not with ``crop``).  ``crop``: as ``batch_tokenize_cropped``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     padlen = _default_padlen(batch, tokenizer, padlen)
     kind, dtype = _dtype_of(destchar)
-    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base))
+    crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
+    if crop is not None and mask is not None:
+        raise ValueError("mask covers the uncropped residues: it cannot be combined with crop")
+    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop)
     try:
         _check_lengths(r, padlen, tok, onehot=True)
         d_mask = None
@@ -248,22 +337,24 @@ def batch_onehot_encode_bcl(tokenizer, batch, padlen=-1, destchar="f", mask=None
 
 
 def batch_embed(tokenizer, batch, weight, padlen=-1, batch_first=True, device=None, *, augment=0, augment_frac=1.0, seed=0,
-                seq_index_base=0):
+                seq_index_base=0, crop=None, crop_len=None):
     """``weight[tokens]`` for the tokens of ``batch_tokenize(batch, padlen, batch_first=batch_first)`` without
     materialising them: ``(batch, padlen, dim)`` or ``(padlen, batch, dim)``, dtype and device of ``weight``.
 
     ``weight``: ``(rows >= alphabet_size, dim)`` CUDA tensor (an ``nn.Embedding.weight``); ``dim * itemsize`` must be
-    a multiple of 16 bytes.  Forward only (no autograd graph is recorded)."""
+    a multiple of 16 bytes.  Forward only (no autograd graph is recorded).  ``crop``: as ``batch_tokenize_cropped``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     padlen = _default_padlen(batch, tokenizer, padlen)
+    crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
     w = weight.detach()
     if not w.is_cuda or w.dim() != 2:
         raise ValueError("weight must be a 2-D CUDA tensor")
     if not w.is_contiguous():
         w = w.contiguous()
     row_bytes = w.shape[1] * w.element_size()
-    r = _resolve(batch, w.device if device is None else device, _augment_args(augment, augment_frac, seed, seq_index_base))
+    r = _resolve(batch, w.device if device is None else device, _augment_args(augment, augment_frac, seed, seq_index_base),
+                 crop=crop)
     try:
         if r.device != w.device.index:
             raise ValueError("weight and batch live on different devices")
@@ -288,6 +379,63 @@ def augment_packed(bytes_cuda, offsets_cuda, augment=1, augment_frac=1.0, seed=0
     capi.augment_blosum62(dev, torch.cuda.current_stream(dev).cuda_stream, bytes_cuda, offsets_cuda, offsets_cuda.numel() - 1,
                           int(augment), float(augment_frac), int(seed), int(seq_index_base))
     return bytes_cuda
+
+
+CroppedBatch = collections.namedtuple("CroppedBatch", ["bytes", "offsets", "starts"])
+CroppedBatch.__doc__ = """A cropped packed batch: ``bytes`` (uint8) and ``offsets`` (int64, from 0) of the windows, and ``starts``
+(int64, one per sequence: where its window begins in the sequence -- what a caller needs to crop per-residue labels or
+coordinates the same way)."""
+
+
+def crop_packed(bytes_cuda, offsets_cuda, crop_len, *, crop="random", seed=0, seq_index_base=0):
+    """Every sequence of a packed CUDA batch cropped to at most ``crop_len`` residues: a :class:`CroppedBatch`.
+
+    ``crop="random"``: a window drawn from Philox4x32-10 keyed by ``seed`` at sequence ``seq_index_base + i`` (the same
+    window whatever the batch's slicing; redraw with another seed); ``crop="head"``: the first ``crop_len`` residues.
+    A sequence no longer than ``crop_len`` is kept whole.  The exact rule is documented with ``bsq_crop`` in
+    include/bsq.h.  One synchronisation: the output's size is read back, and the offsets are validated."""
+    torch = _torch()
+    if not (isinstance(bytes_cuda, torch.Tensor) and bytes_cuda.is_cuda and bytes_cuda.dtype == torch.uint8 and
+            isinstance(offsets_cuda, torch.Tensor) and offsets_cuda.is_cuda and offsets_cuda.dtype == torch.int64 and
+            bytes_cuda.device == offsets_cuda.device and bytes_cuda.is_contiguous() and offsets_cuda.is_contiguous()):
+        raise ValueError("crop_packed: contiguous uint8 bytes and int64 offsets CUDA tensors on one device expected")
+    if crop is None:
+        raise ValueError("crop_packed: crop must be 'head' or 'random'")
+    random, crop_len, seed, base = _crop_spec(crop, crop_len, seed, seq_index_base)
+    if offsets_cuda.numel() < 1:
+        raise ValueError("offsets needs at least one entry")
+    dev = bytes_cuda.device
+    stream = torch.cuda.current_stream(dev.index).cuda_stream
+    n = offsets_cuda.numel() - 1
+    total, _ = capi.crop_extent_device(dev.index, stream, offsets_cuda, n, crop_len, nbytes=bytes_cuda.numel())
+    out_b = torch.empty(max(total, 1), dtype=torch.uint8, device=dev)
+    out_o = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    starts = torch.empty(n, dtype=torch.int64, device=dev)
+    src = bytes_cuda if bytes_cuda.numel() > 0 else out_b  # (an all-empty batch: nothing is read)
+    capi.crop(dev.index, stream, src, offsets_cuda, n, crop_len, random, seed, base, out_b, out_o, starts)
+    return CroppedBatch(out_b[:total], out_o, starts)
+
+
+def batch_tokenize_cropped(tokenizer, batch, padlen, destchar="B", batch_first=True, device=None, *, crop="random", crop_len=None,
+                           seed=0, seq_index_base=0, augment=0, augment_frac=1.0):
+    """``batch_tokenize`` of the batch with every sequence cropped to ``crop_len`` residues on the device (default and
+    maximum: ``padlen - bos - eos``): stage -> crop -> augment -> tokenize.  ``crop``: ``"random"`` or ``"head"``, as
+    :func:`crop_packed` (same ``seed`` / ``seq_index_base``)."""
+    torch = _torch()
+    tok = descriptor(tokenizer)
+    padlen = _default_padlen(batch, tokenizer, padlen)
+    kind, dtype = _dtype_of(destchar)
+    if crop is None:
+        raise ValueError("batch_tokenize_cropped: crop must be 'head' or 'random'")
+    crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
+    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop)
+    try:
+        shape = (r.nseq, padlen) if batch_first else (padlen, r.nseq)
+        out = torch.empty(shape, dtype=dtype, device=torch.device("cuda", r.device))
+        capi.tokenize(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, padlen, tok, batch_first, kind, out)
+        return out
+    finally:
+        r.release()
 
 
 def batch_tokenize_augmented(tokenizer, batch, padlen=-1, destchar="B", batch_first=False, device=None, *, augment=1,
@@ -334,28 +482,35 @@ def _varlen_extent_host(h_offs, n, k):
     return total, int(lens.max()) + k
 
 
-def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None):
+def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None, *, crop=None, crop_len=None, seed=0, seq_index_base=0):
     """Tokens of every sequence of ``batch`` back to back, without padding: a :class:`VarlenBatch`.
 
     Row ``i`` (``tokens[cu_seqlens[i]:cu_seqlens[i + 1]]``) equals ``batch_tokenize(batch, padlen=P, batch_first=True,
     destchar=destchar)[i, :len_i + bos + eos]`` for any large enough ``P``: ``[BOS] residues [EOS]``, no PAD token
     whatever ``padchar`` is.  ``cu_seqlens[i] = (offsets[i] - offsets[0]) + i * (bos + eos)`` as int32; a batch of more
     than 2^31 - 1 tokens raises ``ValueError``.  Host batches are sized from their host offsets without synchronising;
-    CUDA batches pay one synchronisation (the extent is read back)."""
-    return _tokenize_varlen(tokenizer, batch, destchar, device)
+    CUDA batches pay one synchronisation (the extent is read back).  ``crop`` / ``crop_len`` (required with ``crop``):
+    every sequence is cropped first, as :func:`crop_packed` does."""
+    return _tokenize_varlen(tokenizer, batch, destchar, device, crop=_crop_spec(crop, crop_len, seed, seq_index_base))
 
 
-def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None, mlm=None):
+def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None, mlm=None, crop=None):
     """batch_tokenize_varlen; ``augment``: BLOSUM62 arguments as ``_augment_args`` makes them (FlatFileDataset);
-    ``mlm``: a ``capi.MLMDesc`` -- then ``(VarlenBatch, labels)`` is returned."""
+    ``mlm``: a ``capi.MLMDesc`` -- then ``(VarlenBatch, labels)`` is returned; ``crop``: from ``_crop_spec``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
     k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
     extent = []
-    r = _resolve(batch, device, augment, before_stage=lambda h_offs, n: extent.extend(_varlen_extent_host(h_offs, n, k)))
+    r = _resolve(batch, device, augment, before_stage=lambda h_offs, n: extent.extend(_varlen_extent_host(h_offs, n, k)),
+                 crop=crop)
     try:
-        if r.h_offs is None:
+        if r.h_offs is None and r.extent is not None:  # a cropped CUDA batch: sized by the crop's one read-back
+            total, max_seqlen = r.extent[0] + r.nseq * k, (r.extent[1] + k if r.nseq > 0 else 0)
+            if total > _INT32_MAX:
+                raise ValueError(f"varlen batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one "
+                                 "batch; split the batch")
+        elif r.h_offs is None:
             nbytes = -1
             if isinstance(batch, tuple) and len(batch) == 2:
                 nbytes = batch[0].numel()
@@ -432,7 +587,7 @@ def _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignor
 
 def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *, varlen=False, maskfrac=0.15, mask_prob=0.8,
                        random_prob=0.1, mask_token=None, ignore_index=-100, seed=0, seq_index_base=0, augment=0,
-                       augment_frac=1.0):
+                       augment_frac=1.0, crop=None, crop_len=None):
     """A masked-language-model batch in one launch: :class:`MLMBatch` ``(inputs, labels)``.
 
     ``inputs`` start from ``batch_tokenize(batch, padlen, batch_first=True, destchar=destchar)`` (``varlen=False``:
@@ -446,7 +601,8 @@ def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *
     The draw is Philox4x32-10 keyed by ``seed`` at (``seq_index_base + i``, residue position): the same sequence gets
     the same mask padded or padding-free, in any slice (the exact rule is documented with ``bsq_tokenize_mlm`` in
     include/bsq.h).  ``augment``: BLOSUM62 point mutations first (as ``batch_tokenize_augmented``, same seed), then the
-    mask."""
+    mask.  ``crop`` / ``crop_len``: every sequence is cropped before both (as :func:`batch_tokenize_cropped`, same seed;
+    ``varlen=True`` needs an explicit ``crop_len``); residue positions are then positions within the window."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
@@ -455,10 +611,12 @@ def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *
     if varlen:
         if padlen is not None and padlen != -1:
             raise ValueError("batch_tokenize_mlm(varlen=True) writes no padding: padlen must not be given")
-        vb, labels = _tokenize_varlen(tokenizer, batch, destchar, device, augment, mlm)
+        crop = _crop_spec(crop, crop_len, seed, seq_index_base)
+        vb, labels = _tokenize_varlen(tokenizer, batch, destchar, device, augment, mlm, crop)
         return MLMBatch(vb, labels)
     padlen = _default_padlen(batch, tokenizer, padlen)
-    r = _resolve(batch, device, augment)
+    crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
+    r = _resolve(batch, device, augment, crop=crop)
     try:
         _check_lengths(r, padlen, tok, onehot=False)
         dev = torch.device("cuda", r.device)

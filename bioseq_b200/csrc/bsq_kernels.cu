@@ -14,7 +14,8 @@
 //   K4 decode_*             tokens -> characters: pass 1 decode_len16p_kernel (lengths, validation, where each row's
 //                           trailing <PAD> run starts) + scan, pass 2 decode_chars_kernel (text); bsq_decode_text
 //                           enqueues both behind one another.
-//   K0 maxlen_kernel        length and offsets validation for device-resident packed input.
+//   K0 maxlen_kernel        length and offsets validation for device-resident packed input (K0c crop_extent_kernel: the
+//                           same for a crop, bsq_crop_extent_device).
 //   (K1s, the batch-first one-byte kernel for padlen >= 257 -- the headline path -- lives in bsq_span.cu.)
 //
 // Reference semantics: src/tokenize.h:381-485 (K1/K2), :283-371 (K3), :131-179 (K4).
@@ -683,6 +684,34 @@ __global__ void maxlen_kernel(const int64_t *__restrict__ offs, int64_t nseq, in
     }
 }
 
+// K0c: K0's sibling for bsq_crop_extent_device -- the same validation bits, the longest cropped length min(len, W) in
+// out[0] and the sum of the cropped lengths in out[2].
+__global__ void crop_extent_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, int64_t W,
+                                   unsigned long long *out) {
+    long long best = 0, sum = 0;
+    unsigned bad = 0;
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const long long len = static_cast<long long>(offs[i + 1] - offs[i]);
+        if (len < 0) bad |= 1u;
+        if (i == 0 && offs[0] < 0) bad |= 2u;
+        if (i == nseq - 1 && nbytes >= 0 && offs[nseq] > nbytes) bad |= 4u;
+        const long long kept = min(max(len, 0ll), static_cast<long long>(W));
+        best = max(best, kept);
+        sum += kept;
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
+        sum += __shfl_xor_sync(0xffffffffu, sum, o);
+    }
+    bad = __reduce_or_sync(0xffffffffu, bad);
+    if ((threadIdx.x & 31) == 0) {
+        if (best > 0) atomicMax(out, static_cast<unsigned long long>(best));
+        if (bad) atomicOr(out + 1, static_cast<unsigned long long>(bad));
+        if (sum > 0) atomicAdd(out + 2, static_cast<unsigned long long>(sum));
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // K4: decode.  inv[key + 128] for key in [-128, 384): 0..255 = character, 0x100 + k = the
 // 5-character special k (0 <BOS>, 1 <EOS>, 2 <PAD>), 0xFFFF = no entry.
@@ -984,29 +1013,6 @@ __global__ void fill_i32_kernel(int32_t *p, int64_t n, int32_t v) {
 
 // exclusive scan of row_len (three small kernels; rows can be millions)
 constexpr int kScanBlock = 1024;
-__device__ __forceinline__ int64_t block_exclusive_scan(int64_t x, int64_t *s_warp, int64_t *total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    int64_t incl = x;
-    for (int o = 1; o < 32; o <<= 1) {
-        const int64_t y = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += y;
-    }
-    if (lane == 31) s_warp[warp] = incl;
-    __syncthreads();
-    if (warp == 0) {
-        int64_t wv = lane < (blockDim.x >> 5) ? s_warp[lane] : 0;
-        int64_t wi = wv;
-        for (int o = 1; o < 32; o <<= 1) {
-            const int64_t y = __shfl_up_sync(0xffffffffu, wi, o);
-            if (lane >= o) wi += y;
-        }
-        s_warp[lane] = wi - wv;  // exclusive prefix of the warp totals
-        if (lane == 31) *total = wi;
-    }
-    __syncthreads();
-    return s_warp[warp] + incl - x;
-}
-
 __global__ void __launch_bounds__(kScanBlock)
 scan_local_kernel(int64_t *__restrict__ data, int64_t n, int64_t *__restrict__ block_tot) {
     __shared__ int64_t s_warp[32];
@@ -1923,13 +1929,18 @@ int scratch_alloc(int device, void **p, size_t bytes, cudaStream_t st) {
 }
 
 // K0 and its read-back: h_res = {longest sequence, error bits, offsets[nseq] - offsets[0]}; fails on bad offsets.
-int reduce_offsets(int device, cudaStream_t st, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, unsigned long long h_res[3]) {
+// crop_len >= 1: K0c instead, h_res = {longest cropped length, error bits, sum of the cropped lengths}.
+int reduce_offsets(int device, cudaStream_t st, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, unsigned long long h_res[3],
+                   int64_t crop_len = 0) {
     BSQ_CUDA_TRY(cudaSetDevice(device));
     unsigned long long *d_res = nullptr;
     if (int rc = scratch_alloc(device, reinterpret_cast<void **>(&d_res), 3 * sizeof(*d_res), st)) return rc;
     BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, 3 * sizeof(*d_res), st));
     const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
-    maxlen_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, d_res, reinterpret_cast<long long *>(d_res + 2));
+    if (crop_len >= 1)
+        crop_extent_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, crop_len, d_res);
+    else
+        maxlen_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, d_res, reinterpret_cast<long long *>(d_res + 2));
     count_launch();
     BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, 3 * sizeof(*d_res), cudaMemcpyDeviceToHost, st));
     BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
@@ -1967,6 +1978,21 @@ int bsq_varlen_extent_device(int device, void *stream, const int64_t *d_offsets,
     const int64_t k = (tok->bos_id >= 0) + (tok->eos_id >= 0);
     *total = static_cast<int64_t>(h_res[2]) + nseq * k;
     *max_seqlen = static_cast<int64_t>(h_res[0]) + k;
+    return BSQ_OK;
+}
+
+int bsq_crop_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, int64_t crop_len,
+                           int64_t *total, int64_t *max_len) {
+    bsq::DeviceRestore restore_device;
+    if (total == nullptr || max_len == nullptr) return fail(BSQ_ERR_ARG, "null argument");
+    if (crop_len < 1) return fail(BSQ_ERR_ARG, "crop_len must be >= 1");
+    if (nseq < 0 || (nseq > 0 && d_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
+    *total = *max_len = 0;
+    if (nseq == 0) return BSQ_OK;
+    unsigned long long h_res[3] = {0, 0, 0};
+    if (int rc = reduce_offsets(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, h_res, crop_len)) return rc;
+    *total = static_cast<int64_t>(h_res[2]);
+    *max_len = static_cast<int64_t>(h_res[0]);
     return BSQ_OK;
 }
 

@@ -318,6 +318,32 @@ __device__ __forceinline__ Philox philox4x32_10(uint32_t c0, uint32_t c1, uint32
     return p;
 }
 
+// Exclusive prefix sum of one int64 per thread over the whole block (blockDim.x a multiple of 32, at most 1024);
+// *total receives the block's sum.  s_warp: 32 entries of shared memory.  Every thread of the block must call it.
+// Used by the decode scan (K4) and the crop's output offsets (K9).
+__device__ __forceinline__ int64_t block_exclusive_scan(int64_t x, int64_t *s_warp, int64_t *total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int64_t incl = x;
+    for (int o = 1; o < 32; o <<= 1) {
+        const int64_t y = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += y;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        int64_t wv = lane < (blockDim.x >> 5) ? s_warp[lane] : 0;
+        int64_t wi = wv;
+        for (int o = 1; o < 32; o <<= 1) {
+            const int64_t y = __shfl_up_sync(0xffffffffu, wi, o);
+            if (lane >= o) wi += y;
+        }
+        s_warp[lane] = wi - wv;  // exclusive prefix of the warp totals
+        if (lane == 31) *total = wi;
+    }
+    __syncthreads();
+    return s_warp[warp] + incl - x;
+}
+
 #endif  // __CUDACC__
 
 }  // namespace bsq

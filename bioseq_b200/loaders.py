@@ -5,7 +5,9 @@ on the CPU and move the numpy result to the device.  Here a range of the file go
 packed bytes + offsets (``Tokenizer.batch_tokenize_flatfile``), so no per-sequence host work is
 left.  BLOSUM62 augmentation (``augment=``; bioseq/blosum.py:63-87) runs on the device between the copy and
 the tokeniser (``consumers``; Philox streams keyed by the dataset seed, the draw number and the sequence index),
-and ``cnn=True`` batches are written directly in the ``(batch, emb, length)`` float layout.
+and ``cnn=True`` batches are written directly in the ``(batch, emb, length)`` float layout.  ``max_seq_len=`` crops
+over-long sequences on the device (``consumers.crop_packed``) so that a file with a few very long sequences still
+yields batches of the model's context.
 """
 import numpy as np
 
@@ -62,13 +64,20 @@ class FlatFileDataset(_dataset_base()):
     masked (id ``alphabet_size()``) / randomised / kept, labels ``-100`` elsewhere.  Like augmentation, every fetch is a
     new draw: the mask is keyed by the dataset seed, the draw number and the sequence's index in the file.
 
-    ``fetch(index, return_items=True)`` also hands back the raw sequence(s) (bioseq/loaders.py:60-84).  Two quirks of
+    ``max_seq_len=L`` makes rows ``L`` wide whatever the file holds: every sequence is cropped on the device to a window of
+    at most ``L - bos - eos`` residues before augmentation, masking or tokenization (the padding-free forms use the same
+    window length).  ``crop="random"`` (the default) draws a new window every fetch from the same per-fetch seed as
+    augmentation and masking (ESM-style); ``crop="head"`` keeps the first residues (truncation).  Without
+    ``max_seq_len`` rows are as wide as the file's longest sequence and nothing is cropped.
+
+    ``fetch(index, return_items=True)`` also hands back the raw sequence(s) (bioseq/loaders.py:60-84), as stored in the
+    file: uncropped, like they are unaugmented.  Two quirks of
     the reference's ``fetch`` are NOT reproduced: with ``cnn=True`` and ``return_items=False`` it falls off the end and
     returns ``None``, and without ``cnn`` it ignores ``return_items``; here both modes honour the flag.
     """
 
     def __init__(self, ff, tokenizer, *, augment=0, augment_frac=0.5, cnn=False, device=None, maskfrac=0.15, seed=13,
-                 varlen=False, mlm=False):
+                 varlen=False, mlm=False, max_seq_len=None, crop="random"):
         super().__init__()
         assert isinstance(ff, cbioseq.FlatFile)
         assert isinstance(tokenizer, cbioseq.Tokenizer)
@@ -80,7 +89,16 @@ class FlatFileDataset(_dataset_base()):
         self.ff, self.tokenizer = ff, tokenizer
         self.seed, self._draw = int(seed), 0  # the reference seeds its generator with 13 (bioseq/loaders.py:49-50)
         self.maskfrac, self.augment, self.augment_frac, self.cnn, self.device = maskfrac, augment, augment_frac, cnn, device
-        self.max_seq_len = ff.maxseqlen + tokenizer.includes_bos() + tokenizer.includes_eos()
+        k = tokenizer.includes_bos() + tokenizer.includes_eos()
+        self.crop, self.crop_len = None, None
+        if max_seq_len is None:
+            self.max_seq_len = ff.maxseqlen + k
+        else:
+            if crop not in ("head", "random"):
+                raise ValueError(f"FlatFileDataset: crop must be 'head' or 'random', got {crop!r}")
+            if max_seq_len < k + 1:
+                raise ValueError(f"FlatFileDataset: max_seq_len {max_seq_len} leaves no room for a residue next to bos + eos")
+            self.max_seq_len, self.crop, self.crop_len = int(max_seq_len), crop, int(max_seq_len) - k
         self.maxseqlen = self.max_seq_len
 
     def _range(self, index):
@@ -107,31 +125,38 @@ class FlatFileDataset(_dataset_base()):
     def __getitem__(self, index):
         import torch
         start, stop, many = self._range(index)
+        crop = dict(crop=self.crop, crop_len=self.crop_len) if self.crop else {}
         if self.mlm:
-            # one draw per fetch, shared by the augmentation (counter word 3 = 0) and the mask (words 1, 2)
+            # one draw per fetch, shared by the augmentation (counter word 3 = 0), the mask (words 1, 2) and the crop (3)
             kw = self._augment_kwargs(start)
             mb = consumers.batch_tokenize_mlm(self.tokenizer, (self.ff, start, stop),
                                               padlen=-1 if self.varlen else self.max_seq_len, destchar="l",
                                               device=self.device, varlen=self.varlen, maskfrac=self.maskfrac,
-                                              mask_token=self.tokenizer.alphabet_size(), **kw)
+                                              mask_token=self.tokenizer.alphabet_size(), **kw, **crop)
             if many:
                 return mb
             return consumers.MLMBatch(mb.inputs.tokens if self.varlen else mb.inputs[0], mb.labels if self.varlen else mb.labels[0])
-        aug = self._augment_kwargs(start) if self.augment else {}
+        aug = self._augment_kwargs(start) if self.augment or self.crop else {}
         if self.cnn:
             if many:  # (batch, emb, length) float, written in that layout by one kernel
                 return consumers.batch_onehot_encode_bcl(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
-                                                         destchar='f', device=self.device, **aug)
+                                                         destchar='f', device=self.device, **aug, **crop)
             if aug:
-                # (mutated on the device: the batched path at padlen = max_seq_len; a mutated sequence keeps its length,
-                # so only the reference's extra bos + eos pad rows of the single-sequence encoder are missing here)
+                # (mutated or cropped on the device: the batched path at padlen = max_seq_len; a mutated sequence keeps its
+                # length, so only the reference's extra bos + eos pad rows of the single-sequence encoder are missing here)
                 return consumers.batch_onehot_encode_bcl(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
-                                                         destchar='f', device=self.device, **aug)[0].t()
+                                                         destchar='f', device=self.device, **aug, **crop)[0].t()
             return self.tokenizer.onehot_encode(bytes(self.ff[start]), padlen=self.max_seq_len, destchar='f', device=self.device)
         if self.varlen:
             vb = consumers._tokenize_varlen(self.tokenizer, (self.ff, start, stop), "l", self.device,
-                                            consumers._augment_args(**aug) if aug else None)
+                                            consumers._augment_args(**aug) if aug else None,
+                                            crop=consumers._crop_spec(self.crop, self.crop_len, aug.get("seed", 0), start)
+                                            if crop else None)
             return vb if many else vb.tokens
+        if crop:
+            toks = consumers.batch_tokenize_cropped(self.tokenizer, (self.ff, start, stop), self.max_seq_len, batch_first=True,
+                                                    destchar='B', device=self.device, **aug, **crop).to(torch.long)
+            return toks if many else toks[0]
         if aug:
             toks = consumers.batch_tokenize_augmented(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
                                                       batch_first=True, destchar='B', device=self.device, **aug).to(torch.long)

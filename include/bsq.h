@@ -192,6 +192,37 @@ int bsq_tokenize_varlen_mlm(int device, void *stream, const uint8_t *d_bytes, co
                             const bsq_tokenizer *tok, int kind, const bsq_mlm *mlm, void *d_inputs, int64_t *d_labels,
                             int32_t *d_cu_seqlens);
 
+/* Cropping over-long sequences (protein / DNA language-model training crops each sequence to the model's context):
+ * a packed batch in, a packed batch of windows out, which every entry point above then takes unchanged.
+ * Let W = crop_len >= 1, len_i = offsets[i+1] - offsets[i] and len'_i = min(len_i, W).
+ *   - start_i = 0 if len_i <= W or the mode is head (random == 0).
+ *   - Random mode: with span = len_i - W + 1, g = seq_index_base + i, and (x0, x1, x2, x3) = Philox4x32-10 at counter
+ *     (g_lo, g_hi, 0, 3) under key (seed_lo, seed_hi):
+ *       start_i = floor(d * span / 2^64) with d = x0 | x1 << 32 (__umul64hi; exact integers, nothing in floating point).
+ *   - Output: out_offsets[0] = 0, out_offsets[i+1] = out_offsets[i] + len'_i, and
+ *     out_bytes[out_offsets[i] + j] = bytes[offsets[i] + start_i + j] for j < len'_i.  Optionally, starts[i] = start_i
+ *     (int64).
+ *   - Counter word 3 = 3 keeps these draws disjoint from augmentation (0) and MLM (1, 2) under the same seed.  The window
+ *     depends only on (seed, global sequence index, length, W).  It does not depend on padlen, on the padded or
+ *     padding-free form, or on how the data is sliced.
+ *   - A sequence no longer than W is copied unchanged, and no draw is used for it.
+ * Order inside a consumer: stage -> crop -> augment -> tokenize / mask.  For augmentation and MLM, "residue position"
+ * then means position within the window, and the sequence index is unchanged.
+ *
+ * bsq_crop enqueues only (at most three kernels; nseq == 0: an 8-byte memset of out_offsets), keeps no state between
+ * launches and is capturable into a CUDA graph.  The caller has validated the offsets (bsq_crop_extent_device does) and
+ * sized d_out_bytes to at least sum(len'_i) bytes (any alignment); d_out_offsets has nseq + 1 entries; d_starts (nseq
+ * entries) may be NULL.  BSQ_ERR_ARG for crop_len < 1, nseq < 0, or NULL pointers with nseq > 0, before any device call.
+ * The output must not overlap the input. */
+int bsq_crop(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq, int64_t crop_len,
+             int random, uint64_t seed, int64_t seq_index_base, uint8_t *d_out_bytes, int64_t *d_out_offsets, int64_t *d_starts);
+/* The extent of that output for device-resident offsets: *total = sum(len'_i) and *max_len = max(len'_i) (0 for
+ * nseq == 0), from one reduction kernel and one read-back (synchronises `stream`).  Validates the offsets like
+ * bsq_check_offsets_device, with no padlen limit (BSQ_ERR_ARG: negative length, offsets[0] < 0, offsets[nseq] > nbytes
+ * when nbytes >= 0); BSQ_ERR_ARG for crop_len < 1. */
+int bsq_crop_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, int64_t crop_len,
+                           int64_t *total, int64_t *max_len);
+
 /* Several batches that share padlen and tokenizer in one launch (batch-first one-byte tokens; other layouts / element
  * types fall back to one launch per batch): batch k = (d_bytes[k], d_offsets[k], nseq[k]) -> d_out[k].  The reference's
  * per-step callers tokenise small batches (training/cnnpretrain.py:123-125,145, bioseq/decoders.py:505): a 4096 x 1000
