@@ -106,6 +106,9 @@ def lib():
         "bsq_tokenize_varlen_mlm": (i32, [i32, vp, vp, vp, i64, tokp, i32, C.POINTER(MLMDesc), vp, vp, vp]),
         "bsq_crop": (i32, [i32, vp, vp, vp, i64, i64, i32, C.c_uint64, i64, vp, vp, vp]),
         "bsq_crop_extent_device": (i32, [i32, vp, vp, i64, i64, i64, C.POINTER(i64), C.POINTER(i64)]),
+        "bsq_seqpack_plan": (i32, [vp, i64, i32, i64, i64, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), vp, vp, vp, vp]),
+        "bsq_tokenize_seqpack": (i32, [i32, vp, vp, vp, tokp, i32, i64, i64, vp, vp, vp, vp]),
+        "bsq_tokenize_seqpack_mlm": (i32, [i32, vp, vp, vp, tokp, i32, C.POINTER(MLMDesc), i64, i64, vp, vp, vp, vp, vp]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(L, name)
@@ -124,7 +127,8 @@ EXPORTS = ("bsq_abi_version bsq_last_error bsq_launch_count bsq_launch_count_res
            "bsq_free bsq_stage_host bsq_stage_release bsq_stager_set_augment bsq_onehot_bcl bsq_embed bsq_augment_blosum62 "
            "bsq_blosum62_thresholds bsq_tokenize_items bsq_onehot_items bsq_fetch_rows bsq_parallel_for "
            "bsq_tokenize_stream_items bsq_onehot_stream_items bsq_shard_bounds bsq_tokenize_host_sharded bsq_memcpy_d2d bsq_tokenize_many "
-           "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm bsq_crop bsq_crop_extent_device").split()
+           "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm bsq_crop bsq_crop_extent_device "
+           "bsq_seqpack_plan bsq_tokenize_seqpack bsq_tokenize_seqpack_mlm").split()
 
 
 def last_error():
@@ -226,6 +230,31 @@ def crop_extent_device(device, stream, d_offsets, nseq, crop_len, nbytes=-1):
     check(lib().bsq_crop_extent_device(device, stream, _ptr(d_offsets), nseq, nbytes, crop_len, C.byref(total),
                                        C.byref(maxlen)))
     return total.value, maxlen.value
+
+
+def seqpack_plan(h_offsets, nseq, k, row_len, rows=0, starts=None, row_ptr=None, row_seq=None, cu_seqlens=None):
+    """Best-fit-decreasing layout of host offsets in rows of row_len (bsq_seqpack_plan) -> (R, nsegments, max_seqlen).
+    Without the four arrays only the sizes are computed; with them (host pointers or arrays: starts[nseq],
+    row_ptr[R + 1], row_seq[nseq] int64, cu_seqlens[nsegments + 1] int32) the layout is written as well."""
+    R, nseg, mx = C.c_int64(), C.c_int64(), C.c_int64()
+    check(lib().bsq_seqpack_plan(_ptr(h_offsets), nseq, k, row_len, rows, C.byref(R), C.byref(nseg), C.byref(mx), _ptr(starts),
+                                 _ptr(row_ptr), _ptr(row_seq), _ptr(cu_seqlens)))
+    return R.value, nseg.value, mx.value
+
+
+def tokenize_seqpack(device, stream, d_bytes, d_offsets, tok, kind, row_len, nrows, d_row_ptr, d_row_seq, d_tokens,
+                     d_position_ids):
+    """(nrows, row_len) tokens + int32 position ids of a plan (bsq_tokenize_seqpack)."""
+    check(lib().bsq_tokenize_seqpack(device, stream, _ptr(d_bytes), _ptr(d_offsets), C.byref(tok), kind, row_len, nrows,
+                                     _ptr(d_row_ptr), _ptr(d_row_seq), _ptr(d_tokens), _ptr(d_position_ids)))
+
+
+def tokenize_seqpack_mlm(device, stream, d_bytes, d_offsets, tok, kind, mlm, row_len, nrows, d_row_ptr, d_row_seq, d_inputs,
+                         d_position_ids, d_labels):
+    """The same with masked inputs + int64 labels (bsq_tokenize_seqpack_mlm); ``mlm``: an MLMDesc."""
+    check(lib().bsq_tokenize_seqpack_mlm(device, stream, _ptr(d_bytes), _ptr(d_offsets), C.byref(tok), kind, C.byref(mlm), row_len,
+                                         nrows, _ptr(d_row_ptr), _ptr(d_row_seq), _ptr(d_inputs), _ptr(d_position_ids),
+                                         _ptr(d_labels)))
 
 
 def onehot(device, stream, d_bytes, d_offsets, d_mask, nseq, padlen, tok, kind, d_out):

@@ -16,6 +16,9 @@ Reference counterparts:
 * ``batch_tokenize_mlm`` -- a masked-language-model batch (the objective of ``training/cnnpretrain.py:119-125``; BERT /
   ESM pretraining): masked input tokens and ``cross_entropy``-ready int64 labels, padded or padding-free, written by
   one kernel instead of tokenize + the HuggingFace-collator recipe in torch (rand, where, index_put, casts).
+* ``batch_tokenize_seqpack`` -- sequence packing: whole sequences best-fit into fixed-width ``(rows, L)`` rows with
+  position ids that restart per sequence and ``cu_seqlens`` (optionally MLM inputs and labels), written by one kernel
+  from a host plan instead of varlen tokenize + a torch scatter + ``repeat_interleave`` position ids.
 * ``crop_packed`` / ``crop=`` -- every sequence cropped to a window of the model's context on the device (ESM-style
   seeded random windows, or the heads as HF ``truncation=True`` does) instead of slicing Python strings or gathering
   in torch; the consumers above take ``crop=`` and ``crop_len=`` and run unchanged on the cropped batch.
@@ -109,7 +112,7 @@ class _Resolved:
             self.ctx = None
 
 
-def _resolve(batch, device, augment=None, before_stage=None, crop=None):
+def _resolve(batch, device, augment=None, before_stage=None, crop=None, crop_extent=None):
     """-> _Resolved.  Host batches are staged (and, with ``augment``, mutated on the device after the copy);
     device batches are used in place (with ``augment``: a mutated clone).  ``before_stage(host_offsets, n)`` checks a
     host batch before anything is copied to the device.
@@ -117,7 +120,8 @@ def _resolve(batch, device, augment=None, before_stage=None, crop=None):
     ``crop`` (from ``_crop_spec``): the batch is cropped on the device after staging and the result describes the
     cropped batch, with ``extent = (sum, max)`` of its lengths; ``augment`` then mutates the crop's fresh buffer in
     place.  Host batches are sized from their host offsets (``before_stage`` sees the cropped offsets); device
-    batches pay one ``bsq_crop_extent_device`` (which also validates their offsets)."""
+    batches pay one ``bsq_crop_extent_device`` (which also validates their offsets), unless the caller has read their
+    offsets back already and passes ``crop_extent``."""
     torch = _torch()
     r = _Resolved()
     r.ctx, r.keep, r.h_offs, r.base, r.extent = None, [], None, 0, None
@@ -138,7 +142,8 @@ def _resolve(batch, device, augment=None, before_stage=None, crop=None):
             if crop is not None:
                 r.d_bytes, r.d_offs, r.nseq = b.data_ptr(), o.data_ptr(), o.numel() - 1
                 r.keep += [b, o]
-                r.extent = capi.crop_extent_device(r.device, r.stream, o, r.nseq, crop[1], nbytes=b.numel())
+                r.extent = crop_extent if crop_extent is not None else capi.crop_extent_device(r.device, r.stream, o, r.nseq, crop[1],
+                                                                                                nbytes=b.numel())
                 _apply_crop(r, crop, augment)
                 return r
             if augment:
@@ -624,5 +629,132 @@ def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *
         labels = torch.empty((r.nseq, padlen), dtype=torch.int64, device=dev)
         capi.tokenize_mlm(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, padlen, tok, kind, mlm, inputs, labels)
         return MLMBatch(inputs, labels)
+    finally:
+        r.release()
+
+
+SeqPackBatch = collections.namedtuple("SeqPackBatch", ["tokens", "position_ids", "cu_seqlens", "max_seqlen", "starts", "labels"])
+SeqPackBatch.__doc__ = """Whole sequences packed into fixed-width rows: ``tokens`` ``(rows, L)`` (MLM inputs with ``mlm=True``),
+``position_ids`` int32 ``(rows, L)`` (0 at the start of every sequence and of every row's padding run), ``cu_seqlens`` (int32:
+the flat start of every segment -- a sequence or a padding run -- then ``rows * L``), ``max_seqlen`` (int, the longest
+segment), ``starts`` (int64, one per sequence: its flat position in ``tokens.view(-1)``, -1 for a sequence that occupies
+nothing) and ``labels`` (int64 ``(rows, L)`` with ``mlm=True``, else None)."""
+
+
+def _seqpack_host_offsets(batch):
+    """Host offsets to plan a batch from before it is staged: a CUDA batch's are read back and validated (one
+    synchronisation); host arrays and FlatFile ranges are used as they are.  None for a list of items (planned once
+    ``_resolve`` has gathered it)."""
+    torch = _torch()
+    if isinstance(batch, tuple) and len(batch) == 3 and isinstance(batch[0], cbioseq.FlatFile):
+        return batch[0].packed(batch[1], batch[2])[1]
+    if not (isinstance(batch, tuple) and len(batch) == 2 and hasattr(batch[0], "dtype")):
+        return None
+    b, o = batch
+    if not (isinstance(b, torch.Tensor) and b.is_cuda):
+        o = o.numpy() if isinstance(o, torch.Tensor) else np.asarray(o)
+        return o if o.dtype == np.int64 and o.ndim == 1 and o.size >= 1 else None  # (anything else: _resolve raises)
+    if not (isinstance(o, torch.Tensor) and o.is_cuda and o.device == b.device):
+        raise ValueError("bytes and offsets must live on the same side (all host or all CUDA)")
+    if b.dtype != torch.uint8 or o.dtype != torch.int64 or not b.is_contiguous() or not o.is_contiguous():
+        raise ValueError("packed batch: contiguous uint8 bytes and int64 offsets expected")
+    if o.numel() < 1:
+        raise ValueError("offsets needs at least one entry")
+    h = o.cpu().numpy()
+    n = h.size - 1
+    if n > 0 and (int(h[0]) < 0 or int(np.diff(h).min()) < 0):
+        raise ValueError("offsets must start at or after 0 and be non-decreasing")
+    if int(h[n]) > b.numel():
+        raise ValueError("offsets run past the end of bytes")
+    return h
+
+
+class _SeqPackPlan:
+    """The host plan (bsq_seqpack_plan) in one pinned int64 buffer: row_ptr | row_seq | starts | cu_seqlens (int32)."""
+
+    def __init__(self, h_offs, n, k, row_len, rows):
+        torch = _torch()
+        h_offs = np.ascontiguousarray(h_offs[:n + 1], dtype=np.int64)
+        R, nseg, self.max_seqlen = capi.seqpack_plan(h_offs, n, k, row_len, rows)  # (sizes; ValueError on a bad layout)
+        self.R, self.nseg, self.n = R, nseg, n
+        self.o_seq, self.o_starts, self.o_cu = R + 1, R + 1 + n, R + 1 + 2 * n
+        self.buf = torch.empty(self.o_cu + (nseg + 2) // 2, dtype=torch.int64, pin_memory=True)
+        a = self.buf.numpy()
+        capi.seqpack_plan(h_offs, n, k, row_len, rows, a[self.o_starts:], a, a[self.o_seq:], a[self.o_cu:])
+
+    def to_device(self, dev):
+        """One cudaMemcpyAsync from pinned memory on the current stream."""
+        self.dbuf = self.buf.to(dev, non_blocking=True)
+        d = self.dbuf
+        return (d[:self.o_seq], d[self.o_seq:self.o_starts], d[self.o_starts:self.o_cu],
+                d[self.o_cu:].view(_torch().int32)[:self.nseg + 1])
+
+
+def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None, *, rows=None, mlm=False, maskfrac=0.15,
+                           mask_prob=0.8, random_prob=0.1, mask_token=None, ignore_index=-100, crop=None, crop_len=None,
+                           augment=0, augment_frac=1.0, seed=0, seq_index_base=0):
+    """Sequence packing: every sequence of ``batch`` whole, laid end to end in rows of ``row_len`` tokens -- a
+    :class:`SeqPackBatch` of fixed shape ``(rows, row_len)`` with almost no padding.
+
+    Placement is best-fit decreasing (longest first, each into the fullest row that still fits it; the exact,
+    deterministic rule is documented with ``bsq_seqpack_plan`` in include/bsq.h).  The tokens of sequence ``i`` at
+    ``starts[i]`` equal row ``i`` of :func:`batch_tokenize_varlen`: ``[BOS] residues [EOS]``; the rest of a row is what
+    ``batch_tokenize`` writes after EOS.  ``position_ids`` restart at 0 for every sequence and padding run, and
+    ``cu_seqlens`` lists them all, so the batch feeds ``flash_attn_varlen_func`` (flattened), SDPA with a block mask
+    (``(position_ids == 0).cumsum(-1)``) or models that find packed sequences from position ids.
+
+    ``rows``: exactly that many rows (extra rows are padding; ValueError if the batch needs more), else as many as
+    needed.  ``mlm=True``: inputs and int64 labels as :func:`batch_tokenize_mlm` (``varlen=True``, same seed and
+    ``seq_index_base``) writes them per sequence, padding labels ``ignore_index``.  ``crop`` / ``crop_len`` (default
+    ``row_len - bos - eos``) and ``augment`` as for the other consumers: stage -> crop -> augment -> pack.  Every
+    sequence must fit a row (ValueError otherwise).  Host batches are planned from their host offsets without
+    synchronising; CUDA batches pay one read-back of their offsets, which also validates them."""
+    torch = _torch()
+    tok = descriptor(tokenizer)
+    kind, dtype = _dtype_of(destchar)
+    k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
+    try:
+        row_len = operator.index(row_len)
+        rows = None if rows is None else operator.index(rows)
+    except TypeError:
+        raise ValueError("row_len and rows must be integers") from None
+    if row_len < 1:
+        raise ValueError(f"row_len must be >= 1, got {row_len}")
+    if rows is not None and rows < 1:
+        raise ValueError(f"rows must be >= 1, got {rows}")
+    rows = rows or 0  # (the planner's "as many as needed")
+    mlm = _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignore_index, seed, seq_index_base) if mlm else None
+    crop = _crop_spec(crop, crop_len, seed, seq_index_base, row_len - k)
+    augment = _augment_args(augment, augment_frac, seed, seq_index_base)
+    plan = []
+
+    def make_plan(h_offs, n):
+        plan.append(_SeqPackPlan(h_offs, n, k, row_len, rows))
+
+    h = _seqpack_host_offsets(batch)
+    crop_extent = None
+    if h is not None:  # planned before anything is staged (a CUDA batch: from its offsets, read back once)
+        n = h.size - 1
+        if crop is not None:
+            h, crop_extent = _crop_host_extent(h, n, crop[1])
+        make_plan(h, n)
+    r = _resolve(batch, device, augment, before_stage=None if h is not None else make_plan, crop=crop, crop_extent=crop_extent)
+    try:
+        p = plan[0]
+        dev = torch.device("cuda", r.device)
+        with torch.cuda.device(r.device):
+            d_row_ptr, d_row_seq, starts, cu_seqlens = p.to_device(dev)
+        tokens = torch.empty((p.R, row_len), dtype=dtype, device=dev)
+        position_ids = torch.empty((p.R, row_len), dtype=torch.int32, device=dev)
+        labels = None
+        if mlm is not None:
+            labels = torch.empty((p.R, row_len), dtype=torch.int64, device=dev)
+            capi.tokenize_seqpack_mlm(r.device, r.stream, r.d_bytes, r.d_offs, tok, kind, mlm, row_len, p.R, d_row_ptr, d_row_seq,
+                                      tokens, position_ids, labels)
+        else:
+            capi.tokenize_seqpack(r.device, r.stream, r.d_bytes, r.d_offs, tok, kind, row_len, p.R, d_row_ptr, d_row_seq, tokens,
+                                  position_ids)
+        r.keep.append(p)
+        return SeqPackBatch(tokens, position_ids, cu_seqlens, p.max_seqlen, starts, labels)
     finally:
         r.release()

@@ -15,6 +15,7 @@
 #include <stdint.h>
 
 struct bsq_tokenizer;
+struct bsq_mlm;
 
 namespace bsq {
 
@@ -90,6 +91,19 @@ void span_magic(uint32_t d, uint32_t *mul, uint32_t *shift);
 constexpr int kSpanManyMax = 32;  // batches per launch of launch_tokenize_span_many
 int launch_tokenize_span_many(int device, cudaStream_t st, int nbatch, const uint8_t *const *d_bytes, const int64_t *const *d_offs,
                               const int64_t *nseqs, int64_t padlen, const Prepared &p, uint8_t *const *outs);
+
+// Masked-language-model parameters (include/bsq.h, bsq_mlm) in kernel form, and below the per-residue selection and
+// corruption shared by K8 (bsq_mlm.cu) and K10 (bsq_seqpack.cu).
+struct MlmParam {
+    uint32_t k0, k1;      // Philox key (seed)
+    uint64_t ts, tm, tr;  // t_select, t_mask, t_random, each in [0, 2^32]
+    int64_t base;         // global index of this launch's sequence 0
+    int64_t ignore;       // label of positions that are not selected
+    int32_t mask_id;
+    uint32_t nchars;
+};
+// Validates a bsq_mlm for `kind` (BSQ_ERR_ARG with the message of include/bsq.h) and fills *m (bsq_mlm.cu).
+int check_mlm_param(const bsq_tokenizer *tok, int kind, const bsq_mlm *mlm, MlmParam *m);
 
 #ifdef __CUDACC__
 
@@ -342,6 +356,147 @@ __device__ __forceinline__ int64_t block_exclusive_scan(int64_t x, int64_t *s_wa
     }
     __syncthreads();
     return s_warp[warp] + incl - x;
+}
+
+// word w (0..3) of a block, with selects (a run-time index into the block would put it in local memory)
+__device__ __forceinline__ uint32_t pick4(const Philox &p, uint32_t w) {
+    const uint32_t lo = (w & 1u) ? p.c[1] : p.c[0], hi = (w & 1u) ? p.c[3] : p.c[2];
+    return (w & 2u) ? hi : lo;
+}
+
+__device__ __forceinline__ Philox mlm_block(uint64_t g, uint32_t blk, uint32_t stream, const MlmParam &m) {
+    return philox4x32_10(static_cast<uint32_t>(g), static_cast<uint32_t>(g >> 32), blk, stream, m.k0, m.k1);
+}
+
+__device__ __forceinline__ uint32_t mlm_random_id(uint64_t g, uint32_t j, const MlmParam &m) {
+    return __umulhi(pick4(mlm_block(g, j >> 2, 2u, m), j & 3u), m.nchars);
+}
+
+template <typename T>
+__device__ __forceinline__ T code_value(uint32_t code, const Expand &ex) {
+    // one-byte kinds: codes are the output bytes; wider kinds: ids through Expand
+    if (sizeof(T) == 1) return static_cast<T>(static_cast<uint8_t>(code));
+    return static_cast<T>(expand_code(code, ex));
+}
+
+// The decisions for 16 consecutive positions p of one row whose position 0 is residue j0 (position p is a residue
+// iff 0 <= j0 + p < len): bit p of sel (selected), msk (-> mask_id) and rnd (-> random id), the random ids one per
+// byte of rid.
+struct Mlm16 {
+    uint32_t sel, msk, rnd;
+    uint32_t rid[4];
+};
+
+__device__ __forceinline__ Mlm16 mlm_decide16(int j0, int len, uint64_t g, const MlmParam &m) {
+    Mlm16 d;
+    d.sel = d.msk = d.rnd = 0u;
+    d.rid[0] = d.rid[1] = d.rid[2] = d.rid[3] = 0u;
+    const int lo = max(-j0, 0), hi = min(len - j0, 16);
+    if (hi <= lo) return d;  // no residue (padding, or only BOS / EOS)
+    // selection words of blocks j0 >> 2 .. +4 that hold a residue of the chunk (j0 = -1: block -1 holds none)
+    const int b0 = j0 >> 2, jlo = j0 + lo, jhi = j0 + hi - 1;
+    uint32_t W[20];
+#pragma unroll
+    for (int b = 0; b < 5; ++b) {
+        const int blk = b0 + b;
+        W[4 * b] = W[4 * b + 1] = W[4 * b + 2] = W[4 * b + 3] = 0u;
+        if (4 * blk + 3 >= jlo && 4 * blk <= jhi) {
+            const Philox p = mlm_block(g, static_cast<uint32_t>(blk), 1u, m);
+            W[4 * b] = p.c[0]; W[4 * b + 1] = p.c[1]; W[4 * b + 2] = p.c[2]; W[4 * b + 3] = p.c[3];
+        }
+    }
+    // u[p] = W[(j0 & 3) + p]: a two-step shift with selects
+    const uint32_t a = static_cast<uint32_t>(j0) & 3u;
+    uint32_t X[18];
+#pragma unroll
+    for (int q = 0; q < 18; ++q) X[q] = (a & 2u) ? W[q + 2] : W[q];
+#pragma unroll
+    for (int p = 0; p < 16; ++p) {
+        const uint64_t u = (a & 1u) ? X[p + 1] : X[p];
+        if (p >= lo && p < hi && u < m.ts) {
+            d.sel |= 1u << p;
+            if (u < m.tm) d.msk |= 1u << p;
+            else if (u < m.tr) d.rnd |= 1u << p;
+        }
+    }
+    // random ids: rare (random_prob of the selected share), one block each, only where needed
+    uint32_t need = d.rnd;
+    while (need) {
+        const int p = __ffs(need) - 1;
+        need &= need - 1u;
+        const uint32_t v = mlm_random_id(g, static_cast<uint32_t>(j0 + p), m) << (8 * (p & 3));
+        const int w = p >> 2;
+        d.rid[0] |= w == 0 ? v : 0u;
+        d.rid[1] |= w == 1 ? v : 0u;
+        d.rid[2] |= w == 2 ? v : 0u;
+        d.rid[3] |= w == 3 ? v : 0u;
+    }
+    return d;
+}
+
+// bits 0..3 of x -> 0x000000ff / 0x0000ff00 / 0x00ff0000 / 0xff000000
+__device__ __forceinline__ uint32_t byte_mask4(uint32_t x) { return (((x & 0xfu) * 0x00204081u) & 0x01010101u) * 0xffu; }
+
+// 16 codes t (bytes) + decisions -> inputs at `in` and labels at `lab`.  VEC: 16 elements, both pointers 16-byte
+// aligned; otherwise the first cnt elements, one by one.
+template <typename T, bool VEC>
+__device__ __forceinline__ void mlm_emit16(T *in, int64_t *lab, const uint32_t t[4], const Mlm16 &d, int cnt, const MlmParam &m,
+                                           const Expand &ex) {
+    if (sizeof(T) == 1) {
+        const uint32_t mrep = (static_cast<uint32_t>(m.mask_id) & 0xffu) * 0x01010101u;
+        uint32_t o[4];
+#pragma unroll
+        for (int w = 0; w < 4; ++w) {
+            const uint32_t mm = byte_mask4(d.msk >> (4 * w)), rm = byte_mask4(d.rnd >> (4 * w));
+            o[w] = (t[w] & ~(mm | rm)) | (mrep & mm) | (d.rid[w] & rm);
+        }
+        if (VEC) {
+            __stcs(reinterpret_cast<uint4 *>(in), make_uint4(o[0], o[1], o[2], o[3]));
+        } else {
+#pragma unroll
+            for (int p = 0; p < 16; ++p)
+                if (p < cnt) reinterpret_cast<uint8_t *>(in)[p] = static_cast<uint8_t>(o[p >> 2] >> (8 * (p & 3)));
+        }
+    } else {
+        constexpr int EPV = 16 / sizeof(T);
+#pragma unroll
+        for (int s = 0; s < 16 / EPV; ++s) {
+            T vals[EPV];
+#pragma unroll
+            for (int j = 0; j < EPV; ++j) {
+                const int p = s * EPV + j;
+                const uint32_t code = (t[p >> 2] >> (8 * (p & 3))) & 0xffu;
+                const uint32_t rid = (d.rid[p >> 2] >> (8 * (p & 3))) & 0xffu;
+                vals[j] = (d.msk >> p) & 1u ? static_cast<T>(m.mask_id)
+                                            : ((d.rnd >> p) & 1u ? static_cast<T>(static_cast<int32_t>(rid)) : code_value<T>(code, ex));
+            }
+            if (VEC) {
+                __stcs(reinterpret_cast<uint4 *>(in) + s, *reinterpret_cast<const uint4 *>(vals));
+            } else {
+#pragma unroll
+                for (int j = 0; j < EPV; ++j)
+                    if (s * EPV + j < cnt) in[s * EPV + j] = vals[j];
+            }
+        }
+    }
+    // labels: the residue's code (< 0x80 in every mode) where selected
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+        int64_t l[2];
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+            const int p = 2 * q + h;
+            l[h] = (d.sel >> p) & 1u ? static_cast<int64_t>((t[p >> 2] >> (8 * (p & 3))) & 0xffu) : m.ignore;
+        }
+        if (VEC) {
+            __stcs(reinterpret_cast<uint4 *>(lab) + q,
+                   make_uint4(static_cast<uint32_t>(l[0]), static_cast<uint32_t>(static_cast<uint64_t>(l[0]) >> 32),
+                              static_cast<uint32_t>(l[1]), static_cast<uint32_t>(static_cast<uint64_t>(l[1]) >> 32)));
+        } else {
+            if (2 * q < cnt) lab[2 * q] = l[0];
+            if (2 * q + 1 < cnt) lab[2 * q + 1] = l[1];
+        }
+    }
 }
 
 #endif  // __CUDACC__

@@ -70,6 +70,11 @@ class FlatFileDataset(_dataset_base()):
     augmentation and masking (ESM-style); ``crop="head"`` keeps the first residues (truncation).  Without
     ``max_seq_len`` rows are as wide as the file's longest sequence and nothing is cropped.
 
+    With ``seqpack=True`` a slice is a ``consumers.SeqPackBatch``: its sequences packed whole, best-fit, into as few rows of
+    ``max_seq_len`` as they need, with ``long`` tokens, position ids that restart per sequence and ``cu_seqlens`` (and
+    labels with ``mlm=True``); a single index is the same with one row.  Crop, augmentation and masking draw from the
+    per-fetch seed as above.  ``seqpack=True`` cannot be combined with ``varlen=True`` or ``cnn=True``.
+
     ``fetch(index, return_items=True)`` also hands back the raw sequence(s) (bioseq/loaders.py:60-84), as stored in the
     file: uncropped, like they are unaugmented.  Two quirks of
     the reference's ``fetch`` are NOT reproduced: with ``cnn=True`` and ``return_items=False`` it falls off the end and
@@ -77,7 +82,7 @@ class FlatFileDataset(_dataset_base()):
     """
 
     def __init__(self, ff, tokenizer, *, augment=0, augment_frac=0.5, cnn=False, device=None, maskfrac=0.15, seed=13,
-                 varlen=False, mlm=False, max_seq_len=None, crop="random"):
+                 varlen=False, mlm=False, max_seq_len=None, crop="random", seqpack=False):
         super().__init__()
         assert isinstance(ff, cbioseq.FlatFile)
         assert isinstance(tokenizer, cbioseq.Tokenizer)
@@ -85,7 +90,10 @@ class FlatFileDataset(_dataset_base()):
             raise ValueError("FlatFileDataset: varlen=True yields tokens, cnn=True one-hot; choose one")
         if mlm and cnn:
             raise ValueError("FlatFileDataset: mlm=True yields masked tokens and labels, cnn=True one-hot; choose one")
-        self.varlen, self.mlm = bool(varlen), bool(mlm)
+        if seqpack and (varlen or cnn):
+            raise ValueError("FlatFileDataset: seqpack=True yields packed fixed-width rows; it cannot be combined with varlen=True "
+                             "or cnn=True")
+        self.varlen, self.mlm, self.seqpack = bool(varlen), bool(mlm), bool(seqpack)
         self.ff, self.tokenizer = ff, tokenizer
         self.seed, self._draw = int(seed), 0  # the reference seeds its generator with 13 (bioseq/loaders.py:49-50)
         self.maskfrac, self.augment, self.augment_frac, self.cnn, self.device = maskfrac, augment, augment_frac, cnn, device
@@ -126,6 +134,11 @@ class FlatFileDataset(_dataset_base()):
         import torch
         start, stop, many = self._range(index)
         crop = dict(crop=self.crop, crop_len=self.crop_len) if self.crop else {}
+        if self.seqpack:
+            kw = self._augment_kwargs(start) if self.mlm or self.augment or self.crop else {}
+            mlm = dict(mlm=True, maskfrac=self.maskfrac, mask_token=self.tokenizer.alphabet_size()) if self.mlm else {}
+            return consumers.batch_tokenize_seqpack(self.tokenizer, (self.ff, start, stop), self.max_seq_len, "l", self.device,
+                                                    rows=None if many else 1, **mlm, **kw, **crop)
         if self.mlm:
             # one draw per fetch, shared by the augmentation (counter word 3 = 0), the mask (words 1, 2) and the crop (3)
             kw = self._augment_kwargs(start)
@@ -182,7 +195,7 @@ class FlatFileDataset(_dataset_base()):
 
     def batches(self, batch_size, prefetch=0):
         """Consecutive ``(batch, max_seq_len)`` token batches (``VarlenBatch``es with ``varlen=True``, ``MLMBatch``es with
-        ``mlm=True``) covering the file.
+        ``mlm=True``, ``SeqPackBatch``es of ``batch_size`` sequences with ``seqpack=True``) covering the file.
 
         ``prefetch=k`` (k > 0) keeps k batches ahead of the consumer on a side stream: the host-to-device copy and the
         tokeniser of batch i+1 .. i+k run while the caller's stream is still busy with batch i (the reference's
@@ -203,7 +216,7 @@ class FlatFileDataset(_dataset_base()):
         def record(x, cur):
             if isinstance(x, torch.Tensor):
                 x.record_stream(cur)  # (allocated on the side stream, used on the caller's)
-            elif isinstance(x, tuple):  # VarlenBatch, MLMBatch(VarlenBatch, labels), ...
+            elif isinstance(x, tuple):  # VarlenBatch, MLMBatch(VarlenBatch, labels), SeqPackBatch (int / None fields skipped)
                 for y in x:
                     record(y, cur)
 

@@ -223,6 +223,55 @@ int bsq_crop(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_
 int bsq_crop_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, int64_t crop_len,
                            int64_t *total, int64_t *max_len);
 
+/* Sequence packing (padding-free batches of a fixed shape: SDPA with a block-diagonal mask, position-id packing as in
+ * HF's DataCollatorWithFlattening, CUDA graphs, torch.compile): whole sequences laid end to end in R rows of L tokens.
+ * With k = bos + eos and the (already cropped) lengths len_i, sequence i occupies need_i = len_i + k tokens; every
+ * need_i must be <= L (BSQ_ERR_ARG "seq len + bos + eos > padlen: N, vs padlen L" otherwise).
+ *   Placement is best-fit decreasing, fully deterministic:
+ *     1. sequences with need_i > 0 are placed in order of decreasing need_i, ties to the lower index (a stable sort);
+ *     2. each goes into the open row with the least remaining space that still fits it, ties to the lowest row index;
+ *     3. if no open row fits, a new row is opened with the next row index;
+ *     4. within a row, sequences lie in placement order from column 0 without gaps: a sequence's column is the row's
+ *        fill when it is placed;
+ *     5. sequences with need_i == 0 (empty, k = 0) occupy nothing: starts[i] = -1.
+ *   Layout: R rows are used; with rows = R0 > 0 exactly R0 (the extra rows are padding), BSQ_ERR_ARG if the layout needs
+ *   more.  R * L must be <= 2^31 - 1 (cu_seqlens is int32), BSQ_ERR_ARG otherwise.
+ *   Output: a placed sequence starts at flat position s = starts[i] = row * L + column of the (R, L) tokens;
+ *   tokens[s .. s + need_i) = row i of bsq_tokenize_varlen on the same batch ([BOS] lut(residues) [EOS]) and
+ *   position_ids over that span are 0 .. need_i - 1.  A segment is a placed sequence or the non-empty padding run at the
+ *   end of a row; a padding run holds what bsq_tokenize writes after EOS (pad_id with padchar, else 0) and its position
+ *   ids restart at 0 too.  cu_seqlens (int32) lists the flat start of every segment in order, then R * L; max_seqlen is
+ *   the longest segment.  So varlen attention runs on the flattened tokens as they are, and a block mask is
+ *   (position_ids == 0).cumsum(-1) compared within a row.
+ *   MLM: inputs and int64 labels of a placed sequence equal bsq_tokenize_varlen_mlm's under the same bsq_mlm -- the draw
+ *   is keyed by the global sequence index, not by the placement; padding labels are ignore_index.
+ *   Crop and augmentation: stage -> crop -> augment -> pack, as for the other consumers.
+ *
+ * bsq_seqpack_plan (host only, no device call) computes that layout from host offsets (the cropped ones when a crop
+ * applies): O(n log L).  *nrows = R, *nsegments = the number of segments, *max_seqlen.  A first call with starts,
+ * row_ptr, row_seq and cu_seqlens all NULL only sizes; otherwise all four are written: starts[nseq] (int64), row_ptr[R + 1]
+ * and row_seq[row_ptr[R]] (at most nseq entries: the sequences of each row in column order, the CSR the kernel walks),
+ * cu_seqlens[nsegments + 1].  rows <= 0: as many rows as the layout needs.  BSQ_ERR_ARG for nseq < 0, k outside 0..2,
+ * row_len < 1, NULL offsets with nseq > 0, NULL size outputs, only some of the four arrays, negative lengths, and the
+ * cases above. */
+int bsq_seqpack_plan(const int64_t *h_offsets, int64_t nseq, int k, int64_t row_len, int64_t rows, int64_t *nrows,
+                     int64_t *nsegments, int64_t *max_seqlen, int64_t *starts, int64_t *row_ptr, int64_t *row_seq,
+                     int32_t *cu_seqlens);
+/* The packed rows of a plan: d_tokens (nrows, row_len) `kind` elements and d_position_ids (nrows, row_len) int32, both
+ * 16-byte aligned (any row_len); every element is written once (no memset).  d_row_ptr / d_row_seq: the plan's CSR on
+ * the device, for the batch given by d_bytes / d_offsets (the offsets the plan was made from, up to a constant shift;
+ * d_bytes, d_offsets and d_row_seq are only read for placed sequences, so a plan of padding rows alone may pass NULL).
+ * One kernel (nrows == 0: nothing); enqueues only, keeps no state between launches, capturable into a CUDA graph.
+ * BSQ_ERR_ARG for a NULL d_row_ptr, NULL or misaligned outputs, row_len < 1, nrows < 0 or nrows * row_len > 2^31 - 1. */
+int bsq_tokenize_seqpack(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, const bsq_tokenizer *tok,
+                         int kind, int64_t row_len, int64_t nrows, const int64_t *d_row_ptr, const int64_t *d_row_seq,
+                         void *d_tokens, int32_t *d_position_ids);
+/* The same rows with the masked-language-model rule of bsq_tokenize_mlm: d_inputs as d_tokens, plus d_labels
+ * (nrows, row_len) int64, 16-byte aligned.  BSQ_ERR_ARG also for a bsq_mlm bsq_tokenize_mlm rejects. */
+int bsq_tokenize_seqpack_mlm(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, const bsq_tokenizer *tok,
+                             int kind, const bsq_mlm *mlm, int64_t row_len, int64_t nrows, const int64_t *d_row_ptr,
+                             const int64_t *d_row_seq, void *d_inputs, int32_t *d_position_ids, int64_t *d_labels);
+
 /* Several batches that share padlen and tokenizer in one launch (batch-first one-byte tokens; other layouts / element
  * types fall back to one launch per batch): batch k = (d_bytes[k], d_offsets[k], nseq[k]) -> d_out[k].  The reference's
  * per-step callers tokenise small batches (training/cnnpretrain.py:123-125,145, bioseq/decoders.py:505): a 4096 x 1000
