@@ -21,6 +21,16 @@ class MLMDesc(C.Structure):
                 ("t_random", C.c_uint64), ("mask_id", C.c_int64), ("ignore_index", C.c_int64)]
 
 
+class KmerDesc(C.Structure):
+    """struct bsq_kmer"""
+    _fields_ = [("k", C.c_int32), ("stride", C.c_int32), ("tail", C.c_int32), ("nchars", C.c_int32), ("bos", C.c_int32),
+                ("eos", C.c_int32), ("padchar", C.c_int32), ("nkmers", C.c_int64), ("unk_id", C.c_int64), ("bos_id", C.c_int64),
+                ("eos_id", C.c_int64), ("pad_id", C.c_int64), ("vocab_size", C.c_int64)]
+
+
+KMER_DROP, KMER_SINGLE = 0, 1
+
+
 class TokenizerDesc(C.Structure):
     """struct bsq_tokenizer"""
     _fields_ = [("lut", C.c_int8 * 256), ("nchars", C.c_int32), ("bos_id", C.c_int32), ("eos_id", C.c_int32),
@@ -109,6 +119,11 @@ def lib():
         "bsq_seqpack_plan": (i32, [vp, i64, i32, i64, i64, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), vp, vp, vp, vp]),
         "bsq_tokenize_seqpack": (i32, [i32, vp, vp, vp, tokp, i32, i64, i64, vp, vp, vp, vp]),
         "bsq_tokenize_seqpack_mlm": (i32, [i32, vp, vp, vp, tokp, i32, C.POINTER(MLMDesc), i64, i64, vp, vp, vp, vp, vp]),
+        "bsq_kmer_init": (i32, [C.POINTER(KmerDesc), tokp, i32, i32, i32]),
+        "bsq_tokenize_kmer": (i32, [i32, vp, vp, vp, i64, i64, tokp, C.POINTER(KmerDesc), i32, vp]),
+        "bsq_tokenize_kmer_varlen": (i32, [i32, vp, vp, vp, i64, tokp, C.POINTER(KmerDesc), i32, vp, vp]),
+        "bsq_kmer_extent_host": (i32, [vp, i64, C.POINTER(KmerDesc), C.POINTER(i64), C.POINTER(i64)]),
+        "bsq_kmer_extent_device": (i32, [i32, vp, vp, i64, i64, C.POINTER(KmerDesc), C.POINTER(i64), C.POINTER(i64)]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(L, name)
@@ -128,7 +143,8 @@ EXPORTS = ("bsq_abi_version bsq_last_error bsq_launch_count bsq_launch_count_res
            "bsq_blosum62_thresholds bsq_tokenize_items bsq_onehot_items bsq_fetch_rows bsq_parallel_for "
            "bsq_tokenize_stream_items bsq_onehot_stream_items bsq_shard_bounds bsq_tokenize_host_sharded bsq_memcpy_d2d bsq_tokenize_many "
            "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm bsq_crop bsq_crop_extent_device "
-           "bsq_seqpack_plan bsq_tokenize_seqpack bsq_tokenize_seqpack_mlm").split()
+           "bsq_seqpack_plan bsq_tokenize_seqpack bsq_tokenize_seqpack_mlm bsq_kmer_init bsq_tokenize_kmer bsq_tokenize_kmer_varlen "
+           "bsq_kmer_extent_host bsq_kmer_extent_device").split()
 
 
 def last_error():
@@ -255,6 +271,39 @@ def tokenize_seqpack_mlm(device, stream, d_bytes, d_offsets, tok, kind, mlm, row
     check(lib().bsq_tokenize_seqpack_mlm(device, stream, _ptr(d_bytes), _ptr(d_offsets), C.byref(tok), kind, C.byref(mlm), row_len,
                                          nrows, _ptr(d_row_ptr), _ptr(d_row_seq), _ptr(d_inputs), _ptr(d_position_ids),
                                          _ptr(d_labels)))
+
+
+def kmer_desc(tok, k, stride=1, tail=KMER_DROP):
+    """struct bsq_kmer of a tokenizer descriptor (bsq_kmer_init: ValueError on a bad k, stride, tail or alphabet)."""
+    km = KmerDesc()
+    check(lib().bsq_kmer_init(C.byref(km), C.byref(tok), k, stride, tail))
+    return km
+
+
+def tokenize_kmer(device, stream, d_bytes, d_offsets, nseq, padlen, tok, km, kind, d_out):
+    """(nseq, padlen) k-mer tokens, batch-first (bsq_tokenize_kmer); ``km``: a KmerDesc."""
+    check(lib().bsq_tokenize_kmer(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, padlen, C.byref(tok), C.byref(km), kind,
+                                  _ptr(d_out)))
+
+
+def tokenize_kmer_varlen(device, stream, d_bytes, d_offsets, nseq, tok, km, kind, d_out, d_cu_seqlens):
+    """Padding-free k-mer tokens + int32 cu_seqlens (bsq_tokenize_kmer_varlen)."""
+    check(lib().bsq_tokenize_kmer_varlen(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, C.byref(tok), C.byref(km), kind,
+                                         _ptr(d_out), _ptr(d_cu_seqlens)))
+
+
+def kmer_extent_host(h_offsets, nseq, km):
+    """-> (sum, max) of the k-mer row lengths T(len_i) of host offsets (bsq_kmer_extent_host; no device call)."""
+    total, mx = C.c_int64(), C.c_int64()
+    check(lib().bsq_kmer_extent_host(_ptr(h_offsets), nseq, C.byref(km), C.byref(total), C.byref(mx)))
+    return total.value, mx.value
+
+
+def kmer_extent_device(device, stream, d_offsets, nseq, km, nbytes=-1):
+    """-> (sum, max) of T(len_i) over device-resident offsets (bsq_kmer_extent_device: validates them; synchronises)."""
+    total, mx = C.c_int64(), C.c_int64()
+    check(lib().bsq_kmer_extent_device(device, stream, _ptr(d_offsets), nseq, nbytes, C.byref(km), C.byref(total), C.byref(mx)))
+    return total.value, mx.value
 
 
 def onehot(device, stream, d_bytes, d_offsets, d_mask, nseq, padlen, tok, kind, d_out):

@@ -758,3 +758,127 @@ def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None,
         return SeqPackBatch(tokens, position_ids, cu_seqlens, p.max_seqlen, starts, labels)
     finally:
         r.release()
+
+
+KmerIds = collections.namedtuple("KmerIds", ["nkmers", "single_base", "unk", "bos", "eos", "pad", "vocab_size"])
+KmerIds.__doc__ = """The ids of a k-mer vocabulary (include/bsq.h, bsq_kmer): k-mers are ``0 .. nkmers - 1`` (``nkmers = b^k``),
+the single residue of code ``c`` is ``single_base + c``, ``unk`` stands for anything with an invalid byte, then ``bos`` /
+``eos`` (None when the tokenizer has none) and ``pad``; ``vocab_size`` ids in all -- the size of an ``nn.Embedding``."""
+
+_KMER_TAILS = {"drop": capi.KMER_DROP, "single": capi.KMER_SINGLE}
+
+
+def _kmer_desc(tokenizer, k, stride=1, tail="drop"):
+    """capi.KmerDesc of (tokenizer, k, stride, tail); ValueError on anything bsq_kmer_init rejects."""
+    if tail not in _KMER_TAILS:
+        raise ValueError(f"tail must be 'drop' or 'single', got {tail!r}")
+    try:
+        k, stride = operator.index(k), operator.index(stride)
+    except TypeError:
+        raise ValueError("k and stride must be integers") from None
+    if not (-2 ** 31 <= k < 2 ** 31 and -2 ** 31 <= stride < 2 ** 31):
+        raise ValueError(f"k = {k} or stride = {stride} out of range")
+    return capi.kmer_desc(descriptor(tokenizer), k, stride, _KMER_TAILS[tail])
+
+
+def kmer_ids(tokenizer, k):
+    """The ids of ``tokenizer``'s k-mer vocabulary: a :class:`KmerIds`.  They depend on the tokenizer and ``k`` only (not on
+    the stride or the tail mode), so one embedding serves every way of cutting the sequences."""
+    km = _kmer_desc(tokenizer, k)
+    return KmerIds(km.nkmers, km.nkmers, km.unk_id, km.bos_id if km.bos else None, km.eos_id if km.eos else None, km.pad_id,
+                   km.vocab_size)
+
+
+def kmer_vocab(tokenizer, k):
+    """The string of every id of ``tokenizer``'s k-mer vocabulary, in id order (for HF vocab files and for inspection).
+
+    K-mers and single residues are spelled with the letter ``decode_tokens`` prints for each residue code (so a k-mer is
+    its k letters, first residue first); the specials are ``"<UNK>"``, ``"<BOS>"``, ``"<EOS>"`` and ``"<PAD>"`` (those the
+    tokenizer has).  Its length is ``vocab_size = b^k + b + 1 + bos + eos + padchar``: it grows as b^k (4 096 k-mers for
+    DNA with k = 6, about 10^9 with k = 15), so build it only for the k a model uses."""
+    import itertools
+    tok = descriptor(tokenizer)
+    ids = kmer_ids(tokenizer, k)
+    buf = capi.C.create_string_buffer(8)
+    letters = []
+    for c in range(int(tok.nchars)):
+        n = capi.lib().bsq_tokenizer_lookup(capi.C.byref(tok), c, buf, 8)
+        letters.append(buf.value.decode("latin-1") if n else "?")
+    vocab = ["".join(p) for p in itertools.product(letters, repeat=int(k))]
+    vocab += letters + ["<UNK>"]
+    vocab += ["<BOS>"] * (ids.bos is not None) + ["<EOS>"] * (ids.eos is not None) + ["<PAD>"] * bool(tok.padchar)
+    assert len(vocab) == ids.vocab_size
+    return vocab
+
+
+def _kmer_check_extent(extent, padlen, varlen):
+    total, longest = extent
+    if varlen and total > _INT32_MAX:
+        raise ValueError(f"k-mer batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one batch; "
+                         "split the batch")
+    if not varlen and longest > padlen:
+        raise ValueError(f"k-mer tokens + bos + eos > padlen: {longest}, vs padlen {padlen}")
+
+
+def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=None, *, stride=1, tail="drop", varlen=False,
+                        crop=None, crop_len=None, seed=0, seq_index_base=0):
+    """K-mer tokens of every sequence of ``batch``, written by one kernel (padding-free: three small ones).
+
+    Sequence ``i`` of ``n`` residues gives ``[BOS] k-mer ids [single-residue ids] [EOS]``: ``m = (n - k) // stride + 1``
+    k-mers (none when ``n < k``) starting at residues ``0, stride, 2 * stride, ...``; with ``tail="single"`` the residues
+    after the last k-mer follow one token each, with ``tail="drop"`` they are dropped.  ``stride=1`` gives DNABERT's
+    overlapping k-mers, ``stride=k, tail="single"`` Nucleotide Transformer's.  Ids are those of :func:`kmer_ids`: a k-mer is
+    its codes read as a base-``b`` number, first residue most significant; anything holding an invalid byte is ``unk``.
+    The exact rule is documented with ``bsq_kmer`` in include/bsq.h.
+
+    ``varlen=False``: a padded ``(n, padlen)`` tensor (``padlen`` required), after EOS ``pad`` with ``padchar`` and 0
+    without; a row longer than ``padlen`` raises ValueError.  ``varlen=True``: a :class:`VarlenBatch` (``padlen`` must not
+    be given); more than 2^31 - 1 tokens raise ValueError.  ``destchar`` defaults to int32 (``"i"``), which holds every
+    vocabulary the rule allows; a kind too narrow for ``vocab_size`` raises ValueError.  ``crop`` / ``crop_len`` (required
+    with ``crop``, in residues): every sequence is cropped first, as :func:`crop_packed` does.  Host batches are sized from
+    their host offsets without synchronising; CUDA batches pay one read-back (two when cropped)."""
+    torch = _torch()
+    tok = descriptor(tokenizer)
+    kind, dtype = _dtype_of(destchar)
+    km = _kmer_desc(tokenizer, k, stride, tail)
+    limit = _mask_token_limit(destchar)
+    if km.vocab_size - 1 > limit:
+        raise ValueError(f"k-mer ids up to {km.vocab_size - 1} do not fit destchar {destchar!r} (0..{limit})")
+    if varlen:
+        if padlen is not None and padlen != -1:
+            raise ValueError("batch_tokenize_kmer(varlen=True) writes no padding: padlen must not be given")
+        padlen = 0
+    else:
+        try:
+            padlen = operator.index(padlen) if padlen is not None else -1
+        except TypeError:
+            raise ValueError("padlen must be an integer") from None
+        if padlen <= 0:
+            raise ValueError("batch_tokenize_kmer requires padlen (or varlen=True)")
+    crop = _crop_spec(crop, crop_len, seed, seq_index_base)
+    extent = []
+
+    def before_stage(h_offs, n):
+        e = capi.kmer_extent_host(np.ascontiguousarray(h_offs[:n + 1], dtype=np.int64), n, km)
+        _kmer_check_extent(e, padlen, varlen)
+        extent.extend(e)
+
+    r = _resolve(batch, device, before_stage=before_stage, crop=crop)
+    try:
+        if r.h_offs is None:  # a CUDA batch: one reduction and read-back, which also validates its offsets
+            nbytes = batch[0].numel() if r.extent is None else -1
+            extent = capi.kmer_extent_device(r.device, r.stream, r.d_offs, r.nseq, km, nbytes=nbytes)
+            _kmer_check_extent(extent, padlen, varlen)
+        dev = torch.device("cuda", r.device)
+        if varlen:
+            tokens = torch.empty(extent[0], dtype=dtype, device=dev)
+            cu_seqlens = torch.empty(r.nseq + 1, dtype=torch.int32, device=dev)
+            # an all-empty batch may have no residue buffer at all; nothing is read from it then
+            capi.tokenize_kmer_varlen(r.device, r.stream, r.d_bytes or cu_seqlens, r.d_offs, r.nseq, tok, km, kind, tokens,
+                                      cu_seqlens)
+            return VarlenBatch(tokens, cu_seqlens, extent[1])
+        out = torch.empty((r.nseq, padlen), dtype=dtype, device=dev)
+        capi.tokenize_kmer(r.device, r.stream, r.d_bytes or out, r.d_offs, r.nseq, padlen, tok, km, kind, out)
+        return out
+    finally:
+        r.release()

@@ -5,10 +5,10 @@
 // (g_lo, g_hi, 0, 3), g = seq_index_base + i.  out_offsets is the exclusive scan of len'_i (out_offsets[0] = 0).
 //
 // Three launches, no scratch memory and no state between launches (capturable into a CUDA graph):
-//   crop_scan_kernel    one thread per row, kCScan rows per CTA: len'_i, the CTA's inclusive scan of them
+//   row_scan_kernel     one thread per row, kCScan rows per CTA: len'_i, the CTA's inclusive scan of them
 //                       (block_exclusive_scan) written to out_offsets[i + 1].  The entry at the end of each CTA's rows
-//                       is then that CTA's total.
-//   crop_carry_kernel   one CTA (only when there is more than one scan CTA): scans the CTA totals in place, so every
+//                       is then that CTA's total.  (Shared with K11's cu_seqlens, bsq_kernels.cuh.)
+//   row_carry_kernel    one CTA (only when there is more than one scan CTA): scans the CTA totals in place, so every
 //                       entry at the end of a scan CTA's rows becomes final.
 //   crop_gather_kernel  one warp per row: adds the carry (the final entry at the end of the previous scan CTA, never
 //                       written by this kernel) to the row's own entry, draws the start (one Philox block, cropped
@@ -29,7 +29,7 @@ namespace bsq {
 
 namespace {
 
-constexpr int kCScan = 1024;    // rows per crop_scan_kernel CTA (block_exclusive_scan handles up to 1024 threads)
+constexpr int kCScan = kRowScan;  // rows per row_scan_kernel CTA
 constexpr int kCThreads = 256;  // crop_gather_kernel: 8 warps, one row each
 
 struct CropParam {
@@ -47,33 +47,11 @@ __device__ __forceinline__ int64_t crop_start(int64_t len, int64_t i, const Crop
     return static_cast<int64_t>(__umul64hi(d, static_cast<uint64_t>(len - c.W + 1)));
 }
 
-__global__ void __launch_bounds__(kCScan)
-crop_scan_kernel(const int64_t *__restrict__ offs, int64_t n, int64_t W, int64_t *__restrict__ out_offs) {
-    __shared__ int64_t s_warp[32];
-    __shared__ int64_t s_total;
-    const int64_t i = static_cast<int64_t>(blockIdx.x) * kCScan + threadIdx.x;
-    const int64_t kept = i < n ? min(__ldg(offs + i + 1) - __ldg(offs + i), W) : 0;
-    const int64_t ex = block_exclusive_scan(kept, s_warp, &s_total);
-    if (i < n) out_offs[i + 1] = ex + kept;
-    if (i == 0) out_offs[0] = 0;
-}
-
-// entry e = min((b + 1) * kCScan, n) holds scan CTA b's total; it becomes the inclusive prefix over CTAs 0 .. b
-__global__ void __launch_bounds__(kCScan)
-crop_carry_kernel(int64_t *__restrict__ out_offs, int64_t n, int64_t nblocks) {
-    __shared__ int64_t s_warp[32];
-    __shared__ int64_t s_total;
-    int64_t carry = 0;
-    for (int64_t base = 0; base < nblocks; base += kCScan) {
-        const int64_t b = base + threadIdx.x;
-        const int64_t e = min((b + 1) * kCScan, n);
-        const int64_t x = b < nblocks ? out_offs[e] : 0;
-        const int64_t ex = block_exclusive_scan(x, s_warp, &s_total);
-        if (b < nblocks) out_offs[e] = carry + ex + x;
-        carry += s_total;
-        __syncthreads();
-    }
-}
+// the per-row count of the scan (bsq_kernels.cuh): the kept length min(len_i, W)
+struct CropCount {
+    int64_t W;
+    __device__ __forceinline__ int64_t operator()(int64_t len) const { return min(len, W); }
+};
 
 __global__ void __launch_bounds__(kCThreads)
 crop_gather_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__ offs, int64_t n, CropParam c,
@@ -142,11 +120,11 @@ extern "C" int bsq_crop(int device, void *stream, const uint8_t *d_bytes, const 
         return BSQ_OK;
     }
     const int64_t nblocks = (nseq + kCScan - 1) / kCScan;
-    crop_scan_kernel<<<static_cast<unsigned>(nblocks), kCScan, 0, st>>>(d_offsets, nseq, crop_len, d_out_offsets);
+    row_scan_kernel<<<static_cast<unsigned>(nblocks), kCScan, 0, st>>>(d_offsets, nseq, CropCount{crop_len}, d_out_offsets);
     count_launch();
     BSQ_CUDA_TRY(cudaGetLastError());
     if (nblocks > 1) {
-        crop_carry_kernel<<<1, kCScan, 0, st>>>(d_out_offsets, nseq, nblocks);
+        row_carry_kernel<<<1, kCScan, 0, st>>>(d_out_offsets, nseq, nblocks);
         count_launch();
         BSQ_CUDA_TRY(cudaGetLastError());
     }

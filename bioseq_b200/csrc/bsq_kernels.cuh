@@ -105,6 +105,31 @@ struct MlmParam {
 // Validates a bsq_mlm for `kind` (BSQ_ERR_ARG with the message of include/bsq.h) and fills *m (bsq_mlm.cu).
 int check_mlm_param(const bsq_tokenizer *tok, int kind, const bsq_mlm *mlm, MlmParam *m);
 
+// The token count of one k-mer row (include/bsq.h, bsq_kmer): the only statement of T(n), used by the host extent, the
+// device extent and K11 (bsq_kmer.cu).  sdiv divides by the stride.
+struct KmerShape {
+    int32_t k, s, single, bos, eos;
+    FastDiv sdiv;
+};
+struct KmerCount {
+    int64_t m;        // k-mers, starting at residues 0, s, 2s, ...
+    int64_t covered;  // residues they cover
+    int64_t tail;     // residues after them that become single tokens (0 when dropped)
+};
+__host__ __device__ inline KmerCount kmer_count(int64_t n, const KmerShape &ks) {
+    KmerCount c;
+    const int64_t d = n - ks.k;
+    c.m = d < 0 ? 0 : (d < (int64_t(1) << 31) ? static_cast<int64_t>(fd_div(static_cast<uint32_t>(d), ks.sdiv)) : d / ks.s) + 1;
+    c.covered = c.m > 0 ? (c.m - 1) * ks.s + ks.k : 0;
+    c.tail = ks.single ? n - c.covered : 0;
+    return c;
+}
+// T(n) = m + (single ? r : 0) + bos + eos
+__host__ __device__ inline int64_t kmer_tokens(int64_t n, const KmerShape &ks) {
+    const KmerCount c = kmer_count(n, ks);
+    return c.m + c.tail + ks.bos + ks.eos;
+}
+
 #ifdef __CUDACC__
 
 __device__ __forceinline__ uint4 ldg16(uintptr_t addr) {
@@ -356,6 +381,45 @@ __device__ __forceinline__ int64_t block_exclusive_scan(int64_t x, int64_t *s_wa
     }
     __syncthreads();
     return s_warp[warp] + incl - x;
+}
+
+// Exclusive scan of a per-row count over a packed batch, in two launches without scratch memory (K9's crop offsets, K11's
+// cu_seqlens).  count(len) is the row's count from its length; Out the element type of the offsets array.
+//   row_scan_kernel   one thread per row, kRowScan rows per CTA: the CTA's inclusive scan of count(len_i) goes to
+//                     out[i + 1] (and out[0] = 0), so the entry at the end of each CTA's rows is that CTA's total.
+//   row_carry_kernel  one CTA, only when there is more than one scan CTA: scans the CTA totals in place, so every entry
+//                     at the end of a scan CTA's rows becomes final.
+// The consumer then finishes row i's entry itself (row_scan_final).
+constexpr int kRowScan = 1024;  // block_exclusive_scan handles up to 1024 threads
+
+template <typename Count, typename Out>
+__global__ void __launch_bounds__(kRowScan)
+row_scan_kernel(const int64_t *__restrict__ offs, int64_t n, Count count, Out *__restrict__ out_offs) {
+    __shared__ int64_t s_warp[32];
+    __shared__ int64_t s_total;
+    const int64_t i = static_cast<int64_t>(blockIdx.x) * kRowScan + threadIdx.x;
+    const int64_t kept = i < n ? count(__ldg(offs + i + 1) - __ldg(offs + i)) : 0;
+    const int64_t ex = block_exclusive_scan(kept, s_warp, &s_total);
+    if (i < n) out_offs[i + 1] = static_cast<Out>(ex + kept);
+    if (i == 0) out_offs[0] = 0;
+}
+
+// entry e = min((b + 1) * kRowScan, n) holds scan CTA b's total; it becomes the inclusive prefix over CTAs 0 .. b
+template <typename Out>
+__global__ void __launch_bounds__(kRowScan)
+row_carry_kernel(Out *__restrict__ out_offs, int64_t n, int64_t nblocks) {
+    __shared__ int64_t s_warp[32];
+    __shared__ int64_t s_total;
+    int64_t carry = 0;
+    for (int64_t base = 0; base < nblocks; base += kRowScan) {
+        const int64_t b = base + threadIdx.x;
+        const int64_t e = min((b + 1) * kRowScan, n);
+        const int64_t x = b < nblocks ? static_cast<int64_t>(out_offs[e]) : 0;
+        const int64_t ex = block_exclusive_scan(x, s_warp, &s_total);
+        if (b < nblocks) out_offs[e] = static_cast<Out>(carry + ex + x);
+        carry += s_total;
+        __syncthreads();
+    }
 }
 
 // word w (0..3) of a block, with selects (a run-time index into the block would put it in local memory)

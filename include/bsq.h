@@ -272,6 +272,72 @@ int bsq_tokenize_seqpack_mlm(int device, void *stream, const uint8_t *d_bytes, c
                              int kind, const bsq_mlm *mlm, int64_t row_len, int64_t nrows, const int64_t *d_row_ptr,
                              const int64_t *d_row_seq, void *d_inputs, int32_t *d_position_ids, int64_t *d_labels);
 
+/* K-mer tokens (DNABERT's overlapping k-mers, Nucleotide Transformer's non-overlapping 6-mers with single-residue
+ * tails, reduced-alphabet protein k-mers).  Take a tokenizer with b = nchars codes, its LUT (byte -> code, -1 invalid;
+ * bytes >= 0x80 are invalid) and its bos / eos / padchar flags; choose k >= 1, a stride 1 <= s <= k and a tail mode.
+ *   Ids depend on (tokenizer, k) only, not on the stride or tail mode:
+ *     0 .. b^k - 1      k-mer c_0 ... c_{k-1} -> sum_t c_t * b^(k-1-t)   (the first residue is the most significant)
+ *     b^k + c           single residue of code c (tail mode BSQ_KMER_SINGLE)
+ *     unk = b^k + b     any k-mer or single residue that contains an invalid byte
+ *     unk + 1, ...      BOS (if bos), EOS (if eos), PAD = unk + 1 + bos + eos (always defined, written only with padchar)
+ *   vocab_size = b^k + b + 1 + bos + eos + padchar.  BSQ_ERR_ARG when vocab_size - 1 > 2^31 - 1, for the BYTES alphabet
+ *   (nchars == 256: its LUT is not a code table), k < 1 or s outside 1..k; the compute calls also reject an output kind
+ *   that cannot hold vocab_size - 1 (255 for BSQ_I8, 32767 for BSQ_I16, 2^24 for BSQ_F32, 2^31 - 1 otherwise, as for
+ *   bsq_mlm's mask_id).  So DNA allows k <= 15, PROTEIN k <= 7 and the two-letter alphabets k <= 30.
+ *   Tokens of one sequence of n residues, before the specials:
+ *     m = n >= k ? (n - k) / s + 1 : 0 k-mers, starting at residues 0, s, 2s, ...;
+ *     covered = m > 0 ? (m - 1) * s + k : 0 and r = n - covered;
+ *     BSQ_KMER_SINGLE: the r residues after `covered` follow, one token each; BSQ_KMER_DROP: they are dropped;
+ *     T(n) = m + (single ? r : 0) + bos + eos.
+ *   Padded, batch-first (nseq, padlen): row i = [BOS] tokens [EOS], then pad_id with padchar and 0 without (as
+ *   bsq_tokenize); T(len_i) <= padlen is the caller's check ("k-mer tokens + bos + eos > padlen: N, vs padlen P").
+ *   Padding-free: the rows back to back, int32 cu_seqlens with cu[0] = 0 and cu[i+1] - cu[i] = T(len_i); no PAD.  The
+ *   caller has checked that the total is <= 2^31 - 1.
+ *   Crop: stage -> crop -> k-mer, with crop_len counted in residues, as for the other consumers.
+ * Worked answers: Tokenizer("DNA", bos, eos, padchar) with k = 3: b^k = 64, singles 64..67, unk 68, BOS 69, EOS 70,
+ * PAD 71, vocab_size 72 (N is invalid in DNA):
+ *     "ACGTNAG"  s = 1, either tail  [69, 6, 27, 68, 68, 68, 70]
+ *     "ACGTNAG"  s = 3, single       [69, 6, 68, 66, 70]
+ *     "ACGTNAG"  s = 3, drop         [69, 6, 68, 70]
+ *     "AC"       any s, single       [69, 64, 65, 70]
+ *     "AC"       any s, drop         [69, 70]
+ *     ""         any s, either tail  [69, 70]
+ */
+#define BSQ_KMER_DROP 0
+#define BSQ_KMER_SINGLE 1
+typedef struct bsq_kmer {
+    int32_t k, stride, tail; /* tail: BSQ_KMER_DROP or BSQ_KMER_SINGLE                                        */
+    int32_t nchars;          /* b                                                                             */
+    int32_t bos, eos, padchar;
+    int64_t nkmers;          /* b^k, also the id of the single residue of code 0                            */
+    int64_t unk_id;          /* b^k + b                                                                       */
+    int64_t bos_id, eos_id;  /* -1 when absent                                                                */
+    int64_t pad_id;          /* unk + 1 + bos + eos                                                           */
+    int64_t vocab_size;
+} bsq_kmer;
+/* Host only, no device call: validates (tok, k, stride, tail) as above and fills *km.  The only place the ids are
+ * computed. */
+int bsq_kmer_init(bsq_kmer *km, const bsq_tokenizer *tok, int k, int stride, int tail);
+/* Padded tokens: d_out (nseq, padlen) `kind` elements, batch-first, 16-byte aligned; every element is written once (no
+ * memset).  `km` must come from bsq_kmer_init with `tok`.  Enqueues only (one kernel); keeps no state between launches and
+ * is capturable into a CUDA graph.  BSQ_ERR_ARG for NULL or misaligned pointers, padlen < 1, nseq < 0 or a kind too
+ * narrow for the vocabulary, before any device call. */
+int bsq_tokenize_kmer(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq, int64_t padlen,
+                      const bsq_tokenizer *tok, const bsq_kmer *km, int kind, void *d_out);
+/* Padding-free tokens: d_out holds exactly the total (16-byte aligned; may be NULL when it is 0) and d_cu_seqlens nseq + 1
+ * int32 entries, both written by this call (at most three kernels; nseq == 0: a 4-byte memset of cu_seqlens).  Enqueues
+ * only, keeps no state between launches, capturable into a CUDA graph. */
+int bsq_tokenize_kmer_varlen(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq,
+                             const bsq_tokenizer *tok, const bsq_kmer *km, int kind, void *d_out, int32_t *d_cu_seqlens);
+/* *total = sum of T(len_i) and *max_tokens = max T(len_i) (both 0 for nseq == 0) of host offsets, with no device call.
+ * BSQ_ERR_ARG for a negative length or offsets[0] < 0. */
+int bsq_kmer_extent_host(const int64_t *h_offsets, int64_t nseq, const bsq_kmer *km, int64_t *total, int64_t *max_tokens);
+/* The same for device-resident offsets, from one reduction kernel and one read-back (synchronises `stream`); validates
+ * the offsets like bsq_crop_extent_device (BSQ_ERR_ARG: negative length, offsets[0] < 0, offsets[nseq] > nbytes when
+ * nbytes >= 0). */
+int bsq_kmer_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, const bsq_kmer *km,
+                           int64_t *total, int64_t *max_tokens);
+
 /* Several batches that share padlen and tokenizer in one launch (batch-first one-byte tokens; other layouts / element
  * types fall back to one launch per batch): batch k = (d_bytes[k], d_offsets[k], nseq[k]) -> d_out[k].  The reference's
  * per-step callers tokenise small batches (training/cnnpretrain.py:123-125,145, bioseq/decoders.py:505): a 4096 x 1000
