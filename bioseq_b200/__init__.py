@@ -127,6 +127,7 @@ from .consumers import batch_tokenize_mlm, MLMBatch  # noqa: E402
 from .consumers import crop_packed, batch_tokenize_cropped, CroppedBatch  # noqa: E402
 from .consumers import batch_tokenize_seqpack, SeqPackBatch  # noqa: E402
 from .consumers import batch_tokenize_kmer, kmer_ids, kmer_vocab, KmerIds  # noqa: E402
+from .consumers import revcomp_packed, batch_tokenize_revcomp, RevCompBatch  # noqa: E402
 
 
 def __getattr__(name):
@@ -147,4 +148,5 @@ __all__ = ["onehot_encode", "cbioseq", "f_encode", "Tokenizer", "make_embedding"
            "PyViewFF", "loaders", "consumers", "batch_onehot_encode_bcl", "batch_embed", "augment_packed",
            "batch_tokenize_augmented", "batch_tokenize_varlen", "VarlenBatch", "batch_tokenize_mlm", "MLMBatch", "crop_packed",
            "batch_tokenize_cropped", "CroppedBatch", "batch_tokenize_seqpack", "SeqPackBatch", "batch_tokenize_kmer", "kmer_ids", "kmer_vocab", "KmerIds",
+           "revcomp_packed", "batch_tokenize_revcomp", "RevCompBatch",
            "TokenizerLayer", "EmbeddingTokenizerLayer"]

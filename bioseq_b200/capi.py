@@ -29,6 +29,7 @@ class KmerDesc(C.Structure):
 
 
 KMER_DROP, KMER_SINGLE = 0, 1
+RC_ALWAYS, RC_RANDOM, RC_BOTH = 0, 1, 2
 
 
 class TokenizerDesc(C.Structure):
@@ -124,6 +125,8 @@ def lib():
         "bsq_tokenize_kmer_varlen": (i32, [i32, vp, vp, vp, i64, tokp, C.POINTER(KmerDesc), i32, vp, vp]),
         "bsq_kmer_extent_host": (i32, [vp, i64, C.POINTER(KmerDesc), C.POINTER(i64), C.POINTER(i64)]),
         "bsq_kmer_extent_device": (i32, [i32, vp, vp, i64, i64, C.POINTER(KmerDesc), C.POINTER(i64), C.POINTER(i64)]),
+        "bsq_revcomp": (i32, [i32, vp, vp, vp, i64, i32, C.c_double, C.c_uint64, i64, vp, vp, vp]),
+        "bsq_revcomp_table": (i32, [vp]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(L, name)
@@ -144,7 +147,7 @@ EXPORTS = ("bsq_abi_version bsq_last_error bsq_launch_count bsq_launch_count_res
            "bsq_tokenize_stream_items bsq_onehot_stream_items bsq_shard_bounds bsq_tokenize_host_sharded bsq_memcpy_d2d bsq_tokenize_many "
            "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm bsq_crop bsq_crop_extent_device "
            "bsq_seqpack_plan bsq_tokenize_seqpack bsq_tokenize_seqpack_mlm bsq_kmer_init bsq_tokenize_kmer bsq_tokenize_kmer_varlen "
-           "bsq_kmer_extent_host bsq_kmer_extent_device").split()
+           "bsq_kmer_extent_host bsq_kmer_extent_device bsq_revcomp bsq_revcomp_table").split()
 
 
 def last_error():
@@ -246,6 +249,21 @@ def crop_extent_device(device, stream, d_offsets, nseq, crop_len, nbytes=-1):
     check(lib().bsq_crop_extent_device(device, stream, _ptr(d_offsets), nseq, nbytes, crop_len, C.byref(total),
                                        C.byref(maxlen)))
     return total.value, maxlen.value
+
+
+def revcomp(device, stream, d_bytes, d_offsets, nseq, mode, rc_prob, seed, seq_index_base, d_out_bytes, d_out_offsets,
+            d_flipped=None):
+    """Reverse complement of a packed batch (bsq_revcomp); ``mode``: RC_ALWAYS, RC_RANDOM or RC_BOTH."""
+    check(lib().bsq_revcomp(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, mode, float(rc_prob), seed & 0xFFFFFFFFFFFFFFFF,
+                            seq_index_base, _ptr(d_out_bytes), _ptr(d_out_offsets), _ptr(d_flipped)))
+
+
+def revcomp_table():
+    """The complement table of bsq_revcomp: a uint8 numpy array of 256 entries (no device call)."""
+    import numpy as np
+    t = np.zeros(256, np.uint8)
+    check(lib().bsq_revcomp_table(t.ctypes.data))
+    return t
 
 
 def seqpack_plan(h_offsets, nseq, k, row_len, rows=0, starts=None, row_ptr=None, row_seq=None, cu_seqlens=None):

@@ -22,6 +22,9 @@ Reference counterparts:
 * ``crop_packed`` / ``crop=`` -- every sequence cropped to a window of the model's context on the device (ESM-style
   seeded random windows, or the heads as HF ``truncation=True`` does) instead of slicing Python strings or gathering
   in torch; the consumers above take ``crop=`` and ``crop_len=`` and run unchanged on the cropped batch.
+* ``revcomp_packed`` / ``rc=`` -- the reverse complement of every DNA / RNA sequence on the device (seeded strand flips
+  for training, both strands for test-time averaging) instead of flipping Python strings or gathering in torch; every
+  consumer takes ``rc=`` and ``rc_prob=`` and runs unchanged on the flipped batch.
 
 All of these call the C ABI (``include/bsq.h``) through ``capi``; torch supplies memory and the stream.
 A *batch* is one of
@@ -112,7 +115,7 @@ class _Resolved:
             self.ctx = None
 
 
-def _resolve(batch, device, augment=None, before_stage=None, crop=None, crop_extent=None):
+def _resolve(batch, device, augment=None, before_stage=None, crop=None, crop_extent=None, rc=None, validated=False):
     """-> _Resolved.  Host batches are staged (and, with ``augment``, mutated on the device after the copy);
     device batches are used in place (with ``augment``: a mutated clone).  ``before_stage(host_offsets, n)`` checks a
     host batch before anything is copied to the device.
@@ -121,7 +124,13 @@ def _resolve(batch, device, augment=None, before_stage=None, crop=None, crop_ext
     cropped batch, with ``extent = (sum, max)`` of its lengths; ``augment`` then mutates the crop's fresh buffer in
     place.  Host batches are sized from their host offsets (``before_stage`` sees the cropped offsets); device
     batches pay one ``bsq_crop_extent_device`` (which also validates their offsets), unless the caller has read their
-    offsets back already and passes ``crop_extent``."""
+    offsets back already and passes ``crop_extent``.
+
+    ``rc`` (from ``_rc_spec``): after the crop, the batch is flipped on the device into fresh buffers (``_apply_rc``).
+    Uncropped batches then also get ``extent``: host batches from their host offsets, device batches from one
+    ``bsq_crop_extent_device`` with no window (which validates their offsets), unless the caller has validated them
+    already (``crop_extent``, or ``validated`` when it needs no extent).  ``rc="both"`` doubles the batch:
+    ``before_stage`` and ``h_offs`` then see the doubled offsets."""
     torch = _torch()
     r = _Resolved()
     r.ctx, r.keep, r.h_offs, r.base, r.extent = None, [], None, 0, None
@@ -145,6 +154,15 @@ def _resolve(batch, device, augment=None, before_stage=None, crop=None, crop_ext
                 r.extent = crop_extent if crop_extent is not None else capi.crop_extent_device(r.device, r.stream, o, r.nseq, crop[1],
                                                                                                 nbytes=b.numel())
                 _apply_crop(r, crop, augment)
+                _apply_rc(r, rc, r.extent[0])
+                return r
+            if rc is not None:
+                r.d_bytes, r.d_offs, r.nseq = b.data_ptr(), o.data_ptr(), o.numel() - 1
+                r.keep += [b, o]
+                if crop_extent is not None or not validated:
+                    r.extent = crop_extent if crop_extent is not None else capi.crop_extent_device(r.device, r.stream, o, r.nseq,
+                                                                                                    _UNCROPPED, nbytes=b.numel())
+                _apply_rc(r, rc, b.numel())
                 return r
             if augment:
                 with torch.cuda.device(r.device):
@@ -189,14 +207,15 @@ def _resolve(batch, device, augment=None, before_stage=None, crop=None, crop_ext
                 raise ValueError("offsets run past the end of bytes")
             hb_ptr = host_b.ctypes.data
             r.keep += [host_b, host_o]
-        if crop is not None:
-            cropped_o, r.extent = _crop_host_extent(host_o, n, crop[1])
+        if crop is not None or rc is not None:
+            cropped_o, r.extent = _crop_host_extent(host_o, n, crop[1] if crop is not None else _UNCROPPED)
             if before_stage is not None:
-                before_stage(cropped_o, n)
+                before_stage(*_rc_host_offsets(cropped_o, n, rc))
             r.d_bytes, r.d_offs = ctx.stager.stage(r.stream, hb_ptr, host_o.ctypes.data, n)
-            r.nseq, r.ctx = n, ctx
-            _apply_crop(r, crop, augment)
-            r.h_offs = cropped_o
+            r.nseq, r.ctx, r.h_offs = n, ctx, cropped_o
+            if crop is not None:
+                _apply_crop(r, crop, augment)
+            _apply_rc(r, rc, r.extent[0])
             return r
         if before_stage is not None:
             before_stage(host_o, n)
@@ -215,7 +234,8 @@ def _resolve(batch, device, augment=None, before_stage=None, crop=None, crop_ext
 
 
 def _check_lengths(r, padlen, tok, onehot):
-    if r.extent is not None:  # cropped: _crop_spec capped crop_len at padlen - bos - eos, and the crop validated the offsets
+    if r.extent is not None:  # cropped or flipped: the offsets are validated and the longest length is known
+        capi.check_lengths_host(np.array([0, r.extent[1]], np.int64), 1, padlen, tok, onehot=onehot)
         return
     if r.h_offs is not None:
         capi.check_lengths_host(r.h_offs, r.nseq, padlen, tok, onehot=onehot)
@@ -294,17 +314,80 @@ def _apply_crop(r, crop, augment):
         capi.augment_blosum62(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, *augment)
 
 
+_RC_MODES = {None: None, "always": capi.RC_ALWAYS, "random": capi.RC_RANDOM, "both": capi.RC_BOTH}
+# the nucleotide alphabets: the complement table is meaningless for protein codes and raw bytes
+_RC_KEYS = ("DNA", "DNA4", "DNA5", "DNAMETH", "C", "KETO", "PURPYR")
+_UNCROPPED = (1 << 63) - 1  # a window no sequence exceeds: bsq_crop_extent_device then only validates and measures
+
+
+def _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer=None, augment=None, mlm=False):
+    """Validate the reverse-complement arguments (ValueError before anything is staged) -> None (no flip) or
+    ``(mode, rc_prob, seed, seq_index_base)``.  ``tokenizer`` (None for ``revcomp_packed``) must be nucleotide; ``augment``
+    (BLOSUM62, for proteins) and ``rc="both"`` with ``mlm`` are rejected."""
+    if not isinstance(rc, (str, type(None))) or rc not in _RC_MODES:
+        raise ValueError(f"rc must be one of None, 'always', 'random', 'both', got {rc!r}")
+    if rc_prob is not None and rc != "random":
+        raise ValueError("rc_prob is given without rc='random'")
+    if rc is None:
+        return None
+    if rc == "random":
+        try:
+            rc_prob = float(0.5 if rc_prob is None else rc_prob)
+        except (TypeError, ValueError):
+            raise ValueError(f"rc_prob must be a number in [0, 1], got {rc_prob!r}") from None
+        if not 0.0 <= rc_prob <= 1.0:
+            raise ValueError(f"rc_prob must lie in [0, 1], got {rc_prob}")
+    if tokenizer is not None:
+        key = descriptor(tokenizer).key.decode("latin-1").upper()
+        if key not in _RC_KEYS:
+            raise ValueError(f"rc needs a nucleotide tokenizer ({', '.join(_RC_KEYS)}), got {key}")
+    if augment:
+        raise ValueError("rc cannot be combined with augment: BLOSUM62 substitutions are for proteins")
+    if mlm and rc == "both":
+        raise ValueError("rc='both' doubles the batch for inference; it cannot be combined with mlm")
+    return (_RC_MODES[rc], rc_prob or 0.0, int(seed), int(seq_index_base))
+
+
+def _rc_host_offsets(h_offs, n, rc):
+    """-> (offsets, n) of the batch ``rc`` makes from host offsets that start at 0: the same, or doubled for "both"."""
+    if rc is None or rc[0] != capi.RC_BOTH:
+        return h_offs, n
+    h = np.asarray(h_offs[:n + 1], dtype=np.int64)
+    return np.concatenate([h, h[n] + h[1:]]), 2 * n
+
+
+def _apply_rc(r, rc, nbytes):
+    """Flip the resolved batch (validated offsets, ``nbytes`` >= its residues) into fresh device buffers; r then
+    describes the flipped batch (doubled for "both")."""
+    if rc is None:
+        return
+    torch = _torch()
+    mode, rc_prob, seed, base = rc
+    both = mode == capi.RC_BOTH
+    dev = torch.device("cuda", r.device)
+    out_b = torch.empty(max(nbytes * (2 if both else 1), 1), dtype=torch.uint8, device=dev)  # (never a null pointer)
+    out_o = torch.empty(r.nseq * (2 if both else 1) + 1, dtype=torch.int64, device=dev)
+    capi.revcomp(r.device, r.stream, r.d_bytes or out_b, r.d_offs, r.nseq, mode, rc_prob, seed, base, out_b, out_o)
+    r.keep += [out_b, out_o]
+    if r.h_offs is not None:
+        r.h_offs = _rc_host_offsets(np.asarray(r.h_offs, np.int64) - int(r.h_offs[0]), r.nseq, rc)[0]
+    r.d_bytes, r.d_offs, r.base, r.nseq = out_b.data_ptr(), out_o.data_ptr(), 0, out_o.numel() - 1
+    if both and r.extent is not None:
+        r.extent = (2 * r.extent[0], r.extent[1])
+
+
 def _row_residues(tokenizer, padlen):
     return padlen - int(tokenizer.includes_bos()) - int(tokenizer.includes_eos())
 
 
 def batch_onehot_encode_bcl(tokenizer, batch, padlen=-1, destchar="f", mask=None, device=None, *, augment=0, augment_frac=1.0,
-                            seed=0, seq_index_base=0, crop=None, crop_len=None):
+                            seed=0, seq_index_base=0, crop=None, crop_len=None, rc=None, rc_prob=None):
     """One-hot ``(batch, alphabet_size, padlen)`` tensor (CNN layout), default float32.
 
     Element ``[i, c, p]`` equals ``batch_onehot_encode(...)[p, i, c]`` (src/tokenize.h:345-368), i.e. the result of the
     reference's rearrange + float (bioseq/loaders.py:74-75).  ``mask``: uint8, one entry per residue of ``bytes``
-    (packed batches only, not with ``crop``).  ``crop``: as ``batch_tokenize_cropped``."""
+    (packed batches only, not with ``crop`` or ``rc``).  ``crop``: as ``batch_tokenize_cropped``; ``rc`` / ``rc_prob``: as
+    ``batch_tokenize_revcomp``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     padlen = _default_padlen(batch, tokenizer, padlen)
@@ -312,7 +395,10 @@ def batch_onehot_encode_bcl(tokenizer, batch, padlen=-1, destchar="f", mask=None
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
     if crop is not None and mask is not None:
         raise ValueError("mask covers the uncropped residues: it cannot be combined with crop")
-    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop)
+    rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment)
+    if rc is not None and mask is not None:
+        raise ValueError("mask covers the unflipped residues: it cannot be combined with rc")
+    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop, rc=rc)
     try:
         _check_lengths(r, padlen, tok, onehot=True)
         d_mask = None
@@ -342,16 +428,18 @@ def batch_onehot_encode_bcl(tokenizer, batch, padlen=-1, destchar="f", mask=None
 
 
 def batch_embed(tokenizer, batch, weight, padlen=-1, batch_first=True, device=None, *, augment=0, augment_frac=1.0, seed=0,
-                seq_index_base=0, crop=None, crop_len=None):
+                seq_index_base=0, crop=None, crop_len=None, rc=None, rc_prob=None):
     """``weight[tokens]`` for the tokens of ``batch_tokenize(batch, padlen, batch_first=batch_first)`` without
     materialising them: ``(batch, padlen, dim)`` or ``(padlen, batch, dim)``, dtype and device of ``weight``.
 
     ``weight``: ``(rows >= alphabet_size, dim)`` CUDA tensor (an ``nn.Embedding.weight``); ``dim * itemsize`` must be
-    a multiple of 16 bytes.  Forward only (no autograd graph is recorded).  ``crop``: as ``batch_tokenize_cropped``."""
+    a multiple of 16 bytes.  Forward only (no autograd graph is recorded).  ``crop``: as ``batch_tokenize_cropped``; ``rc`` /
+    ``rc_prob``: as ``batch_tokenize_revcomp``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     padlen = _default_padlen(batch, tokenizer, padlen)
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
+    rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment)
     w = weight.detach()
     if not w.is_cuda or w.dim() != 2:
         raise ValueError("weight must be a 2-D CUDA tensor")
@@ -359,7 +447,7 @@ def batch_embed(tokenizer, batch, weight, padlen=-1, batch_first=True, device=No
         w = w.contiguous()
     row_bytes = w.shape[1] * w.element_size()
     r = _resolve(batch, w.device if device is None else device, _augment_args(augment, augment_frac, seed, seq_index_base),
-                 crop=crop)
+                 crop=crop, rc=rc)
     try:
         if r.device != w.device.index:
             raise ValueError("weight and batch live on different devices")
@@ -422,25 +510,88 @@ def crop_packed(bytes_cuda, offsets_cuda, crop_len, *, crop="random", seed=0, se
 
 
 def batch_tokenize_cropped(tokenizer, batch, padlen, destchar="B", batch_first=True, device=None, *, crop="random", crop_len=None,
-                           seed=0, seq_index_base=0, augment=0, augment_frac=1.0):
+                           seed=0, seq_index_base=0, augment=0, augment_frac=1.0, rc=None, rc_prob=None):
     """``batch_tokenize`` of the batch with every sequence cropped to ``crop_len`` residues on the device (default and
     maximum: ``padlen - bos - eos``): stage -> crop -> augment -> tokenize.  ``crop``: ``"random"`` or ``"head"``, as
-    :func:`crop_packed` (same ``seed`` / ``seq_index_base``)."""
+    :func:`crop_packed` (same ``seed`` / ``seq_index_base``).  ``rc`` / ``rc_prob``: the windows are then flipped, as
+    :func:`batch_tokenize_revcomp` does."""
+    if crop is None:
+        raise ValueError("batch_tokenize_cropped: crop must be 'head' or 'random'")
+    return _tokenize_padded(tokenizer, batch, padlen, destchar, batch_first, device, crop, crop_len, seed, seq_index_base,
+                            augment, augment_frac, rc, rc_prob)
+
+
+def batch_tokenize_revcomp(tokenizer, batch, padlen, destchar="B", batch_first=True, device=None, *, rc="random", rc_prob=None,
+                           seed=0, seq_index_base=0, crop=None, crop_len=None):
+    """``batch_tokenize`` of the batch's reverse complements, flipped on the device: stage -> crop -> flip -> tokenize.
+
+    ``rc="random"``: each sequence is flipped with probability ``rc_prob`` (default 0.5) by a coin drawn from
+    Philox4x32-10 keyed by ``seed`` at sequence ``seq_index_base + i`` (the same coin whatever the slicing); ``"always"``:
+    every sequence; ``"both"``: ``2n`` rows, the batch as is and then its reverse complements (average the model's outputs
+    over ``y[:n]`` and the flipped ``y[n:]``).  The complement keeps case and maps IUPAC codes (U -> A); the exact rule is
+    documented with ``bsq_revcomp`` in include/bsq.h.  Nucleotide tokenizers only (DNA, DNA4, DNA5, DNAMETH, C, KETO,
+    PURPYR).  ``crop`` / ``crop_len``: as :func:`batch_tokenize_cropped`, applied before the flip.  CUDA batches pay one
+    read-back, which validates their offsets and replaces the length check."""
+    if rc is None:
+        raise ValueError("batch_tokenize_revcomp: rc must be 'always', 'random' or 'both'")
+    return _tokenize_padded(tokenizer, batch, padlen, destchar, batch_first, device, crop, crop_len, seed, seq_index_base, 0, 1.0,
+                            rc, rc_prob)
+
+
+def _tokenize_padded(tokenizer, batch, padlen, destchar, batch_first, device, crop, crop_len, seed, seq_index_base, augment,
+                     augment_frac, rc, rc_prob):
     torch = _torch()
     tok = descriptor(tokenizer)
     padlen = _default_padlen(batch, tokenizer, padlen)
     kind, dtype = _dtype_of(destchar)
-    if crop is None:
-        raise ValueError("batch_tokenize_cropped: crop must be 'head' or 'random'")
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
-    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop)
+    rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment)
+    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop, rc=rc)
     try:
+        _check_lengths(r, padlen, tok, onehot=False)
         shape = (r.nseq, padlen) if batch_first else (padlen, r.nseq)
         out = torch.empty(shape, dtype=dtype, device=torch.device("cuda", r.device))
         capi.tokenize(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, padlen, tok, batch_first, kind, out)
         return out
     finally:
         r.release()
+
+
+RevCompBatch = collections.namedtuple("RevCompBatch", ["bytes", "offsets", "flipped"])
+RevCompBatch.__doc__ = """A reverse-complemented packed batch: ``bytes`` (uint8) and ``offsets`` (int64, from 0) of the output
+sequences, and ``flipped`` (bool, one per output sequence: whether it is a reverse complement -- what a caller needs to
+flip per-position labels the same way)."""
+
+
+def revcomp_packed(bytes_cuda, offsets_cuda, *, rc="always", rc_prob=None, seed=0, seq_index_base=0):
+    """The reverse complement of a packed CUDA batch: a :class:`RevCompBatch`; the input is not modified.
+
+    ``rc="always"``: every sequence is flipped; ``"random"``: each with probability ``rc_prob`` (default 0.5), the coin
+    drawn from Philox4x32-10 keyed by ``seed`` at sequence ``seq_index_base + i``; ``"both"``: ``2n`` sequences, the batch
+    unchanged and then flipped.  The exact rule is documented with ``bsq_revcomp`` in include/bsq.h.  For per-position
+    labels: crop with :func:`crop_packed`, flip with this, then reverse the labels of the rows ``flipped`` marks.  One
+    synchronisation: the offsets are validated and the output's size is read back."""
+    torch = _torch()
+    if not (isinstance(bytes_cuda, torch.Tensor) and bytes_cuda.is_cuda and bytes_cuda.dtype == torch.uint8 and
+            isinstance(offsets_cuda, torch.Tensor) and offsets_cuda.is_cuda and offsets_cuda.dtype == torch.int64 and
+            bytes_cuda.device == offsets_cuda.device and bytes_cuda.is_contiguous() and offsets_cuda.is_contiguous()):
+        raise ValueError("revcomp_packed: contiguous uint8 bytes and int64 offsets CUDA tensors on one device expected")
+    if rc is None:
+        raise ValueError("revcomp_packed: rc must be 'always', 'random' or 'both'")
+    mode, rc_prob, seed, base = _rc_spec(rc, rc_prob, seed, seq_index_base)
+    if offsets_cuda.numel() < 1:
+        raise ValueError("offsets needs at least one entry")
+    dev = bytes_cuda.device
+    stream = torch.cuda.current_stream(dev.index).cuda_stream
+    n = offsets_cuda.numel() - 1
+    total, _ = capi.crop_extent_device(dev.index, stream, offsets_cuda, n, _UNCROPPED, nbytes=bytes_cuda.numel())
+    m = 2 if mode == capi.RC_BOTH else 1
+    out_b = torch.empty(max(m * total, 1), dtype=torch.uint8, device=dev)
+    out_o = torch.empty(m * n + 1, dtype=torch.int64, device=dev)
+    flipped = torch.empty(m * n, dtype=torch.uint8, device=dev)
+    src = bytes_cuda if bytes_cuda.numel() > 0 else out_b  # (an all-empty batch: nothing is read)
+    capi.revcomp(dev.index, stream, src, offsets_cuda, n, mode, rc_prob, seed, base, out_b, out_o, flipped)
+    return RevCompBatch(out_b[:m * total], out_o, flipped.view(torch.bool))
 
 
 def batch_tokenize_augmented(tokenizer, batch, padlen=-1, destchar="B", batch_first=False, device=None, *, augment=1,
@@ -487,7 +638,8 @@ def _varlen_extent_host(h_offs, n, k):
     return total, int(lens.max()) + k
 
 
-def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None, *, crop=None, crop_len=None, seed=0, seq_index_base=0):
+def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None, *, crop=None, crop_len=None, seed=0, seq_index_base=0,
+                          rc=None, rc_prob=None):
     """Tokens of every sequence of ``batch`` back to back, without padding: a :class:`VarlenBatch`.
 
     Row ``i`` (``tokens[cu_seqlens[i]:cu_seqlens[i + 1]]``) equals ``batch_tokenize(batch, padlen=P, batch_first=True,
@@ -495,22 +647,25 @@ def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None, *, crop=N
     whatever ``padchar`` is.  ``cu_seqlens[i] = (offsets[i] - offsets[0]) + i * (bos + eos)`` as int32; a batch of more
     than 2^31 - 1 tokens raises ``ValueError``.  Host batches are sized from their host offsets without synchronising;
     CUDA batches pay one synchronisation (the extent is read back).  ``crop`` / ``crop_len`` (required with ``crop``):
-    every sequence is cropped first, as :func:`crop_packed` does."""
-    return _tokenize_varlen(tokenizer, batch, destchar, device, crop=_crop_spec(crop, crop_len, seed, seq_index_base))
+    every sequence is cropped first, as :func:`crop_packed` does.  ``rc`` / ``rc_prob``: then flipped, as
+    :func:`batch_tokenize_revcomp` does (``"both"`` gives ``2n`` rows)."""
+    return _tokenize_varlen(tokenizer, batch, destchar, device, crop=_crop_spec(crop, crop_len, seed, seq_index_base),
+                            rc=_rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer))
 
 
-def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None, mlm=None, crop=None):
+def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None, mlm=None, crop=None, rc=None):
     """batch_tokenize_varlen; ``augment``: BLOSUM62 arguments as ``_augment_args`` makes them (FlatFileDataset);
-    ``mlm``: a ``capi.MLMDesc`` -- then ``(VarlenBatch, labels)`` is returned; ``crop``: from ``_crop_spec``."""
+    ``mlm``: a ``capi.MLMDesc`` -- then ``(VarlenBatch, labels)`` is returned; ``crop``: from ``_crop_spec``; ``rc``: from
+    ``_rc_spec``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
     k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
     extent = []
     r = _resolve(batch, device, augment, before_stage=lambda h_offs, n: extent.extend(_varlen_extent_host(h_offs, n, k)),
-                 crop=crop)
+                 crop=crop, rc=rc)
     try:
-        if r.h_offs is None and r.extent is not None:  # a cropped CUDA batch: sized by the crop's one read-back
+        if r.h_offs is None and r.extent is not None:  # a cropped or flipped CUDA batch: sized by its one read-back
             total, max_seqlen = r.extent[0] + r.nseq * k, (r.extent[1] + k if r.nseq > 0 else 0)
             if total > _INT32_MAX:
                 raise ValueError(f"varlen batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one "
@@ -592,7 +747,7 @@ def _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignor
 
 def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *, varlen=False, maskfrac=0.15, mask_prob=0.8,
                        random_prob=0.1, mask_token=None, ignore_index=-100, seed=0, seq_index_base=0, augment=0,
-                       augment_frac=1.0, crop=None, crop_len=None):
+                       augment_frac=1.0, crop=None, crop_len=None, rc=None, rc_prob=None):
     """A masked-language-model batch in one launch: :class:`MLMBatch` ``(inputs, labels)``.
 
     ``inputs`` start from ``batch_tokenize(batch, padlen, batch_first=True, destchar=destchar)`` (``varlen=False``:
@@ -607,21 +762,24 @@ def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *
     the same mask padded or padding-free, in any slice (the exact rule is documented with ``bsq_tokenize_mlm`` in
     include/bsq.h).  ``augment``: BLOSUM62 point mutations first (as ``batch_tokenize_augmented``, same seed), then the
     mask.  ``crop`` / ``crop_len``: every sequence is cropped before both (as :func:`batch_tokenize_cropped`, same seed;
-    ``varlen=True`` needs an explicit ``crop_len``); residue positions are then positions within the window."""
+    ``varlen=True`` needs an explicit ``crop_len``); residue positions are then positions within the window.  ``rc`` /
+    ``rc_prob``: "always" or "random" (not "both"), after the crop and before the mask, as :func:`batch_tokenize_revcomp`
+    does; residue positions are then positions in the flipped window."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
     mlm = _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignore_index, seed, seq_index_base)
+    rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment, mlm=True)
     augment = _augment_args(augment, augment_frac, seed, seq_index_base)
     if varlen:
         if padlen is not None and padlen != -1:
             raise ValueError("batch_tokenize_mlm(varlen=True) writes no padding: padlen must not be given")
         crop = _crop_spec(crop, crop_len, seed, seq_index_base)
-        vb, labels = _tokenize_varlen(tokenizer, batch, destchar, device, augment, mlm, crop)
+        vb, labels = _tokenize_varlen(tokenizer, batch, destchar, device, augment, mlm, crop, rc)
         return MLMBatch(vb, labels)
     padlen = _default_padlen(batch, tokenizer, padlen)
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
-    r = _resolve(batch, device, augment, crop=crop)
+    r = _resolve(batch, device, augment, crop=crop, rc=rc)
     try:
         _check_lengths(r, padlen, tok, onehot=False)
         dev = torch.device("cuda", r.device)
@@ -669,6 +827,21 @@ def _seqpack_host_offsets(batch):
     return h
 
 
+def _cuda_pair(batch):
+    """(bytes, offsets) of a packed CUDA batch, checked as ``_resolve`` checks them; None for any other batch form."""
+    torch = _torch()
+    if not (isinstance(batch, tuple) and len(batch) == 2 and isinstance(batch[0], torch.Tensor) and batch[0].is_cuda):
+        return None
+    b, o = batch
+    if not (isinstance(o, torch.Tensor) and o.is_cuda and o.device == b.device):
+        raise ValueError("bytes and offsets must live on the same side (all host or all CUDA)")
+    if b.dtype != torch.uint8 or o.dtype != torch.int64 or not b.is_contiguous() or not o.is_contiguous():
+        raise ValueError("packed batch: contiguous uint8 bytes and int64 offsets expected")
+    if o.numel() < 1:
+        raise ValueError("offsets needs at least one entry")
+    return b, o
+
+
 class _SeqPackPlan:
     """The host plan (bsq_seqpack_plan) in one pinned int64 buffer: row_ptr | row_seq | starts | cu_seqlens (int32)."""
 
@@ -692,7 +865,7 @@ class _SeqPackPlan:
 
 def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None, *, rows=None, mlm=False, maskfrac=0.15,
                            mask_prob=0.8, random_prob=0.1, mask_token=None, ignore_index=-100, crop=None, crop_len=None,
-                           augment=0, augment_frac=1.0, seed=0, seq_index_base=0):
+                           augment=0, augment_frac=1.0, seed=0, seq_index_base=0, rc=None, rc_prob=None):
     """Sequence packing: every sequence of ``batch`` whole, laid end to end in rows of ``row_len`` tokens -- a
     :class:`SeqPackBatch` of fixed shape ``(rows, row_len)`` with almost no padding.
 
@@ -707,8 +880,10 @@ def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None,
     needed.  ``mlm=True``: inputs and int64 labels as :func:`batch_tokenize_mlm` (``varlen=True``, same seed and
     ``seq_index_base``) writes them per sequence, padding labels ``ignore_index``.  ``crop`` / ``crop_len`` (default
     ``row_len - bos - eos``) and ``augment`` as for the other consumers: stage -> crop -> augment -> pack.  Every
-    sequence must fit a row (ValueError otherwise).  Host batches are planned from their host offsets without
-    synchronising; CUDA batches pay one read-back of their offsets, which also validates them."""
+    sequence must fit a row (ValueError otherwise).  ``rc`` / ``rc_prob``: sequences are flipped after the crop, as
+    :func:`batch_tokenize_revcomp` does (``"both"``, not with ``mlm``, packs ``2n`` sequences).  Host batches are planned
+    from their host offsets without synchronising; CUDA batches pay one read-back of their offsets, which also validates
+    them."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
@@ -725,6 +900,7 @@ def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None,
     rows = rows or 0  # (the planner's "as many as needed")
     mlm = _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignore_index, seed, seq_index_base) if mlm else None
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, row_len - k)
+    rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment, mlm=mlm is not None)
     augment = _augment_args(augment, augment_frac, seed, seq_index_base)
     plan = []
 
@@ -735,10 +911,11 @@ def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None,
     crop_extent = None
     if h is not None:  # planned before anything is staged (a CUDA batch: from its offsets, read back once)
         n = h.size - 1
-        if crop is not None:
-            h, crop_extent = _crop_host_extent(h, n, crop[1])
-        make_plan(h, n)
-    r = _resolve(batch, device, augment, before_stage=None if h is not None else make_plan, crop=crop, crop_extent=crop_extent)
+        if crop is not None or rc is not None:
+            h, crop_extent = _crop_host_extent(h, n, crop[1] if crop is not None else _UNCROPPED)
+        make_plan(*_rc_host_offsets(h, n, rc))
+    r = _resolve(batch, device, augment, before_stage=None if h is not None else make_plan, crop=crop, crop_extent=crop_extent,
+                 rc=rc)
     try:
         p = plan[0]
         dev = torch.device("cuda", r.device)
@@ -821,7 +998,7 @@ def _kmer_check_extent(extent, padlen, varlen):
 
 
 def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=None, *, stride=1, tail="drop", varlen=False,
-                        crop=None, crop_len=None, seed=0, seq_index_base=0):
+                        crop=None, crop_len=None, seed=0, seq_index_base=0, rc=None, rc_prob=None):
     """K-mer tokens of every sequence of ``batch``, written by one kernel (padding-free: three small ones).
 
     Sequence ``i`` of ``n`` residues gives ``[BOS] k-mer ids [single-residue ids] [EOS]``: ``m = (n - k) // stride + 1``
@@ -835,8 +1012,9 @@ def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=Non
     without; a row longer than ``padlen`` raises ValueError.  ``varlen=True``: a :class:`VarlenBatch` (``padlen`` must not
     be given); more than 2^31 - 1 tokens raise ValueError.  ``destchar`` defaults to int32 (``"i"``), which holds every
     vocabulary the rule allows; a kind too narrow for ``vocab_size`` raises ValueError.  ``crop`` / ``crop_len`` (required
-    with ``crop``, in residues): every sequence is cropped first, as :func:`crop_packed` does.  Host batches are sized from
-    their host offsets without synchronising; CUDA batches pay one read-back (two when cropped)."""
+    with ``crop``, in residues): every sequence is cropped first, as :func:`crop_packed` does.  ``rc`` / ``rc_prob``: then
+    flipped, as :func:`batch_tokenize_revcomp` does, so the k-mers are those of the reverse complement.  Host batches are
+    sized from their host offsets without synchronising; CUDA batches pay one read-back (two when cropped)."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
@@ -856,6 +1034,7 @@ def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=Non
         if padlen <= 0:
             raise ValueError("batch_tokenize_kmer requires padlen (or varlen=True)")
     crop = _crop_spec(crop, crop_len, seed, seq_index_base)
+    rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer)
     extent = []
 
     def before_stage(h_offs, n):
@@ -863,9 +1042,19 @@ def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=Non
         _kmer_check_extent(e, padlen, varlen)
         extent.extend(e)
 
-    r = _resolve(batch, device, before_stage=before_stage, crop=crop)
+    validated = False
+    if rc is not None and crop is None and _cuda_pair(batch) is not None:
+        # the extent of the unflipped offsets is the flipped batch's (doubled by "both"), and reading it validates them:
+        # the flip needs no read-back of its own
+        b, o = _cuda_pair(batch)
+        total, longest = capi.kmer_extent_device(b.device.index, torch.cuda.current_stream(b.device.index).cuda_stream, o,
+                                                 o.numel() - 1, km, nbytes=b.numel())
+        extent = [total * (2 if rc[0] == capi.RC_BOTH else 1), longest]
+        _kmer_check_extent(extent, padlen, varlen)
+        validated = True
+    r = _resolve(batch, device, before_stage=before_stage, crop=crop, rc=rc, validated=validated)
     try:
-        if r.h_offs is None:  # a CUDA batch: one reduction and read-back, which also validates its offsets
+        if r.h_offs is None and not validated:  # a CUDA batch: one reduction and read-back, which also validates its offsets
             nbytes = batch[0].numel() if r.extent is None else -1
             extent = capi.kmer_extent_device(r.device, r.stream, r.d_offs, r.nseq, km, nbytes=nbytes)
             _kmer_check_extent(extent, padlen, varlen)

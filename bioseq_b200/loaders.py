@@ -7,7 +7,8 @@ left.  BLOSUM62 augmentation (``augment=``; bioseq/blosum.py:63-87) runs on the 
 the tokeniser (``consumers``; Philox streams keyed by the dataset seed, the draw number and the sequence index),
 and ``cnn=True`` batches are written directly in the ``(batch, emb, length)`` float layout.  ``max_seq_len=`` crops
 over-long sequences on the device (``consumers.crop_packed``) so that a file with a few very long sequences still
-yields batches of the model's context.
+yields batches of the model's context, and ``rc="random"`` flips DNA sequences to their reverse complement on the device
+(``consumers.revcomp_packed``).
 """
 import numpy as np
 
@@ -75,14 +76,19 @@ class FlatFileDataset(_dataset_base()):
     labels with ``mlm=True``); a single index is the same with one row.  Crop, augmentation and masking draw from the
     per-fetch seed as above.  ``seqpack=True`` cannot be combined with ``varlen=True`` or ``cnn=True``.
 
+    ``rc="random"`` (nucleotide tokenizers, not with ``augment``) flips each sequence to its reverse complement with
+    probability ``rc_prob`` after the crop and before masking or tokenization: strand augmentation, usually together with
+    ``crop="random"`` as the random shift.  Like the crop, every fetch is a new draw from the per-fetch seed.  Datasets
+    are for training, so the inference modes (``"always"``, ``"both"``) are rejected: call the consumers directly.
+
     ``fetch(index, return_items=True)`` also hands back the raw sequence(s) (bioseq/loaders.py:60-84), as stored in the
-    file: uncropped, like they are unaugmented.  Two quirks of
+    file: uncropped and unflipped, like they are unaugmented.  Two quirks of
     the reference's ``fetch`` are NOT reproduced: with ``cnn=True`` and ``return_items=False`` it falls off the end and
     returns ``None``, and without ``cnn`` it ignores ``return_items``; here both modes honour the flag.
     """
 
     def __init__(self, ff, tokenizer, *, augment=0, augment_frac=0.5, cnn=False, device=None, maskfrac=0.15, seed=13,
-                 varlen=False, mlm=False, max_seq_len=None, crop="random", seqpack=False):
+                 varlen=False, mlm=False, max_seq_len=None, crop="random", seqpack=False, rc=None, rc_prob=0.5):
         super().__init__()
         assert isinstance(ff, cbioseq.FlatFile)
         assert isinstance(tokenizer, cbioseq.Tokenizer)
@@ -108,6 +114,10 @@ class FlatFileDataset(_dataset_base()):
                 raise ValueError(f"FlatFileDataset: max_seq_len {max_seq_len} leaves no room for a residue next to bos + eos")
             self.max_seq_len, self.crop, self.crop_len = int(max_seq_len), crop, int(max_seq_len) - k
         self.maxseqlen = self.max_seq_len
+        if rc not in (None, "random"):
+            raise ValueError(f"FlatFileDataset: rc must be None or 'random' (a dataset is for training), got {rc!r}")
+        consumers._rc_spec(rc, rc_prob if rc else None, 0, 0, tokenizer, augment)  # ValueError now rather than per fetch
+        self.rc, self.rc_prob = rc, rc_prob
 
     def _range(self, index):
         n = len(self)
@@ -134,41 +144,50 @@ class FlatFileDataset(_dataset_base()):
         import torch
         start, stop, many = self._range(index)
         crop = dict(crop=self.crop, crop_len=self.crop_len) if self.crop else {}
+        rc = dict(rc=self.rc, rc_prob=self.rc_prob) if self.rc else {}
         if self.seqpack:
-            kw = self._augment_kwargs(start) if self.mlm or self.augment or self.crop else {}
+            kw = self._augment_kwargs(start) if self.mlm or self.augment or self.crop or self.rc else {}
             mlm = dict(mlm=True, maskfrac=self.maskfrac, mask_token=self.tokenizer.alphabet_size()) if self.mlm else {}
             return consumers.batch_tokenize_seqpack(self.tokenizer, (self.ff, start, stop), self.max_seq_len, "l", self.device,
-                                                    rows=None if many else 1, **mlm, **kw, **crop)
+                                                    rows=None if many else 1, **mlm, **kw, **crop, **rc)
         if self.mlm:
-            # one draw per fetch, shared by the augmentation (counter word 3 = 0), the mask (words 1, 2) and the crop (3)
+            # one draw per fetch, shared by the augmentation (counter word 3 = 0), the mask (words 1, 2), the crop (3) and the
+            # strand flip (4)
             kw = self._augment_kwargs(start)
             mb = consumers.batch_tokenize_mlm(self.tokenizer, (self.ff, start, stop),
                                               padlen=-1 if self.varlen else self.max_seq_len, destchar="l",
                                               device=self.device, varlen=self.varlen, maskfrac=self.maskfrac,
-                                              mask_token=self.tokenizer.alphabet_size(), **kw, **crop)
+                                              mask_token=self.tokenizer.alphabet_size(), **kw, **crop, **rc)
             if many:
                 return mb
             return consumers.MLMBatch(mb.inputs.tokens if self.varlen else mb.inputs[0], mb.labels if self.varlen else mb.labels[0])
-        aug = self._augment_kwargs(start) if self.augment or self.crop else {}
+        aug = self._augment_kwargs(start) if self.augment or self.crop or self.rc else {}
         if self.cnn:
             if many:  # (batch, emb, length) float, written in that layout by one kernel
                 return consumers.batch_onehot_encode_bcl(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
-                                                         destchar='f', device=self.device, **aug, **crop)
+                                                         destchar='f', device=self.device, **aug, **crop, **rc)
             if aug:
-                # (mutated or cropped on the device: the batched path at padlen = max_seq_len; a mutated sequence keeps its
-                # length, so only the reference's extra bos + eos pad rows of the single-sequence encoder are missing here)
+                # (mutated, cropped or flipped on the device: the batched path at padlen = max_seq_len; such a sequence is no
+                # longer than before, so only the reference's extra bos + eos pad rows of the single-sequence encoder are
+                # missing here)
                 return consumers.batch_onehot_encode_bcl(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
-                                                         destchar='f', device=self.device, **aug, **crop)[0].t()
+                                                         destchar='f', device=self.device, **aug, **crop, **rc)[0].t()
             return self.tokenizer.onehot_encode(bytes(self.ff[start]), padlen=self.max_seq_len, destchar='f', device=self.device)
         if self.varlen:
             vb = consumers._tokenize_varlen(self.tokenizer, (self.ff, start, stop), "l", self.device,
                                             consumers._augment_args(**aug) if aug else None,
                                             crop=consumers._crop_spec(self.crop, self.crop_len, aug.get("seed", 0), start)
-                                            if crop else None)
+                                            if crop else None,
+                                            rc=consumers._rc_spec(self.rc, self.rc_prob, aug.get("seed", 0), start) if rc else None)
             return vb if many else vb.tokens
         if crop:
             toks = consumers.batch_tokenize_cropped(self.tokenizer, (self.ff, start, stop), self.max_seq_len, batch_first=True,
-                                                    destchar='B', device=self.device, **aug, **crop).to(torch.long)
+                                                    destchar='B', device=self.device, **aug, **crop, **rc).to(torch.long)
+            return toks if many else toks[0]
+        if rc:
+            seed = dict(seed=aug["seed"], seq_index_base=start)
+            toks = consumers.batch_tokenize_revcomp(self.tokenizer, (self.ff, start, stop), self.max_seq_len, batch_first=True,
+                                                    destchar='B', device=self.device, **seed, **rc).to(torch.long)
             return toks if many else toks[0]
         if aug:
             toks = consumers.batch_tokenize_augmented(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,

@@ -223,6 +223,46 @@ int bsq_crop(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_
 int bsq_crop_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, int64_t crop_len,
                            int64_t *total, int64_t *max_len);
 
+/* Reverse complement (strand augmentation for DNA / RNA models in training, both-strand averaging at inference): a
+ * packed batch in, a packed batch out, which every entry point above then takes unchanged.
+ *   Complement table comp[256], defined on every byte value and case-preserving: A<->T, C<->G, R<->Y, K<->M, B<->V, D<->H;
+ *   S, W and N map to themselves; U -> A (RNA gives its DNA reverse complement); the same pairs in lower case.  Every
+ *   other byte maps to itself (gaps, '*', digits, bytes >= 0x80), so a byte a tokenizer rejects is still rejected after
+ *   the flip.  bsq_revcomp_table copies it out.
+ *   Flip of a sequence of len bytes: out[j] = comp[in[len - 1 - j]].
+ *   Modes:
+ *     BSQ_RC_ALWAYS  every sequence is flipped;
+ *     BSQ_RC_RANDOM  sequence i is flipped iff x0 < gate, with x0 = word 0 of Philox4x32-10 at counter (g_lo, g_hi, 0, 4)
+ *                    under key (seed_lo, seed_hi), g = seq_index_base + i, and gate = rc_prob >= 1 ? 2^32 :
+ *                    floor(rc_prob * 2^32) (in double precision, on the host).  Counter word 3 = 4 keeps the draw
+ *                    disjoint from augmentation (0), MLM (1, 2) and crop (3) under the same seed: the flip depends only on
+ *                    (seed, global sequence index), not on the length, padlen, the padded or padding-free form or slicing;
+ *     BSQ_RC_BOTH    2n output sequences: sequence i is input sequence i unchanged, sequence n + i its reverse complement
+ *                    (the torch.cat([x, x_rc]) layout that both-strand inference averages over).
+ *   Output: out_offsets start at 0; out_offsets[i] = offsets[i] - offsets[0] for i = 0 .. n, and in BOTH mode, with
+ *   T = offsets[n] - offsets[0], out_offsets[n + i] = T + offsets[i] - offsets[0].  d_flipped (optional, may be NULL): one
+ *   byte (0 / 1) per output sequence.
+ *   Order inside a consumer: stage -> crop -> reverse complement -> tokenize / mask / pack / k-mer.  MLM positions are
+ *   positions in the flipped window; the sequence index is unchanged.
+ * Worked answers: "ACGTN" -> "NACGT", "GATTACA" -> "TGTAATC", "ACGU" -> "ACGT", "acgRYkmBDHVswn-*" -> "*-nwsBDHVkmRYcgt",
+ * "" -> "".  RANDOM, rc_prob 0.5, sequences 0 .. 7: seed 7, seq_index_base 0 flips [1,0,1,1,1,1,1,1] (x0 = 407685168,
+ * 3339964855, 305774060, ...); seed 0x123456789ABCDEF0, seq_index_base 2^32 + 11 flips [1,0,0,0,1,0,1,1].
+ *
+ * bsq_revcomp enqueues only (one kernel; nseq == 0: an 8-byte memset of out_offsets), uses no scratch memory, keeps no
+ * state between launches and is capturable into a CUDA graph.  The caller has validated the offsets (as for bsq_crop).
+ * d_out_bytes (any alignment, not overlapping the input) holds at least T bytes, 2T in BOTH mode -- a caller with a
+ * device batch can size it from the byte buffer's size, with no read-back; BOTH writes its forward half too.
+ * d_out_offsets has n + 1 entries (2n + 1 in BOTH mode).  BSQ_ERR_ARG, before any device call, for a bad mode, rc_prob
+ * NaN or < 0 (read in RANDOM mode only, checked in every mode), nseq < 0, a NULL d_out_offsets, or NULL bytes, offsets or
+ * output bytes with nseq > 0. */
+#define BSQ_RC_ALWAYS 0
+#define BSQ_RC_RANDOM 1
+#define BSQ_RC_BOTH 2
+int bsq_revcomp(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq, int mode, double rc_prob,
+                uint64_t seed, int64_t seq_index_base, uint8_t *d_out_bytes, int64_t *d_out_offsets, uint8_t *d_flipped);
+/* Host only, no device call: out[b] = comp[b] for every byte value b.  BSQ_ERR_ARG for a NULL out. */
+int bsq_revcomp_table(uint8_t out[256]);
+
 /* Sequence packing (padding-free batches of a fixed shape: SDPA with a block-diagonal mask, position-id packing as in
  * HF's DataCollatorWithFlattening, CUDA graphs, torch.compile): whole sequences laid end to end in R rows of L tokens.
  * With k = bos + eos and the (already cropped) lengths len_i, sequence i occupies need_i = len_i + k tokens; every
