@@ -30,6 +30,8 @@ class KmerDesc(C.Structure):
 
 KMER_DROP, KMER_SINGLE = 0, 1
 RC_ALWAYS, RC_RANDOM, RC_BOTH = 0, 1, 2
+TILE_SHORT, TILE_END, TILE_DROP = 0, 1, 2
+UNTILE_F32, UNTILE_BF16, UNTILE_F16 = 0, 1, 2
 
 
 class TokenizerDesc(C.Structure):
@@ -127,6 +129,10 @@ def lib():
         "bsq_kmer_extent_device": (i32, [i32, vp, vp, i64, i64, C.POINTER(KmerDesc), C.POINTER(i64), C.POINTER(i64)]),
         "bsq_revcomp": (i32, [i32, vp, vp, vp, i64, i32, C.c_double, C.c_uint64, i64, vp, vp, vp]),
         "bsq_revcomp_table": (i32, [vp]),
+        "bsq_tile_extent_host": (i32, [vp, i64, i64, i64, i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
+        "bsq_tile_extent_device": (i32, [i32, vp, vp, i64, i64, i64, i64, i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
+        "bsq_tile": (i32, [i32, vp, vp, vp, i64, i64, i64, i32, vp, vp, vp, vp, vp]),
+        "bsq_untile_mean": (i32, [i32, vp, i32, vp, i64, i64, vp, i64, vp, i64, i64, i64, i32, vp, i64, i32, vp, vp]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(L, name)
@@ -147,7 +153,8 @@ EXPORTS = ("bsq_abi_version bsq_last_error bsq_launch_count bsq_launch_count_res
            "bsq_tokenize_stream_items bsq_onehot_stream_items bsq_shard_bounds bsq_tokenize_host_sharded bsq_memcpy_d2d bsq_tokenize_many "
            "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm bsq_crop bsq_crop_extent_device "
            "bsq_seqpack_plan bsq_tokenize_seqpack bsq_tokenize_seqpack_mlm bsq_kmer_init bsq_tokenize_kmer bsq_tokenize_kmer_varlen "
-           "bsq_kmer_extent_host bsq_kmer_extent_device bsq_revcomp bsq_revcomp_table").split()
+           "bsq_kmer_extent_host bsq_kmer_extent_device bsq_revcomp bsq_revcomp_table bsq_tile_extent_host bsq_tile_extent_device "
+           "bsq_tile bsq_untile_mean").split()
 
 
 def last_error():
@@ -264,6 +271,36 @@ def revcomp_table():
     t = np.zeros(256, np.uint8)
     check(lib().bsq_revcomp_table(t.ctypes.data))
     return t
+
+
+def tile_extent_host(h_offsets, nseq, window, stride, tail):
+    """-> (windows, bytes, longest window) of host offsets (bsq_tile_extent_host; no device call)."""
+    w, b, m = C.c_int64(), C.c_int64(), C.c_int64()
+    check(lib().bsq_tile_extent_host(_ptr(h_offsets), nseq, window, stride, tail, C.byref(w), C.byref(b), C.byref(m)))
+    return w.value, b.value, m.value
+
+
+def tile_extent_device(device, stream, d_offsets, nseq, window, stride, tail, nbytes=-1):
+    """-> (windows, bytes, longest window) of device-resident offsets (bsq_tile_extent_device: validates them;
+    synchronises)."""
+    w, b, m = C.c_int64(), C.c_int64(), C.c_int64()
+    check(lib().bsq_tile_extent_device(device, stream, _ptr(d_offsets), nseq, nbytes, window, stride, tail, C.byref(w), C.byref(b),
+                                       C.byref(m)))
+    return w.value, b.value, m.value
+
+
+def tile(device, stream, d_bytes, d_offsets, nseq, window, stride, tail, d_out_bytes, d_out_offsets, d_seq_ptr=None,
+         d_seq_index=None, d_starts=None):
+    """Every window of every sequence (bsq_tile); ``tail``: TILE_SHORT, TILE_END or TILE_DROP."""
+    check(lib().bsq_tile(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, window, stride, tail, _ptr(d_out_bytes),
+                         _ptr(d_out_offsets), _ptr(d_seq_ptr), _ptr(d_seq_index), _ptr(d_starts)))
+
+
+def untile_mean(device, stream, dtype, d_y, channels, row_stride, d_cu, col0, d_src_offsets, nseq, window, stride, tail, d_seq_ptr,
+                nwin, strands, d_flipped, d_out):
+    """Per-residue mean of window outputs (bsq_untile_mean); ``dtype``: UNTILE_F32, UNTILE_BF16 or UNTILE_F16."""
+    check(lib().bsq_untile_mean(device, stream, dtype, _ptr(d_y), channels, row_stride, _ptr(d_cu), col0, _ptr(d_src_offsets), nseq,
+                                window, stride, tail, _ptr(d_seq_ptr), nwin, strands, _ptr(d_flipped), _ptr(d_out)))
 
 
 def seqpack_plan(h_offsets, nseq, k, row_len, rows=0, starts=None, row_ptr=None, row_seq=None, cu_seqlens=None):

@@ -25,6 +25,10 @@ Reference counterparts:
 * ``revcomp_packed`` / ``rc=`` -- the reverse complement of every DNA / RNA sequence on the device (seeded strand flips
   for training, both strands for test-time averaging) instead of flipping Python strings or gathering in torch; every
   consumer takes ``rc=`` and ``rc_prob=`` and runs unchanged on the flipped batch.
+* ``tile_packed`` / ``batch_tokenize_tiled`` / ``untile`` -- every window of every sequence at a stride (inference over
+  whole long sequences, chunked datasets) on the device instead of slicing Python strings or a ragged gather in torch,
+  and the per-residue mean of the model's window outputs stitched back deterministically instead of ``index_add_`` and
+  counts.
 
 All of these call the C ABI (``include/bsq.h``) through ``capi``; torch supplies memory and the stream.
 A *batch* is one of
@@ -1071,3 +1075,225 @@ def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=Non
         return out
     finally:
         r.release()
+
+
+_TILE_TAILS = {"short": capi.TILE_SHORT, "end": capi.TILE_END, "drop": capi.TILE_DROP}
+
+
+def _tile_spec(window, stride, tail):
+    """Validate the tiling arguments (ValueError before anything is staged) -> ``(window, stride, tail code)``; ``stride``
+    defaults to ``window`` (windows side by side)."""
+    if not isinstance(tail, str) or tail not in _TILE_TAILS:
+        raise ValueError(f"tail must be 'short', 'end' or 'drop', got {tail!r}")
+    try:
+        window = operator.index(window)
+        stride = window if stride is None else operator.index(stride)
+    except TypeError:
+        raise ValueError("window and stride must be integers") from None
+    if not 1 <= window <= _INT64_MAX:
+        raise ValueError(f"window must be >= 1, got {window}")
+    if not 1 <= stride <= window:
+        raise ValueError(f"stride must lie in 1..window = {window}, got {stride}")
+    return int(window), int(stride), _TILE_TAILS[tail]
+
+
+TiledBatch = collections.namedtuple("TiledBatch", ["bytes", "offsets", "seq_index", "starts", "seq_ptr", "seq_offsets"])
+TiledBatch.__doc__ = """Every window of a packed batch, as a packed batch: ``bytes`` (uint8) and ``offsets`` (int64, from 0) of the
+windows; ``seq_index`` (int64, one per window: its sequence -- HF's ``overflow_to_sample_mapping``); ``starts`` (int64, one
+per window: where it begins in its sequence); ``seq_ptr`` (int64, ``n + 1``: sequence ``i``'s windows are
+``seq_ptr[i] .. seq_ptr[i + 1] - 1``); ``seq_offsets`` (int64, ``n + 1``: the source offsets from 0, the layout
+:func:`untile` writes)."""
+
+
+def tile_packed(bytes_cuda, offsets_cuda, window, *, stride=None, tail="short"):
+    """Every window of ``window`` residues, every ``stride`` residues (default ``window``), of every sequence of a packed
+    CUDA batch: a :class:`TiledBatch`; the input is not modified.
+
+    A sequence of at most ``window`` residues is one window (an empty sequence one empty window).  A longer one gives
+    windows at ``0, stride, 2 * stride, ...``; ``tail`` decides the last: ``"short"`` keeps a shorter last window,
+    ``"end"`` ends the last window at the sequence's end (every window is ``window`` long), ``"drop"`` drops the residues
+    after the last full window.  The exact rule is documented with ``bsq_tile`` in include/bsq.h.  ``(tb.bytes,
+    tb.offsets)`` is a packed CUDA batch that every consumer takes, ``rc=`` included; their seeded draws are then keyed by
+    window index (``seq_index_base + w``).  One synchronisation: the offsets are validated and the output's size is read
+    back."""
+    torch = _torch()
+    if not (isinstance(bytes_cuda, torch.Tensor) and bytes_cuda.is_cuda and bytes_cuda.dtype == torch.uint8 and
+            isinstance(offsets_cuda, torch.Tensor) and offsets_cuda.is_cuda and offsets_cuda.dtype == torch.int64 and
+            bytes_cuda.device == offsets_cuda.device and bytes_cuda.is_contiguous() and offsets_cuda.is_contiguous()):
+        raise ValueError("tile_packed: contiguous uint8 bytes and int64 offsets CUDA tensors on one device expected")
+    window, stride, tail = _tile_spec(window, stride, tail)
+    if offsets_cuda.numel() < 1:
+        raise ValueError("offsets needs at least one entry")
+    dev = bytes_cuda.device
+    stream = torch.cuda.current_stream(dev.index).cuda_stream
+    n = offsets_cuda.numel() - 1
+    M, nbytes, _ = capi.tile_extent_device(dev.index, stream, offsets_cuda, n, window, stride, tail, nbytes=bytes_cuda.numel())
+    out = _tile_into(dev, stream, bytes_cuda.data_ptr(), offsets_cuda, n, window, stride, tail, M, nbytes)
+    return out._replace(seq_offsets=offsets_cuda - offsets_cuda[:1])
+
+
+def _tile_into(dev, stream, d_bytes, d_offs, n, window, stride, tail, M, nbytes):
+    """bsq_tile into fresh buffers (a TiledBatch without seq_offsets)."""
+    torch = _torch()
+    out_b = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)  # (never a null pointer)
+    out_o = torch.empty(M + 1, dtype=torch.int64, device=dev)
+    seq_ptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    seq_index = torch.empty(M, dtype=torch.int64, device=dev)
+    starts = torch.empty(M, dtype=torch.int64, device=dev)
+    # an all-empty batch may have no residue buffer at all; nothing is read from it then
+    capi.tile(dev.index, stream, d_bytes or out_b, d_offs, n, window, stride, tail, out_b, out_o, seq_ptr, seq_index, starts)
+    return TiledBatch(out_b[:nbytes], out_o, seq_index, starts, seq_ptr, None)
+
+
+TiledTokens = collections.namedtuple("TiledTokens", ["tokens", "seq_index", "starts", "seq_ptr", "seq_offsets", "flipped", "strands",
+                                                     "window", "stride", "tail", "bos"])
+TiledTokens.__doc__ = """Tokens of every window of a batch: ``tokens`` (padded ``(strands * M, padlen)`` or a :class:`VarlenBatch`),
+``seq_index`` / ``starts`` / ``seq_ptr`` / ``seq_offsets`` as in :class:`TiledBatch` (for the ``M`` windows of one strand:
+with ``strands == 2`` rows ``M .. 2M - 1`` are rows ``0 .. M - 1`` reverse-complemented), ``flipped`` (bool, one per row,
+or None without ``rc``), ``strands`` (1, or 2 for ``rc="both"``), ``window`` / ``stride`` / ``tail`` (the tiling) and
+``bos`` (leading special tokens per row: :func:`untile`'s default ``col0``)."""
+
+UntiledBatch = collections.namedtuple("UntiledBatch", ["values", "offsets"])
+UntiledBatch.__doc__ = """Per-residue values stitched back onto the sequences: ``values`` (float32 ``(sum len_i, C)``, sequence
+``i``'s residues in rows ``offsets[i] .. offsets[i + 1] - 1``) and ``offsets`` (int64, from 0)."""
+
+
+def batch_tokenize_tiled(tokenizer, batch, window, stride=None, padlen=None, destchar="B", device=None, *, tail="short",
+                         varlen=False, rc=None, rc_prob=None, seed=0, crop=None):
+    """Tokens of every window of every sequence of ``batch``: stage -> tile -> reverse complement -> tokenize, on the
+    device.  A :class:`TiledTokens`.
+
+    Windows as :func:`tile_packed` cuts them (``stride`` defaults to ``window``; ``tail`` ``"short"``, ``"end"`` or
+    ``"drop"``).  ``varlen=False``: a padded ``(rows, padlen)`` tensor, one row per window as ``batch_tokenize(...,
+    batch_first=True)`` writes it; ``padlen`` defaults to ``window + bos + eos`` and may not be smaller.  ``varlen=True``:
+    a :class:`VarlenBatch` (``padlen`` must not be given).  ``rc`` / ``rc_prob`` / ``seed``: the windows are flipped as
+    :func:`batch_tokenize_revcomp` does, with the coins keyed by window index; ``"both"`` gives ``2M`` rows, the windows
+    and then their reverse complements -- the layout :func:`untile` averages over.  A tile is a crop, so ``crop`` is
+    rejected.  Host batches are sized from their host offsets without synchronising; CUDA batches pay one read-back,
+    which also validates their offsets."""
+    torch = _torch()
+    if crop is not None:
+        raise ValueError("batch_tokenize_tiled: a tile is already a crop of the sequence; crop cannot be combined with it")
+    tok = descriptor(tokenizer)
+    kind, dtype = _dtype_of(destchar)
+    window, stride, tail_code = _tile_spec(window, stride, tail)
+    k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
+    if varlen:
+        if padlen is not None and padlen != -1:
+            raise ValueError("batch_tokenize_tiled(varlen=True) writes no padding: padlen must not be given")
+    else:
+        try:
+            padlen = window + k if padlen is None or padlen == -1 else operator.index(padlen)
+        except TypeError:
+            raise ValueError("padlen must be an integer") from None
+        if padlen < window + k:
+            raise ValueError(f"padlen {padlen} is shorter than window + bos + eos = {window + k}")
+    rc = _rc_spec(rc, rc_prob, seed, 0, tokenizer)
+    strands = 2 if rc is not None and rc[0] == capi.RC_BOTH else 1
+    extent = []
+    seq_offsets = []
+
+    def before_stage(h_offs, n):
+        h = np.ascontiguousarray(h_offs[:n + 1], dtype=np.int64)
+        e = capi.tile_extent_host(h, n, window, stride, tail_code)
+        if varlen and strands * (e[1] + e[0] * k) > _INT32_MAX:
+            raise ValueError(f"varlen batch of {strands * (e[1] + e[0] * k)} tokens: cu_seqlens is int32, so at most 2^31 - 1 "
+                             "tokens fit one batch; split the batch")
+        extent.extend(e)
+        seq_offsets.append(h - h[0] if n >= 0 else h)
+
+    r = _resolve(batch, device, before_stage=before_stage)
+    try:
+        dev = torch.device("cuda", r.device)
+        if r.h_offs is None:  # a CUDA batch: one reduction and read-back, which also validates its offsets
+            b, o = batch
+            extent = capi.tile_extent_device(r.device, r.stream, o, r.nseq, window, stride, tail_code, nbytes=b.numel())
+            if varlen and strands * (extent[1] + extent[0] * k) > _INT32_MAX:
+                raise ValueError(f"varlen batch of {strands * (extent[1] + extent[0] * k)} tokens: cu_seqlens is int32, so at "
+                                 "most 2^31 - 1 tokens fit one batch; split the batch")
+            so = o - o[:1]
+        else:
+            so = torch.from_numpy(seq_offsets[0]).to(dev)
+        M, nbytes, longest = extent
+        tb = _tile_into(dev, r.stream, r.d_bytes, r.d_offs, r.nseq, window, stride, tail_code, M, nbytes)
+        d_bytes, d_offs, rows, flipped = tb.bytes, tb.offsets, M, None
+        if rc is not None:
+            mode, rc_prob, seed_, _ = rc
+            out_b = torch.empty(max(strands * nbytes, 1), dtype=torch.uint8, device=dev)
+            out_o = torch.empty(strands * M + 1, dtype=torch.int64, device=dev)
+            flipped = torch.empty(strands * M, dtype=torch.uint8, device=dev)
+            capi.revcomp(r.device, r.stream, d_bytes, d_offs, M, mode, rc_prob, seed_, 0, out_b, out_o, flipped)
+            d_bytes, d_offs, rows, flipped = out_b, out_o, strands * M, flipped.view(torch.bool)
+        if varlen:
+            total = strands * nbytes + rows * k
+            tokens = torch.empty(total, dtype=dtype, device=dev)
+            cu_seqlens = torch.empty(rows + 1, dtype=torch.int32, device=dev)
+            capi.tokenize_varlen(r.device, r.stream, d_bytes, d_offs, rows, tok, kind, tokens, cu_seqlens)
+            tokens = VarlenBatch(tokens, cu_seqlens, longest + k if rows > 0 else 0)
+        else:
+            tokens = torch.empty((rows, padlen), dtype=dtype, device=dev)
+            if rows > 0:
+                capi.tokenize(r.device, r.stream, d_bytes, d_offs, rows, padlen, tok, True, kind, tokens)
+        return TiledTokens(tokens, tb.seq_index, tb.starts, tb.seq_ptr, so, flipped, strands, window, stride, tail,
+                           int(tokenizer.includes_bos()))
+    finally:
+        r.release()
+
+
+_UNTILE_DTYPES = None
+
+
+def untile(values, tiled, *, col0=None):
+    """The per-residue mean of model outputs over every window (and strand) that covers each residue: an
+    :class:`UntiledBatch`.
+
+    ``values``: the outputs for ``tiled.tokens`` (a :class:`TiledTokens`), float32, bfloat16 or float16, contiguous, on the
+    tokens' device: ``(rows, P, C)`` or ``(rows, P)`` (C = 1) for padded tokens (``P >= col0 + window``), ``(T, C)`` or
+    ``(T,)`` for a :class:`VarlenBatch` of ``T`` tokens.  Position ``col0 + t`` of a window's row (``col0`` defaults to
+    ``tiled.bos``) is its residue ``t``; in a flipped window that is residue ``len - 1 - t`` of the window's span.  The sum
+    runs in float32 in a fixed order (strand 0 before strand 1, windows in ascending order), so the result is
+    deterministic; a residue no window covers (``tail="drop"``) gets NaN.  The exact rule is documented with
+    ``bsq_untile_mean`` in include/bsq.h.  One synchronisation: the residue count is read back."""
+    global _UNTILE_DTYPES
+    torch = _torch()
+    if _UNTILE_DTYPES is None:
+        _UNTILE_DTYPES = {torch.float32: capi.UNTILE_F32, torch.bfloat16: capi.UNTILE_BF16, torch.float16: capi.UNTILE_F16}
+    if not isinstance(tiled, TiledTokens):
+        raise ValueError("untile: tiled must be the TiledTokens of batch_tokenize_tiled")
+    if not isinstance(values, torch.Tensor) or values.dtype not in _UNTILE_DTYPES:
+        raise ValueError("untile: values must be a float32, bfloat16 or float16 tensor")
+    if not values.is_contiguous():
+        raise ValueError("untile: values must be contiguous")
+    varlen = isinstance(tiled.tokens, VarlenBatch)
+    tokens = tiled.tokens.tokens if varlen else tiled.tokens
+    if values.device != tokens.device:
+        raise ValueError("untile: values must live on the tokens' device")
+    try:
+        col0 = tiled.bos if col0 is None else operator.index(col0)
+    except TypeError:
+        raise ValueError("col0 must be an integer") from None
+    if col0 < 0:
+        raise ValueError(f"col0 must be >= 0, got {col0}")
+    rows = tiled.seq_index.numel() * tiled.strands
+    if varlen:
+        if values.dim() not in (1, 2) or values.shape[0] != tokens.numel():
+            raise ValueError(f"untile: padding-free values must be (T,) or (T, C) with T = {tokens.numel()}, got {tuple(values.shape)}")
+        C, stride, cu = (values.shape[1] if values.dim() == 2 else 1), 0, tiled.tokens.cu_seqlens
+    else:
+        if values.dim() not in (2, 3) or values.shape[0] != rows:
+            raise ValueError(f"untile: padded values must be (rows, P) or (rows, P, C) with rows = {rows}, got {tuple(values.shape)}")
+        C, stride, cu = (values.shape[2] if values.dim() == 3 else 1), values.shape[1], None
+        if stride < col0 + tiled.window:
+            raise ValueError(f"untile: P = {stride} is shorter than col0 + window = {col0 + tiled.window}")
+    if C < 1:
+        raise ValueError("untile: values have no channels")
+    dev = values.device
+    n = tiled.seq_ptr.numel() - 1
+    R = int(tiled.seq_offsets[-1].item()) if n > 0 else 0
+    out = torch.empty((R, C), dtype=torch.float32, device=dev)
+    if n > 0 and R > 0:
+        flipped = tiled.flipped.view(torch.uint8) if tiled.flipped is not None else None
+        capi.untile_mean(dev.index, torch.cuda.current_stream(dev.index).cuda_stream, _UNTILE_DTYPES[values.dtype], values, C,
+                         stride, cu, col0, tiled.seq_offsets, n, tiled.window, tiled.stride, _TILE_TAILS[tiled.tail], tiled.seq_ptr,
+                         tiled.seq_index.numel(), tiled.strands, flipped, out)
+    return UntiledBatch(out, tiled.seq_offsets)

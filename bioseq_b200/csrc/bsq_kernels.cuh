@@ -136,6 +136,25 @@ __device__ __forceinline__ uint4 ldg16(uintptr_t addr) {
     return __ldg(reinterpret_cast<const uint4 *>(addr));
 }
 
+__device__ __forceinline__ uintptr_t clamp_word(uintptr_t a, uintptr_t lo, uintptr_t hi) { return a < lo ? lo : (a > hi ? hi : a); }
+
+// The 16 bytes at address X (any alignment) as four little-endian words, from the aligned words at X & ~15 and the next
+// one, each clamped to [lo, hi] (16-byte aligned).  The shift may vary from thread to thread, so the words are picked
+// with selects.  Used by K12 (bsq_revcomp.cu) and K13 (bsq_tile.cu).
+__device__ __forceinline__ void fetch16_clamped(uintptr_t X, uintptr_t lo, uintptr_t hi, uint32_t t[4]) {
+    const uintptr_t a0 = X & ~uintptr_t(15);
+    const uint32_t s = static_cast<uint32_t>(X) & 15u;
+    const uint4 v0 = ldg16(clamp_word(a0, lo, hi));
+    const uint4 v1 = s != 0 ? ldg16(clamp_word(a0 + 16, lo, hi)) : make_uint4(0u, 0u, 0u, 0u);
+    const bool q2 = (s & 8u) != 0, q1 = (s & 4u) != 0;
+    const uint32_t a_0 = q2 ? v0.z : v0.x, a_1 = q2 ? v0.w : v0.y, a_2 = q2 ? v1.x : v0.z, a_3 = q2 ? v1.y : v0.w;
+    const uint32_t a_4 = q2 ? v1.z : v1.x, a_5 = q2 ? v1.w : v1.y;
+    const uint32_t x[5] = {q1 ? a_1 : a_0, q1 ? a_2 : a_1, q1 ? a_3 : a_2, q1 ? a_4 : a_3, q1 ? a_5 : a_4};
+    const uint32_t sh = (s & 3u) * 8u;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) t[k] = __funnelshift_r(x[k], x[k + 1], sh);
+}
+
 __device__ __forceinline__ void load_lut(uint8_t *lut_smem, const LutParam &p) {
     if (threadIdx.x < 64) reinterpret_cast<uint32_t *>(lut_smem)[threadIdx.x] = p.w[threadIdx.x];
 }

@@ -81,25 +81,6 @@ __device__ __forceinline__ bool rc_flip(int64_t r, int64_t n, const RcParam &p) 
     return x.c[0] < p.gate;
 }
 
-__device__ __forceinline__ uintptr_t clamp_word(uintptr_t a, uintptr_t lo, uintptr_t hi) { return a < lo ? lo : (a > hi ? hi : a); }
-
-// The 16 bytes at address X (any alignment) as four little-endian words, from the aligned words at X & ~15 and the next
-// one, each clamped to [lo, hi] (16-byte aligned).  The shift varies from row to row in flipped rows, so the words are
-// picked with selects.
-__device__ __forceinline__ void rc_fetch16(uintptr_t X, uintptr_t lo, uintptr_t hi, uint32_t t[4]) {
-    const uintptr_t a0 = X & ~uintptr_t(15);
-    const uint32_t s = static_cast<uint32_t>(X) & 15u;
-    const uint4 v0 = ldg16(clamp_word(a0, lo, hi));
-    const uint4 v1 = s != 0 ? ldg16(clamp_word(a0 + 16, lo, hi)) : make_uint4(0u, 0u, 0u, 0u);
-    const bool q2 = (s & 8u) != 0, q1 = (s & 4u) != 0;
-    const uint32_t a_0 = q2 ? v0.z : v0.x, a_1 = q2 ? v0.w : v0.y, a_2 = q2 ? v1.x : v0.z, a_3 = q2 ? v1.y : v0.w;
-    const uint32_t a_4 = q2 ? v1.z : v1.x, a_5 = q2 ? v1.w : v1.y;
-    const uint32_t x[5] = {q1 ? a_1 : a_0, q1 ? a_2 : a_1, q1 ? a_3 : a_2, q1 ? a_4 : a_3, q1 ? a_5 : a_4};
-    const uint32_t sh = (s & 3u) * 8u;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) t[k] = __funnelshift_r(x[k], x[k + 1], sh);
-}
-
 struct RcBatch {
     const uint8_t *bytes;
     const uint8_t *comp;  // complement table in shared memory
@@ -124,7 +105,7 @@ __device__ __forceinline__ void rc_vector(int64_t q, int64_t r, const RcBatch &b
             // mirror the 16 source bytes that end at s + e - 1 + sb - q
             const bool flip = flip_of(r);
             uint32_t t[4];
-            rc_fetch16(base + static_cast<uintptr_t>(flip ? s + e - 16 + sb - q : q + sb), lo, hi, t);
+            fetch16_clamped(base + static_cast<uintptr_t>(flip ? s + e - 16 + sb - q : q + sb), lo, hi, t);
             if (flip) {
                 const uint32_t w0 = t[0], w1 = t[1];
                 t[0] = translate4(__byte_perm(t[3], 0u, 0x0123), b.comp);

@@ -1,0 +1,565 @@
+// K13: sliding-window tiling of a packed batch and per-residue stitching of model outputs (sm_100a).
+//
+// Semantics (include/bsq.h, bsq_tile / bsq_untile_mean): sequence i of len_i residues gives m_i windows of at most W
+// residues starting every S residues (W >= S >= 1); the tail mode decides the last one.  Everything about one sequence's
+// windows -- count, starts, lengths, byte total -- is the arithmetic of tile_count / tile_start / tile_len below, the only
+// statement of the rule in the library (host extent, device extent and both kernels use it).
+//
+// K13a, bsq_tile (no state between launches, capturable into a CUDA graph):
+//   row_scan_kernel x2  (+ row_carry_kernel x2 past 1024 sequences, bsq_kernels.cuh) the per-sequence window counts into
+//                       seq_ptr, and the per-sequence output byte totals (closed form: (m - 1) W + len_last for SHORT,
+//                       m W otherwise) into byte_ptr.  byte_ptr, and seq_ptr when the caller passes none, live in
+//                       stream-ordered scratch (cudaMallocAsync / cudaFreeAsync on the call's stream).
+//   tile_fix_kernel     one thread per sequence adds the carry of its scan CTA to both entries (as K9's gather does).
+//   tile_gather_kernel  a grid-stride pass over the windows writes out_offsets, seq_index and starts (a binary search of
+//                       seq_ptr per window), then the bytes: a flat map over the 16-byte aligned output vectors in tiles
+//                       of 64 KiB on a persistent grid.  Per tile the CTA finds the tile's first sequence with K12's
+//                       256-ary search over byte_ptr and stages the tile's byte_ptr entries in shared memory (over-full
+//                       tiles search global memory).  Per vector a binary search of that table gives the sequence, and a
+//                       FastDiv by W the window (every window but a sequence's last is exactly W bytes of output).  Each
+//                       window piece the vector touches is two aligned ld.global.nc loads of its source, realigned with
+//                       funnel shifts and merged in with a byte mask; a vector inside the output leaves as one 16-byte
+//                       store, the at most two partial vectors at the ends of the output (any alignment) as byte stores.
+//   With S < W, overlapping windows re-read their shared source bytes; those re-reads hit L2 (a tile's source span is
+//   about 64 KiB * S / W + W bytes).
+//
+// K13b, bsq_untile_mean: one thread per (residue, channel vector): the residue's sequence by a binary search of the
+// source offsets, then the covering windows by arithmetic -- j from ceil((p - W + 1) / S) to floor(p / S), and END's last
+// window -- strand 0 before strand 1, ascending within a strand; a float32 sum divided by the count (NaN for none).
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+#include <cuda_runtime.h>
+
+#include <algorithm>
+#include <cmath>
+#include <string>
+#include <type_traits>
+
+#include "bsq_internal.h"
+#include "bsq_kernels.cuh"
+
+namespace bsq {
+
+namespace {
+
+struct TileShape {
+    int64_t W, S;
+    int tail;
+};
+
+// windows of a sequence of len >= 0 residues
+__host__ __device__ __forceinline__ int64_t tile_count(int64_t len, const TileShape &t) {
+    if (len <= t.W) return 1;
+    const int64_t d = len - t.W;
+    return (t.tail == BSQ_TILE_DROP ? d : d + t.S - 1) / t.S + 1;
+}
+// output bytes of those windows (I: int64_t in the kernels, whose totals are validated; __int128 in the extents)
+template <typename I>
+__host__ __device__ __forceinline__ I tile_bytes(int64_t len, int64_t m, const TileShape &t) {
+    if (len <= t.W) return static_cast<I>(len);
+    if (t.tail == BSQ_TILE_SHORT) return static_cast<I>(m - 1) * t.W + (len - (m - 1) * t.S);
+    return static_cast<I>(m) * t.W;
+}
+__host__ __device__ __forceinline__ int64_t tile_start(int64_t j, int64_t m, int64_t len, const TileShape &t) {
+    return (t.tail == BSQ_TILE_END && j == m - 1 && len > t.W) ? len - t.W : j * t.S;
+}
+__host__ __device__ __forceinline__ int64_t tile_len(int64_t j, int64_t len, const TileShape &t) {
+    if (len <= t.W) return len;
+    return t.tail == BSQ_TILE_SHORT ? min(t.W, len - j * t.S) : t.W;
+}
+
+struct WinCount {
+    TileShape t;
+    __device__ __forceinline__ int64_t operator()(int64_t len) const { return tile_count(len, t); }
+};
+struct ByteCount {
+    TileShape t;
+    __device__ __forceinline__ int64_t operator()(int64_t len) const { return tile_bytes<int64_t>(len, tile_count(len, t), t); }
+};
+
+// the scan entries that are not the last of their scan CTA get that CTA's carry (the last ones are final already and are
+// only read here, so no thread reads an entry another thread writes)
+__global__ void tile_fix_kernel(int64_t n, int64_t *__restrict__ seq_ptr, int64_t *__restrict__ byte_ptr) {
+    const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int64_t e = i + 1, blk = i / kRowScan;
+    if ((e % kRowScan) == 0 || e == n || blk == 0) return;
+    seq_ptr[e] += seq_ptr[blk * kRowScan];
+    byte_ptr[e] += byte_ptr[blk * kRowScan];
+}
+
+constexpr int kTThreads = 256;
+constexpr int kTVecs = 16;                  // output vectors per thread and tile
+constexpr int kTTile = kTThreads * kTVecs;  // 4096 vectors: 64 KiB of output per tile
+constexpr int kTRowCap = 2048;              // sequences a tile's table holds
+constexpr int kTMinBlocks = 4;
+
+struct TileArgs {
+    const uint8_t *bytes;
+    const int64_t *offs;
+    const int64_t *seq_ptr;
+    const int64_t *byte_ptr;
+    int64_t n, total;
+    TileShape t;
+    FastDiv wdiv;  // W, when W < 2^31
+};
+
+__device__ __forceinline__ int64_t div_w(int64_t x, const TileArgs &a) {
+    return (x < (int64_t(1) << 31) && a.t.W < (int64_t(1) << 31)) ? static_cast<int64_t>(fd_div(static_cast<uint32_t>(x), a.wdiv))
+                                                                   : x / a.t.W;
+}
+
+// Output bytes [q, q + 16) (out + q is 16-byte aligned), whose first byte in [0, total) lies in sequence i.
+// base_of(i) is byte_ptr[i] (from the tile's table or global memory).
+template <typename BASE>
+__device__ __forceinline__ void tile_vector(int64_t q, int64_t i, const TileArgs &a, const BASE &base_of, uint8_t *dst) {
+    uint32_t res[4] = {0u, 0u, 0u, 0u};
+    const uintptr_t src0 = reinterpret_cast<uintptr_t>(a.bytes);
+    int64_t b = base_of(i);
+    const int64_t x = max(q, int64_t(0));
+    for (;;) {
+        const int64_t be = base_of(i + 1);
+        if (be > b) {  // (an empty sequence has no bytes)
+            const int64_t s = __ldg(a.offs + i), len = __ldg(a.offs + i + 1) - s;
+            const int64_t m = tile_count(len, a.t);
+            int64_t j = div_w(max(x, b) - b, a);
+            for (; j < m; ++j) {
+                const int64_t ws = b + j * a.t.W;  // the window's first output byte
+                if (ws >= q + 16) break;
+                const int64_t wl = tile_len(j, len, a.t);
+                const int64_t src = s + tile_start(j, m, len, a.t);  // its first source byte
+                const uintptr_t lo = (src0 + static_cast<uintptr_t>(src)) & ~uintptr_t(15);
+                const uintptr_t hi = (src0 + static_cast<uintptr_t>(src + wl - 1)) & ~uintptr_t(15);
+                uint32_t t[4];
+                fetch16_clamped(src0 + static_cast<uintptr_t>(src + (q - ws)), lo, hi, t);
+                const int k0 = static_cast<int>(min(max(ws - q, int64_t(0)), int64_t(16)));
+                const int k1 = static_cast<int>(min(max(ws + wl - q, int64_t(0)), int64_t(16)));
+#pragma unroll
+                for (int w = 0; w < 4; ++w) {
+                    const uint32_t mk = lt_mask(k1, w) & ~lt_mask(k0, w);
+                    res[w] = (res[w] & ~mk) | (t[w] & mk);
+                }
+            }
+        }
+        if (be >= q + 16 || i + 1 >= a.n) break;
+        ++i;
+        b = be;
+    }
+    if (q >= 0 && q + 16 <= a.total) {
+        __stcs(reinterpret_cast<uint4 *>(dst), make_uint4(res[0], res[1], res[2], res[3]));
+    } else {
+#pragma unroll
+        for (int k = 0; k < 16; ++k)
+            if (q + k >= 0 && q + k < a.total) dst[k] = static_cast<uint8_t>(res[k >> 2] >> (8 * (k & 3)));
+    }
+}
+
+__global__ void __launch_bounds__(kTThreads, kTMinBlocks)
+tile_gather_kernel(TileArgs a, uint8_t *__restrict__ out, int64_t *__restrict__ out_offs, int64_t *__restrict__ seq_index,
+                   int64_t *__restrict__ starts) {
+    __shared__ int64_t tab[kTRowCap];  // byte_ptr of sequences i0, i0 + 1, ...
+    const int tid = threadIdx.x;
+    a.total = __ldg(a.byte_ptr + a.n);
+    // window table: out_offsets, seq_index, starts
+    const int64_t M = __ldg(a.seq_ptr + a.n);
+    for (int64_t w = blockIdx.x * static_cast<int64_t>(kTThreads) + tid; w <= M; w += static_cast<int64_t>(gridDim.x) * kTThreads) {
+        if (w == M) {
+            out_offs[M] = a.total;
+            break;
+        }
+        int64_t lo = 0, hi = a.n;  // the largest i with seq_ptr[i] <= w
+        while (hi - lo > 1) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (__ldg(a.seq_ptr + mid) <= w) lo = mid;
+            else hi = mid;
+        }
+        const int64_t j = w - __ldg(a.seq_ptr + lo);
+        out_offs[w] = __ldg(a.byte_ptr + lo) + j * a.t.W;
+        if (seq_index != nullptr) seq_index[w] = lo;
+        if (starts != nullptr) {
+            const int64_t len = __ldg(a.offs + lo + 1) - __ldg(a.offs + lo);
+            starts[w] = tile_start(j, tile_count(len, a.t), len, a.t);
+        }
+    }
+    const int al = static_cast<int>(reinterpret_cast<uintptr_t>(out) & 15u);  // out - al is 16-byte aligned
+    const int64_t nvec = a.total > 0 ? (a.total - 1 + al) / 16 + 1 : 0;      // vector v holds bytes [16v - al, 16v - al + 16)
+    const int64_t ntiles = (nvec + kTTile - 1) / kTTile;
+    auto base_g = [&](int64_t i) { return __ldg(a.byte_ptr + i); };
+    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        const int64_t v0 = tile * kTTile;
+        const int64_t p0 = max(16 * v0 - al, int64_t(0)), p1 = min(16 * (v0 + kTTile) - al, a.total);
+        // 1. first sequence: the largest i in [0, n) with byte_ptr[i] <= p0
+        int64_t lo = 0, hi = a.n;
+        while (hi - lo > 1) {
+            const int64_t w = hi - lo;
+            const int64_t pr = lo + (static_cast<int64_t>(tid) + 1) * w / (kTThreads + 1);
+            const int cnt = __syncthreads_count(base_g(pr) <= p0);
+            const int64_t nlo = cnt > 0 ? lo + static_cast<int64_t>(cnt) * w / (kTThreads + 1) : lo;
+            const int64_t nhi = cnt < kTThreads ? lo + (static_cast<int64_t>(cnt) + 1) * w / (kTThreads + 1) : hi;
+            lo = nlo;
+            hi = nhi;
+        }
+        const int64_t i0 = lo;
+        // 2. table up to the first sequence that starts at or after the tile's end (byte_ptr[n] = total >= p1 closes it)
+        int nrows = -1;
+        for (int base = 0; base < kTRowCap; base += kTThreads) {
+            const int j = base + tid;
+            const int64_t i = i0 + j;
+            bool past = true;
+            if (i <= a.n) {
+                const int64_t s = base_g(i);
+                tab[j] = s;
+                past = s >= p1;
+            }
+            const int cnt = __syncthreads_count(past);
+            if (cnt > 0) {
+                nrows = base + kTThreads - cnt;
+                break;
+            }
+        }
+        for (int k = 0; k < kTVecs; ++k) {
+            const int64_t v = v0 + k * kTThreads + tid;
+            if (v >= nvec) break;
+            const int64_t q = 16 * v - al, x = max(q, int64_t(0));
+            if (nrows > 0) {
+                int l = 0, h = nrows;  // the largest j < nrows with tab[j] <= x
+                while (h - l > 1) {
+                    const int mid = (l + h) >> 1;
+                    if (tab[mid] <= x) l = mid;
+                    else h = mid;
+                }
+                const int64_t r0 = i0;
+                tile_vector(q, i0 + l, a, [&](int64_t i) { return i - r0 <= nrows ? tab[i - r0] : base_g(i); }, out + q);
+            } else {
+                int64_t l = i0, h = a.n;
+                while (h - l > 1) {
+                    const int64_t mid = (l + h) >> 1;
+                    if (base_g(mid) <= x) l = mid;
+                    else h = mid;
+                }
+                tile_vector(q, l, a, base_g, out + q);
+            }
+        }
+        __syncthreads();  // the table is refilled by the next tile
+    }
+}
+
+// ---- K13b -------------------------------------------------------------------------------------------------------------
+
+struct UntileArgs {
+    const void *y;
+    const int32_t *cu;   // per-window first row, or nullptr: w * stride
+    int64_t stride, col0, C;
+    const int64_t *offs;  // source offsets
+    int64_t n;
+    const int64_t *seq_ptr;
+    int64_t nwin;
+    int strands;
+    const uint8_t *flipped;
+    TileShape t;
+    int64_t nc;  // channel vectors per row
+    FastDiv ncdiv;
+};
+
+template <typename T>
+__device__ __forceinline__ float to_f32(T v);
+template <>
+__device__ __forceinline__ float to_f32<float>(float v) { return v; }
+template <>
+__device__ __forceinline__ float to_f32<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <>
+__device__ __forceinline__ float to_f32<__half>(__half v) { return __half2float(v); }
+
+// V consecutive elements of type T (V * sizeof(T) is 4, 8 or 16 bytes with V > 1: one load, aligned by the host's checks)
+template <typename T, int V>
+__device__ __forceinline__ void load_v(const T *p, float f[V]) {
+    if constexpr (V == 1) {
+        f[0] = to_f32<T>(p[0]);
+    } else {
+        constexpr int kBytes = V * sizeof(T);
+        using L = typename std::conditional<kBytes == 16, uint4, typename std::conditional<kBytes == 8, uint2, uint32_t>::type>::type;
+        const L raw = __ldg(reinterpret_cast<const L *>(p));
+        const T *e = reinterpret_cast<const T *>(&raw);
+#pragma unroll
+        for (int k = 0; k < V; ++k) f[k] = to_f32<T>(e[k]);
+    }
+}
+
+template <typename T, int V>
+__global__ void __launch_bounds__(256) untile_kernel(UntileArgs a, float *__restrict__ out) {
+    const int64_t R = __ldg(a.offs + a.n) - __ldg(a.offs);
+    const int64_t items = R * a.nc;
+    const int64_t M = a.nwin;
+    for (int64_t it = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; it < items;
+         it += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int64_t row = it < (int64_t(1) << 31) ? static_cast<int64_t>(fd_div(static_cast<uint32_t>(it), a.ncdiv)) : it / a.nc;
+        const int64_t c = (it - row * a.nc) * V;
+        const int64_t gpos = row + __ldg(a.offs);
+        int64_t lo = 0, hi = a.n;  // the largest i with offs[i] <= gpos (the first of equal offsets is an empty sequence)
+        while (hi - lo > 1) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (__ldg(a.offs + mid) <= gpos) lo = mid;
+            else hi = mid;
+        }
+        const int64_t s = __ldg(a.offs + lo), len = __ldg(a.offs + lo + 1) - s, p = gpos - s;
+        const int64_t m = tile_count(len, a.t), w0 = __ldg(a.seq_ptr + lo);
+        // regular windows (all but END's last) cover p for j in [jlo, jhi]
+        const int64_t mreg = (a.t.tail == BSQ_TILE_END && len > a.t.W) ? m - 1 : m;
+        const int64_t jlo = p >= a.t.W ? (p - a.t.W) / a.t.S + 1 : 0;
+        const int64_t jhi = min(p / a.t.S, mreg - 1);
+        const bool last = mreg < m && p >= len - a.t.W;  // END's last window
+        float acc[V];
+#pragma unroll
+        for (int k = 0; k < V; ++k) acc[k] = 0.0f;
+        int cnt = 0;
+        for (int strand = 0; strand < a.strands; ++strand) {
+            auto add = [&](int64_t j) {
+                const int64_t w = w0 + j + strand * M;
+                const int64_t st = tile_start(j, m, len, a.t), wl = tile_len(j, len, a.t);
+                const bool fl = a.flipped != nullptr && a.flipped[w] != 0;
+                const int64_t tpos = fl ? wl - 1 - (p - st) : p - st;
+                const int64_t yrow = (a.cu != nullptr ? __ldg(a.cu + w) : w * a.stride) + a.col0 + tpos;
+                float f[V];
+                load_v<T, V>(static_cast<const T *>(a.y) + yrow * a.C + c, f);
+#pragma unroll
+                for (int k = 0; k < V; ++k) acc[k] += f[k];
+                ++cnt;
+            };
+            for (int64_t j = jlo; j <= jhi; ++j) add(j);
+            if (last) add(m - 1);
+        }
+        float *o = out + row * a.C + c;
+#pragma unroll
+        for (int k = 0; k < V; ++k) o[k] = cnt > 0 ? acc[k] / static_cast<float>(cnt) : __int_as_float(0x7fc00000);
+    }
+}
+
+// a persistent grid: the row count lives on the device, and the kernel strides over whatever it is
+template <typename T, int V>
+int launch_untile(cudaStream_t st, const UntileArgs &a, float *out) {
+    untile_kernel<T, V><<<cur_sms() * 8, 256, 0, st>>>(a, out);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    return BSQ_OK;
+}
+
+int check_shape(int64_t W, int64_t S, int tail) {
+    if (W < 1) return fail(BSQ_ERR_ARG, "window must be >= 1, got " + std::to_string(W));
+    if (S < 1 || S > W) return fail(BSQ_ERR_ARG, "stride must lie in 1..window = " + std::to_string(W) + ", got " + std::to_string(S));
+    if (tail != BSQ_TILE_SHORT && tail != BSQ_TILE_END && tail != BSQ_TILE_DROP)
+        return fail(BSQ_ERR_ARG, "tail must be BSQ_TILE_SHORT, BSQ_TILE_END or BSQ_TILE_DROP");
+    return BSQ_OK;
+}
+
+constexpr __int128 kI64Max = (__int128(1) << 63) - 1;
+
+// the bsq_tile_extent_device reduction: validation bits in out[0] (1: negative length, 2: offsets[0] < 0, 4: past nbytes,
+// 8: a total past INT64_MAX), sum m in out[1], sum bytes in out[2], max window length in out[3]
+__device__ __forceinline__ void sat_add(unsigned long long *p, unsigned long long v, unsigned *bad) {
+    unsigned long long old = *reinterpret_cast<volatile unsigned long long *>(p), assumed;
+    do {
+        assumed = old;
+        unsigned long long nv = assumed + v;  // both <= INT64_MAX: no wrap
+        if (nv > static_cast<unsigned long long>(kI64Max)) {
+            nv = static_cast<unsigned long long>(kI64Max);
+            *bad |= 8u;
+        }
+        old = atomicCAS(p, assumed, nv);
+    } while (old != assumed);
+}
+
+__global__ void tile_extent_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, TileShape t,
+                                   unsigned long long *out) {
+    unsigned long long wins = 0, byts = 0;
+    long long best = 0;
+    unsigned bad = 0;
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int64_t a = offs[i], b = offs[i + 1];
+        if (b < a) bad |= 1u;
+        if (i == 0 && a < 0) bad |= 2u;
+        if (i == nseq - 1 && nbytes >= 0 && b > nbytes) bad |= 4u;
+        const __int128 len128 = static_cast<__int128>(b) - a;
+        if (len128 < 0 || len128 > kI64Max) continue;
+        const int64_t len = static_cast<int64_t>(len128);
+        const int64_t m = tile_count(len, t);
+        const __int128 nb = tile_bytes<__int128>(len, m, t);
+        const __int128 sw = static_cast<__int128>(wins) + m, sb = static_cast<__int128>(byts) + nb;
+        if (sw > kI64Max || sb > kI64Max) bad |= 8u;
+        wins = static_cast<unsigned long long>(sw > kI64Max ? kI64Max : sw);
+        byts = static_cast<unsigned long long>(sb > kI64Max ? kI64Max : sb);
+        best = max(best, static_cast<long long>(min(len, t.W)));
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
+        const unsigned long long w2 = __shfl_xor_sync(0xffffffffu, wins, o), b2 = __shfl_xor_sync(0xffffffffu, byts, o);
+        if (wins + w2 > static_cast<unsigned long long>(kI64Max) || byts + b2 > static_cast<unsigned long long>(kI64Max)) bad |= 8u;
+        wins = min(wins + w2, static_cast<unsigned long long>(kI64Max));
+        byts = min(byts + b2, static_cast<unsigned long long>(kI64Max));
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (wins > 0) sat_add(out + 1, wins, &bad);
+        if (byts > 0) sat_add(out + 2, byts, &bad);
+        if (best > 0) atomicMax(out + 3, static_cast<unsigned long long>(best));
+    }
+    bad = __reduce_or_sync(0xffffffffu, bad);
+    if ((threadIdx.x & 31) == 0 && bad) atomicOr(out, static_cast<unsigned long long>(bad));
+}
+
+}  // namespace
+
+}  // namespace bsq
+
+using namespace bsq;
+
+extern "C" int bsq_tile_extent_host(const int64_t *h_offsets, int64_t nseq, int64_t window, int64_t stride, int tail, int64_t *nwin,
+                                    int64_t *nbytes, int64_t *max_len) {
+    if (int rc = check_shape(window, stride, tail)) return rc;
+    if (nwin == nullptr || nbytes == nullptr || max_len == nullptr) return fail(BSQ_ERR_ARG, "null output");
+    if (nseq < 0 || (nseq > 0 && h_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
+    *nwin = *nbytes = *max_len = 0;
+    if (nseq == 0) return BSQ_OK;
+    if (h_offsets[0] < 0) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
+    const TileShape t{window, stride, tail};
+    __int128 sw = 0, sb = 0;
+    int64_t best = 0;
+    for (int64_t i = 0; i < nseq; ++i) {
+        const int64_t len = h_offsets[i + 1] - h_offsets[i];  // (both in [0, INT64_MAX]: no overflow)
+        if (len < 0) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
+        const int64_t m = tile_count(len, t);
+        sw += m;
+        sb += tile_bytes<__int128>(len, m, t);
+        if (sw > kI64Max || sb > kI64Max) return fail(BSQ_ERR_ARG, "the windows' count or bytes exceed INT64_MAX");
+        best = std::max(best, std::min(len, window));
+    }
+    *nwin = static_cast<int64_t>(sw);
+    *nbytes = static_cast<int64_t>(sb);
+    *max_len = best;
+    return BSQ_OK;
+}
+
+extern "C" int bsq_tile_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, int64_t window,
+                                      int64_t stride, int tail, int64_t *nwin, int64_t *out_nbytes, int64_t *max_len) {
+    bsq::DeviceRestore restore_device;
+    if (int rc = check_shape(window, stride, tail)) return rc;
+    if (nwin == nullptr || out_nbytes == nullptr || max_len == nullptr) return fail(BSQ_ERR_ARG, "null output");
+    if (nseq < 0 || (nseq > 0 && d_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
+    *nwin = *out_nbytes = *max_len = 0;
+    if (nseq == 0) return BSQ_OK;
+    BSQ_CUDA_TRY(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    unsigned long long *d_res = nullptr, h_res[4] = {0, 0, 0, 0};
+    BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&d_res), sizeof(h_res), st));
+    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, sizeof(h_res), st));
+    const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
+    tile_extent_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, TileShape{window, stride, tail}, d_res);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, sizeof(h_res), cudaMemcpyDeviceToHost, st));
+    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
+    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
+    if (h_res[0] & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
+    if (h_res[0] & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
+    if (h_res[0] & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
+    if (h_res[0] & 8u) return fail(BSQ_ERR_ARG, "the windows' count or bytes exceed INT64_MAX");
+    *nwin = static_cast<int64_t>(h_res[1]);
+    *out_nbytes = static_cast<int64_t>(h_res[2]);
+    *max_len = static_cast<int64_t>(h_res[3]);
+    return BSQ_OK;
+}
+
+extern "C" int bsq_tile(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq, int64_t window,
+                        int64_t stride, int tail, uint8_t *d_out_bytes, int64_t *d_out_offsets, int64_t *d_seq_ptr,
+                        int64_t *d_seq_index, int64_t *d_starts) {
+    bsq::DeviceRestore restore_device;
+    if (int rc = check_shape(window, stride, tail)) return rc;
+    if (nseq < 0) return fail(BSQ_ERR_ARG, "negative batch size");
+    if (d_out_offsets == nullptr) return fail(BSQ_ERR_ARG, "null output offsets");
+    if (nseq > 0 && (d_bytes == nullptr || d_offsets == nullptr || d_out_bytes == nullptr))
+        return fail(BSQ_ERR_ARG, "null bytes, offsets or output bytes");
+    BSQ_CUDA_TRY(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (nseq == 0) {
+        BSQ_CUDA_TRY(cudaMemsetAsync(d_out_offsets, 0, sizeof(int64_t), st));
+        if (d_seq_ptr != nullptr) BSQ_CUDA_TRY(cudaMemsetAsync(d_seq_ptr, 0, sizeof(int64_t), st));
+        return BSQ_OK;
+    }
+    const TileShape t{window, stride, tail};
+    int64_t *scratch = nullptr;
+    const size_t ns = static_cast<size_t>(nseq + 1) * (d_seq_ptr != nullptr ? 1 : 2);
+    BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&scratch), ns * sizeof(int64_t), st));
+    int64_t *byte_ptr = scratch, *seq_ptr = d_seq_ptr != nullptr ? d_seq_ptr : scratch + nseq + 1;
+    const int64_t nblocks = (nseq + kRowScan - 1) / kRowScan;
+    row_scan_kernel<<<static_cast<unsigned>(nblocks), kRowScan, 0, st>>>(d_offsets, nseq, WinCount{t}, seq_ptr);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    row_scan_kernel<<<static_cast<unsigned>(nblocks), kRowScan, 0, st>>>(d_offsets, nseq, ByteCount{t}, byte_ptr);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    if (nblocks > 1) {
+        row_carry_kernel<<<1, kRowScan, 0, st>>>(seq_ptr, nseq, nblocks);
+        count_launch();
+        BSQ_CUDA_TRY(cudaGetLastError());
+        row_carry_kernel<<<1, kRowScan, 0, st>>>(byte_ptr, nseq, nblocks);
+        count_launch();
+        BSQ_CUDA_TRY(cudaGetLastError());
+        tile_fix_kernel<<<static_cast<unsigned>((nseq + 255) / 256), 256, 0, st>>>(nseq, seq_ptr, byte_ptr);
+        count_launch();
+        BSQ_CUDA_TRY(cudaGetLastError());
+    }
+    TileArgs a;
+    a.bytes = d_bytes;
+    a.offs = d_offsets;
+    a.seq_ptr = seq_ptr;
+    a.byte_ptr = byte_ptr;
+    a.n = nseq;
+    a.total = 0;  // (byte_ptr[n]: read by the kernel)
+    a.t = t;
+    a.wdiv = make_fastdiv(static_cast<uint32_t>(std::min<int64_t>(window, (int64_t(1) << 31) - 1)));
+    tile_gather_kernel<<<cur_sms() * kTMinBlocks, kTThreads, 0, st>>>(a, d_out_bytes, d_out_offsets, d_seq_index, d_starts);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    BSQ_CUDA_TRY(cudaFreeAsync(scratch, st));
+    return BSQ_OK;
+}
+
+extern "C" int bsq_untile_mean(int device, void *stream, int dtype, const void *d_y, int64_t channels, int64_t row_stride,
+                               const int32_t *d_cu, int64_t col0, const int64_t *d_src_offsets, int64_t nseq, int64_t window,
+                               int64_t stride, int tail, const int64_t *d_seq_ptr, int64_t nwin, int strands,
+                               const uint8_t *d_flipped, float *d_out) {
+    bsq::DeviceRestore restore_device;
+    if (int rc = check_shape(window, stride, tail)) return rc;
+    if (dtype != BSQ_UNTILE_F32 && dtype != BSQ_UNTILE_BF16 && dtype != BSQ_UNTILE_F16)
+        return fail(BSQ_ERR_ARG, "dtype must be BSQ_UNTILE_F32, BSQ_UNTILE_BF16 or BSQ_UNTILE_F16");
+    if (channels < 1) return fail(BSQ_ERR_ARG, "channels must be >= 1");
+    if (col0 < 0) return fail(BSQ_ERR_ARG, "col0 must be >= 0");
+    if (strands != 1 && strands != 2) return fail(BSQ_ERR_ARG, "strands must be 1 or 2");
+    if (nseq < 0 || nwin < nseq) return fail(BSQ_ERR_ARG, "negative batch size, or fewer windows than sequences");
+    if (d_cu == nullptr && row_stride <= col0) return fail(BSQ_ERR_ARG, "row_stride must exceed col0 without cu_seqlens");
+    if (nseq == 0) return BSQ_OK;
+    if (d_y == nullptr || d_src_offsets == nullptr || d_seq_ptr == nullptr || d_out == nullptr)
+        return fail(BSQ_ERR_ARG, "null values, offsets, seq_ptr or output");
+    const size_t es = dtype == BSQ_UNTILE_F32 ? 4 : 2;
+    UntileArgs a;
+    a.y = d_y;
+    a.cu = d_cu;
+    a.stride = row_stride;
+    a.col0 = col0;
+    a.C = channels;
+    a.offs = d_src_offsets;
+    a.n = nseq;
+    a.seq_ptr = d_seq_ptr;
+    a.nwin = nwin;
+    a.strands = strands;
+    a.flipped = d_flipped;
+    a.t = TileShape{window, stride, tail};
+    // channel vectors: 16 bytes of input when every row and both pointers allow it, else one element
+    const bool al16 = ((reinterpret_cast<uintptr_t>(d_y) | reinterpret_cast<uintptr_t>(d_out)) & 15u) == 0;
+    const int V = (al16 && (channels * static_cast<int64_t>(es)) % 16 == 0) ? static_cast<int>(16 / es) : 1;
+    a.nc = channels / V;
+    a.ncdiv = make_fastdiv(static_cast<uint32_t>(std::min<int64_t>(a.nc, (int64_t(1) << 31) - 1)));
+    BSQ_CUDA_TRY(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (dtype == BSQ_UNTILE_F32) return V == 4 ? launch_untile<float, 4>(st, a, d_out) : launch_untile<float, 1>(st, a, d_out);
+    if (dtype == BSQ_UNTILE_BF16) return V == 8 ? launch_untile<__nv_bfloat16, 8>(st, a, d_out) : launch_untile<__nv_bfloat16, 1>(st, a, d_out);
+    return V == 8 ? launch_untile<__half, 8>(st, a, d_out) : launch_untile<__half, 1>(st, a, d_out);
+}

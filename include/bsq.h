@@ -263,6 +263,77 @@ int bsq_revcomp(int device, void *stream, const uint8_t *d_bytes, const int64_t 
 /* Host only, no device call: out[b] = comp[b] for every byte value b.  BSQ_ERR_ARG for a NULL out. */
 int bsq_revcomp_table(uint8_t out[256]);
 
+/* Sliding-window tiling (inference over whole long sequences, dataset construction by chunking -- HF's
+ * return_overflowing_tokens=True with stride=): a packed batch in, a packed batch of all its windows out, which every
+ * entry point above then takes unchanged, with the maps that connect the two.  Nothing is drawn at random: the windows
+ * depend only on (len_i, W, S, tail).
+ * Let W = window >= 1, S = stride with 1 <= S <= W, len_i = offsets[i+1] - offsets[i] and tail one of BSQ_TILE_*:
+ *   - len_i <= W (0 included): one window, the whole sequence (start 0, length len_i), under every tail.  An empty
+ *     sequence gives one empty window, so every sequence has at least one window.
+ *   - len_i > W:
+ *       SHORT  m_i = ceil((len_i - W) / S) + 1 windows; window j starts at j*S and has length min(W, len_i - j*S) (only
+ *              the last can be shorter than W);
+ *       END    the same m_i; windows j < m_i - 1 start at j*S, the last at len_i - W; every window is W long (the last
+ *              overlaps its predecessor by more than W - S; identical to SHORT when S divides len_i - W);
+ *       DROP   m_i = floor((len_i - W) / S) + 1 windows at j*S, all W long; the last len_i - ((m_i - 1)*S + W) residues
+ *              are in no window.
+ *   - Output order: the windows of sequence 0 by start, then those of sequence 1, ...; M = sum m_i.
+ *     seq_ptr[i] (int64, n + 1 entries, seq_ptr[0] = 0): index of sequence i's first window;
+ *     seq_index[w] (int64, M): the sequence of window w (HF's overflow_to_sample_mapping);
+ *     starts[w] (int64, M): where window w begins in its sequence;
+ *     out_offsets (int64, M + 1, from 0) and out_bytes[out_offsets[w] + t] = bytes[offsets[seq_index[w]] + starts[w] + t].
+ * Worked answers, W = 4, S = 3: "ACGTACGTACG" (11) -> SHORT starts 0, 3, 6, 9: ACGT, TACG, GTAC, CG; END 0, 3, 6, 7: ACGT,
+ * TACG, GTAC, TACG; DROP 0, 3, 6: ACGT, TACG, GTAC.  Length 5: SHORT (0, 4), (3, 2); END (0, 4), (1, 4); DROP (0, 4).
+ * Lengths 4 and 0: one window each, under every tail.
+ *
+ * bsq_tile_extent_host (no device call): *nwin = M, *nbytes = sum of the window lengths, *max_len = the longest window
+ * (all 0 for nseq == 0).  BSQ_ERR_ARG for W < 1, S < 1, S > W, a bad tail, NULL outputs, negative lengths, offsets[0] < 0,
+ * and a window count or byte total past INT64_MAX (the arithmetic does not overflow for any int64 lengths). */
+#define BSQ_TILE_SHORT 0
+#define BSQ_TILE_END 1
+#define BSQ_TILE_DROP 2
+int bsq_tile_extent_host(const int64_t *h_offsets, int64_t nseq, int64_t window, int64_t stride, int tail, int64_t *nwin,
+                         int64_t *nbytes, int64_t *max_len);
+/* The same for device-resident offsets, from one reduction kernel and one read-back (synchronises `stream`); it validates
+ * the offsets like bsq_crop_extent_device (BSQ_ERR_ARG: negative length, offsets[0] < 0, offsets[nseq] > nbytes when
+ * nbytes >= 0). */
+int bsq_tile_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, int64_t window,
+                           int64_t stride, int tail, int64_t *nwin, int64_t *out_nbytes, int64_t *max_len);
+/* bsq_tile enqueues only (nseq == 0: out_offsets[0] = 0 and seq_ptr[0] = 0 by 8-byte memsets), keeps no state between
+ * launches and is capturable into a CUDA graph.  Scratch: 8 (n + 1) bytes, 16 (n + 1) when d_seq_ptr is NULL, allocated
+ * and freed in stream order (cudaMallocAsync / cudaFreeAsync from the device's default memory pool).  The caller has
+ * validated the offsets (bsq_tile_extent_device does) and sized d_out_bytes (any alignment, not overlapping the input) to
+ * the extent's nbytes and d_out_offsets to nwin + 1 entries; d_seq_ptr (n + 1), d_seq_index and d_starts (nwin each) may
+ * be NULL.  BSQ_ERR_ARG, before any device call, for a bad W, S or tail, nseq < 0, a NULL d_out_offsets, or NULL bytes,
+ * offsets or output bytes with nseq > 0. */
+int bsq_tile(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq, int64_t window, int64_t stride,
+             int tail, uint8_t *d_out_bytes, int64_t *d_out_offsets, int64_t *d_seq_ptr, int64_t *d_seq_index, int64_t *d_starts);
+
+/* Stitching per-residue model outputs of the windows back onto the sequences: the mean over every covering window.
+ *   d_y: the outputs, C channels per position of element type dtype (BSQ_UNTILE_*), channels contiguous.  Window w's
+ *   residue t is row base_w + col0 + t of the 2-D (rows, C) view: base_w = w * row_stride for padded batch-first outputs
+ *   (M', P, C) (d_cu NULL, row_stride = P > col0), base_w = d_cu[w] for padding-free outputs (T, C) (d_cu: int32 window starts,
+ *   a padding-free token batch's cu_seqlens); col0 is the number of leading special tokens (BOS).
+ *   strands 1 or 2: with 2 (the layout BSQ_RC_BOTH makes), windows M .. 2M - 1 are windows 0 .. M - 1 again.
+ *   d_flipped (strands * M bytes, or NULL): windows that were reverse-complemented; in a flipped window of length l,
+ *   residue t is source position starts + l - 1 - t.
+ *   Output d_out: float32 (offsets[n] - offsets[0], C), row offsets[i] - offsets[0] + p for residue p of sequence i: the
+ *   sum over every covering window (of every strand) in float32 -- strand 0 before strand 1, windows in ascending order
+ *   within a strand -- divided by their count; a residue no window covers (DROP) gets a quiet NaN.  Channels are averaged
+ *   as they are (swapping strand-specific channels of a flipped window is the caller's business).
+ * Worked answer: "ACGTACGTACG", W = 4, S = 3, C = 1, every window reporting its index w at every position: SHORT gives
+ * [0, 0, 0, 0.5, 1, 1, 1.5, 2, 2, 2.5, 3], END [0, 0, 0, 0.5, 1, 1, 1.5, 2.5, 2.5, 2.5, 3], DROP [0, 0, 0, 0.5, 1, 1, 1.5,
+ * 2, 2, 2, NaN].
+ * Enqueues one kernel, keeps no state between launches and is capturable into a CUDA graph.  d_seq_ptr is bsq_tile's
+ * (n + 1 entries), nwin = M.  BSQ_ERR_ARG, before any device call, for a bad W, S, tail or dtype, C < 1, col0 < 0,
+ * strands not 1 or 2, nseq < 0, nwin < nseq, row_stride <= col0 without d_cu, or NULL pointers with nseq > 0. */
+#define BSQ_UNTILE_F32 0
+#define BSQ_UNTILE_BF16 1
+#define BSQ_UNTILE_F16 2
+int bsq_untile_mean(int device, void *stream, int dtype, const void *d_y, int64_t channels, int64_t row_stride, const int32_t *d_cu,
+                    int64_t col0, const int64_t *d_src_offsets, int64_t nseq, int64_t window, int64_t stride, int tail,
+                    const int64_t *d_seq_ptr, int64_t nwin, int strands, const uint8_t *d_flipped, float *d_out);
+
 /* Sequence packing (padding-free batches of a fixed shape: SDPA with a block-diagonal mask, position-id packing as in
  * HF's DataCollatorWithFlattening, CUDA graphs, torch.compile): whole sequences laid end to end in R rows of L tokens.
  * With k = bos + eos and the (already cropped) lengths len_i, sequence i occupies need_i = len_i + k tokens; every
