@@ -119,122 +119,143 @@ class _Resolved:
             self.ctx = None
 
 
-def _resolve(batch, device, augment=None, before_stage=None, crop=None, crop_extent=None, rc=None, validated=False):
-    """-> _Resolved.  Host batches are staged (and, with ``augment``, mutated on the device after the copy);
-    device batches are used in place (with ``augment``: a mutated clone).  ``before_stage(host_offsets, n)`` checks a
-    host batch before anything is copied to the device.
+_Batch = collections.namedtuple("_Batch", ["bytes", "offsets", "keep"])
 
-    ``crop`` (from ``_crop_spec``): the batch is cropped on the device after staging and the result describes the
-    cropped batch, with ``extent = (sum, max)`` of its lengths; ``augment`` then mutates the crop's fresh buffer in
-    place.  Host batches are sized from their host offsets (``before_stage`` sees the cropped offsets); device
-    batches pay one ``bsq_crop_extent_device`` (which also validates their offsets), unless the caller has read their
-    offsets back already and passes ``crop_extent``.
 
-    ``rc`` (from ``_rc_spec``): after the crop, the batch is flipped on the device into fresh buffers (``_apply_rc``).
-    Uncropped batches then also get ``extent``: host batches from their host offsets, device batches from one
-    ``bsq_crop_extent_device`` with no window (which validates their offsets), unless the caller has validated them
-    already (``crop_extent``, or ``validated`` when it needs no extent).  ``rc="both"`` doubles the batch:
-    ``before_stage`` and ``h_offs`` then see the doubled offsets."""
+def _parse(batch):
+    """-> _Batch: checked CUDA tensors (``offsets`` is a torch tensor), checked host numpy arrays (``keep``: the FlatFile
+    they view), or ``bytes`` None and ``offsets`` the items as ``bytes``, gathered when the batch is staged.  The
+    offsets of a CUDA batch are validated on the device, by the reduction that sizes or checks it."""
     torch = _torch()
-    r = _Resolved()
-    r.ctx, r.keep, r.h_offs, r.base, r.extent = None, [], None, 0, None
-    host_b = host_o = None
+    keep = None
     if isinstance(batch, tuple) and len(batch) == 3 and isinstance(batch[0], cbioseq.FlatFile):
-        ff, start, stop = batch
-        host_b, host_o = ff.packed(start, stop)
-        r.keep.append(ff)
+        keep = batch[0]
+        b, o = keep.packed(batch[1], batch[2])
     elif isinstance(batch, tuple) and len(batch) == 2 and hasattr(batch[0], "dtype"):
         b, o = batch
         if isinstance(b, torch.Tensor) and b.is_cuda:
             if not (isinstance(o, torch.Tensor) and o.is_cuda and o.device == b.device):
                 raise ValueError("bytes and offsets must live on the same side (all host or all CUDA)")
-            if b.dtype != torch.uint8 or o.dtype != torch.int64 or not b.is_contiguous() or not o.is_contiguous():
-                raise ValueError("packed batch: contiguous uint8 bytes and int64 offsets expected")
-            r.device = b.device.index
-            r.stream = torch.cuda.current_stream(r.device).cuda_stream
-            if crop is not None:
-                r.d_bytes, r.d_offs, r.nseq = b.data_ptr(), o.data_ptr(), o.numel() - 1
-                r.keep += [b, o]
-                r.extent = crop_extent if crop_extent is not None else capi.crop_extent_device(r.device, r.stream, o, r.nseq, crop[1],
-                                                                                                nbytes=b.numel())
-                _apply_crop(r, crop, augment)
-                _apply_rc(r, rc, r.extent[0])
-                return r
-            if rc is not None:
-                r.d_bytes, r.d_offs, r.nseq = b.data_ptr(), o.data_ptr(), o.numel() - 1
-                r.keep += [b, o]
-                if crop_extent is not None or not validated:
-                    r.extent = crop_extent if crop_extent is not None else capi.crop_extent_device(r.device, r.stream, o, r.nseq,
-                                                                                                    _UNCROPPED, nbytes=b.numel())
-                _apply_rc(r, rc, b.numel())
-                return r
-            if augment:
-                with torch.cuda.device(r.device):
-                    b = b.clone()  # never mutate the caller's residues
-            r.d_bytes, r.d_offs, r.nseq = b.data_ptr(), o.data_ptr(), o.numel() - 1
-            r.keep += [b, o]
-            if augment:
-                capi.augment_blosum62(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, *augment)
-            return r
-        host_b = b.numpy() if isinstance(b, torch.Tensor) else np.asarray(b)
-        host_o = o.numpy() if isinstance(o, torch.Tensor) else np.asarray(o)
-        if host_b.dtype != np.uint8 or host_o.dtype != np.int64 or not host_b.flags.c_contiguous or not host_o.flags.c_contiguous:
-            raise ValueError("packed batch: contiguous uint8 bytes and int64 offsets expected")
-    r.device = _resolve_device(device)
-    r.stream = torch.cuda.current_stream(r.device).cuda_stream
-    ctx = _device_ctx(r.device)
-    ctx.lock.acquire()
-    try:
-        if host_o is None:  # list of str / bytes / bytearray
-            if not isinstance(batch, (list, tuple)):
-                raise ValueError("item was none of string, bytes, or numpy array of 8-bit integers. ")
-            seqs = []
-            for s in batch:
-                if isinstance(s, str):
-                    s = s.encode("utf-8")
-                elif not isinstance(s, (bytes, bytearray)):
-                    raise ValueError("item was none of string, bytes, or numpy array of 8-bit integers. ")
-                seqs.append(s)
-            if ctx.pack is None:
-                ctx.pack = capi.Pack(pinned=True)
-            ctx.stager.sync_copies()  # the pinned pack buffer may still be in flight
-            ctx.pack.gather(seqs, nthreads=4)
-            n = ctx.pack.nseq
-            pb, po = ctx.pack.bytes_ptr or 0, ctx.pack.offsets_ptr
-            host_o = np.ctypeslib.as_array(capi.C.cast(po, capi.C.POINTER(capi.C.c_int64)), shape=(n + 1,))
-            hb_ptr = pb
+            ok = b.dtype == torch.uint8 and o.dtype == torch.int64 and b.is_contiguous() and o.is_contiguous()
         else:
-            if host_o.size < 1:
-                raise ValueError("offsets needs at least one entry")
-            n = host_o.size - 1
-            if n > 0 and int(host_o[n]) > host_b.size:
-                raise ValueError("offsets run past the end of bytes")
-            hb_ptr = host_b.ctypes.data
-            r.keep += [host_b, host_o]
-        if crop is not None or rc is not None:
-            cropped_o, r.extent = _crop_host_extent(host_o, n, crop[1] if crop is not None else _UNCROPPED)
+            b = b.numpy() if isinstance(b, torch.Tensor) else np.asarray(b)
+            o = o.numpy() if isinstance(o, torch.Tensor) else np.asarray(o)
+            ok = b.dtype == np.uint8 and o.dtype == np.int64 and b.flags.c_contiguous and o.flags.c_contiguous
+        if not ok:
+            raise ValueError("packed batch: contiguous uint8 bytes and int64 offsets expected")
+        if isinstance(o, torch.Tensor):
+            return _Batch(b, o, None)
+    else:  # list of str / bytes / bytearray (any other batch fails as an item)
+        items = []
+        for s in (batch if isinstance(batch, (list, tuple)) else [None]):
+            if isinstance(s, str):
+                s = s.encode("utf-8")
+            elif not isinstance(s, (bytes, bytearray)):
+                raise ValueError("item was none of string, bytes, or numpy array of 8-bit integers. ")
+            items.append(s)
+        return _Batch(None, items, None)
+    _nseq(o, b.size)
+    return _Batch(b, o, keep)
+
+
+def _nseq(offsets, nbytes=None):
+    """The number of sequences ``offsets`` (numpy or torch) delimit; with ``nbytes`` (host offsets), they must end
+    within that many bytes."""
+    n = (offsets.numel() if isinstance(offsets, _torch().Tensor) else offsets.size) - 1
+    if n < 0:
+        raise ValueError("offsets needs at least one entry")
+    if nbytes is not None and n > 0 and int(offsets[n]) > nbytes:
+        raise ValueError("offsets run past the end of bytes")
+    return n
+
+
+def _packed_cuda(name, bytes_cuda, offsets_cuda):
+    """Check the packed CUDA batch of entry point ``name``."""
+    torch = _torch()
+    if not (isinstance(bytes_cuda, torch.Tensor) and bytes_cuda.is_cuda and bytes_cuda.dtype == torch.uint8 and
+            isinstance(offsets_cuda, torch.Tensor) and offsets_cuda.is_cuda and offsets_cuda.dtype == torch.int64 and
+            bytes_cuda.device == offsets_cuda.device and bytes_cuda.is_contiguous() and offsets_cuda.is_contiguous()):
+        raise ValueError(f"{name}: contiguous uint8 bytes and int64 offsets CUDA tensors on one device expected")
+
+
+def _resolve(batch, device, augment=None, before_stage=None, crop=None, rc=None, checked=None):
+    """-> _Resolved of a batch (or of its ``_parse``), in these steps: size the crop and flip, ``before_stage``, stage (or
+    use in place), crop, augment, flip.
+
+    Host batches are staged; CUDA batches are used in place (with ``augment`` and no crop: a clone).
+    ``before_stage(host_offsets, n)`` checks a host batch before anything is copied to the device.  ``crop`` (from
+    ``_crop_spec``): the batch is cropped into fresh device buffers.  ``augment``: BLOSUM62 mutations, by the stager's
+    copy of an uncropped host batch, else in place on the device.  ``rc`` (from ``_rc_spec``): the batch is then
+    flipped into fresh device buffers (``_apply_rc``); ``"both"`` doubles it.
+
+    With a crop or a flip the result has ``extent = (sum, max)`` of its lengths, and ``before_stage`` and ``h_offs``
+    see the cropped and flipped offsets from 0.  Host batches are sized from their host offsets; CUDA batches pay one
+    ``bsq_crop_extent_device`` (which also validates their offsets), unless ``checked`` says the caller has validated
+    them already: it is then their ``(sum, max)`` after the crop, or True when the caller has no such extent."""
+    torch = _torch()
+    p = batch if isinstance(batch, _Batch) else _parse(batch)
+    cuda = isinstance(p.offsets, torch.Tensor)
+    sized = crop is not None or rc is not None
+    crop_len = crop[1] if crop is not None else _UNCROPPED
+    r = _Resolved()
+    r.ctx, r.keep, r.h_offs, r.base, r.extent = None, [p], None, 0, None
+    ctx = None
+    if cuda:
+        b, o = p.bytes, p.offsets
+        r.device = b.device.index
+        r.stream = torch.cuda.current_stream(r.device).cuda_stream
+        if sized and checked is None:
+            r.extent = capi.crop_extent_device(r.device, r.stream, o, o.numel() - 1, crop_len, nbytes=b.numel())
+        elif sized and checked is not True:
+            r.extent = checked
+        if augment and crop is None:
+            with torch.cuda.device(r.device):
+                b = b.clone()  # never mutate the caller's residues
+            r.keep.append(b)
+        r.d_bytes, r.d_offs, r.nseq = b.data_ptr(), o.data_ptr(), o.numel() - 1
+    else:
+        r.device = _resolve_device(device)
+        r.stream = torch.cuda.current_stream(r.device).cuda_stream
+        ctx = _device_ctx(r.device)
+        ctx.lock.acquire()
+    try:
+        if not cuda:
+            if p.bytes is None:
+                if ctx.pack is None:
+                    ctx.pack = capi.Pack(pinned=True)
+                ctx.stager.sync_copies()  # the pinned pack buffer may still be in flight
+                ctx.pack.gather(p.offsets, nthreads=4)
+                n = ctx.pack.nseq
+                hb_ptr = ctx.pack.bytes_ptr or 0
+                h = np.ctypeslib.as_array(capi.C.cast(ctx.pack.offsets_ptr, capi.C.POINTER(capi.C.c_int64)), shape=(n + 1,))
+            else:
+                n, hb_ptr, h = p.offsets.size - 1, p.bytes.ctypes.data, p.offsets
+            if sized:
+                r.h_offs, r.extent = _crop_host_extent(h, n, crop_len)
+            else:
+                r.h_offs, r.base = h, int(h[0])
             if before_stage is not None:
-                before_stage(*_rc_host_offsets(cropped_o, n, rc))
-            r.d_bytes, r.d_offs = ctx.stager.stage(r.stream, hb_ptr, host_o.ctypes.data, n)
-            r.nseq, r.ctx, r.h_offs = n, ctx, cropped_o
-            if crop is not None:
-                _apply_crop(r, crop, augment)
-            _apply_rc(r, rc, r.extent[0])
-            return r
-        if before_stage is not None:
-            before_stage(host_o, n)
-        if augment:
-            ctx.stager.set_augment(*augment)
-        try:
-            r.d_bytes, r.d_offs = ctx.stager.stage(r.stream, hb_ptr, host_o.ctypes.data, n)
-        finally:
-            if augment:
-                ctx.stager.set_augment(0)
-        r.nseq, r.h_offs, r.ctx, r.base = n, host_o, ctx, int(host_o[0]) if n >= 0 else 0
-        return r
+                before_stage(*_rc_host_offsets(r.h_offs, n, rc))
+            stager_augment = augment and crop is None
+            if stager_augment:
+                ctx.stager.set_augment(*augment)
+            try:
+                r.d_bytes, r.d_offs = ctx.stager.stage(r.stream, hb_ptr, h.ctypes.data, n)
+            finally:
+                if stager_augment:
+                    ctx.stager.set_augment(0)
+            r.nseq, r.ctx = n, ctx
+        if crop is not None:
+            _apply_crop(r, crop)
+        if augment and (cuda or crop is not None):
+            capi.augment_blosum62(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, *augment)
+        if rc is not None:
+            _apply_rc(r, rc, r.extent[0] if r.extent is not None else p.bytes.numel())
     except BaseException:
-        ctx.lock.release()
+        if ctx is not None:
+            ctx.lock.release()
         raise
+    return r
 
 
 def _check_lengths(r, padlen, tok, onehot):
@@ -253,6 +274,21 @@ def _default_padlen(batch, tokenizer, padlen):
     if isinstance(batch, tuple) and len(batch) == 3 and isinstance(batch[0], cbioseq.FlatFile):
         return int(batch[0].maxseqlen + tokenizer.includes_bos() + tokenizer.includes_eos())
     raise ValueError("batch tokenize requires padlen is provded.")  # src/tokenize.h:383
+
+
+def _padlen(name, padlen, varlen, default=None):
+    """``padlen`` of a consumer that writes padded or padding-free output: None or -1 give ``default``, anything else
+    must be an integer; with ``varlen`` (no padding is written) None, and giving one is an error."""
+    if varlen:
+        if padlen is not None and padlen != -1:
+            raise ValueError(f"{name}(varlen=True) writes no padding: padlen must not be given")
+        return None
+    if padlen is None or padlen == -1:
+        return default
+    try:
+        return operator.index(padlen)
+    except TypeError:
+        raise ValueError("padlen must be an integer") from None
 
 
 def _augment_args(augment, augment_frac, seed, seq_index_base):
@@ -302,9 +338,9 @@ def _crop_host_extent(h_offs, n, crop_len):
     return out, (int(out[n]), int(kept.max()) if n > 0 else 0)
 
 
-def _apply_crop(r, crop, augment):
-    """Crop the resolved batch into fresh device buffers (r.extent already holds their size), then augment them in
-    place; r then describes the cropped batch."""
+def _apply_crop(r, crop):
+    """Crop the resolved batch into fresh device buffers (r.extent already holds their size); r then describes the
+    cropped batch."""
     torch = _torch()
     random, crop_len, seed, base = crop
     dev = torch.device("cuda", r.device)
@@ -314,8 +350,6 @@ def _apply_crop(r, crop, augment):
     capi.crop(r.device, r.stream, r.d_bytes or out_b, r.d_offs, r.nseq, crop_len, random, seed, base, out_b, out_o)
     r.keep += [out_b, out_o]
     r.d_bytes, r.d_offs, r.base = out_b.data_ptr(), out_o.data_ptr(), 0
-    if augment:
-        capi.augment_blosum62(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, *augment)
 
 
 _RC_MODES = {None: None, "always": capi.RC_ALWAYS, "random": capi.RC_RANDOM, "both": capi.RC_BOTH}
@@ -360,24 +394,24 @@ def _rc_host_offsets(h_offs, n, rc):
     return np.concatenate([h, h[n] + h[1:]]), 2 * n
 
 
-def _apply_rc(r, rc, nbytes):
+def _apply_rc(r, rc, nbytes, flipped=False):
     """Flip the resolved batch (validated offsets, ``nbytes`` >= its residues) into fresh device buffers; r then
-    describes the flipped batch (doubled for "both")."""
-    if rc is None:
-        return
+    describes the flipped batch (doubled for "both").  ``flipped``: return the bool mask of the flipped sequences."""
     torch = _torch()
     mode, rc_prob, seed, base = rc
-    both = mode == capi.RC_BOTH
+    m = 2 if mode == capi.RC_BOTH else 1
     dev = torch.device("cuda", r.device)
-    out_b = torch.empty(max(nbytes * (2 if both else 1), 1), dtype=torch.uint8, device=dev)  # (never a null pointer)
-    out_o = torch.empty(r.nseq * (2 if both else 1) + 1, dtype=torch.int64, device=dev)
-    capi.revcomp(r.device, r.stream, r.d_bytes or out_b, r.d_offs, r.nseq, mode, rc_prob, seed, base, out_b, out_o)
+    out_b = torch.empty(max(nbytes * m, 1), dtype=torch.uint8, device=dev)  # (never a null pointer)
+    out_o = torch.empty(r.nseq * m + 1, dtype=torch.int64, device=dev)
+    flipped = torch.empty(r.nseq * m, dtype=torch.uint8, device=dev) if flipped else None
+    capi.revcomp(r.device, r.stream, r.d_bytes or out_b, r.d_offs, r.nseq, mode, rc_prob, seed, base, out_b, out_o, flipped)
     r.keep += [out_b, out_o]
     if r.h_offs is not None:
         r.h_offs = _rc_host_offsets(np.asarray(r.h_offs, np.int64) - int(r.h_offs[0]), r.nseq, rc)[0]
     r.d_bytes, r.d_offs, r.base, r.nseq = out_b.data_ptr(), out_o.data_ptr(), 0, out_o.numel() - 1
-    if both and r.extent is not None:
+    if m == 2 and r.extent is not None:
         r.extent = (2 * r.extent[0], r.extent[1])
+    return None if flipped is None else flipped.view(torch.bool)
 
 
 def _row_residues(tokenizer, padlen):
@@ -407,14 +441,12 @@ def batch_onehot_encode_bcl(tokenizer, batch, padlen=-1, destchar="f", mask=None
         _check_lengths(r, padlen, tok, onehot=True)
         d_mask = None
         if mask is not None:
-            if isinstance(mask, torch.Tensor) and mask.is_cuda:
-                if r.h_offs is not None:
-                    raise ValueError("bytes, offsets and mask must live on the same side (all host or all CUDA)")
+            if (isinstance(mask, torch.Tensor) and mask.is_cuda) != (r.h_offs is None):
+                raise ValueError("bytes, offsets and mask must live on the same side (all host or all CUDA)")
+            if r.h_offs is None:
                 m = mask
                 d_mask = m.data_ptr()
             else:
-                if r.h_offs is None:
-                    raise ValueError("bytes, offsets and mask must live on the same side (all host or all CUDA)")
                 hm = mask.numpy() if isinstance(mask, torch.Tensor) else np.asarray(mask, dtype=np.uint8)
                 end = int(r.h_offs[r.nseq])
                 if hm.size < end:
@@ -492,18 +524,13 @@ def crop_packed(bytes_cuda, offsets_cuda, crop_len, *, crop="random", seed=0, se
     A sequence no longer than ``crop_len`` is kept whole.  The exact rule is documented with ``bsq_crop`` in
     include/bsq.h.  One synchronisation: the output's size is read back, and the offsets are validated."""
     torch = _torch()
-    if not (isinstance(bytes_cuda, torch.Tensor) and bytes_cuda.is_cuda and bytes_cuda.dtype == torch.uint8 and
-            isinstance(offsets_cuda, torch.Tensor) and offsets_cuda.is_cuda and offsets_cuda.dtype == torch.int64 and
-            bytes_cuda.device == offsets_cuda.device and bytes_cuda.is_contiguous() and offsets_cuda.is_contiguous()):
-        raise ValueError("crop_packed: contiguous uint8 bytes and int64 offsets CUDA tensors on one device expected")
+    _packed_cuda("crop_packed", bytes_cuda, offsets_cuda)
     if crop is None:
         raise ValueError("crop_packed: crop must be 'head' or 'random'")
     random, crop_len, seed, base = _crop_spec(crop, crop_len, seed, seq_index_base)
-    if offsets_cuda.numel() < 1:
-        raise ValueError("offsets needs at least one entry")
+    n = _nseq(offsets_cuda)
     dev = bytes_cuda.device
     stream = torch.cuda.current_stream(dev.index).cuda_stream
-    n = offsets_cuda.numel() - 1
     total, _ = capi.crop_extent_device(dev.index, stream, offsets_cuda, n, crop_len, nbytes=bytes_cuda.numel())
     out_b = torch.empty(max(total, 1), dtype=torch.uint8, device=dev)
     out_o = torch.empty(n + 1, dtype=torch.int64, device=dev)
@@ -576,18 +603,13 @@ def revcomp_packed(bytes_cuda, offsets_cuda, *, rc="always", rc_prob=None, seed=
     labels: crop with :func:`crop_packed`, flip with this, then reverse the labels of the rows ``flipped`` marks.  One
     synchronisation: the offsets are validated and the output's size is read back."""
     torch = _torch()
-    if not (isinstance(bytes_cuda, torch.Tensor) and bytes_cuda.is_cuda and bytes_cuda.dtype == torch.uint8 and
-            isinstance(offsets_cuda, torch.Tensor) and offsets_cuda.is_cuda and offsets_cuda.dtype == torch.int64 and
-            bytes_cuda.device == offsets_cuda.device and bytes_cuda.is_contiguous() and offsets_cuda.is_contiguous()):
-        raise ValueError("revcomp_packed: contiguous uint8 bytes and int64 offsets CUDA tensors on one device expected")
+    _packed_cuda("revcomp_packed", bytes_cuda, offsets_cuda)
     if rc is None:
         raise ValueError("revcomp_packed: rc must be 'always', 'random' or 'both'")
     mode, rc_prob, seed, base = _rc_spec(rc, rc_prob, seed, seq_index_base)
-    if offsets_cuda.numel() < 1:
-        raise ValueError("offsets needs at least one entry")
+    n = _nseq(offsets_cuda)
     dev = bytes_cuda.device
     stream = torch.cuda.current_stream(dev.index).cuda_stream
-    n = offsets_cuda.numel() - 1
     total, _ = capi.crop_extent_device(dev.index, stream, offsets_cuda, n, _UNCROPPED, nbytes=bytes_cuda.numel())
     m = 2 if mode == capi.RC_BOTH else 1
     out_b = torch.empty(max(m * total, 1), dtype=torch.uint8, device=dev)
@@ -602,19 +624,8 @@ def batch_tokenize_augmented(tokenizer, batch, padlen=-1, destchar="B", batch_fi
                              augment_frac=1.0, seed=0, seq_index_base=0):
     """``batch_tokenize`` of the BLOSUM62-augmented batch: copy -> mutate on the device -> tokenize
     (what FlatFileDataset does per item with Python strings, bioseq/loaders.py:99-101)."""
-    torch = _torch()
-    tok = descriptor(tokenizer)
-    padlen = _default_padlen(batch, tokenizer, padlen)
-    kind, dtype = _dtype_of(destchar)
-    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base))
-    try:
-        _check_lengths(r, padlen, tok, onehot=False)
-        shape = (r.nseq, padlen) if batch_first else (padlen, r.nseq)
-        out = torch.empty(shape, dtype=dtype, device=torch.device("cuda", r.device))
-        capi.tokenize(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, padlen, tok, batch_first, kind, out)
-        return out
-    finally:
-        r.release()
+    return _tokenize_padded(tokenizer, batch, padlen, destchar, batch_first, device, None, None, seed, seq_index_base, augment,
+                            augment_frac, None, None)
 
 
 VarlenBatch = collections.namedtuple("VarlenBatch", ["tokens", "cu_seqlens", "max_seqlen"])
@@ -623,6 +634,13 @@ entries: row ``i`` is ``tokens[cu_seqlens[i]:cu_seqlens[i + 1]]``) and ``max_seq
 attention (``flash_attn_varlen_func(q, k, v, cu_seqlens, cu_seqlens, max_seqlen, max_seqlen)``)."""
 
 _INT32_MAX = 2 ** 31 - 1
+
+
+def _check_cu_seqlens(total, what="varlen"):
+    """ValueError unless ``total`` tokens of a ``what`` batch can be indexed by int32 ``cu_seqlens``."""
+    if total > _INT32_MAX:
+        raise ValueError(f"{what} batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one batch; "
+                         "split the batch")
 
 
 def _varlen_extent_host(h_offs, n, k):
@@ -636,9 +654,7 @@ def _varlen_extent_host(h_offs, n, k):
     if lens.size and int(lens.min()) < 0:
         raise ValueError("offsets must be non-decreasing")
     total = int(o[n]) - int(o[0]) + n * k
-    if total > _INT32_MAX:
-        raise ValueError(f"varlen batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one batch; "
-                         "split the batch")
+    _check_cu_seqlens(total)
     return total, int(lens.max()) + k
 
 
@@ -669,21 +685,14 @@ def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None, mlm=None,
     r = _resolve(batch, device, augment, before_stage=lambda h_offs, n: extent.extend(_varlen_extent_host(h_offs, n, k)),
                  crop=crop, rc=rc)
     try:
-        if r.h_offs is None and r.extent is not None:  # a cropped or flipped CUDA batch: sized by its one read-back
-            total, max_seqlen = r.extent[0] + r.nseq * k, (r.extent[1] + k if r.nseq > 0 else 0)
-            if total > _INT32_MAX:
-                raise ValueError(f"varlen batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one "
-                                 "batch; split the batch")
-        elif r.h_offs is None:
-            nbytes = -1
-            if isinstance(batch, tuple) and len(batch) == 2:
-                nbytes = batch[0].numel()
-            total, max_seqlen = capi.varlen_extent_device(r.device, r.stream, r.d_offs, r.nseq, tok, nbytes=nbytes)
-            if total > _INT32_MAX:
-                raise ValueError(f"varlen batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one "
-                                 "batch; split the batch")
-        else:
+        if r.h_offs is not None:
             total, max_seqlen = extent
+        else:
+            if r.extent is not None:  # a cropped or flipped CUDA batch: sized by its one read-back
+                total, max_seqlen = r.extent[0] + r.nseq * k, (r.extent[1] + k if r.nseq > 0 else 0)
+            else:
+                total, max_seqlen = capi.varlen_extent_device(r.device, r.stream, r.d_offs, r.nseq, tok, nbytes=batch[0].numel())
+            _check_cu_seqlens(total)
         dev = torch.device("cuda", r.device)
         tokens = torch.empty(total, dtype=dtype, device=dev)
         cu_seqlens = torch.empty(r.nseq + 1, dtype=torch.int32, device=dev)
@@ -776,8 +785,7 @@ def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *
     rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment, mlm=True)
     augment = _augment_args(augment, augment_frac, seed, seq_index_base)
     if varlen:
-        if padlen is not None and padlen != -1:
-            raise ValueError("batch_tokenize_mlm(varlen=True) writes no padding: padlen must not be given")
+        _padlen("batch_tokenize_mlm", padlen, varlen)
         crop = _crop_spec(crop, crop_len, seed, seq_index_base)
         vb, labels = _tokenize_varlen(tokenizer, batch, destchar, device, augment, mlm, crop, rc)
         return MLMBatch(vb, labels)
@@ -801,49 +809,6 @@ SeqPackBatch.__doc__ = """Whole sequences packed into fixed-width rows: ``tokens
 the flat start of every segment -- a sequence or a padding run -- then ``rows * L``), ``max_seqlen`` (int, the longest
 segment), ``starts`` (int64, one per sequence: its flat position in ``tokens.view(-1)``, -1 for a sequence that occupies
 nothing) and ``labels`` (int64 ``(rows, L)`` with ``mlm=True``, else None)."""
-
-
-def _seqpack_host_offsets(batch):
-    """Host offsets to plan a batch from before it is staged: a CUDA batch's are read back and validated (one
-    synchronisation); host arrays and FlatFile ranges are used as they are.  None for a list of items (planned once
-    ``_resolve`` has gathered it)."""
-    torch = _torch()
-    if isinstance(batch, tuple) and len(batch) == 3 and isinstance(batch[0], cbioseq.FlatFile):
-        return batch[0].packed(batch[1], batch[2])[1]
-    if not (isinstance(batch, tuple) and len(batch) == 2 and hasattr(batch[0], "dtype")):
-        return None
-    b, o = batch
-    if not (isinstance(b, torch.Tensor) and b.is_cuda):
-        o = o.numpy() if isinstance(o, torch.Tensor) else np.asarray(o)
-        return o if o.dtype == np.int64 and o.ndim == 1 and o.size >= 1 else None  # (anything else: _resolve raises)
-    if not (isinstance(o, torch.Tensor) and o.is_cuda and o.device == b.device):
-        raise ValueError("bytes and offsets must live on the same side (all host or all CUDA)")
-    if b.dtype != torch.uint8 or o.dtype != torch.int64 or not b.is_contiguous() or not o.is_contiguous():
-        raise ValueError("packed batch: contiguous uint8 bytes and int64 offsets expected")
-    if o.numel() < 1:
-        raise ValueError("offsets needs at least one entry")
-    h = o.cpu().numpy()
-    n = h.size - 1
-    if n > 0 and (int(h[0]) < 0 or int(np.diff(h).min()) < 0):
-        raise ValueError("offsets must start at or after 0 and be non-decreasing")
-    if int(h[n]) > b.numel():
-        raise ValueError("offsets run past the end of bytes")
-    return h
-
-
-def _cuda_pair(batch):
-    """(bytes, offsets) of a packed CUDA batch, checked as ``_resolve`` checks them; None for any other batch form."""
-    torch = _torch()
-    if not (isinstance(batch, tuple) and len(batch) == 2 and isinstance(batch[0], torch.Tensor) and batch[0].is_cuda):
-        return None
-    b, o = batch
-    if not (isinstance(o, torch.Tensor) and o.is_cuda and o.device == b.device):
-        raise ValueError("bytes and offsets must live on the same side (all host or all CUDA)")
-    if b.dtype != torch.uint8 or o.dtype != torch.int64 or not b.is_contiguous() or not o.is_contiguous():
-        raise ValueError("packed batch: contiguous uint8 bytes and int64 offsets expected")
-    if o.numel() < 1:
-        raise ValueError("offsets needs at least one entry")
-    return b, o
 
 
 class _SeqPackPlan:
@@ -911,15 +876,18 @@ def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None,
     def make_plan(h_offs, n):
         plan.append(_SeqPackPlan(h_offs, n, k, row_len, rows))
 
-    h = _seqpack_host_offsets(batch)
-    crop_extent = None
-    if h is not None:  # planned before anything is staged (a CUDA batch: from its offsets, read back once)
+    p = _parse(batch)
+    checked = None
+    if p.bytes is not None:  # planned before anything is staged (a CUDA batch: from its offsets, read back once)
+        cuda, sized, h = isinstance(p.offsets, torch.Tensor), crop is not None or rc is not None, p.offsets
+        if cuda:
+            h = h.cpu().numpy()
+            _nseq(h, p.bytes.numel())
         n = h.size - 1
-        if crop is not None or rc is not None:
-            h, crop_extent = _crop_host_extent(h, n, crop[1] if crop is not None else _UNCROPPED)
-        make_plan(*_rc_host_offsets(h, n, rc))
-    r = _resolve(batch, device, augment, before_stage=None if h is not None else make_plan, crop=crop, crop_extent=crop_extent,
-                 rc=rc)
+        if cuda or sized:  # (this also validates the offsets)
+            cropped, checked = _crop_host_extent(h, n, crop[1] if crop is not None else _UNCROPPED)
+        make_plan(*_rc_host_offsets(cropped if sized else h, n, rc))
+    r = _resolve(p, device, augment, before_stage=None if plan else make_plan, crop=crop, rc=rc, checked=checked)
     try:
         p = plan[0]
         dev = torch.device("cuda", r.device)
@@ -994,10 +962,9 @@ def kmer_vocab(tokenizer, k):
 
 def _kmer_check_extent(extent, padlen, varlen):
     total, longest = extent
-    if varlen and total > _INT32_MAX:
-        raise ValueError(f"k-mer batch of {total} tokens: cu_seqlens is int32, so at most 2^31 - 1 tokens fit one batch; "
-                         "split the batch")
-    if not varlen and longest > padlen:
+    if varlen:
+        _check_cu_seqlens(total, "k-mer")
+    elif longest > padlen:
         raise ValueError(f"k-mer tokens + bos + eos > padlen: {longest}, vs padlen {padlen}")
 
 
@@ -1026,17 +993,9 @@ def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=Non
     limit = _mask_token_limit(destchar)
     if km.vocab_size - 1 > limit:
         raise ValueError(f"k-mer ids up to {km.vocab_size - 1} do not fit destchar {destchar!r} (0..{limit})")
-    if varlen:
-        if padlen is not None and padlen != -1:
-            raise ValueError("batch_tokenize_kmer(varlen=True) writes no padding: padlen must not be given")
-        padlen = 0
-    else:
-        try:
-            padlen = operator.index(padlen) if padlen is not None else -1
-        except TypeError:
-            raise ValueError("padlen must be an integer") from None
-        if padlen <= 0:
-            raise ValueError("batch_tokenize_kmer requires padlen (or varlen=True)")
+    padlen = _padlen("batch_tokenize_kmer", padlen, varlen, -1)
+    if not varlen and padlen <= 0:
+        raise ValueError("batch_tokenize_kmer requires padlen (or varlen=True)")
     crop = _crop_spec(crop, crop_len, seed, seq_index_base)
     rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer)
     extent = []
@@ -1046,21 +1005,21 @@ def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=Non
         _kmer_check_extent(e, padlen, varlen)
         extent.extend(e)
 
-    validated = False
-    if rc is not None and crop is None and _cuda_pair(batch) is not None:
+    p = _parse(batch)
+    checked = None
+    if rc is not None and crop is None and isinstance(p.offsets, torch.Tensor):
         # the extent of the unflipped offsets is the flipped batch's (doubled by "both"), and reading it validates them:
         # the flip needs no read-back of its own
-        b, o = _cuda_pair(batch)
-        total, longest = capi.kmer_extent_device(b.device.index, torch.cuda.current_stream(b.device.index).cuda_stream, o,
-                                                 o.numel() - 1, km, nbytes=b.numel())
+        d = p.bytes.device.index
+        total, longest = capi.kmer_extent_device(d, torch.cuda.current_stream(d).cuda_stream, p.offsets, _nseq(p.offsets), km,
+                                                 nbytes=p.bytes.numel())
         extent = [total * (2 if rc[0] == capi.RC_BOTH else 1), longest]
         _kmer_check_extent(extent, padlen, varlen)
-        validated = True
-    r = _resolve(batch, device, before_stage=before_stage, crop=crop, rc=rc, validated=validated)
+        checked = True
+    r = _resolve(p, device, before_stage=before_stage, crop=crop, rc=rc, checked=checked)
     try:
-        if r.h_offs is None and not validated:  # a CUDA batch: one reduction and read-back, which also validates its offsets
-            nbytes = batch[0].numel() if r.extent is None else -1
-            extent = capi.kmer_extent_device(r.device, r.stream, r.d_offs, r.nseq, km, nbytes=nbytes)
+        if r.h_offs is None and checked is None:  # a CUDA batch: one reduction and read-back, which also validates its offsets
+            extent = capi.kmer_extent_device(r.device, r.stream, r.d_offs, r.nseq, km, nbytes=-1 if crop is not None else p.bytes.numel())
             _kmer_check_extent(extent, padlen, varlen)
         dev = torch.device("cuda", r.device)
         if varlen:
@@ -1117,16 +1076,11 @@ def tile_packed(bytes_cuda, offsets_cuda, window, *, stride=None, tail="short"):
     window index (``seq_index_base + w``).  One synchronisation: the offsets are validated and the output's size is read
     back."""
     torch = _torch()
-    if not (isinstance(bytes_cuda, torch.Tensor) and bytes_cuda.is_cuda and bytes_cuda.dtype == torch.uint8 and
-            isinstance(offsets_cuda, torch.Tensor) and offsets_cuda.is_cuda and offsets_cuda.dtype == torch.int64 and
-            bytes_cuda.device == offsets_cuda.device and bytes_cuda.is_contiguous() and offsets_cuda.is_contiguous()):
-        raise ValueError("tile_packed: contiguous uint8 bytes and int64 offsets CUDA tensors on one device expected")
+    _packed_cuda("tile_packed", bytes_cuda, offsets_cuda)
     window, stride, tail = _tile_spec(window, stride, tail)
-    if offsets_cuda.numel() < 1:
-        raise ValueError("offsets needs at least one entry")
+    n = _nseq(offsets_cuda)
     dev = bytes_cuda.device
     stream = torch.cuda.current_stream(dev.index).cuda_stream
-    n = offsets_cuda.numel() - 1
     M, nbytes, _ = capi.tile_extent_device(dev.index, stream, offsets_cuda, n, window, stride, tail, nbytes=bytes_cuda.numel())
     out = _tile_into(dev, stream, bytes_cuda.data_ptr(), offsets_cuda, n, window, stride, tail, M, nbytes)
     return out._replace(seq_offsets=offsets_cuda - offsets_cuda[:1])
@@ -1178,28 +1132,22 @@ def batch_tokenize_tiled(tokenizer, batch, window, stride=None, padlen=None, des
     kind, dtype = _dtype_of(destchar)
     window, stride, tail_code = _tile_spec(window, stride, tail)
     k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
-    if varlen:
-        if padlen is not None and padlen != -1:
-            raise ValueError("batch_tokenize_tiled(varlen=True) writes no padding: padlen must not be given")
-    else:
-        try:
-            padlen = window + k if padlen is None or padlen == -1 else operator.index(padlen)
-        except TypeError:
-            raise ValueError("padlen must be an integer") from None
-        if padlen < window + k:
-            raise ValueError(f"padlen {padlen} is shorter than window + bos + eos = {window + k}")
+    padlen = _padlen("batch_tokenize_tiled", padlen, varlen, window + k)
+    if not varlen and padlen < window + k:
+        raise ValueError(f"padlen {padlen} is shorter than window + bos + eos = {window + k}")
     rc = _rc_spec(rc, rc_prob, seed, 0, tokenizer)
     strands = 2 if rc is not None and rc[0] == capi.RC_BOTH else 1
     extent = []
     seq_offsets = []
 
+    def checked(e):
+        if varlen:
+            _check_cu_seqlens(strands * (e[1] + e[0] * k))
+        return e
+
     def before_stage(h_offs, n):
         h = np.ascontiguousarray(h_offs[:n + 1], dtype=np.int64)
-        e = capi.tile_extent_host(h, n, window, stride, tail_code)
-        if varlen and strands * (e[1] + e[0] * k) > _INT32_MAX:
-            raise ValueError(f"varlen batch of {strands * (e[1] + e[0] * k)} tokens: cu_seqlens is int32, so at most 2^31 - 1 "
-                             "tokens fit one batch; split the batch")
-        extent.extend(e)
+        extent.extend(checked(capi.tile_extent_host(h, n, window, stride, tail_code)))
         seq_offsets.append(h - h[0] if n >= 0 else h)
 
     r = _resolve(batch, device, before_stage=before_stage)
@@ -1207,33 +1155,23 @@ def batch_tokenize_tiled(tokenizer, batch, window, stride=None, padlen=None, des
         dev = torch.device("cuda", r.device)
         if r.h_offs is None:  # a CUDA batch: one reduction and read-back, which also validates its offsets
             b, o = batch
-            extent = capi.tile_extent_device(r.device, r.stream, o, r.nseq, window, stride, tail_code, nbytes=b.numel())
-            if varlen and strands * (extent[1] + extent[0] * k) > _INT32_MAX:
-                raise ValueError(f"varlen batch of {strands * (extent[1] + extent[0] * k)} tokens: cu_seqlens is int32, so at "
-                                 "most 2^31 - 1 tokens fit one batch; split the batch")
+            extent = checked(capi.tile_extent_device(r.device, r.stream, o, r.nseq, window, stride, tail_code, nbytes=b.numel()))
             so = o - o[:1]
         else:
             so = torch.from_numpy(seq_offsets[0]).to(dev)
         M, nbytes, longest = extent
         tb = _tile_into(dev, r.stream, r.d_bytes, r.d_offs, r.nseq, window, stride, tail_code, M, nbytes)
-        d_bytes, d_offs, rows, flipped = tb.bytes, tb.offsets, M, None
-        if rc is not None:
-            mode, rc_prob, seed_, _ = rc
-            out_b = torch.empty(max(strands * nbytes, 1), dtype=torch.uint8, device=dev)
-            out_o = torch.empty(strands * M + 1, dtype=torch.int64, device=dev)
-            flipped = torch.empty(strands * M, dtype=torch.uint8, device=dev)
-            capi.revcomp(r.device, r.stream, d_bytes, d_offs, M, mode, rc_prob, seed_, 0, out_b, out_o, flipped)
-            d_bytes, d_offs, rows, flipped = out_b, out_o, strands * M, flipped.view(torch.bool)
+        r.d_bytes, r.d_offs, r.nseq, r.h_offs = tb.bytes.data_ptr(), tb.offsets.data_ptr(), M, None  # r: the windows
+        flipped = None if rc is None else _apply_rc(r, rc, nbytes, flipped=True)
         if varlen:
-            total = strands * nbytes + rows * k
-            tokens = torch.empty(total, dtype=dtype, device=dev)
-            cu_seqlens = torch.empty(rows + 1, dtype=torch.int32, device=dev)
-            capi.tokenize_varlen(r.device, r.stream, d_bytes, d_offs, rows, tok, kind, tokens, cu_seqlens)
-            tokens = VarlenBatch(tokens, cu_seqlens, longest + k if rows > 0 else 0)
+            tokens = torch.empty(strands * nbytes + r.nseq * k, dtype=dtype, device=dev)
+            cu_seqlens = torch.empty(r.nseq + 1, dtype=torch.int32, device=dev)
+            capi.tokenize_varlen(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, tok, kind, tokens, cu_seqlens)
+            tokens = VarlenBatch(tokens, cu_seqlens, longest + k if r.nseq > 0 else 0)
         else:
-            tokens = torch.empty((rows, padlen), dtype=dtype, device=dev)
-            if rows > 0:
-                capi.tokenize(r.device, r.stream, d_bytes, d_offs, rows, padlen, tok, True, kind, tokens)
+            tokens = torch.empty((r.nseq, padlen), dtype=dtype, device=dev)
+            if r.nseq > 0:
+                capi.tokenize(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, padlen, tok, True, kind, tokens)
         return TiledTokens(tokens, tb.seq_index, tb.starts, tb.seq_ptr, so, flipped, strands, window, stride, tail,
                            int(tokenizer.includes_bos()))
     finally:
