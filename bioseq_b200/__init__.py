@@ -129,6 +129,7 @@ from .consumers import batch_tokenize_seqpack, SeqPackBatch  # noqa: E402
 from .consumers import batch_tokenize_kmer, kmer_ids, kmer_vocab, KmerIds  # noqa: E402
 from .consumers import revcomp_packed, batch_tokenize_revcomp, RevCompBatch  # noqa: E402
 from .consumers import tile_packed, batch_tokenize_tiled, untile, TiledBatch, TiledTokens, UntiledBatch  # noqa: E402
+from .consumers import translate_packed, batch_tokenize_translated, TranslatedBatch  # noqa: E402
 
 
 def __getattr__(name):
@@ -151,4 +152,5 @@ __all__ = ["onehot_encode", "cbioseq", "f_encode", "Tokenizer", "make_embedding"
            "batch_tokenize_cropped", "CroppedBatch", "batch_tokenize_seqpack", "SeqPackBatch", "batch_tokenize_kmer", "kmer_ids", "kmer_vocab", "KmerIds",
            "revcomp_packed", "batch_tokenize_revcomp", "RevCompBatch",
            "tile_packed", "batch_tokenize_tiled", "untile", "TiledBatch", "TiledTokens", "UntiledBatch",
+           "translate_packed", "batch_tokenize_translated", "TranslatedBatch",
            "TokenizerLayer", "EmbeddingTokenizerLayer"]

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 ROOT = os.path.dirname(HERE)
 
-LIB_SOURCES = ["bsq_kernels.cu", "bsq_span.cu", "bsq_varlen.cu", "bsq_mlm.cu", "bsq_crop.cu", "bsq_seqpack.cu", "bsq_kmer.cu", "bsq_revcomp.cu", "bsq_tile.cu", "bsq_consumers.cu", "bsq_host.cu", "bsq_flatfile.cu", "bsq_alphabet.cpp"]
+LIB_SOURCES = ["bsq_kernels.cu", "bsq_span.cu", "bsq_varlen.cu", "bsq_mlm.cu", "bsq_crop.cu", "bsq_seqpack.cu", "bsq_kmer.cu", "bsq_revcomp.cu", "bsq_tile.cu", "bsq_translate.cu", "bsq_consumers.cu", "bsq_host.cu", "bsq_flatfile.cu", "bsq_alphabet.cpp"]
 NVCC_COMPILE = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
                 "-Xcompiler", "-fPIC,-Wall"]
 

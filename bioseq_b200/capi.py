@@ -133,6 +133,11 @@ def lib():
         "bsq_tile_extent_device": (i32, [i32, vp, vp, i64, i64, i64, i64, i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
         "bsq_tile": (i32, [i32, vp, vp, vp, i64, i64, i64, i32, vp, vp, vp, vp, vp]),
         "bsq_untile_mean": (i32, [i32, vp, i32, vp, i64, i64, vp, i64, vp, i64, i64, i64, i32, vp, i64, i32, vp, vp]),
+        "bsq_genetic_code": (i32, [i32, vp]),
+        "bsq_translate_table": (i32, [C.c_char_p, vp, vp]),
+        "bsq_translate_extent_host": (i32, [vp, i64, vp, i32, i64, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
+        "bsq_translate_extent_device": (i32, [i32, vp, vp, i64, i64, vp, i32, i64, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
+        "bsq_translate": (i32, [i32, vp, vp, vp, i64, vp, i32, C.c_char_p, vp, vp]),
     }
     for name, (res, args) in sigs.items():
         fn = getattr(L, name)
@@ -154,7 +159,8 @@ EXPORTS = ("bsq_abi_version bsq_last_error bsq_launch_count bsq_launch_count_res
            "bsq_tokenize_varlen bsq_varlen_extent_device bsq_tokenize_mlm bsq_tokenize_varlen_mlm bsq_crop bsq_crop_extent_device "
            "bsq_seqpack_plan bsq_tokenize_seqpack bsq_tokenize_seqpack_mlm bsq_kmer_init bsq_tokenize_kmer bsq_tokenize_kmer_varlen "
            "bsq_kmer_extent_host bsq_kmer_extent_device bsq_revcomp bsq_revcomp_table bsq_tile_extent_host bsq_tile_extent_device "
-           "bsq_tile bsq_untile_mean").split()
+           "bsq_tile bsq_untile_mean bsq_genetic_code bsq_translate_table bsq_translate_extent_host bsq_translate_extent_device "
+           "bsq_translate").split()
 
 
 def last_error():
@@ -301,6 +307,52 @@ def untile_mean(device, stream, dtype, d_y, channels, row_stride, d_cu, col0, d_
     """Per-residue mean of window outputs (bsq_untile_mean); ``dtype``: UNTILE_F32, UNTILE_BF16 or UNTILE_F16."""
     check(lib().bsq_untile_mean(device, stream, dtype, _ptr(d_y), channels, row_stride, _ptr(d_cu), col0, _ptr(d_src_offsets), nseq,
                                 window, stride, tail, _ptr(d_seq_ptr), nwin, strands, _ptr(d_flipped), _ptr(d_out)))
+
+
+def genetic_code(code_id):
+    """The built-in genetic code ``code_id`` as 64 bytes in TCAG order (bsq_genetic_code; no device call)."""
+    buf = C.create_string_buffer(64)
+    check(lib().bsq_genetic_code(code_id, buf))
+    return buf.raw
+
+
+def translate_table(code64):
+    """-> (masks, codons): uint8 numpy arrays of 256 and 4096 entries, the rule of bsq_translate (no device call)."""
+    import numpy as np
+    masks, codons = np.zeros(256, np.uint8), np.zeros(4096, np.uint8)
+    check(lib().bsq_translate_table(code64, masks.ctypes.data, codons.ctypes.data))
+    return masks, codons
+
+
+def _frames_arg(frames):
+    return (C.c_int8 * max(len(frames), 1))(*frames), len(frames)
+
+
+_NO_CROP = (1 << 63) - 1
+
+
+def translate_extent_host(h_offsets, nseq, frames, crop_len=_NO_CROP):
+    """-> (total, total after the crop, longest kept row) of host offsets (bsq_translate_extent_host; no device call)."""
+    t, c, m = C.c_int64(), C.c_int64(), C.c_int64()
+    fa, nf = _frames_arg(frames)
+    check(lib().bsq_translate_extent_host(_ptr(h_offsets), nseq, fa, nf, crop_len, C.byref(t), C.byref(c), C.byref(m)))
+    return t.value, c.value, m.value
+
+
+def translate_extent_device(device, stream, d_offsets, nseq, frames, crop_len=_NO_CROP, nbytes=-1):
+    """The same of device-resident offsets (bsq_translate_extent_device: validates them; synchronises)."""
+    t, c, m = C.c_int64(), C.c_int64(), C.c_int64()
+    fa, nf = _frames_arg(frames)
+    check(lib().bsq_translate_extent_device(device, stream, _ptr(d_offsets), nseq, nbytes, fa, nf, crop_len, C.byref(t), C.byref(c),
+                                            C.byref(m)))
+    return t.value, c.value, m.value
+
+
+def translate(device, stream, d_bytes, d_offsets, nseq, frames, code64, d_out_bytes, d_out_offsets):
+    """Reading frames ``frames`` of every sequence under the 64-letter genetic code ``code64`` (bsq_translate)."""
+    fa, nf = _frames_arg(frames)
+    check(lib().bsq_translate(device, stream, _ptr(d_bytes), _ptr(d_offsets), nseq, fa, nf, code64, _ptr(d_out_bytes),
+                              _ptr(d_out_offsets)))
 
 
 def seqpack_plan(h_offsets, nseq, k, row_len, rows=0, starts=None, row_ptr=None, row_seq=None, cu_seqlens=None):

@@ -178,37 +178,45 @@ def _packed_cuda(name, bytes_cuda, offsets_cuda):
         raise ValueError(f"{name}: contiguous uint8 bytes and int64 offsets CUDA tensors on one device expected")
 
 
-def _resolve(batch, device, augment=None, before_stage=None, crop=None, rc=None, checked=None):
-    """-> _Resolved of a batch (or of its ``_parse``), in these steps: size the crop and flip, ``before_stage``, stage (or
-    use in place), crop, augment, flip.
+def _resolve(batch, device, augment=None, before_stage=None, crop=None, rc=None, checked=None, translate=None):
+    """-> _Resolved of a batch (or of its ``_parse``), in these steps: size the translation, crop and flip,
+    ``before_stage``, stage (or use in place), translate, crop, augment, flip.
 
-    Host batches are staged; CUDA batches are used in place (with ``augment`` and no crop: a clone).
-    ``before_stage(host_offsets, n)`` checks a host batch before anything is copied to the device.  ``crop`` (from
+    Host batches are staged; CUDA batches are used in place (with ``augment`` and no crop or translation: a clone).
+    ``before_stage(host_offsets, n)`` checks a host batch before anything is copied to the device.  ``translate`` (from
+    ``_translate_spec``): the batch is translated into fresh device buffers, n F protein sequences.  ``crop`` (from
     ``_crop_spec``): the batch is cropped into fresh device buffers.  ``augment``: BLOSUM62 mutations, by the stager's
-    copy of an uncropped host batch, else in place on the device.  ``rc`` (from ``_rc_spec``): the batch is then
-    flipped into fresh device buffers (``_apply_rc``); ``"both"`` doubles it.
+    copy of an uncropped, untranslated host batch, else in place on the device.  ``rc`` (from ``_rc_spec``): the batch is
+    then flipped into fresh device buffers (``_apply_rc``); ``"both"`` doubles it.
 
-    With a crop or a flip the result has ``extent = (sum, max)`` of its lengths, and ``before_stage`` and ``h_offs``
-    see the cropped and flipped offsets from 0.  Host batches are sized from their host offsets; CUDA batches pay one
-    ``bsq_crop_extent_device`` (which also validates their offsets), unless ``checked`` says the caller has validated
-    them already: it is then their ``(sum, max)`` after the crop, or True when the caller has no such extent."""
+    With a translation, crop or flip the result has ``extent = (sum, max)`` of its lengths, and ``before_stage`` and
+    ``h_offs`` see the translated, cropped and flipped offsets from 0.  Host batches are sized from their host offsets;
+    CUDA batches pay one ``bsq_crop_extent_device`` or ``bsq_translate_extent_device`` (which also validates their
+    offsets), unless ``checked`` says the caller has validated them already: it is then their ``(sum, max)`` after the
+    crop (``(sum, max, translated bytes)`` with ``translate``), or True when the caller has no such extent."""
     torch = _torch()
     p = batch if isinstance(batch, _Batch) else _parse(batch)
     cuda = isinstance(p.offsets, torch.Tensor)
-    sized = crop is not None or rc is not None
+    sized = crop is not None or rc is not None or translate is not None
     crop_len = crop[1] if crop is not None else _UNCROPPED
     r = _Resolved()
     r.ctx, r.keep, r.h_offs, r.base, r.extent = None, [p], None, 0, None
+    tr_total = None
     ctx = None
     if cuda:
         b, o = p.bytes, p.offsets
         r.device = b.device.index
         r.stream = torch.cuda.current_stream(r.device).cuda_stream
-        if sized and checked is None:
+        if sized and checked is None and translate is not None:
+            tr_total, kept, longest = capi.translate_extent_device(r.device, r.stream, o, o.numel() - 1, translate[0], crop_len,
+                                                                   nbytes=b.numel())
+            r.extent = (kept, longest)
+        elif sized and checked is None:
             r.extent = capi.crop_extent_device(r.device, r.stream, o, o.numel() - 1, crop_len, nbytes=b.numel())
         elif sized and checked is not True:
-            r.extent = checked
-        if augment and crop is None:
+            r.extent = tuple(checked[:2])
+            tr_total = checked[2] if translate is not None else None
+        if augment and crop is None and translate is None:
             with torch.cuda.device(r.device):
                 b = b.clone()  # never mutate the caller's residues
             r.keep.append(b)
@@ -231,12 +239,12 @@ def _resolve(batch, device, augment=None, before_stage=None, crop=None, rc=None,
             else:
                 n, hb_ptr, h = p.offsets.size - 1, p.bytes.ctypes.data, p.offsets
             if sized:
-                r.h_offs, r.extent = _crop_host_extent(h, n, crop_len)
+                r.h_offs, r.extent, tr_total = _sized_host(h, n, crop_len, translate)
             else:
                 r.h_offs, r.base = h, int(h[0])
             if before_stage is not None:
-                before_stage(*_rc_host_offsets(r.h_offs, n, rc))
-            stager_augment = augment and crop is None
+                before_stage(*_rc_host_offsets(r.h_offs, n * len(translate[0]) if translate is not None else n, rc))
+            stager_augment = augment and crop is None and translate is None
             if stager_augment:
                 ctx.stager.set_augment(*augment)
             try:
@@ -245,9 +253,11 @@ def _resolve(batch, device, augment=None, before_stage=None, crop=None, rc=None,
                 if stager_augment:
                     ctx.stager.set_augment(0)
             r.nseq, r.ctx = n, ctx
+        if translate is not None:
+            _apply_translate(r, translate, tr_total)
         if crop is not None:
             _apply_crop(r, crop)
-        if augment and (cuda or crop is not None):
+        if augment and (cuda or crop is not None or translate is not None):
             capi.augment_blosum62(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, *augment)
         if rc is not None:
             _apply_rc(r, rc, r.extent[0] if r.extent is not None else p.bytes.numel())
@@ -414,29 +424,142 @@ def _apply_rc(r, rc, nbytes, flipped=False):
     return None if flipped is None else flipped.view(torch.bool)
 
 
+_FRAME_SETS = {"forward": (1, 2, 3), "six": (1, 2, 3, -1, -2, -3)}
+_GENETIC_CODES = (1, 2, 4, 5, 6, 11)
+# the alphabets a translated batch can be tokenized with: the protein and reduced protein codes, and raw bytes
+_TRANSLATE_KEYS = ("AMINO", "AMINO20", "PROTEIN", "DAYHOFF", "LIA10", "LIB10", "MURPHY", "SEB6", "SEB8", "SEB10", "SEB14", "SEV10",
+                   "BYTES")
+
+
+def _frames(frames):
+    """-> tuple of 1..6 distinct frames from ``frames`` (one of +-1, +-2, +-3, a list / tuple of them, "forward", "six")."""
+    if isinstance(frames, str):
+        if frames not in _FRAME_SETS:
+            raise ValueError(f"frames must be 'forward', 'six', one of +-1, +-2, +-3 or a list of them, got {frames!r}")
+        return _FRAME_SETS[frames]
+    items = list(frames) if isinstance(frames, (list, tuple)) else [frames]
+    out = []
+    for f in items:
+        try:
+            f = operator.index(f)
+        except TypeError:
+            raise ValueError(f"frames must be integers among +-1, +-2, +-3, got {f!r}") from None
+        if f not in (1, 2, 3, -1, -2, -3):
+            raise ValueError(f"frames must lie among +-1, +-2, +-3, got {f}")
+        if f in out:
+            raise ValueError(f"frame {f} is given twice")
+        out.append(int(f))
+    if not 1 <= len(out) <= 6:
+        raise ValueError("frames: 1 to 6 frames expected")
+    return tuple(out)
+
+
+def _genetic_code(code):
+    """-> the 64 bytes of a built-in NCBI table id or of a 64-character code string (TCAG order)."""
+    if isinstance(code, (str, bytes)):
+        b = code.encode("latin-1") if isinstance(code, str) else code
+        if len(b) != 64 or not all(0x21 <= x <= 0x7E for x in b):
+            raise ValueError("genetic_code: a string of 64 printable ASCII characters (TCAG order) expected")
+        return b
+    try:
+        code = operator.index(code)
+    except TypeError:
+        raise ValueError(f"genetic_code must be one of {_GENETIC_CODES} or a 64-character string, got {code!r}") from None
+    if code not in _GENETIC_CODES:
+        raise ValueError(f"genetic_code must be one of {_GENETIC_CODES} or a 64-character string, got {code}")
+    return capi.genetic_code(code)
+
+
+def _translate_spec(translate, genetic_code, tokenizer=None, rc=None, seq_index_base=0):
+    """Validate the translation arguments (ValueError before anything is staged) -> None (no translation) or ``(frames,
+    code64)``.  ``tokenizer`` (None for ``translate_packed``) must be a protein alphabet or BYTES; ``rc`` must be None (the
+    reverse frames are the other strand); ``seq_index_base * F`` must fit int64 (seeded draws use the output index)."""
+    if translate is None:
+        if not (isinstance(genetic_code, int) and genetic_code == 1):
+            raise ValueError("genetic_code is given without translate=")
+        return None
+    frames, code = _frames(translate), _genetic_code(genetic_code)
+    if tokenizer is not None:
+        key = descriptor(tokenizer).key.decode("latin-1").upper()
+        if key not in _TRANSLATE_KEYS:
+            raise ValueError(f"translate= gives proteins: it needs a protein tokenizer or BYTES ({', '.join(_TRANSLATE_KEYS)}), "
+                             f"got {key}")
+    if rc is not None:
+        raise ValueError("rc cannot be combined with translate=: the reverse frames (-1, -2, -3) are the other strand")
+    if not _INT64_MIN <= int(seq_index_base) * len(frames) <= _INT64_MAX:
+        raise ValueError(f"seq_index_base * frames = {int(seq_index_base) * len(frames)} overflows int64")
+    return frames, code
+
+
+def _out_base(seq_index_base, tr):
+    """The global index of a consumer's first output sequence: seeded draws of a translated batch are keyed by
+    (seq_index_base + i) * F + f."""
+    return seq_index_base if tr is None else int(seq_index_base) * len(tr[0])
+
+
+def _translate_host_offsets(h_offs, n, frames):
+    """-> the translated batch's offsets (n F + 1, from 0) of host offsets, in numpy; ValueError on offsets the kernels
+    must not index with."""
+    o = np.asarray(h_offs[:n + 1], dtype=np.int64)
+    lens = np.diff(o)
+    if n > 0 and (int(o[0]) < 0 or int(lens.min()) < 0):
+        raise ValueError("offsets must start at or after 0 and be non-decreasing")
+    L = np.stack([np.maximum(lens - (abs(f) - 1), 0) // 3 for f in frames], 1)
+    out = np.zeros(n * len(frames) + 1, dtype=np.int64)
+    np.cumsum(L.reshape(-1), out=out[1:])
+    return out
+
+
+def _sized_host(h_offs, n, crop_len, tr):
+    """-> (offsets from 0 of the batch after translation and crop, (sum, max) of its lengths, translated bytes or None) of
+    host offsets."""
+    if tr is None:
+        return (*_crop_host_extent(h_offs, n, crop_len), None)
+    t = _translate_host_offsets(h_offs, n, tr[0])
+    return (*_crop_host_extent(t, n * len(tr[0]), crop_len), int(t[-1]))
+
+
+def _apply_translate(r, tr, total):
+    """Translate the resolved batch (validated offsets, ``total`` output bytes) into fresh device buffers; r then
+    describes the n F protein sequences."""
+    torch = _torch()
+    frames, code = tr
+    dev = torch.device("cuda", r.device)
+    out_b = torch.empty(max(total, 1), dtype=torch.uint8, device=dev)  # (never a null pointer)
+    out_o = torch.empty(r.nseq * len(frames) + 1, dtype=torch.int64, device=dev)
+    # an all-empty batch may have no residue buffer at all; nothing is read from it then
+    capi.translate(r.device, r.stream, r.d_bytes or out_b, r.d_offs, r.nseq, frames, code, out_b, out_o)
+    r.keep += [out_b, out_o]
+    r.d_bytes, r.d_offs, r.base, r.nseq = out_b.data_ptr(), out_o.data_ptr(), 0, out_o.numel() - 1
+
+
 def _row_residues(tokenizer, padlen):
     return padlen - int(tokenizer.includes_bos()) - int(tokenizer.includes_eos())
 
 
 def batch_onehot_encode_bcl(tokenizer, batch, padlen=-1, destchar="f", mask=None, device=None, *, augment=0, augment_frac=1.0,
-                            seed=0, seq_index_base=0, crop=None, crop_len=None, rc=None, rc_prob=None):
+                            seed=0, seq_index_base=0, crop=None, crop_len=None, rc=None, rc_prob=None, translate=None, genetic_code=1):
     """One-hot ``(batch, alphabet_size, padlen)`` tensor (CNN layout), default float32.
 
     Element ``[i, c, p]`` equals ``batch_onehot_encode(...)[p, i, c]`` (src/tokenize.h:345-368), i.e. the result of the
     reference's rearrange + float (bioseq/loaders.py:74-75).  ``mask``: uint8, one entry per residue of ``bytes``
-    (packed batches only, not with ``crop`` or ``rc``).  ``crop``: as ``batch_tokenize_cropped``; ``rc`` / ``rc_prob``: as
-    ``batch_tokenize_revcomp``."""
+    (packed batches only, not with ``crop``, ``rc`` or ``translate``).  ``crop``: as ``batch_tokenize_cropped``; ``rc`` /
+    ``rc_prob``: as ``batch_tokenize_revcomp``; ``translate`` / ``genetic_code``: as ``batch_tokenize_translated``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     padlen = _default_padlen(batch, tokenizer, padlen)
     kind, dtype = _dtype_of(destchar)
+    tr = _translate_spec(translate, genetic_code, tokenizer, rc, seq_index_base)
+    if tr is not None and mask is not None:
+        raise ValueError("mask covers the nucleotides: it cannot be combined with translate")
+    seq_index_base = _out_base(seq_index_base, tr)
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
     if crop is not None and mask is not None:
         raise ValueError("mask covers the uncropped residues: it cannot be combined with crop")
     rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment)
     if rc is not None and mask is not None:
         raise ValueError("mask covers the unflipped residues: it cannot be combined with rc")
-    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop, rc=rc)
+    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop, rc=rc, translate=tr)
     try:
         _check_lengths(r, padlen, tok, onehot=True)
         d_mask = None
@@ -464,16 +587,18 @@ def batch_onehot_encode_bcl(tokenizer, batch, padlen=-1, destchar="f", mask=None
 
 
 def batch_embed(tokenizer, batch, weight, padlen=-1, batch_first=True, device=None, *, augment=0, augment_frac=1.0, seed=0,
-                seq_index_base=0, crop=None, crop_len=None, rc=None, rc_prob=None):
+                seq_index_base=0, crop=None, crop_len=None, rc=None, rc_prob=None, translate=None, genetic_code=1):
     """``weight[tokens]`` for the tokens of ``batch_tokenize(batch, padlen, batch_first=batch_first)`` without
     materialising them: ``(batch, padlen, dim)`` or ``(padlen, batch, dim)``, dtype and device of ``weight``.
 
     ``weight``: ``(rows >= alphabet_size, dim)`` CUDA tensor (an ``nn.Embedding.weight``); ``dim * itemsize`` must be
     a multiple of 16 bytes.  Forward only (no autograd graph is recorded).  ``crop``: as ``batch_tokenize_cropped``; ``rc`` /
-    ``rc_prob``: as ``batch_tokenize_revcomp``."""
+    ``rc_prob``: as ``batch_tokenize_revcomp``; ``translate`` / ``genetic_code``: as ``batch_tokenize_translated``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     padlen = _default_padlen(batch, tokenizer, padlen)
+    tr = _translate_spec(translate, genetic_code, tokenizer, rc, seq_index_base)
+    seq_index_base = _out_base(seq_index_base, tr)
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
     rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment)
     w = weight.detach()
@@ -483,7 +608,7 @@ def batch_embed(tokenizer, batch, weight, padlen=-1, batch_first=True, device=No
         w = w.contiguous()
     row_bytes = w.shape[1] * w.element_size()
     r = _resolve(batch, w.device if device is None else device, _augment_args(augment, augment_frac, seed, seq_index_base),
-                 crop=crop, rc=rc)
+                 crop=crop, rc=rc, translate=tr)
     try:
         if r.device != w.device.index:
             raise ValueError("weight and batch live on different devices")
@@ -541,15 +666,17 @@ def crop_packed(bytes_cuda, offsets_cuda, crop_len, *, crop="random", seed=0, se
 
 
 def batch_tokenize_cropped(tokenizer, batch, padlen, destchar="B", batch_first=True, device=None, *, crop="random", crop_len=None,
-                           seed=0, seq_index_base=0, augment=0, augment_frac=1.0, rc=None, rc_prob=None):
+                           seed=0, seq_index_base=0, augment=0, augment_frac=1.0, rc=None, rc_prob=None, translate=None,
+                           genetic_code=1):
     """``batch_tokenize`` of the batch with every sequence cropped to ``crop_len`` residues on the device (default and
     maximum: ``padlen - bos - eos``): stage -> crop -> augment -> tokenize.  ``crop``: ``"random"`` or ``"head"``, as
     :func:`crop_packed` (same ``seed`` / ``seq_index_base``).  ``rc`` / ``rc_prob``: the windows are then flipped, as
-    :func:`batch_tokenize_revcomp` does."""
+    :func:`batch_tokenize_revcomp` does.  ``translate`` / ``genetic_code``: the DNA is first translated, as
+    :func:`batch_tokenize_translated` does, and the proteins are cropped (``crop_len`` in amino acids)."""
     if crop is None:
         raise ValueError("batch_tokenize_cropped: crop must be 'head' or 'random'")
     return _tokenize_padded(tokenizer, batch, padlen, destchar, batch_first, device, crop, crop_len, seed, seq_index_base,
-                            augment, augment_frac, rc, rc_prob)
+                            augment, augment_frac, rc, rc_prob, translate, genetic_code)
 
 
 def batch_tokenize_revcomp(tokenizer, batch, padlen, destchar="B", batch_first=True, device=None, *, rc="random", rc_prob=None,
@@ -570,14 +697,16 @@ def batch_tokenize_revcomp(tokenizer, batch, padlen, destchar="B", batch_first=T
 
 
 def _tokenize_padded(tokenizer, batch, padlen, destchar, batch_first, device, crop, crop_len, seed, seq_index_base, augment,
-                     augment_frac, rc, rc_prob):
+                     augment_frac, rc, rc_prob, translate=None, genetic_code=1):
     torch = _torch()
     tok = descriptor(tokenizer)
     padlen = _default_padlen(batch, tokenizer, padlen)
     kind, dtype = _dtype_of(destchar)
+    tr = _translate_spec(translate, genetic_code, tokenizer, rc, seq_index_base)
+    seq_index_base = _out_base(seq_index_base, tr)
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
     rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment)
-    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop, rc=rc)
+    r = _resolve(batch, device, _augment_args(augment, augment_frac, seed, seq_index_base), crop=crop, rc=rc, translate=tr)
     try:
         _check_lengths(r, padlen, tok, onehot=False)
         shape = (r.nseq, padlen) if batch_first else (padlen, r.nseq)
@@ -659,7 +788,7 @@ def _varlen_extent_host(h_offs, n, k):
 
 
 def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None, *, crop=None, crop_len=None, seed=0, seq_index_base=0,
-                          rc=None, rc_prob=None):
+                          rc=None, rc_prob=None, translate=None, genetic_code=1):
     """Tokens of every sequence of ``batch`` back to back, without padding: a :class:`VarlenBatch`.
 
     Row ``i`` (``tokens[cu_seqlens[i]:cu_seqlens[i + 1]]``) equals ``batch_tokenize(batch, padlen=P, batch_first=True,
@@ -668,22 +797,25 @@ def batch_tokenize_varlen(tokenizer, batch, destchar="B", device=None, *, crop=N
     than 2^31 - 1 tokens raises ``ValueError``.  Host batches are sized from their host offsets without synchronising;
     CUDA batches pay one synchronisation (the extent is read back).  ``crop`` / ``crop_len`` (required with ``crop``):
     every sequence is cropped first, as :func:`crop_packed` does.  ``rc`` / ``rc_prob``: then flipped, as
-    :func:`batch_tokenize_revcomp` does (``"both"`` gives ``2n`` rows)."""
+    :func:`batch_tokenize_revcomp` does (``"both"`` gives ``2n`` rows).  ``translate`` / ``genetic_code``: the DNA is
+    first translated, as :func:`batch_tokenize_translated` does (``crop_len`` then counts amino acids)."""
+    tr = _translate_spec(translate, genetic_code, tokenizer, rc, seq_index_base)
+    seq_index_base = _out_base(seq_index_base, tr)
     return _tokenize_varlen(tokenizer, batch, destchar, device, crop=_crop_spec(crop, crop_len, seed, seq_index_base),
-                            rc=_rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer))
+                            rc=_rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer), translate=tr)
 
 
-def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None, mlm=None, crop=None, rc=None):
+def _tokenize_varlen(tokenizer, batch, destchar, device, augment=None, mlm=None, crop=None, rc=None, translate=None):
     """batch_tokenize_varlen; ``augment``: BLOSUM62 arguments as ``_augment_args`` makes them (FlatFileDataset);
     ``mlm``: a ``capi.MLMDesc`` -- then ``(VarlenBatch, labels)`` is returned; ``crop``: from ``_crop_spec``; ``rc``: from
-    ``_rc_spec``."""
+    ``_rc_spec``; ``translate``: from ``_translate_spec``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
     k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
     extent = []
     r = _resolve(batch, device, augment, before_stage=lambda h_offs, n: extent.extend(_varlen_extent_host(h_offs, n, k)),
-                 crop=crop, rc=rc)
+                 crop=crop, rc=rc, translate=translate)
     try:
         if r.h_offs is not None:
             total, max_seqlen = extent
@@ -760,7 +892,7 @@ def _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignor
 
 def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *, varlen=False, maskfrac=0.15, mask_prob=0.8,
                        random_prob=0.1, mask_token=None, ignore_index=-100, seed=0, seq_index_base=0, augment=0,
-                       augment_frac=1.0, crop=None, crop_len=None, rc=None, rc_prob=None):
+                       augment_frac=1.0, crop=None, crop_len=None, rc=None, rc_prob=None, translate=None, genetic_code=1):
     """A masked-language-model batch in one launch: :class:`MLMBatch` ``(inputs, labels)``.
 
     ``inputs`` start from ``batch_tokenize(batch, padlen, batch_first=True, destchar=destchar)`` (``varlen=False``:
@@ -777,21 +909,25 @@ def batch_tokenize_mlm(tokenizer, batch, padlen=-1, destchar="B", device=None, *
     mask.  ``crop`` / ``crop_len``: every sequence is cropped before both (as :func:`batch_tokenize_cropped`, same seed;
     ``varlen=True`` needs an explicit ``crop_len``); residue positions are then positions within the window.  ``rc`` /
     ``rc_prob``: "always" or "random" (not "both"), after the crop and before the mask, as :func:`batch_tokenize_revcomp`
-    does; residue positions are then positions in the flipped window."""
+    does; residue positions are then positions in the flipped window.  ``translate`` / ``genetic_code``: the DNA is first
+    translated, as :func:`batch_tokenize_translated` does; positions are then amino acids and the draw for output row
+    ``(i, f)`` is keyed by ``(seq_index_base + i) * F + f``."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
+    tr = _translate_spec(translate, genetic_code, tokenizer, rc, seq_index_base)
+    seq_index_base = _out_base(seq_index_base, tr)
     mlm = _mlm_desc(tok, destchar, maskfrac, mask_prob, random_prob, mask_token, ignore_index, seed, seq_index_base)
     rc = _rc_spec(rc, rc_prob, seed, seq_index_base, tokenizer, augment, mlm=True)
     augment = _augment_args(augment, augment_frac, seed, seq_index_base)
     if varlen:
         _padlen("batch_tokenize_mlm", padlen, varlen)
         crop = _crop_spec(crop, crop_len, seed, seq_index_base)
-        vb, labels = _tokenize_varlen(tokenizer, batch, destchar, device, augment, mlm, crop, rc)
+        vb, labels = _tokenize_varlen(tokenizer, batch, destchar, device, augment, mlm, crop, rc, tr)
         return MLMBatch(vb, labels)
     padlen = _default_padlen(batch, tokenizer, padlen)
     crop = _crop_spec(crop, crop_len, seed, seq_index_base, _row_residues(tokenizer, padlen))
-    r = _resolve(batch, device, augment, crop=crop, rc=rc)
+    r = _resolve(batch, device, augment, crop=crop, rc=rc, translate=tr)
     try:
         _check_lengths(r, padlen, tok, onehot=False)
         dev = torch.device("cuda", r.device)
@@ -834,7 +970,8 @@ class _SeqPackPlan:
 
 def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None, *, rows=None, mlm=False, maskfrac=0.15,
                            mask_prob=0.8, random_prob=0.1, mask_token=None, ignore_index=-100, crop=None, crop_len=None,
-                           augment=0, augment_frac=1.0, seed=0, seq_index_base=0, rc=None, rc_prob=None):
+                           augment=0, augment_frac=1.0, seed=0, seq_index_base=0, rc=None, rc_prob=None, translate=None,
+                           genetic_code=1):
     """Sequence packing: every sequence of ``batch`` whole, laid end to end in rows of ``row_len`` tokens -- a
     :class:`SeqPackBatch` of fixed shape ``(rows, row_len)`` with almost no padding.
 
@@ -850,12 +987,15 @@ def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None,
     ``seq_index_base``) writes them per sequence, padding labels ``ignore_index``.  ``crop`` / ``crop_len`` (default
     ``row_len - bos - eos``) and ``augment`` as for the other consumers: stage -> crop -> augment -> pack.  Every
     sequence must fit a row (ValueError otherwise).  ``rc`` / ``rc_prob``: sequences are flipped after the crop, as
-    :func:`batch_tokenize_revcomp` does (``"both"``, not with ``mlm``, packs ``2n`` sequences).  Host batches are planned
-    from their host offsets without synchronising; CUDA batches pay one read-back of their offsets, which also validates
-    them."""
+    :func:`batch_tokenize_revcomp` does (``"both"``, not with ``mlm``, packs ``2n`` sequences).  ``translate`` /
+    ``genetic_code``: the DNA is first translated, as :func:`batch_tokenize_translated` does, and the ``n F`` proteins are
+    packed.  Host batches are planned from their host offsets without synchronising; CUDA batches pay one read-back of
+    their offsets, which also validates them."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
+    tr = _translate_spec(translate, genetic_code, tokenizer, rc, seq_index_base)
+    seq_index_base = _out_base(seq_index_base, tr)
     k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
     try:
         row_len = operator.index(row_len)
@@ -879,15 +1019,17 @@ def batch_tokenize_seqpack(tokenizer, batch, row_len, destchar="B", device=None,
     p = _parse(batch)
     checked = None
     if p.bytes is not None:  # planned before anything is staged (a CUDA batch: from its offsets, read back once)
-        cuda, sized, h = isinstance(p.offsets, torch.Tensor), crop is not None or rc is not None, p.offsets
+        cuda, sized, h = isinstance(p.offsets, torch.Tensor), crop is not None or rc is not None or tr is not None, p.offsets
         if cuda:
             h = h.cpu().numpy()
             _nseq(h, p.bytes.numel())
         n = h.size - 1
         if cuda or sized:  # (this also validates the offsets)
-            cropped, checked = _crop_host_extent(h, n, crop[1] if crop is not None else _UNCROPPED)
-        make_plan(*_rc_host_offsets(cropped if sized else h, n, rc))
-    r = _resolve(p, device, augment, before_stage=None if plan else make_plan, crop=crop, rc=rc, checked=checked)
+            cropped, checked, tr_total = _sized_host(h, n, crop[1] if crop is not None else _UNCROPPED, tr)
+            if tr is not None:
+                checked = (*checked, tr_total)
+        make_plan(*_rc_host_offsets(cropped if sized else h, n * len(tr[0]) if tr is not None else n, rc))
+    r = _resolve(p, device, augment, before_stage=None if plan else make_plan, crop=crop, rc=rc, checked=checked, translate=tr)
     try:
         p = plan[0]
         dev = torch.device("cuda", r.device)
@@ -969,7 +1111,7 @@ def _kmer_check_extent(extent, padlen, varlen):
 
 
 def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=None, *, stride=1, tail="drop", varlen=False,
-                        crop=None, crop_len=None, seed=0, seq_index_base=0, rc=None, rc_prob=None):
+                        crop=None, crop_len=None, seed=0, seq_index_base=0, rc=None, rc_prob=None, translate=None, genetic_code=1):
     """K-mer tokens of every sequence of ``batch``, written by one kernel (padding-free: three small ones).
 
     Sequence ``i`` of ``n`` residues gives ``[BOS] k-mer ids [single-residue ids] [EOS]``: ``m = (n - k) // stride + 1``
@@ -984,11 +1126,15 @@ def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=Non
     be given); more than 2^31 - 1 tokens raise ValueError.  ``destchar`` defaults to int32 (``"i"``), which holds every
     vocabulary the rule allows; a kind too narrow for ``vocab_size`` raises ValueError.  ``crop`` / ``crop_len`` (required
     with ``crop``, in residues): every sequence is cropped first, as :func:`crop_packed` does.  ``rc`` / ``rc_prob``: then
-    flipped, as :func:`batch_tokenize_revcomp` does, so the k-mers are those of the reverse complement.  Host batches are
-    sized from their host offsets without synchronising; CUDA batches pay one read-back (two when cropped)."""
+    flipped, as :func:`batch_tokenize_revcomp` does, so the k-mers are those of the reverse complement.  ``translate`` /
+    ``genetic_code``: the DNA is first translated, as :func:`batch_tokenize_translated` does, and the k-mers are those of
+    the proteins (a protein tokenizer).  Host batches are sized from their host offsets without synchronising; CUDA
+    batches pay one read-back (two when cropped or translated)."""
     torch = _torch()
     tok = descriptor(tokenizer)
     kind, dtype = _dtype_of(destchar)
+    tr = _translate_spec(translate, genetic_code, tokenizer, rc, seq_index_base)
+    seq_index_base = _out_base(seq_index_base, tr)
     km = _kmer_desc(tokenizer, k, stride, tail)
     limit = _mask_token_limit(destchar)
     if km.vocab_size - 1 > limit:
@@ -1016,10 +1162,11 @@ def batch_tokenize_kmer(tokenizer, batch, k, padlen=-1, destchar="i", device=Non
         extent = [total * (2 if rc[0] == capi.RC_BOTH else 1), longest]
         _kmer_check_extent(extent, padlen, varlen)
         checked = True
-    r = _resolve(p, device, before_stage=before_stage, crop=crop, rc=rc, checked=checked)
+    r = _resolve(p, device, before_stage=before_stage, crop=crop, rc=rc, checked=checked, translate=tr)
     try:
         if r.h_offs is None and checked is None:  # a CUDA batch: one reduction and read-back, which also validates its offsets
-            extent = capi.kmer_extent_device(r.device, r.stream, r.d_offs, r.nseq, km, nbytes=-1 if crop is not None else p.bytes.numel())
+            fresh = crop is not None or tr is not None  # (offsets of buffers _resolve wrote)
+            extent = capi.kmer_extent_device(r.device, r.stream, r.d_offs, r.nseq, km, nbytes=-1 if fresh else p.bytes.numel())
             _kmer_check_extent(extent, padlen, varlen)
         dev = torch.device("cuda", r.device)
         if varlen:
@@ -1235,3 +1382,84 @@ def untile(values, tiled, *, col0=None):
                          stride, cu, col0, tiled.seq_offsets, n, tiled.window, tiled.stride, _TILE_TAILS[tiled.tail], tiled.seq_ptr,
                          tiled.seq_index.numel(), tiled.strands, flipped, out)
     return UntiledBatch(out, tiled.seq_offsets)
+
+
+TranslatedBatch = collections.namedtuple("TranslatedBatch", ["bytes", "offsets", "seq_index", "frame", "frames"])
+TranslatedBatch.__doc__ = """The reading frames of a packed DNA batch, as a packed protein batch: ``bytes`` (uint8 amino-acid letters,
+``*`` for stops, ``X`` where a codon is ambiguous or holds an invalid byte) and ``offsets`` (int64, from 0) of the ``n F``
+output sequences, sequence-major; ``seq_index`` (int64, one per output sequence: ``w // F``, its input sequence); ``frame``
+(int8, one per output sequence: ``frames[w % F]``); ``frames`` (the tuple of the F frames)."""
+
+
+def translate_packed(bytes_cuda, offsets_cuda, *, frames=1, genetic_code=1):
+    """Translate every sequence of a packed CUDA DNA / RNA batch into the reading frames ``frames``: a
+    :class:`TranslatedBatch`; the input is not modified.
+
+    ``frames``: one of 1, 2, 3, -1, -2, -3 (frame +k reads from offset k - 1, frame -k the reverse complement from offset
+    k - 1), a list or tuple of distinct ones (kept in that order), ``"forward"`` = (1, 2, 3) or ``"six"`` = (1, 2, 3, -1,
+    -2, -3).  Output sequence ``w = i * F + f`` is frame ``frames[f]`` of sequence ``i``, ``(len - k + 1) // 3`` amino acids
+    long (a trailing partial codon is dropped; sequences shorter than 3 give empty rows).  ``genetic_code``: an NCBI
+    table id (1 standard, 2 vertebrate mitochondrial, 4 mold / protozoan mitochondrial, 5 invertebrate mitochondrial, 6
+    ciliate, 11 bacterial) or 64 letters in TCAG order.  Residues are case-insensitive IUPAC codes (U = T); a codon whose
+    expansions all give one amino acid gives it, any other gives ``X``.  The exact rule is documented with
+    ``bsq_translate`` in include/bsq.h.  ``(tb.bytes, tb.offsets)`` is a packed CUDA batch that every consumer takes with a
+    protein tokenizer.  One synchronisation: the offsets are validated and the output's size is read back."""
+    torch = _torch()
+    _packed_cuda("translate_packed", bytes_cuda, offsets_cuda)
+    fr, code = _translate_spec(frames, genetic_code)
+    n, F = _nseq(offsets_cuda), len(fr)
+    dev = bytes_cuda.device
+    stream = torch.cuda.current_stream(dev.index).cuda_stream
+    total, _, _ = capi.translate_extent_device(dev.index, stream, offsets_cuda, n, fr, nbytes=bytes_cuda.numel())
+    out_b = torch.empty(max(total, 1), dtype=torch.uint8, device=dev)
+    out_o = torch.empty(n * F + 1, dtype=torch.int64, device=dev)
+    src = bytes_cuda if bytes_cuda.numel() > 0 else out_b  # (an all-empty batch: nothing is read)
+    capi.translate(dev.index, stream, src, offsets_cuda, n, fr, code, out_b, out_o)
+    seq_index = torch.arange(n, dtype=torch.int64, device=dev).repeat_interleave(F)
+    frame = torch.tensor(fr, dtype=torch.int8, device=dev).repeat(n)
+    return TranslatedBatch(out_b[:total], out_o, seq_index, frame, fr)
+
+
+def batch_tokenize_translated(tokenizer, batch, padlen=None, destchar="B", device=None, *, frames=1, genetic_code=1, varlen=False,
+                              crop=None, crop_len=None, seed=0, seq_index_base=0, augment=0, augment_frac=1.0):
+    """Tokens of the reading frames of every DNA / RNA sequence of ``batch``: stage -> translate -> crop -> augment ->
+    tokenize, on the device.
+
+    ``frames`` / ``genetic_code``: as :func:`translate_packed`; row ``w = i * F + f`` is frame ``frames[f]`` of sequence
+    ``i``.  ``tokenizer``: a protein alphabet (PROTEIN, AMINO20 and the reduced ones) or BYTES.  PROTEIN / AMINO20 have no
+    ``*`` or ``X``, so stops and ambiguous codons tokenize as every invalid byte does (id 0).  ``varlen=False``: a padded
+    ``(n F, padlen)`` tensor as ``batch_tokenize(..., batch_first=True)`` writes it; ``padlen`` defaults to the longest
+    translated (and cropped) row + bos + eos.  ``varlen=True``: a :class:`VarlenBatch` (``padlen`` must not be given).
+    ``crop`` / ``crop_len`` (in amino acids; default ``padlen - bos - eos``, required without ``padlen``) and ``augment``
+    (BLOSUM62, on the proteins) as for the other consumers, with seeded draws keyed by the output index
+    ``(seq_index_base + i) * F + f``.  Host batches are sized from their host offsets without synchronising; CUDA batches
+    pay one read-back, which also validates their offsets."""
+    torch = _torch()
+    tok = descriptor(tokenizer)
+    kind, dtype = _dtype_of(destchar)
+    tr = _translate_spec(frames, genetic_code, tokenizer, None, seq_index_base)
+    base = _out_base(seq_index_base, tr)
+    augment = _augment_args(augment, augment_frac, seed, base)
+    padlen = _padlen("batch_tokenize_translated", padlen, varlen)
+    if padlen is not None and padlen < 1:
+        raise ValueError(f"padlen must be >= 1, got {padlen}")
+    if varlen or padlen is None:
+        if crop is not None and crop_len is None:
+            raise ValueError("batch_tokenize_translated: crop without padlen needs an explicit crop_len")
+        crop = _crop_spec(crop, crop_len, seed, base)
+    else:
+        crop = _crop_spec(crop, crop_len, seed, base, _row_residues(tokenizer, padlen))
+    if varlen:
+        return _tokenize_varlen(tokenizer, batch, destchar, device, augment, crop=crop, translate=tr)
+    r = _resolve(batch, device, augment, crop=crop, translate=tr)
+    try:
+        k = int(tokenizer.includes_bos()) + int(tokenizer.includes_eos())
+        if padlen is None:
+            padlen = r.extent[1] + k
+        out = torch.empty((r.nseq, padlen), dtype=dtype, device=torch.device("cuda", r.device))
+        if r.nseq > 0 and padlen > 0:
+            _check_lengths(r, padlen, tok, onehot=False)
+            capi.tokenize(r.device, r.stream, r.d_bytes, r.d_offs, r.nseq, padlen, tok, True, kind, out)
+        return out
+    finally:
+        r.release()

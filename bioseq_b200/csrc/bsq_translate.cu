@@ -1,0 +1,546 @@
+// K14: translation of a packed DNA / RNA batch into protein reading frames under a genetic code (sm_100a).
+//
+// Semantics (include/bsq.h, bsq_translate): every byte is an IUPAC base set (a 4-bit mask, A = 1, C = 2, G = 4, T = 8,
+// invalid = 0) and every codon the one letter all expansions of its three base sets agree on, else 'X'.  Both rules are
+// tables built once on the host by bsq_translate_table -- the only statement of them in the library -- and handed to the
+// kernel as parameters: masks[256] (and their complements, the 4-bit reversals) and codons[4096] indexed by
+// m0 << 8 | m1 << 4 | m2.  Output sequence w = i * F + f is frame frames[f] of input sequence i; frame +k has
+// max(0, (len - k + 1) / 3) amino acids read from offset k - 1, frame -k as many read from the reverse complement.
+// tr_len below is the only statement of that length (host extent, device extent and both kernels use it).
+//
+// K14a: row_scan_kernel (+ row_carry_kernel past 1024 sequences, bsq_kernels.cuh) scans the per-sequence output bytes
+//       (the sum of its F frame lengths, TranslateCount) into stream-ordered scratch S[n + 1].  Entries that do not close a
+//       scan CTA lack their CTA's carry; seq_base adds it where it is read, so no fix-up pass runs.
+// K14b: translate_kernel -- a grid-stride pass over the n * F + 1 output offsets (each sequence's base plus the lengths of
+//       its earlier frames), then the bytes: a flat map over the 16-byte aligned output vectors in tiles of 64 KiB on a
+//       persistent grid in static order, the structure K12 and K13a share.  Per tile the CTA finds the tile's first
+//       sequence with a 256-ary search over S and stages the tile's sequence bases and source starts in shared memory
+//       (over-full tiles read global memory).  Per vector a binary search of that table gives the sequence of its first
+//       byte; every (sequence, frame) piece the vector touches then costs
+//         - one 48-byte source span (16 codons) as four clamped aligned 16-byte loads realigned with selects and funnel
+//           shifts; a reverse frame reads the mirrored span and reverses its bytes with PRMT, as K12 does;
+//         - 48 mask look-ups (the complemented mask table for a reverse frame) and 16 codon look-ups in shared memory;
+//         - a merge into the output vector by byte mask.
+//       A vector inside the output leaves as one st.global.cs.v4, the at most two partial vectors at its ends (any
+//       alignment) as byte stores.
+#include <cuda_runtime.h>
+
+#include <algorithm>
+#include <cstring>
+#include <string>
+
+#include "bsq_internal.h"
+#include "bsq_kernels.cuh"
+
+namespace bsq {
+
+namespace {
+
+// A frame in 4 bits: k - 1 in bits 0-1, bit 3 set for the reverse strand.  F frames are packed 4 bits each, so the kernels
+// index them with shifts instead of a run-time index into a parameter array.
+__host__ __device__ __forceinline__ uint32_t frame_code(uint32_t fcode, int f) { return (fcode >> (4 * f)) & 15u; }
+
+// amino acids of one frame of a sequence of len >= 0 nucleotides
+__host__ __device__ __forceinline__ int64_t tr_len(int64_t len, uint32_t fr) {
+    const int64_t skip = fr & 3u;
+    return len > skip ? (len - skip) / 3 : 0;
+}
+
+struct FrameSet {
+    uint32_t fcode;
+    int F;
+};
+
+__host__ __device__ __forceinline__ int64_t tr_row_total(int64_t len, const FrameSet &fs) {
+    int64_t t = 0;
+    for (int f = 0; f < fs.F; ++f) t += tr_len(len, frame_code(fs.fcode, f));
+    return t;
+}
+
+struct TranslateCount {
+    FrameSet fs;
+    __device__ __forceinline__ int64_t operator()(int64_t len) const { return tr_row_total(len, fs); }
+};
+
+// BSQ_ERR_ARG unless frames holds 1..6 distinct values of +-1, +-2, +-3; fills *fs
+int check_frames(const int8_t *frames, int nframes, FrameSet *fs) {
+    if (frames == nullptr || nframes < 1 || nframes > 6) return fail(BSQ_ERR_ARG, "frames: 1 to 6 distinct values of +-1, +-2, +-3 expected");
+    fs->fcode = 0;
+    fs->F = nframes;
+    for (int f = 0; f < nframes; ++f) {
+        const int v = frames[f];
+        if (v == 0 || v < -3 || v > 3) return fail(BSQ_ERR_ARG, "frames must be +-1, +-2 or +-3, got " + std::to_string(v));
+        for (int g = 0; g < f; ++g)
+            if (frames[g] == v) return fail(BSQ_ERR_ARG, "frame " + std::to_string(v) + " is given twice");
+        const uint32_t c = static_cast<uint32_t>((v > 0 ? v : -v) - 1) | (v < 0 ? 8u : 0u);
+        fs->fcode |= c << (4 * f);
+    }
+    return BSQ_OK;
+}
+
+int check_code(const char *code64) {
+    if (code64 == nullptr) return fail(BSQ_ERR_ARG, "null genetic code");
+    for (int c = 0; c < 64; ++c) {
+        const unsigned char b = static_cast<unsigned char>(code64[c]);
+        if (b < 0x21 || b > 0x7E)
+            return fail(BSQ_ERR_ARG, "genetic code: 64 printable ASCII characters (0x21..0x7E) expected; byte " + std::to_string(c) +
+                                         " is " + std::to_string(static_cast<int>(b)));
+    }
+    return BSQ_OK;
+}
+
+// The rule of include/bsq.h, built once: base sets of every byte and the letter of every triple of base sets.
+struct Tables {
+    uint8_t mask[256];
+    uint8_t codon[4096];
+};
+void build_tables(const char *code64, Tables *t) {
+    // each code, then the bases it stands for (upper and lower case alike)
+    static const char *const kSets[] = {"AA", "CC", "GG", "TT", "UT", "RAG", "YCT", "SCG", "WAT", "KGT", "MAC", "BCGT", "DAGT", "HACT",
+                                        "VACG", "NACGT"};
+    std::memset(t->mask, 0, sizeof(t->mask));
+    auto bit = [](char b) -> uint8_t { return b == 'A' ? 1 : b == 'C' ? 2 : b == 'G' ? 4 : 8; };
+    for (const char *s : kSets) {
+        uint8_t m = 0;
+        for (const char *p = s + 1; *p; ++p) m |= bit(*p);
+        t->mask[static_cast<uint8_t>(s[0])] = m;
+        t->mask[static_cast<uint8_t>(s[0] | 0x20)] = m;
+    }
+    static const int kTcag[4] = {2, 1, 3, 0};  // mask bit (A, C, G, T) -> index in TCAG order
+    for (int m0 = 0; m0 < 16; ++m0)
+        for (int m1 = 0; m1 < 16; ++m1)
+            for (int m2 = 0; m2 < 16; ++m2) {
+                char letter = 0;
+                bool agree = m0 && m1 && m2;
+                for (int b0 = 0; agree && b0 < 4; ++b0)
+                    for (int b1 = 0; agree && b1 < 4; ++b1)
+                        for (int b2 = 0; agree && b2 < 4; ++b2) {
+                            if (!((m0 >> b0) & 1) || !((m1 >> b1) & 1) || !((m2 >> b2) & 1)) continue;
+                            const char c = code64[16 * kTcag[b0] + 4 * kTcag[b1] + kTcag[b2]];
+                            if (letter == 0) letter = c;
+                            else if (letter != c) agree = false;
+                        }
+                t->codon[m0 << 8 | m1 << 4 | m2] = static_cast<uint8_t>(agree ? letter : 'X');
+            }
+}
+
+__host__ __device__ __forceinline__ uint8_t bitrev4(uint8_t m) {
+    return static_cast<uint8_t>(((m & 1) << 3) | ((m & 2) << 1) | ((m & 4) >> 1) | ((m & 8) >> 3));
+}
+
+constexpr int kTrThreads = 256;
+constexpr int kTrVecs = 16;                     // output vectors per thread and tile
+constexpr int kTrTile = kTrThreads * kTrVecs;   // 4096 vectors: 64 KiB of output per tile
+constexpr int kTrRowCap = 2048;                 // sequences a tile's table holds
+constexpr int kTrMinBlocks = 4;
+
+struct TrTables {
+    uint32_t mask[64], cmask[64];  // 256 masks and their complements, 4 per word
+    uint32_t codon[1024];          // 4096 letters, 4 per word
+};
+
+struct TrArgs {
+    const uint8_t *bytes;
+    const int64_t *offs;
+    const int64_t *S;  // K14a's scan (see seq_base)
+    int64_t n, total;
+    FrameSet fs;
+};
+
+// S[e] with its scan CTA's carry: the global exclusive prefix of the per-sequence output bytes (seq_base(n) = total)
+__device__ __forceinline__ int64_t seq_base(const TrArgs &a, int64_t e) {
+    int64_t v = __ldg(a.S + e);
+    if (e > kRowScan && (e % kRowScan) != 0 && e != a.n) v += __ldg(a.S + ((e - 1) / kRowScan) * kRowScan);
+    return v;
+}
+
+// The 48 bytes at address X (any alignment) as 12 little-endian words, from the aligned words at X & ~15 and the three
+// after it, each clamped to [lo, hi] (16-byte aligned); the shift is picked with selects, as in fetch16_clamped.
+__device__ __forceinline__ void fetch48_clamped(uintptr_t X, uintptr_t lo, uintptr_t hi, uint32_t t[12]) {
+    const uintptr_t a0 = X & ~uintptr_t(15);
+    const uint32_t s = static_cast<uint32_t>(X) & 15u;
+    uint32_t w[16];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const uint4 v = ldg16(clamp_word(a0 + 16 * k, lo, hi));
+        w[4 * k] = v.x;
+        w[4 * k + 1] = v.y;
+        w[4 * k + 2] = v.z;
+        w[4 * k + 3] = v.w;
+    }
+    const uint4 v3 = s != 0 ? ldg16(clamp_word(a0 + 48, lo, hi)) : make_uint4(0u, 0u, 0u, 0u);
+    w[12] = v3.x;
+    w[13] = v3.y;
+    w[14] = v3.z;
+    w[15] = v3.w;
+    const bool q2 = (s & 8u) != 0, q1 = (s & 4u) != 0;
+    uint32_t a[14], b[13];
+#pragma unroll
+    for (int k = 0; k < 14; ++k) a[k] = q2 ? w[k + 2] : w[k];
+#pragma unroll
+    for (int k = 0; k < 13; ++k) b[k] = q1 ? a[k + 1] : a[k];
+    const uint32_t sh = (s & 3u) * 8u;
+#pragma unroll
+    for (int k = 0; k < 12; ++k) t[k] = __funnelshift_r(b[k], b[k + 1], sh);
+}
+
+// The 16 letters of one (sequence, frame) piece for output bytes [q, q + 16): amino acid t0 + j of the frame lands in
+// byte j.  s / len: the sequence's source start and length; fr: the frame's code.
+__device__ __forceinline__ void tr_piece(int64_t q, int64_t ws, int64_t s, int64_t len, uint32_t fr, const TrArgs &a,
+                                         const uint8_t *mask, const uint8_t *cmask, const uint8_t *codon, uint32_t t[4]) {
+    const uintptr_t src0 = reinterpret_cast<uintptr_t>(a.bytes);
+    const int64_t t0 = q - ws, skip = fr & 3u;
+    const bool rev = (fr & 8u) != 0;
+    // forward: codon j is nucleotides skip + 3 (t0 + j) .. + 2; reverse: len - skip - 3 (t0 + j) - 3 .. - 1, read right to
+    // left -- byte 47 - 3j .. 45 - 3j of the 48 that end at len - skip - 3 t0
+    const int64_t X = rev ? s + len - skip - 3 * t0 - 48 : s + skip + 3 * t0;
+    const uintptr_t lo = (src0 + static_cast<uintptr_t>(s)) & ~uintptr_t(15);
+    const uintptr_t hi = (src0 + static_cast<uintptr_t>(s + len - 1)) & ~uintptr_t(15);
+    uint32_t w[12];
+    fetch48_clamped(src0 + static_cast<uintptr_t>(X), lo, hi, w);
+    if (rev) {
+#pragma unroll
+        for (int k = 0; k < 6; ++k) {
+            const uint32_t x = w[k];
+            w[k] = __byte_perm(w[11 - k], 0u, 0x0123);
+            w[11 - k] = __byte_perm(x, 0u, 0x0123);
+        }
+    }
+    const uint8_t *m = rev ? cmask : mask;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        uint32_t word = 0;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int p = 3 * (4 * k + j);
+            const uint32_t m0 = m[__byte_perm(w[p >> 2], 0u, 0x4440 + (p & 3))];
+            const uint32_t m1 = m[__byte_perm(w[(p + 1) >> 2], 0u, 0x4440 + ((p + 1) & 3))];
+            const uint32_t m2 = m[__byte_perm(w[(p + 2) >> 2], 0u, 0x4440 + ((p + 2) & 3))];
+            word += static_cast<uint32_t>(codon[m0 << 8 | m1 << 4 | m2]) << (8 * j);
+        }
+        t[k] = word;
+    }
+}
+
+struct SeqRow {
+    int64_t base, next, start, end;  // output bases of this sequence and the next; its source offsets
+};
+
+// Output bytes [q, q + 16) (out + q is 16-byte aligned), whose first byte in [0, total) lies in sequence i; row_of(i) is
+// its SeqRow (from the tile's table or global memory).
+template <typename ROW>
+__device__ __forceinline__ void tr_vector(int64_t q, int64_t i, const TrArgs &a, const ROW &row_of, const uint8_t *mask,
+                                          const uint8_t *cmask, const uint8_t *codon, uint8_t *dst) {
+    uint32_t res[4] = {0u, 0u, 0u, 0u};
+    const int64_t x = max(q, int64_t(0));
+    for (;;) {
+        const SeqRow r = row_of(i);
+        if (r.next > r.base) {
+            const int64_t len = r.end - r.start;
+            int64_t ws = r.base;
+            for (int f = 0; f < a.fs.F && ws < q + 16; ++f) {
+                const uint32_t fr = frame_code(a.fs.fcode, f);
+                const int64_t L = tr_len(len, fr);
+                if (L > 0 && ws + L > x) {
+                    uint32_t t[4];
+                    tr_piece(q, ws, r.start, len, fr, a, mask, cmask, codon, t);
+                    const int k0 = static_cast<int>(min(max(ws - q, int64_t(0)), int64_t(16)));
+                    const int k1 = static_cast<int>(min(max(ws + L - q, int64_t(0)), int64_t(16)));
+#pragma unroll
+                    for (int w = 0; w < 4; ++w) {
+                        const uint32_t mk = lt_mask(k1, w) & ~lt_mask(k0, w);
+                        res[w] = (res[w] & ~mk) | (t[w] & mk);
+                    }
+                }
+                ws += L;
+            }
+        }
+        if (r.next >= q + 16 || i + 1 >= a.n) break;
+        ++i;
+    }
+    if (q >= 0 && q + 16 <= a.total) {
+        __stcs(reinterpret_cast<uint4 *>(dst), make_uint4(res[0], res[1], res[2], res[3]));
+    } else {
+#pragma unroll
+        for (int k = 0; k < 16; ++k)
+            if (q + k >= 0 && q + k < a.total) dst[k] = static_cast<uint8_t>(res[k >> 2] >> (8 * (k & 3)));
+    }
+}
+
+__global__ void __launch_bounds__(kTrThreads, kTrMinBlocks)
+translate_kernel(TrArgs a, const __grid_constant__ TrTables tbl, uint8_t *__restrict__ out, int64_t *__restrict__ out_offs) {
+    __shared__ __align__(16) uint8_t s_mask[256];
+    __shared__ __align__(16) uint8_t s_cmask[256];
+    __shared__ __align__(16) uint8_t s_codon[4096];
+    __shared__ int64_t s_base[kTrRowCap];  // output bases of sequences i0, i0 + 1, ...
+    __shared__ int64_t s_src[kTrRowCap];   // ... and their source starts
+    const int tid = threadIdx.x;
+    if (tid < 64) {
+        reinterpret_cast<uint32_t *>(s_mask)[tid] = tbl.mask[tid];
+        reinterpret_cast<uint32_t *>(s_cmask)[tid] = tbl.cmask[tid];
+    }
+    for (int k = tid; k < 1024; k += kTrThreads) reinterpret_cast<uint32_t *>(s_codon)[k] = tbl.codon[k];
+    a.total = seq_base(a, a.n);
+    // output offsets: sequence i's base, then each frame's length
+    const int64_t nw = a.n * a.fs.F;
+    for (int64_t w = blockIdx.x * static_cast<int64_t>(kTrThreads) + tid; w <= nw; w += static_cast<int64_t>(gridDim.x) * kTrThreads) {
+        if (w == nw) {
+            out_offs[nw] = a.total;
+            break;
+        }
+        const int64_t i = w / a.fs.F;
+        const int f = static_cast<int>(w - i * a.fs.F);
+        const int64_t len = __ldg(a.offs + i + 1) - __ldg(a.offs + i);
+        int64_t o = seq_base(a, i);
+        for (int g = 0; g < f; ++g) o += tr_len(len, frame_code(a.fs.fcode, g));
+        out_offs[w] = o;
+    }
+    __syncthreads();  // the tables are in shared memory
+    const int al = static_cast<int>(reinterpret_cast<uintptr_t>(out) & 15u);  // out - al is 16-byte aligned
+    const int64_t nvec = a.total > 0 ? (a.total - 1 + al) / 16 + 1 : 0;      // vector v holds bytes [16v - al, 16v - al + 16)
+    const int64_t ntiles = (nvec + kTrTile - 1) / kTrTile;
+    auto row_g = [&](int64_t i) { return SeqRow{seq_base(a, i), seq_base(a, i + 1), __ldg(a.offs + i), __ldg(a.offs + i + 1)}; };
+    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        const int64_t v0 = tile * kTrTile;
+        const int64_t p0 = max(16 * v0 - al, int64_t(0)), p1 = min(16 * (v0 + kTrTile) - al, a.total);
+        // 1. first sequence: the largest i in [0, n) with base(i) <= p0
+        int64_t lo = 0, hi = a.n;
+        while (hi - lo > 1) {
+            const int64_t w = hi - lo;
+            const int64_t pr = lo + (static_cast<int64_t>(tid) + 1) * w / (kTrThreads + 1);
+            const int cnt = __syncthreads_count(seq_base(a, pr) <= p0);
+            const int64_t nlo = cnt > 0 ? lo + static_cast<int64_t>(cnt) * w / (kTrThreads + 1) : lo;
+            const int64_t nhi = cnt < kTrThreads ? lo + (static_cast<int64_t>(cnt) + 1) * w / (kTrThreads + 1) : hi;
+            lo = nlo;
+            hi = nhi;
+        }
+        const int64_t i0 = lo;
+        // 2. table up to the first sequence that starts at or after the tile's end (base(n) = total >= p1 closes it)
+        int nrows = -1;
+        for (int b = 0; b < kTrRowCap; b += kTrThreads) {
+            const int j = b + tid;
+            const int64_t i = i0 + j;
+            bool past = true;
+            if (i <= a.n) {
+                const int64_t sb = seq_base(a, i);
+                s_base[j] = sb;
+                s_src[j] = __ldg(a.offs + i);
+                past = sb >= p1;
+            }
+            const int cnt = __syncthreads_count(past);
+            if (cnt > 0) {
+                nrows = b + kTrThreads - cnt;
+                break;
+            }
+        }
+        for (int k = 0; k < kTrVecs; ++k) {
+            const int64_t v = v0 + k * kTrThreads + tid;
+            if (v >= nvec) break;
+            const int64_t q = 16 * v - al, x = max(q, int64_t(0));
+            if (nrows > 0) {
+                int l = 0, h = nrows;  // the largest j < nrows with s_base[j] <= x
+                while (h - l > 1) {
+                    const int mid = (l + h) >> 1;
+                    if (s_base[mid] <= x) l = mid;
+                    else h = mid;
+                }
+                auto row_t = [&](int64_t i) {
+                    const int64_t j = i - i0;
+                    return j < nrows ? SeqRow{s_base[j], s_base[j + 1], s_src[j], s_src[j + 1]} : row_g(i);
+                };
+                tr_vector(q, i0 + l, a, row_t, s_mask, s_cmask, s_codon, out + q);
+            } else {
+                int64_t l = i0, h = a.n;
+                while (h - l > 1) {
+                    const int64_t mid = (l + h) >> 1;
+                    if (seq_base(a, mid) <= x) l = mid;
+                    else h = mid;
+                }
+                tr_vector(q, l, a, row_g, s_mask, s_cmask, s_codon, out + q);
+            }
+        }
+        __syncthreads();  // the table is refilled by the next tile
+    }
+}
+
+// The bsq_translate_extent_device reduction: validation bits in out[0] (1: negative length, 2: offsets[0] < 0, 4: past
+// nbytes), sum of the row totals in out[1], of the cropped frame lengths in out[2], the longest cropped frame in out[3].
+// (Valid offsets hold at most INT64_MAX nucleotides and every row at most twice its length, so the sums fit 64 bits.)
+__global__ void translate_extent_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, FrameSet fs, int64_t crop_len,
+                                        unsigned long long *out) {
+    unsigned long long tot = 0, cropped = 0;
+    long long best = 0;
+    unsigned bad = 0;
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const int64_t a = offs[i], b = offs[i + 1];
+        if (b < a) bad |= 1u;
+        if (i == 0 && a < 0) bad |= 2u;
+        if (i == nseq - 1 && nbytes >= 0 && b > nbytes) bad |= 4u;
+        if (b < a) continue;
+        const int64_t len = b - a;
+        for (int f = 0; f < fs.F; ++f) {
+            const int64_t L = tr_len(len, frame_code(fs.fcode, f)), c = min(L, crop_len);
+            tot += static_cast<unsigned long long>(L);
+            cropped += static_cast<unsigned long long>(c);
+            best = max(best, static_cast<long long>(c));
+        }
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
+        tot += __shfl_xor_sync(0xffffffffu, tot, o);
+        cropped += __shfl_xor_sync(0xffffffffu, cropped, o);
+    }
+    bad = __reduce_or_sync(0xffffffffu, bad);
+    if ((threadIdx.x & 31) == 0) {
+        if (bad) atomicOr(out, static_cast<unsigned long long>(bad));
+        if (tot > 0) atomicAdd(out + 1, tot);
+        if (cropped > 0) atomicAdd(out + 2, cropped);
+        if (best > 0) atomicMax(out + 3, static_cast<unsigned long long>(best));
+    }
+}
+
+constexpr unsigned long long kI64Max = (1ull << 63) - 1;
+
+}  // namespace
+
+}  // namespace bsq
+
+using namespace bsq;
+
+extern "C" int bsq_genetic_code(int id, char out[64]) {
+    if (out == nullptr) return fail(BSQ_ERR_ARG, "null output");
+    const char *s = nullptr;
+    switch (id) {
+        case 1:
+        case 11: s = "FFLLSSSSYY**CC*WLLLLPPPPHHQQRRRRIIIMTTTTNNKKSSRRVVVVAAAADDEEGGGG"; break;
+        case 2: s = "FFLLSSSSYY**CCWWLLLLPPPPHHQQRRRRIIMMTTTTNNKKSS**VVVVAAAADDEEGGGG"; break;
+        case 4: s = "FFLLSSSSYY**CCWWLLLLPPPPHHQQRRRRIIIMTTTTNNKKSSRRVVVVAAAADDEEGGGG"; break;
+        case 5: s = "FFLLSSSSYY**CCWWLLLLPPPPHHQQRRRRIIMMTTTTNNKKSSSSVVVVAAAADDEEGGGG"; break;
+        case 6: s = "FFLLSSSSYYQQCC*WLLLLPPPPHHQQRRRRIIIMTTTTNNKKSSRRVVVVAAAADDEEGGGG"; break;
+        default: return fail(BSQ_ERR_ARG, "no built-in genetic code " + std::to_string(id) + " (built in: 1, 2, 4, 5, 6, 11)");
+    }
+    std::memcpy(out, s, 64);
+    return BSQ_OK;
+}
+
+extern "C" int bsq_translate_table(const char *code64, uint8_t masks[256], uint8_t codons[4096]) {
+    if (int rc = check_code(code64)) return rc;
+    if (masks == nullptr || codons == nullptr) return fail(BSQ_ERR_ARG, "null output table");
+    Tables t;
+    build_tables(code64, &t);
+    std::memcpy(masks, t.mask, 256);
+    std::memcpy(codons, t.codon, 4096);
+    return BSQ_OK;
+}
+
+extern "C" int bsq_translate_extent_host(const int64_t *h_offsets, int64_t nseq, const int8_t *frames, int nframes, int64_t crop_len,
+                                         int64_t *total, int64_t *crop_total, int64_t *max_len) {
+    FrameSet fs;
+    if (int rc = check_frames(frames, nframes, &fs)) return rc;
+    if (crop_len < 1) return fail(BSQ_ERR_ARG, "crop_len must be >= 1");
+    if (total == nullptr || crop_total == nullptr || max_len == nullptr) return fail(BSQ_ERR_ARG, "null output");
+    if (nseq < 0 || (nseq > 0 && h_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
+    *total = *crop_total = *max_len = 0;
+    if (nseq == 0) return BSQ_OK;
+    if (h_offsets[0] < 0) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
+    __int128 st = 0, sc = 0;
+    int64_t best = 0;
+    for (int64_t i = 0; i < nseq; ++i) {
+        const int64_t len = h_offsets[i + 1] - h_offsets[i];  // (both in [0, INT64_MAX]: no overflow)
+        if (len < 0) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
+        for (int f = 0; f < fs.F; ++f) {
+            const int64_t L = tr_len(len, frame_code(fs.fcode, f)), c = std::min(L, crop_len);
+            st += L;
+            sc += c;
+            best = std::max(best, c);
+        }
+    }
+    if (st > static_cast<__int128>(kI64Max)) return fail(BSQ_ERR_ARG, "the translated batch exceeds INT64_MAX bytes");
+    *total = static_cast<int64_t>(st);
+    *crop_total = static_cast<int64_t>(sc);
+    *max_len = best;
+    return BSQ_OK;
+}
+
+extern "C" int bsq_translate_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes,
+                                           const int8_t *frames, int nframes, int64_t crop_len, int64_t *total, int64_t *crop_total,
+                                           int64_t *max_len) {
+    bsq::DeviceRestore restore_device;
+    FrameSet fs;
+    if (int rc = check_frames(frames, nframes, &fs)) return rc;
+    if (crop_len < 1) return fail(BSQ_ERR_ARG, "crop_len must be >= 1");
+    if (total == nullptr || crop_total == nullptr || max_len == nullptr) return fail(BSQ_ERR_ARG, "null output");
+    if (nseq < 0 || (nseq > 0 && d_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
+    *total = *crop_total = *max_len = 0;
+    if (nseq == 0) return BSQ_OK;
+    BSQ_CUDA_TRY(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    unsigned long long *d_res = nullptr, h_res[4] = {0, 0, 0, 0};
+    BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&d_res), sizeof(h_res), st));
+    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, sizeof(h_res), st));
+    const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
+    translate_extent_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, fs, crop_len, d_res);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, sizeof(h_res), cudaMemcpyDeviceToHost, st));
+    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
+    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
+    if (h_res[0] & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
+    if (h_res[0] & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
+    if (h_res[0] & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
+    if (h_res[1] > kI64Max) return fail(BSQ_ERR_ARG, "the translated batch exceeds INT64_MAX bytes");
+    *total = static_cast<int64_t>(h_res[1]);
+    *crop_total = static_cast<int64_t>(h_res[2]);
+    *max_len = static_cast<int64_t>(h_res[3]);
+    return BSQ_OK;
+}
+
+extern "C" int bsq_translate(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq,
+                             const int8_t *frames, int nframes, const char *code64, uint8_t *d_out_bytes, int64_t *d_out_offsets) {
+    bsq::DeviceRestore restore_device;
+    FrameSet fs;
+    if (int rc = check_frames(frames, nframes, &fs)) return rc;
+    if (int rc = check_code(code64)) return rc;
+    if (nseq < 0 || nseq > static_cast<int64_t>(kI64Max / 6) - 1) return fail(BSQ_ERR_ARG, "bad batch size");
+    if (d_out_offsets == nullptr) return fail(BSQ_ERR_ARG, "null output offsets");
+    if (nseq > 0 && (d_bytes == nullptr || d_offsets == nullptr || d_out_bytes == nullptr))
+        return fail(BSQ_ERR_ARG, "null bytes, offsets or output bytes");
+    BSQ_CUDA_TRY(cudaSetDevice(device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (nseq == 0) {
+        BSQ_CUDA_TRY(cudaMemsetAsync(d_out_offsets, 0, sizeof(int64_t), st));
+        return BSQ_OK;
+    }
+    Tables t;
+    build_tables(code64, &t);
+    TrTables tt;
+    for (int w = 0; w < 64; ++w) {
+        const uint8_t *m = t.mask + 4 * w;
+        tt.mask[w] = m[0] | (m[1] << 8) | (m[2] << 16) | (static_cast<uint32_t>(m[3]) << 24);
+        tt.cmask[w] = bitrev4(m[0]) | (bitrev4(m[1]) << 8) | (bitrev4(m[2]) << 16) | (static_cast<uint32_t>(bitrev4(m[3])) << 24);
+    }
+    std::memcpy(tt.codon, t.codon, sizeof(tt.codon));
+    int64_t *S = nullptr;
+    BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&S), static_cast<size_t>(nseq + 1) * sizeof(int64_t), st));
+    const int64_t nblocks = (nseq + kRowScan - 1) / kRowScan;
+    row_scan_kernel<<<static_cast<unsigned>(nblocks), kRowScan, 0, st>>>(d_offsets, nseq, TranslateCount{fs}, S);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    if (nblocks > 1) {
+        row_carry_kernel<<<1, kRowScan, 0, st>>>(S, nseq, nblocks);
+        count_launch();
+        BSQ_CUDA_TRY(cudaGetLastError());
+    }
+    TrArgs a;
+    a.bytes = d_bytes;
+    a.offs = d_offsets;
+    a.S = S;
+    a.n = nseq;
+    a.total = 0;  // (S's last entry: read by the kernel)
+    a.fs = fs;
+    translate_kernel<<<cur_sms() * kTrMinBlocks, kTrThreads, 0, st>>>(a, tt, d_out_bytes, d_out_offsets);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    BSQ_CUDA_TRY(cudaFreeAsync(S, st));
+    return BSQ_OK;
+}

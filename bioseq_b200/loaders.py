@@ -8,7 +8,8 @@ the tokeniser (``consumers``; Philox streams keyed by the dataset seed, the draw
 and ``cnn=True`` batches are written directly in the ``(batch, emb, length)`` float layout.  ``max_seq_len=`` crops
 over-long sequences on the device (``consumers.crop_packed``) so that a file with a few very long sequences still
 yields batches of the model's context, and ``rc="random"`` flips DNA sequences to their reverse complement on the device
-(``consumers.revcomp_packed``).
+(``consumers.revcomp_packed``).  ``translate=`` reads protein rows out of a DNA file: each sequence's reading frames
+are translated on the device (``consumers.translate_packed``) before the crop.
 """
 import numpy as np
 
@@ -81,6 +82,12 @@ class FlatFileDataset(_dataset_base()):
     ``crop="random"`` as the random shift.  Like the crop, every fetch is a new draw from the per-fetch seed.  Datasets
     are for training, so the inference modes (``"always"``, ``"both"``) are rejected: call the consumers directly.
 
+    ``translate=frames`` (with ``genetic_code``, as ``consumers.batch_tokenize_translated``; a protein tokenizer) turns a
+    DNA file into protein rows: F frames per sequence, so a slice ``[start, stop)`` yields ``(stop - start) * F`` rows, and a
+    single index F rows (a 1-D row when F = 1, as without translation).  The default ``max_seq_len`` is then
+    ``maxseqlen // 3 + bos + eos``; ``max_seq_len`` crops the proteins, and every seeded draw is keyed by the output row
+    ``(index * F + f)``.  Not with ``rc`` (the reverse frames are the other strand).
+
     ``fetch(index, return_items=True)`` also hands back the raw sequence(s) (bioseq/loaders.py:60-84), as stored in the
     file: uncropped and unflipped, like they are unaugmented.  Two quirks of
     the reference's ``fetch`` are NOT reproduced: with ``cnn=True`` and ``return_items=False`` it falls off the end and
@@ -88,7 +95,7 @@ class FlatFileDataset(_dataset_base()):
     """
 
     def __init__(self, ff, tokenizer, *, augment=0, augment_frac=0.5, cnn=False, device=None, maskfrac=0.15, seed=13,
-                 varlen=False, mlm=False, max_seq_len=None, crop="random", seqpack=False, rc=None, rc_prob=0.5):
+                 varlen=False, mlm=False, max_seq_len=None, crop="random", seqpack=False, rc=None, rc_prob=0.5, translate=None, genetic_code=1):
         super().__init__()
         assert isinstance(ff, cbioseq.FlatFile)
         assert isinstance(tokenizer, cbioseq.Tokenizer)
@@ -104,9 +111,11 @@ class FlatFileDataset(_dataset_base()):
         self.seed, self._draw = int(seed), 0  # the reference seeds its generator with 13 (bioseq/loaders.py:49-50)
         self.maskfrac, self.augment, self.augment_frac, self.cnn, self.device = maskfrac, augment, augment_frac, cnn, device
         k = tokenizer.includes_bos() + tokenizer.includes_eos()
+        self.tr = consumers._translate_spec(translate, genetic_code, tokenizer, rc)  # ValueError now rather than per fetch
+        self.translate, self.genetic_code = translate, genetic_code
         self.crop, self.crop_len = None, None
         if max_seq_len is None:
-            self.max_seq_len = ff.maxseqlen + k
+            self.max_seq_len = (ff.maxseqlen // 3 if self.tr else ff.maxseqlen) + k
         else:
             if crop not in ("head", "random"):
                 raise ValueError(f"FlatFileDataset: crop must be 'head' or 'random', got {crop!r}")
@@ -145,11 +154,13 @@ class FlatFileDataset(_dataset_base()):
         start, stop, many = self._range(index)
         crop = dict(crop=self.crop, crop_len=self.crop_len) if self.crop else {}
         rc = dict(rc=self.rc, rc_prob=self.rc_prob) if self.rc else {}
+        tr = dict(translate=self.translate, genetic_code=self.genetic_code) if self.tr else {}
+        F = len(self.tr[0]) if self.tr else 1
         if self.seqpack:
             kw = self._augment_kwargs(start) if self.mlm or self.augment or self.crop or self.rc else {}
             mlm = dict(mlm=True, maskfrac=self.maskfrac, mask_token=self.tokenizer.alphabet_size()) if self.mlm else {}
             return consumers.batch_tokenize_seqpack(self.tokenizer, (self.ff, start, stop), self.max_seq_len, "l", self.device,
-                                                    rows=None if many else 1, **mlm, **kw, **crop, **rc)
+                                                    rows=None if many or F > 1 else 1, **mlm, **kw, **crop, **rc, **tr)
         if self.mlm:
             # one draw per fetch, shared by the augmentation (counter word 3 = 0), the mask (words 1, 2), the crop (3) and the
             # strand flip (4)
@@ -157,15 +168,19 @@ class FlatFileDataset(_dataset_base()):
             mb = consumers.batch_tokenize_mlm(self.tokenizer, (self.ff, start, stop),
                                               padlen=-1 if self.varlen else self.max_seq_len, destchar="l",
                                               device=self.device, varlen=self.varlen, maskfrac=self.maskfrac,
-                                              mask_token=self.tokenizer.alphabet_size(), **kw, **crop, **rc)
-            if many:
+                                              mask_token=self.tokenizer.alphabet_size(), **kw, **crop, **rc, **tr)
+            if many or (F > 1 and not self.varlen):
                 return mb
             return consumers.MLMBatch(mb.inputs.tokens if self.varlen else mb.inputs[0], mb.labels if self.varlen else mb.labels[0])
         aug = self._augment_kwargs(start) if self.augment or self.crop or self.rc else {}
         if self.cnn:
             if many:  # (batch, emb, length) float, written in that layout by one kernel
                 return consumers.batch_onehot_encode_bcl(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
-                                                         destchar='f', device=self.device, **aug, **crop, **rc)
+                                                         destchar='f', device=self.device, **aug, **crop, **rc, **tr)
+            if tr:  # F (length, emb) items
+                oh = consumers.batch_onehot_encode_bcl(self.tokenizer, (self.ff, start, stop), padlen=self.max_seq_len,
+                                                       destchar='f', device=self.device, **aug, **crop, **tr).transpose(1, 2)
+                return oh[0] if F == 1 else oh
             if aug:
                 # (mutated, cropped or flipped on the device: the batched path at padlen = max_seq_len; such a sequence is no
                 # longer than before, so only the reference's extra bos + eos pad rows of the single-sequence encoder are
@@ -174,12 +189,20 @@ class FlatFileDataset(_dataset_base()):
                                                          destchar='f', device=self.device, **aug, **crop, **rc)[0].t()
             return self.tokenizer.onehot_encode(bytes(self.ff[start]), padlen=self.max_seq_len, destchar='f', device=self.device)
         if self.varlen:
+            base = consumers._out_base(start, self.tr)  # (the global index of the first output row)
             vb = consumers._tokenize_varlen(self.tokenizer, (self.ff, start, stop), "l", self.device,
-                                            consumers._augment_args(**aug) if aug else None,
-                                            crop=consumers._crop_spec(self.crop, self.crop_len, aug.get("seed", 0), start)
+                                            consumers._augment_args(**dict(aug, seq_index_base=base)) if aug else None,
+                                            crop=consumers._crop_spec(self.crop, self.crop_len, aug.get("seed", 0), base)
                                             if crop else None,
-                                            rc=consumers._rc_spec(self.rc, self.rc_prob, aug.get("seed", 0), start) if rc else None)
+                                            rc=consumers._rc_spec(self.rc, self.rc_prob, aug.get("seed", 0), start) if rc else None,
+                                            translate=self.tr)
             return vb if many else vb.tokens
+        if tr:
+            kw = dict(seed=aug.get("seed", 0), seq_index_base=start, augment=self.augment, augment_frac=self.augment_frac)
+            toks = consumers.batch_tokenize_translated(self.tokenizer, (self.ff, start, stop), self.max_seq_len, 'B', self.device,
+                                                       frames=self.translate, genetic_code=self.genetic_code, **kw,
+                                                       **crop).to(torch.long)
+            return toks if many or F > 1 else toks[0]
         if crop:
             toks = consumers.batch_tokenize_cropped(self.tokenizer, (self.ff, start, stop), self.max_seq_len, batch_first=True,
                                                     destchar='B', device=self.device, **aug, **crop, **rc).to(torch.long)

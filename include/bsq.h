@@ -334,6 +334,66 @@ int bsq_untile_mean(int device, void *stream, int dtype, const void *d_y, int64_
                     int64_t col0, const int64_t *d_src_offsets, int64_t nseq, int64_t window, int64_t stride, int tail,
                     const int64_t *d_seq_ptr, int64_t nwin, int strands, const uint8_t *d_flipped, float *d_out);
 
+/* Translation (protein language models on coding sequences, six-frame searches over reads, gene calls into a protein
+ * model): a packed DNA / RNA batch in, a packed protein batch of its reading frames out, which every entry point above
+ * then takes unchanged.
+ *   Residues -> base sets, case-insensitive IUPAC: A, C, G, T (U = T) stand for themselves; R = AG, Y = CT, S = CG,
+ *   W = AT, K = GT, M = AC, B = CGT, D = AGT, H = ACT, V = ACG, N = ACGT.  Every other byte is invalid (gaps, '*', digits,
+ *   bytes >= 0x80).  As a 4-bit mask: A = 1, C = 2, G = 4, T = 8, invalid = 0; the complement (A <-> T, C <-> G, K12's
+ *   pairs applied to base sets) is then the reversal of the 4 bits.
+ *   Codon -> amino acid: every expansion of the three base sets is looked up in the genetic code; if all give the same
+ *   letter that letter is the result, otherwise -- or if a byte is invalid -- 'X'.  Stops are the code's '*'.  (Biopython's
+ *   B / Z / J ambiguity letters are not produced.)
+ *   Genetic code: 64 characters in TCAG order, codon index 16 b1 + 4 b2 + b3 with T = 0, C = 1, A = 2, G = 3.  Any 64
+ *   printable ASCII characters (0x21..0x7E) are accepted, so a custom table's letters come out as written; the built-in
+ *   NCBI tables (bsq_genetic_code) are upper case.  Every codon translates to its table letter, the first included
+ *   (alternative start codons are not applied).
+ *   Frames: frame +k (k = 1, 2, 3) reads the sequence from offset k - 1, frame -k its reverse complement from offset
+ *   k - 1 (so frame -1 starts at the last base).  Each has max(0, floor((len - (k - 1)) / 3)) amino acids; a trailing
+ *   partial codon is dropped.  Amino acid t of frame +k comes from nucleotides k - 1 + 3t .. k + 1 + 3t, of frame -k from
+ *   len - k - 3t - 2 .. len - k - 3t, read right to left on the complement.
+ *   Output: the caller gives F frames, 1 to 6 distinct values in any order; output sequence w = i F + f is frame frames[f]
+ *   of input sequence i (sequence-major, n F sequences).  out_offsets (int64, n F + 1 entries) start at 0.  Sequences
+ *   shorter than 3 give empty rows, which are kept.
+ *   Order inside a consumer: stage -> translate -> crop -> augment -> tokenize / mask / pack / k-mer.  Crop lengths,
+ *   padlen and MLM positions count amino acids; a seeded draw for output sequence (i, f) is keyed by the global output
+ *   index (seq_index_base + i) F + f, so slicing a batch changes no draw.
+ * Worked answers, standard code, frames +1, +2, +3, -1, -2, -3:
+ *   "ATGGCCATTGTAATGGGCCGCTGAAAGGGTGCCCGATAG" (39 nt) -> "MAIVMGR*KGAR*", "WPL*WAAERVPD", "GHCNGPLKGCPI", "LSGTLSAAHYNGH",
+ *   "YRAPFQRPITMA", "IGHPFSGPLQWP";  "ATGA" -> "M", "*", "", "S", "H", "";  "ATGAA" -> "M", "*", "E", "F", "S", "H";
+ *   "", "A" and "AT" -> six empty rows each.
+ *   Frame +1 under codes 1 / 2, and frame -1 under code 1: GCN A / A, X; TAR * / *, L; TRA * / X, X; YTG L / L, Q;
+ *   atg and AUG M / M, H; A-G X / X, X; TGA * / W, S; AGA R / *, S.  "ATAAGATGA" frame +1: "IR*" (code 1), "M*W" (code 2);
+ *   "TAATAG" frame +1 under code 6: "QQ".
+ *
+ * bsq_genetic_code (host only): the built-in tables -- 1 standard and 11 bacterial (the same amino acids), 2 vertebrate
+ * mitochondrial, 4 mold / protozoan mitochondrial and Mycoplasma, 5 invertebrate mitochondrial, 6 ciliate -- as 64
+ * characters (no terminating NUL).  BSQ_ERR_ARG for any other id.
+ * bsq_translate_table (host only): masks[b] = the base set of byte b, codons[m0 << 8 | m1 << 4 | m2] = the letter of
+ * that triple of base sets (or 'X').  The only place the rule is built in the library; the kernels get these tables.
+ * BSQ_ERR_ARG for a NULL or non-printable code or NULL outputs. */
+int bsq_genetic_code(int id, char out[64]);
+int bsq_translate_table(const char *code64, uint8_t masks[256], uint8_t codons[4096]);
+/* The output's size before a crop (*total bytes) and after a crop of every output row to crop_len amino acids
+ * (*crop_total, *max_len = the longest kept row); crop_len = INT64_MAX means no crop.  All 0 for nseq == 0.  The host
+ * form makes no device call; BSQ_ERR_ARG for bad frames (as bsq_translate), crop_len < 1, NULL outputs, negative lengths,
+ * offsets[0] < 0 or a total past INT64_MAX.  The device form runs one reduction and one read-back (synchronises `stream`)
+ * and validates the offsets like bsq_crop_extent_device (BSQ_ERR_ARG: negative length, offsets[0] < 0, offsets[nseq] >
+ * nbytes when nbytes >= 0). */
+int bsq_translate_extent_host(const int64_t *h_offsets, int64_t nseq, const int8_t *frames, int nframes, int64_t crop_len,
+                              int64_t *total, int64_t *crop_total, int64_t *max_len);
+int bsq_translate_extent_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, const int8_t *frames,
+                                int nframes, int64_t crop_len, int64_t *total, int64_t *crop_total, int64_t *max_len);
+/* bsq_translate enqueues only (two or three kernels; nseq == 0: an 8-byte memset of out_offsets), keeps no state between
+ * launches and is capturable into a CUDA graph.  Scratch: 8 (n + 1) bytes, allocated and freed in stream order
+ * (cudaMallocAsync / cudaFreeAsync from the device's default memory pool).  `frames` (nframes entries) and `code64` are
+ * host memory, read before the call returns.  The caller has validated the offsets (bsq_translate_extent_device does) and
+ * sized d_out_bytes (any alignment, not overlapping the input) to the extent's total and d_out_offsets to n F + 1 entries.
+ * BSQ_ERR_ARG, before any device call, for bad, duplicate, zero or more than six frames, a NULL or non-printable code,
+ * nseq < 0 (or n F + 1 past INT64_MAX), a NULL d_out_offsets, or NULL bytes, offsets or output bytes with nseq > 0. */
+int bsq_translate(int device, void *stream, const uint8_t *d_bytes, const int64_t *d_offsets, int64_t nseq, const int8_t *frames,
+                  int nframes, const char *code64, uint8_t *d_out_bytes, int64_t *d_out_offsets);
+
 /* Sequence packing (padding-free batches of a fixed shape: SDPA with a block-diagonal mask, position-id packing as in
  * HF's DataCollatorWithFlattening, CUDA graphs, torch.compile): whole sequences laid end to end in R rows of L tokens.
  * With k = bos + eos and the (already cropped) lengths len_i, sequence i occupies need_i = len_i + k tokens; every
