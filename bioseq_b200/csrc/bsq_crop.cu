@@ -5,7 +5,7 @@
 // (g_lo, g_hi, 0, 3), g = seq_index_base + i.  out_offsets is the exclusive scan of len'_i (out_offsets[0] = 0).
 //
 // Three launches, no scratch memory and no state between launches (capturable into a CUDA graph):
-//   row_scan_kernel     one thread per row, kCScan rows per CTA: len'_i, the CTA's inclusive scan of them
+//   row_scan_kernel     one thread per row, kCScan rows per CTA: len'_i (CropCount), the CTA's inclusive scan of them
 //                       (block_exclusive_scan) written to out_offsets[i + 1].  The entry at the end of each CTA's rows
 //                       is then that CTA's total.  (Shared with K11's cu_seqlens, bsq_kernels.cuh.)
 //   row_carry_kernel    one CTA (only when there is more than one scan CTA): scans the CTA totals in place, so every
@@ -46,12 +46,6 @@ __device__ __forceinline__ int64_t crop_start(int64_t len, int64_t i, const Crop
     const uint64_t d = static_cast<uint64_t>(p.c[0]) | (static_cast<uint64_t>(p.c[1]) << 32);
     return static_cast<int64_t>(__umul64hi(d, static_cast<uint64_t>(len - c.W + 1)));
 }
-
-// the per-row count of the scan (bsq_kernels.cuh): the kept length min(len_i, W)
-struct CropCount {
-    int64_t W;
-    __device__ __forceinline__ int64_t operator()(int64_t len) const { return min(len, W); }
-};
 
 __global__ void __launch_bounds__(kCThreads)
 crop_gather_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__ offs, int64_t n, CropParam c,
@@ -119,15 +113,7 @@ extern "C" int bsq_crop(int device, void *stream, const uint8_t *d_bytes, const 
         BSQ_CUDA_TRY(cudaMemsetAsync(d_out_offsets, 0, sizeof(int64_t), st));
         return BSQ_OK;
     }
-    const int64_t nblocks = (nseq + kCScan - 1) / kCScan;
-    row_scan_kernel<<<static_cast<unsigned>(nblocks), kCScan, 0, st>>>(d_offsets, nseq, CropCount{crop_len}, d_out_offsets);
-    count_launch();
-    BSQ_CUDA_TRY(cudaGetLastError());
-    if (nblocks > 1) {
-        row_carry_kernel<<<1, kCScan, 0, st>>>(d_out_offsets, nseq, nblocks);
-        count_launch();
-        BSQ_CUDA_TRY(cudaGetLastError());
-    }
+    if (int rc = launch_row_scan(st, d_offsets, nseq, CropCount{crop_len}, d_out_offsets)) return rc;
     const CropParam c{crop_len, seq_index_base, static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32), random != 0};
     const int64_t rows_per_cta = kCThreads / 32;
     crop_gather_kernel<<<static_cast<unsigned>((nseq + rows_per_cta - 1) / rows_per_cta), kCThreads, 0, st>>>(

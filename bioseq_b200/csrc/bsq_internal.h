@@ -24,6 +24,9 @@ int launch_tokenize(cudaStream_t st, const uint8_t *d_bytes, const int64_t *d_of
 int launch_onehot(cudaStream_t st, const uint8_t *d_bytes, const int64_t *d_offs, const uint8_t *d_mask, int64_t nseq,
                   int64_t ld, int64_t padlen, const bsq_tokenizer &tok, int kind, void *d_out);
 int check_launch_args(int device, int64_t nseq, int64_t padlen, const bsq_tokenizer *tok, int kind, const void *d_out);
+// A few bytes of device workspace for an entry point that synchronises before it returns, from a library-owned
+// stream-ordered pool of `device` (bsq_kernels.cu); free it with cudaFreeAsync on st.
+int scratch_alloc(int device, void **p, size_t bytes, cudaStream_t st);
 #endif
 
 }  // namespace bsq

@@ -14,8 +14,8 @@
 //   K4 decode_*             tokens -> characters: pass 1 decode_len16p_kernel (lengths, validation, where each row's
 //                           trailing <PAD> run starts) + scan, pass 2 decode_chars_kernel (text); bsq_decode_text
 //                           enqueues both behind one another.
-//   K0 maxlen_kernel        length and offsets validation for device-resident packed input (K0c crop_extent_kernel: the
-//                           same for a crop, bsq_crop_extent_device).
+//   K0 offsets_extent_kernel<CropCount>  length and offsets validation for device-resident packed input, and the crop's
+//                           and varlen's extents (the template and its launcher are in bsq_kernels.cuh).
 //   (K1s, the batch-first one-byte kernel for padlen >= 257 -- the headline path -- lives in bsq_span.cu.)
 //
 // Reference semantics: src/tokenize.h:381-485 (K1/K2), :283-371 (K3), :131-179 (K4).
@@ -653,62 +653,6 @@ seqfirst_tok8_kernel(SeqView v, int64_t nseq, int64_t ld, int padlen, FastDiv di
         }
     }
     if (TPC > 1 && tp + 1 < TPC) __syncthreads();  // the tile is rewritten by the next position tile
-    }
-}
-
-// ------------------------------------------------------------------------------------------
-// K0: longest sequence of a device-resident offsets array.
-// ------------------------------------------------------------------------------------------
-// out[0] = longest sequence; out[1] = what is wrong with the offsets, if anything: 1 a negative length, 2 offsets[0] < 0,
-// 4 offsets[nseq] > nbytes (nbytes < 0: the size of the byte buffer is not known) -- the kernels index the byte buffer
-// with these offsets, so a bad array must fail here and not read out of bounds.  span (optional): offsets[nseq] -
-// offsets[0], the residue count of a packed token stream (bsq_varlen_extent_device).
-__global__ void maxlen_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, unsigned long long *out,
-                              long long *span) {
-    long long best = 0;
-    unsigned bad = 0;
-    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq;
-         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-        const long long len = static_cast<long long>(offs[i + 1] - offs[i]);
-        best = max(best, len);
-        if (len < 0) bad |= 1u;
-        if (i == 0 && offs[0] < 0) bad |= 2u;
-        if (i == nseq - 1 && nbytes >= 0 && offs[nseq] > nbytes) bad |= 4u;
-        if (i == nseq - 1 && span != nullptr) *span = static_cast<long long>(offs[nseq] - offs[0]);
-    }
-    for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
-    bad = __reduce_or_sync(0xffffffffu, bad);
-    if ((threadIdx.x & 31) == 0) {
-        if (best > 0) atomicMax(out, static_cast<unsigned long long>(best));
-        if (bad) atomicOr(out + 1, static_cast<unsigned long long>(bad));
-    }
-}
-
-// K0c: K0's sibling for bsq_crop_extent_device -- the same validation bits, the longest cropped length min(len, W) in
-// out[0] and the sum of the cropped lengths in out[2].
-__global__ void crop_extent_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, int64_t W,
-                                   unsigned long long *out) {
-    long long best = 0, sum = 0;
-    unsigned bad = 0;
-    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq;
-         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-        const long long len = static_cast<long long>(offs[i + 1] - offs[i]);
-        if (len < 0) bad |= 1u;
-        if (i == 0 && offs[0] < 0) bad |= 2u;
-        if (i == nseq - 1 && nbytes >= 0 && offs[nseq] > nbytes) bad |= 4u;
-        const long long kept = min(max(len, 0ll), static_cast<long long>(W));
-        best = max(best, kept);
-        sum += kept;
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-        best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
-        sum += __shfl_xor_sync(0xffffffffu, sum, o);
-    }
-    bad = __reduce_or_sync(0xffffffffu, bad);
-    if ((threadIdx.x & 31) == 0) {
-        if (best > 0) atomicMax(out, static_cast<unsigned long long>(best));
-        if (bad) atomicOr(out + 1, static_cast<unsigned long long>(bad));
-        if (sum > 0) atomicAdd(out + 2, static_cast<unsigned long long>(sum));
     }
 }
 
@@ -1900,11 +1844,14 @@ int bsq_onehot(int device, void *stream, const uint8_t *d_bytes, const int64_t *
                          d_out);
 }
 
-// Scratch for the entry points that need a few words of device workspace (length check, decode
+}  // extern "C"
+
+namespace bsq {
+
+// Scratch for the entry points that need a few words of device workspace (offsets reductions, decode
 // scan).  A library-owned memory pool per device with an unbounded release threshold: the default
 // pool hands its memory back to the driver at every synchronisation that finds it empty, which made
 // each of these calls pay a fresh physical allocation (measured: decode 1.07 ms -> 11.6 ms per call).
-namespace {
 int scratch_alloc(int device, void **p, size_t bytes, cudaStream_t st) {
     static std::mutex mu;
     static cudaMemPool_t pools[64] = {};
@@ -1928,29 +1875,16 @@ int scratch_alloc(int device, void **p, size_t bytes, cudaStream_t st) {
     return BSQ_OK;
 }
 
-// K0 and its read-back: h_res = {longest sequence, error bits, offsets[nseq] - offsets[0]}; fails on bad offsets.
-// crop_len >= 1: K0c instead, h_res = {longest cropped length, error bits, sum of the cropped lengths}.
-int reduce_offsets(int device, cudaStream_t st, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, unsigned long long h_res[3],
-                   int64_t crop_len = 0) {
-    BSQ_CUDA_TRY(cudaSetDevice(device));
-    unsigned long long *d_res = nullptr;
-    if (int rc = scratch_alloc(device, reinterpret_cast<void **>(&d_res), 3 * sizeof(*d_res), st)) return rc;
-    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, 3 * sizeof(*d_res), st));
-    const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
-    if (crop_len >= 1)
-        crop_extent_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, crop_len, d_res);
-    else
-        maxlen_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, d_res, reinterpret_cast<long long *>(d_res + 2));
-    count_launch();
-    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, 3 * sizeof(*d_res), cudaMemcpyDeviceToHost, st));
-    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
-    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
-    if (h_res[1] & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
-    if (h_res[1] & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
-    if (h_res[1] & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
+int offsets_error(unsigned long long bits) {
+    if (bits & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
+    if (bits & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
+    if (bits & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
     return BSQ_OK;
 }
-}  // namespace
+
+}  // namespace bsq
+
+extern "C" {
 
 int bsq_check_offsets_device(int device, void *stream, const int64_t *d_offsets, int64_t nseq, int64_t nbytes, int64_t padlen,
                              const bsq_tokenizer *tok) {
@@ -1958,9 +1892,9 @@ int bsq_check_offsets_device(int device, void *stream, const int64_t *d_offsets,
     if (tok == nullptr) return fail(BSQ_ERR_ARG, "null tokenizer");
     if (padlen <= 0) return fail(BSQ_ERR_ARG, "batch tokenize requires padlen is provded.");
     if (nseq <= 0) return BSQ_OK;
-    unsigned long long h_res[3] = {0, 0, 0};
-    if (int rc = reduce_offsets(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, h_res)) return rc;
-    const int64_t tl = static_cast<int64_t>(h_res[0]) + (tok->bos_id >= 0) + (tok->eos_id >= 0);
+    Extent e{};
+    if (int rc = reduce_offsets_device(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, CropCount{kI64Max}, &e)) return rc;
+    const int64_t tl = e.max + (tok->bos_id >= 0) + (tok->eos_id >= 0);
     if (tl > padlen)
         return fail(BSQ_ERR_TOO_LONG, "seq len + bos + eos > padlen: " + std::to_string(tl) + ", vs padlen " + std::to_string(padlen));
     return BSQ_OK;
@@ -1973,11 +1907,11 @@ int bsq_varlen_extent_device(int device, void *stream, const int64_t *d_offsets,
     if (nseq < 0 || (nseq > 0 && d_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
     *total = *max_seqlen = 0;
     if (nseq == 0) return BSQ_OK;
-    unsigned long long h_res[3] = {0, 0, 0};
-    if (int rc = reduce_offsets(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, h_res)) return rc;
+    Extent e{};
+    if (int rc = reduce_offsets_device(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, CropCount{kI64Max}, &e)) return rc;
     const int64_t k = (tok->bos_id >= 0) + (tok->eos_id >= 0);
-    *total = static_cast<int64_t>(h_res[2]) + nseq * k;
-    *max_seqlen = static_cast<int64_t>(h_res[0]) + k;
+    *total = e.sum0 + nseq * k;
+    *max_seqlen = e.max + k;
     return BSQ_OK;
 }
 
@@ -1989,10 +1923,10 @@ int bsq_crop_extent_device(int device, void *stream, const int64_t *d_offsets, i
     if (nseq < 0 || (nseq > 0 && d_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
     *total = *max_len = 0;
     if (nseq == 0) return BSQ_OK;
-    unsigned long long h_res[3] = {0, 0, 0};
-    if (int rc = reduce_offsets(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, h_res, crop_len)) return rc;
-    *total = static_cast<int64_t>(h_res[2]);
-    *max_len = static_cast<int64_t>(h_res[0]);
+    Extent e{};
+    if (int rc = reduce_offsets_device(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, CropCount{crop_len}, &e)) return rc;
+    *total = e.sum0;
+    *max_len = e.max;
     return BSQ_OK;
 }
 

@@ -14,6 +14,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
+
+#include "bsq_internal.h"
+
 struct bsq_tokenizer;
 struct bsq_mlm;
 
@@ -124,11 +128,46 @@ __host__ __device__ inline KmerCount kmer_count(int64_t n, const KmerShape &ks) 
     c.tail = ks.single ? n - c.covered : 0;
     return c;
 }
-// T(n) = m + (single ? r : 0) + bos + eos
+// T(n) = m + (single ? r : 0) + bos + eos.  m + r <= n, so only the specials can take T past INT64_MAX (n within two of
+// it): the sum wraps to a negative value then, which KmerCountFn::extent reports.
 __host__ __device__ inline int64_t kmer_tokens(int64_t n, const KmerShape &ks) {
     const KmerCount c = kmer_count(n, ks);
-    return c.m + c.tail + ks.bos + ks.eos;
+    return static_cast<int64_t>(static_cast<uint64_t>(c.m + c.tail) + ks.bos + ks.eos);
 }
+
+// ---- offsets reductions: validate a packed batch's offsets and size an output from them ------------------------------
+// Each feature states its per-row share as a measure, m.extent(len) for a row of len >= 0: two sums and a max, each in
+// [0, INT64_MAX], and whether one had to be clamped.  reduce_offsets_host and reduce_offsets_device (below) add the rows
+// up with the same measure, so host and device extents cannot disagree.
+constexpr int64_t kI64Max = INT64_MAX;
+struct Extent {
+    int64_t sum0, sum1, max;
+    bool over;  // a value passed INT64_MAX (it is clamped there)
+};
+// a + b for a, b in [0, INT64_MAX], clamped to INT64_MAX
+__host__ __device__ __forceinline__ int64_t add_sat(int64_t a, int64_t b, bool *over) {
+    if (a > kI64Max - b) {
+        *over = true;
+        return kI64Max;
+    }
+    return a + b;
+}
+// v >= 0 clamped to INT64_MAX
+__host__ __device__ __forceinline__ int64_t clamp_sat(__int128 v, bool *over) {
+    if (v > kI64Max) {
+        *over = true;
+        return kI64Max;
+    }
+    return static_cast<int64_t>(v);
+}
+
+// The kept length min(len, W) of a crop (K9's scan, K0c), and with W = INT64_MAX the length itself (K0): the sum and the
+// max of the kept lengths.
+struct CropCount {
+    int64_t W;
+    __host__ __device__ __forceinline__ int64_t operator()(int64_t len) const { return len < W ? len : W; }
+    __host__ __device__ __forceinline__ Extent extent(int64_t len) const { return {(*this)(len), 0, (*this)(len), false}; }
+};
 
 #ifdef __CUDACC__
 
@@ -439,6 +478,128 @@ row_carry_kernel(Out *__restrict__ out_offs, int64_t n, int64_t nblocks) {
         carry += s_total;
         __syncthreads();
     }
+}
+
+// row_scan_kernel, and row_carry_kernel past kRowScan rows, enqueued on st
+template <typename Count, typename Out>
+int launch_row_scan(cudaStream_t st, const int64_t *d_offs, int64_t n, Count count, Out *out_offs) {
+    const int64_t nblocks = (n + kRowScan - 1) / kRowScan;
+    row_scan_kernel<<<static_cast<unsigned>(nblocks), kRowScan, 0, st>>>(d_offs, n, count, out_offs);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    if (nblocks > 1) {
+        row_carry_kernel<<<1, kRowScan, 0, st>>>(out_offs, n, nblocks);
+        count_launch();
+        BSQ_CUDA_TRY(cudaGetLastError());
+    }
+    return BSQ_OK;
+}
+
+// K0: the device offsets reduction.  out = {sum0, sum1, max, what is wrong}: 1 a negative length, 2 offsets[0] < 0,
+// 4 offsets[n] > nbytes (nbytes < 0: the size of the byte buffer is not known), 8 a sum or a row's value past INT64_MAX.
+// The kernels index the byte buffer with these offsets, so a bad array must fail here and not read out of bounds.  Sums
+// saturate per thread, warp and CTA; each CTA's atomicAdd then sees in the old value whether the total passed INT64_MAX
+// (the counter only rises, so the CTA whose add crosses 2^63 sees it before any add could wrap 2^64).  One atomic per
+// CTA and word, not per warp: with per-warp atomics a call on a million rows took 45 us instead of 34 us (B200, 1000 W).
+constexpr int kExtentThreads = 256;
+
+template <typename Measure>
+__global__ void __launch_bounds__(kExtentThreads)
+offsets_extent_kernel(const int64_t *__restrict__ offs, int64_t n, int64_t nbytes, Measure m, unsigned long long *out) {
+    constexpr int kWarps = kExtentThreads / 32;
+    __shared__ int64_t s_part[3][kWarps];
+    __shared__ unsigned s_bad[kWarps];
+    int64_t s0 = 0, s1 = 0, best = 0;
+    unsigned bad = 0;
+    bool over = false;
+    for (int64_t i = blockIdx.x * static_cast<int64_t>(kExtentThreads) + threadIdx.x; i < n; i += static_cast<int64_t>(gridDim.x) * kExtentThreads) {
+        const int64_t a = offs[i], b = offs[i + 1];
+        if (b < a) bad |= 1u;
+        if (i == 0 && a < 0) bad |= 2u;
+        if (i == n - 1 && nbytes >= 0 && b > nbytes) bad |= 4u;
+        // negative: b < a, or a < 0 with more than INT64_MAX after it (flagged at offsets[0] or an earlier decrease)
+        const int64_t len = static_cast<int64_t>(static_cast<uint64_t>(b) - static_cast<uint64_t>(a));
+        if (len < 0) continue;
+        const Extent e = m.extent(len);
+        over |= e.over;
+        s0 = add_sat(s0, e.sum0, &over);
+        s1 = add_sat(s1, e.sum1, &over);
+        best = max(best, e.max);
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
+        s0 = add_sat(s0, __shfl_xor_sync(0xffffffffu, s0, o), &over);
+        s1 = add_sat(s1, __shfl_xor_sync(0xffffffffu, s1, o), &over);
+    }
+    bad = __reduce_or_sync(0xffffffffu, bad | (over ? 8u : 0u));
+    const int warp = threadIdx.x >> 5;
+    if ((threadIdx.x & 31) == 0) {
+        s_part[0][warp] = s0;
+        s_part[1][warp] = s1;
+        s_part[2][warp] = best;
+        s_bad[warp] = bad;
+    }
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    for (int w = 1; w < kWarps; ++w) {
+        s0 = add_sat(s0, s_part[0][w], &over);
+        s1 = add_sat(s1, s_part[1][w], &over);
+        best = max(best, s_part[2][w]);
+        bad |= s_bad[w];
+    }
+    const unsigned long long kMax = static_cast<unsigned long long>(kI64Max);
+    if (s0 > 0) {
+        const unsigned long long old = atomicAdd(out, static_cast<unsigned long long>(s0));
+        over |= old > kMax || old + s0 > kMax;
+    }
+    if (s1 > 0) {
+        const unsigned long long old = atomicAdd(out + 1, static_cast<unsigned long long>(s1));
+        over |= old > kMax || old + s1 > kMax;
+    }
+    if (best > 0) atomicMax(out + 2, static_cast<unsigned long long>(best));
+    if (over) bad |= 8u;
+    if (bad) atomicOr(out + 3, static_cast<unsigned long long>(bad));
+}
+
+// BSQ_ERR_ARG for the first of offsets_extent_kernel's validation bits that is set (BSQ_OK when none is)
+int offsets_error(unsigned long long bits);
+
+// The offsets reduction of n rows of device offsets on st: one launch, one read-back, one synchronise.  Fails on bad
+// offsets; a total past INT64_MAX is left to the caller (e->over), whose output it sizes.
+template <typename Measure>
+int reduce_offsets_device(int device, cudaStream_t st, const int64_t *d_offs, int64_t n, int64_t nbytes, const Measure &m, Extent *e) {
+    BSQ_CUDA_TRY(cudaSetDevice(device));
+    unsigned long long *d_res = nullptr, h_res[4] = {0, 0, 0, 0};
+    if (int rc = scratch_alloc(device, reinterpret_cast<void **>(&d_res), sizeof(h_res), st)) return rc;
+    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, sizeof(h_res), st));
+    const int blocks = static_cast<int>(std::min<int64_t>((n + kExtentThreads - 1) / kExtentThreads, static_cast<int64_t>(cur_sms()) * 8));
+    offsets_extent_kernel<<<blocks, kExtentThreads, 0, st>>>(d_offs, n, nbytes, m, d_res);
+    count_launch();
+    BSQ_CUDA_TRY(cudaGetLastError());
+    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, sizeof(h_res), cudaMemcpyDeviceToHost, st));
+    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
+    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
+    if (int rc = offsets_error(h_res[3] & 7u)) return rc;
+    *e = Extent{static_cast<int64_t>(h_res[0]), static_cast<int64_t>(h_res[1]), static_cast<int64_t>(h_res[2]), (h_res[3] & 8u) != 0};
+    return BSQ_OK;
+}
+
+// The same of host offsets: offsets[0] < 0 first, then row by row up to the first negative length (an error) or the
+// first row that takes a total past INT64_MAX (e->over).
+template <typename Measure>
+int reduce_offsets_host(const int64_t *h_offs, int64_t n, const Measure &m, Extent *e) {
+    if (h_offs[0] < 0) return offsets_error(2u);
+    *e = Extent{0, 0, 0, false};
+    for (int64_t i = 0; i < n && !e->over; ++i) {
+        const int64_t len = h_offs[i + 1] - h_offs[i];  // (both >= offsets[0] >= 0 so far: no overflow)
+        if (len < 0) return offsets_error(1u);
+        const Extent r = m.extent(len);
+        e->over |= r.over;
+        e->sum0 = add_sat(e->sum0, r.sum0, &e->over);
+        e->sum1 = add_sat(e->sum1, r.sum1, &e->over);
+        e->max = r.max > e->max ? r.max : e->max;
+    }
+    return BSQ_OK;
 }
 
 // word w (0..3) of a block, with selects (a run-time index into the block would put it in local memory)

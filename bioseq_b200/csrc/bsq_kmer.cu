@@ -41,10 +41,14 @@ struct KmerParam {
     uint32_t pad;    // what follows EOS in a padded row: pad_id with padchar, else 0
 };
 
-// the per-row count of the cu_seqlens scan
+// the per-row count of the cu_seqlens scan, and the extents' measure: the sum and the max of T(len_i)
 struct KmerCountFn {
     KmerShape ks;
-    __device__ __forceinline__ int64_t operator()(int64_t len) const { return kmer_tokens(len, ks); }
+    __host__ __device__ __forceinline__ int64_t operator()(int64_t len) const { return kmer_tokens(len, ks); }
+    __host__ __device__ __forceinline__ Extent extent(int64_t len) const {
+        const int64_t t = kmer_tokens(len, ks);
+        return t < 0 ? Extent{kI64Max, 0, kI64Max, true} : Extent{t, 0, t, false};
+    }
 };
 
 // Ids of columns c_lo + (t - tlo), t in [tlo, thi), of a row of n residues at src, into tok[t].
@@ -178,33 +182,6 @@ kmer_varlen_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict_
     }
 }
 
-// K11's sibling of K0c for bsq_kmer_extent_device: the same validation bits, max T in out[0] and sum T in out[2].
-__global__ void kmer_extent_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, KmerShape ks,
-                                   unsigned long long *out) {
-    long long best = 0, sum = 0;
-    unsigned bad = 0;
-    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq;
-         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-        const long long len = static_cast<long long>(offs[i + 1] - offs[i]);
-        if (len < 0) bad |= 1u;
-        if (i == 0 && offs[0] < 0) bad |= 2u;
-        if (i == nseq - 1 && nbytes >= 0 && offs[nseq] > nbytes) bad |= 4u;
-        const long long t = kmer_tokens(max(len, 0ll), ks);
-        best = max(best, t);
-        sum += t;
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-        best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
-        sum += __shfl_xor_sync(0xffffffffu, sum, o);
-    }
-    bad = __reduce_or_sync(0xffffffffu, bad);
-    if ((threadIdx.x & 31) == 0) {
-        if (best > 0) atomicMax(out, static_cast<unsigned long long>(best));
-        if (bad) atomicOr(out + 1, static_cast<unsigned long long>(bad));
-        if (sum > 0) atomicAdd(out + 2, static_cast<unsigned long long>(sum));
-    }
-}
-
 KmerShape shape_of(const bsq_kmer &km) {
     return KmerShape{km.k, km.stride, km.tail == BSQ_KMER_SINGLE, km.bos, km.eos, make_fastdiv(static_cast<uint32_t>(km.stride))};
 }
@@ -263,15 +240,7 @@ int launch_kmer(cudaStream_t st, const uint8_t *d_bytes, const int64_t *d_offs, 
         BSQ_CUDA_TRY(cudaGetLastError());
         return BSQ_OK;
     }
-    const int64_t nblocks = (nseq + kRowScan - 1) / kRowScan;
-    row_scan_kernel<<<static_cast<unsigned>(nblocks), kRowScan, 0, st>>>(d_offs, nseq, KmerCountFn{p.ks}, d_cu);
-    count_launch();
-    BSQ_CUDA_TRY(cudaGetLastError());
-    if (nblocks > 1) {
-        row_carry_kernel<<<1, kRowScan, 0, st>>>(d_cu, nseq, nblocks);
-        count_launch();
-        BSQ_CUDA_TRY(cudaGetLastError());
-    }
+    if (int rc = launch_row_scan(st, d_offs, nseq, KmerCountFn{p.ks}, d_cu)) return rc;
     const int64_t rows_per_cta = kKThreads / 32;
     kmer_varlen_kernel<T><<<static_cast<unsigned>((nseq + rows_per_cta - 1) / rows_per_cta), kKThreads, 0, st>>>(
         d_bytes, d_offs, nseq, p, lutp, o, d_cu);
@@ -345,18 +314,11 @@ extern "C" int bsq_kmer_extent_host(const int64_t *h_offsets, int64_t nseq, cons
     if (km->k < 1 || km->stride < 1 || km->stride > km->k) return fail(BSQ_ERR_ARG, "bad k-mer descriptor");
     *total = *max_tokens = 0;
     if (nseq == 0) return BSQ_OK;
-    if (h_offsets[0] < 0) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
-    const KmerShape ks = shape_of(*km);
-    int64_t sum = 0, best = 0;
-    for (int64_t i = 0; i < nseq; ++i) {
-        const int64_t len = h_offsets[i + 1] - h_offsets[i];
-        if (len < 0) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
-        const int64_t t = kmer_tokens(len, ks);
-        sum += t;
-        best = std::max(best, t);
-    }
-    *total = sum;
-    *max_tokens = best;
+    Extent e{};
+    if (int rc = reduce_offsets_host(h_offsets, nseq, KmerCountFn{shape_of(*km)}, &e)) return rc;
+    if (e.over) return fail(BSQ_ERR_ARG, "the k-mer tokens exceed INT64_MAX");
+    *total = e.sum0;
+    *max_tokens = e.max;
     return BSQ_OK;
 }
 
@@ -368,23 +330,12 @@ extern "C" int bsq_kmer_extent_device(int device, void *stream, const int64_t *d
     if (km->k < 1 || km->stride < 1 || km->stride > km->k) return fail(BSQ_ERR_ARG, "bad k-mer descriptor");
     *total = *max_tokens = 0;
     if (nseq == 0) return BSQ_OK;
-    BSQ_CUDA_TRY(cudaSetDevice(device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    unsigned long long *d_res = nullptr, h_res[3] = {0, 0, 0};
-    BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&d_res), sizeof(h_res), st));
-    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, sizeof(h_res), st));
-    const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
-    kmer_extent_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, shape_of(*km), d_res);
-    count_launch();
-    BSQ_CUDA_TRY(cudaGetLastError());
-    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, sizeof(h_res), cudaMemcpyDeviceToHost, st));
-    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
-    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
-    if (h_res[1] & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
-    if (h_res[1] & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
-    if (h_res[1] & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
-    *total = static_cast<int64_t>(h_res[2]);
-    *max_tokens = static_cast<int64_t>(h_res[0]);
+    Extent e{};
+    if (int rc = reduce_offsets_device(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, KmerCountFn{shape_of(*km)}, &e))
+        return rc;
+    if (e.over) return fail(BSQ_ERR_ARG, "the k-mer tokens exceed INT64_MAX");
+    *total = e.sum0;
+    *max_tokens = e.max;
     return BSQ_OK;
 }
 

@@ -6,10 +6,10 @@
 // statement of the rule in the library (host extent, device extent and both kernels use it).
 //
 // K13a, bsq_tile (no state between launches, capturable into a CUDA graph):
-//   row_scan_kernel x2  (+ row_carry_kernel x2 past 1024 sequences, bsq_kernels.cuh) the per-sequence window counts into
-//                       seq_ptr, and the per-sequence output byte totals (closed form: (m - 1) W + len_last for SHORT,
-//                       m W otherwise) into byte_ptr.  byte_ptr, and seq_ptr when the caller passes none, live in
-//                       stream-ordered scratch (cudaMallocAsync / cudaFreeAsync on the call's stream).
+//   row_scan_kernel + row_carry_kernel, twice (the carry only past 1024 sequences, bsq_kernels.cuh): the per-sequence
+//                       window counts into seq_ptr, then the per-sequence output byte totals (closed form: (m - 1) W +
+//                       len_last for SHORT, m W otherwise) into byte_ptr.  byte_ptr, and seq_ptr when the caller passes
+//                       none, live in stream-ordered scratch (cudaMallocAsync / cudaFreeAsync on the call's stream).
 //   tile_fix_kernel     one thread per sequence adds the carry of its scan CTA to both entries (as K9's gather does).
 //   tile_gather_kernel  a grid-stride pass over the windows writes out_offsets, seq_index and starts (a binary search of
 //                       seq_ptr per window), then the bytes: a flat map over the 16-byte aligned output vectors in tiles
@@ -75,6 +75,16 @@ struct WinCount {
 struct ByteCount {
     TileShape t;
     __device__ __forceinline__ int64_t operator()(int64_t len) const { return tile_bytes<int64_t>(len, tile_count(len, t), t); }
+};
+// the extents' measure: windows, their bytes, and the longest window
+struct TileMeasure {
+    TileShape t;
+    __host__ __device__ __forceinline__ Extent extent(int64_t len) const {
+        const int64_t m = tile_count(len, t);
+        bool over = false;
+        const int64_t nb = clamp_sat(tile_bytes<__int128>(len, m, t), &over);
+        return {m, nb, len < t.W ? len : t.W, over};
+    }
 };
 
 // the scan entries that are not the last of their scan CTA get that CTA's carry (the last ones are final already and are
@@ -351,60 +361,6 @@ int check_shape(int64_t W, int64_t S, int tail) {
     return BSQ_OK;
 }
 
-constexpr __int128 kI64Max = (__int128(1) << 63) - 1;
-
-// the bsq_tile_extent_device reduction: validation bits in out[0] (1: negative length, 2: offsets[0] < 0, 4: past nbytes,
-// 8: a total past INT64_MAX), sum m in out[1], sum bytes in out[2], max window length in out[3]
-__device__ __forceinline__ void sat_add(unsigned long long *p, unsigned long long v, unsigned *bad) {
-    unsigned long long old = *reinterpret_cast<volatile unsigned long long *>(p), assumed;
-    do {
-        assumed = old;
-        unsigned long long nv = assumed + v;  // both <= INT64_MAX: no wrap
-        if (nv > static_cast<unsigned long long>(kI64Max)) {
-            nv = static_cast<unsigned long long>(kI64Max);
-            *bad |= 8u;
-        }
-        old = atomicCAS(p, assumed, nv);
-    } while (old != assumed);
-}
-
-__global__ void tile_extent_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, TileShape t,
-                                   unsigned long long *out) {
-    unsigned long long wins = 0, byts = 0;
-    long long best = 0;
-    unsigned bad = 0;
-    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-        const int64_t a = offs[i], b = offs[i + 1];
-        if (b < a) bad |= 1u;
-        if (i == 0 && a < 0) bad |= 2u;
-        if (i == nseq - 1 && nbytes >= 0 && b > nbytes) bad |= 4u;
-        const __int128 len128 = static_cast<__int128>(b) - a;
-        if (len128 < 0 || len128 > kI64Max) continue;
-        const int64_t len = static_cast<int64_t>(len128);
-        const int64_t m = tile_count(len, t);
-        const __int128 nb = tile_bytes<__int128>(len, m, t);
-        const __int128 sw = static_cast<__int128>(wins) + m, sb = static_cast<__int128>(byts) + nb;
-        if (sw > kI64Max || sb > kI64Max) bad |= 8u;
-        wins = static_cast<unsigned long long>(sw > kI64Max ? kI64Max : sw);
-        byts = static_cast<unsigned long long>(sb > kI64Max ? kI64Max : sb);
-        best = max(best, static_cast<long long>(min(len, t.W)));
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-        best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
-        const unsigned long long w2 = __shfl_xor_sync(0xffffffffu, wins, o), b2 = __shfl_xor_sync(0xffffffffu, byts, o);
-        if (wins + w2 > static_cast<unsigned long long>(kI64Max) || byts + b2 > static_cast<unsigned long long>(kI64Max)) bad |= 8u;
-        wins = min(wins + w2, static_cast<unsigned long long>(kI64Max));
-        byts = min(byts + b2, static_cast<unsigned long long>(kI64Max));
-    }
-    if ((threadIdx.x & 31) == 0) {
-        if (wins > 0) sat_add(out + 1, wins, &bad);
-        if (byts > 0) sat_add(out + 2, byts, &bad);
-        if (best > 0) atomicMax(out + 3, static_cast<unsigned long long>(best));
-    }
-    bad = __reduce_or_sync(0xffffffffu, bad);
-    if ((threadIdx.x & 31) == 0 && bad) atomicOr(out, static_cast<unsigned long long>(bad));
-}
-
 }  // namespace
 
 }  // namespace bsq
@@ -418,22 +374,12 @@ extern "C" int bsq_tile_extent_host(const int64_t *h_offsets, int64_t nseq, int6
     if (nseq < 0 || (nseq > 0 && h_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
     *nwin = *nbytes = *max_len = 0;
     if (nseq == 0) return BSQ_OK;
-    if (h_offsets[0] < 0) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
-    const TileShape t{window, stride, tail};
-    __int128 sw = 0, sb = 0;
-    int64_t best = 0;
-    for (int64_t i = 0; i < nseq; ++i) {
-        const int64_t len = h_offsets[i + 1] - h_offsets[i];  // (both in [0, INT64_MAX]: no overflow)
-        if (len < 0) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
-        const int64_t m = tile_count(len, t);
-        sw += m;
-        sb += tile_bytes<__int128>(len, m, t);
-        if (sw > kI64Max || sb > kI64Max) return fail(BSQ_ERR_ARG, "the windows' count or bytes exceed INT64_MAX");
-        best = std::max(best, std::min(len, window));
-    }
-    *nwin = static_cast<int64_t>(sw);
-    *nbytes = static_cast<int64_t>(sb);
-    *max_len = best;
+    Extent e{};
+    if (int rc = reduce_offsets_host(h_offsets, nseq, TileMeasure{{window, stride, tail}}, &e)) return rc;
+    if (e.over) return fail(BSQ_ERR_ARG, "the windows' count or bytes exceed INT64_MAX");
+    *nwin = e.sum0;
+    *nbytes = e.sum1;
+    *max_len = e.max;
     return BSQ_OK;
 }
 
@@ -445,25 +391,14 @@ extern "C" int bsq_tile_extent_device(int device, void *stream, const int64_t *d
     if (nseq < 0 || (nseq > 0 && d_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
     *nwin = *out_nbytes = *max_len = 0;
     if (nseq == 0) return BSQ_OK;
-    BSQ_CUDA_TRY(cudaSetDevice(device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    unsigned long long *d_res = nullptr, h_res[4] = {0, 0, 0, 0};
-    BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&d_res), sizeof(h_res), st));
-    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, sizeof(h_res), st));
-    const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
-    tile_extent_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, TileShape{window, stride, tail}, d_res);
-    count_launch();
-    BSQ_CUDA_TRY(cudaGetLastError());
-    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, sizeof(h_res), cudaMemcpyDeviceToHost, st));
-    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
-    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
-    if (h_res[0] & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
-    if (h_res[0] & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
-    if (h_res[0] & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
-    if (h_res[0] & 8u) return fail(BSQ_ERR_ARG, "the windows' count or bytes exceed INT64_MAX");
-    *nwin = static_cast<int64_t>(h_res[1]);
-    *out_nbytes = static_cast<int64_t>(h_res[2]);
-    *max_len = static_cast<int64_t>(h_res[3]);
+    Extent e{};
+    if (int rc = reduce_offsets_device(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, TileMeasure{{window, stride, tail}},
+                                       &e))
+        return rc;
+    if (e.over) return fail(BSQ_ERR_ARG, "the windows' count or bytes exceed INT64_MAX");
+    *nwin = e.sum0;
+    *out_nbytes = e.sum1;
+    *max_len = e.max;
     return BSQ_OK;
 }
 
@@ -488,20 +423,9 @@ extern "C" int bsq_tile(int device, void *stream, const uint8_t *d_bytes, const 
     const size_t ns = static_cast<size_t>(nseq + 1) * (d_seq_ptr != nullptr ? 1 : 2);
     BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&scratch), ns * sizeof(int64_t), st));
     int64_t *byte_ptr = scratch, *seq_ptr = d_seq_ptr != nullptr ? d_seq_ptr : scratch + nseq + 1;
-    const int64_t nblocks = (nseq + kRowScan - 1) / kRowScan;
-    row_scan_kernel<<<static_cast<unsigned>(nblocks), kRowScan, 0, st>>>(d_offsets, nseq, WinCount{t}, seq_ptr);
-    count_launch();
-    BSQ_CUDA_TRY(cudaGetLastError());
-    row_scan_kernel<<<static_cast<unsigned>(nblocks), kRowScan, 0, st>>>(d_offsets, nseq, ByteCount{t}, byte_ptr);
-    count_launch();
-    BSQ_CUDA_TRY(cudaGetLastError());
-    if (nblocks > 1) {
-        row_carry_kernel<<<1, kRowScan, 0, st>>>(seq_ptr, nseq, nblocks);
-        count_launch();
-        BSQ_CUDA_TRY(cudaGetLastError());
-        row_carry_kernel<<<1, kRowScan, 0, st>>>(byte_ptr, nseq, nblocks);
-        count_launch();
-        BSQ_CUDA_TRY(cudaGetLastError());
+    if (int rc = launch_row_scan(st, d_offsets, nseq, WinCount{t}, seq_ptr)) return rc;
+    if (int rc = launch_row_scan(st, d_offsets, nseq, ByteCount{t}, byte_ptr)) return rc;
+    if (nseq > kRowScan) {
         tile_fix_kernel<<<static_cast<unsigned>((nseq + 255) / 256), 256, 0, st>>>(nseq, seq_ptr, byte_ptr);
         count_launch();
         BSQ_CUDA_TRY(cudaGetLastError());

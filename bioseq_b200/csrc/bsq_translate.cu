@@ -61,6 +61,25 @@ struct TranslateCount {
     FrameSet fs;
     __device__ __forceinline__ int64_t operator()(int64_t len) const { return tr_row_total(len, fs); }
 };
+// the extents' measure: the row's amino acids, the same after a crop to crop_len, and its longest cropped frame (a row
+// has at most 2 len amino acids, so the 128-bit sums cannot wrap)
+struct TranslateMeasure {
+    FrameSet fs;
+    int64_t crop_len;
+    __host__ __device__ __forceinline__ Extent extent(int64_t len) const {
+        __int128 t = 0, c = 0;
+        int64_t best = 0;
+        for (int f = 0; f < fs.F; ++f) {
+            const int64_t L = tr_len(len, frame_code(fs.fcode, f)), k = L < crop_len ? L : crop_len;
+            t += L;
+            c += k;
+            best = k > best ? k : best;
+        }
+        bool over = false;
+        const int64_t st = clamp_sat(t, &over), sc = clamp_sat(c, &over);
+        return {st, sc, best, over};
+    }
+};
 
 // BSQ_ERR_ARG unless frames holds 1..6 distinct values of +-1, +-2, +-3; fills *fs
 int check_frames(const int8_t *frames, int nframes, FrameSet *fs) {
@@ -363,44 +382,6 @@ translate_kernel(TrArgs a, const __grid_constant__ TrTables tbl, uint8_t *__rest
     }
 }
 
-// The bsq_translate_extent_device reduction: validation bits in out[0] (1: negative length, 2: offsets[0] < 0, 4: past
-// nbytes), sum of the row totals in out[1], of the cropped frame lengths in out[2], the longest cropped frame in out[3].
-// (Valid offsets hold at most INT64_MAX nucleotides and every row at most twice its length, so the sums fit 64 bits.)
-__global__ void translate_extent_kernel(const int64_t *__restrict__ offs, int64_t nseq, int64_t nbytes, FrameSet fs, int64_t crop_len,
-                                        unsigned long long *out) {
-    unsigned long long tot = 0, cropped = 0;
-    long long best = 0;
-    unsigned bad = 0;
-    for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < nseq; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
-        const int64_t a = offs[i], b = offs[i + 1];
-        if (b < a) bad |= 1u;
-        if (i == 0 && a < 0) bad |= 2u;
-        if (i == nseq - 1 && nbytes >= 0 && b > nbytes) bad |= 4u;
-        if (b < a) continue;
-        const int64_t len = b - a;
-        for (int f = 0; f < fs.F; ++f) {
-            const int64_t L = tr_len(len, frame_code(fs.fcode, f)), c = min(L, crop_len);
-            tot += static_cast<unsigned long long>(L);
-            cropped += static_cast<unsigned long long>(c);
-            best = max(best, static_cast<long long>(c));
-        }
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-        best = max(best, __shfl_xor_sync(0xffffffffu, best, o));
-        tot += __shfl_xor_sync(0xffffffffu, tot, o);
-        cropped += __shfl_xor_sync(0xffffffffu, cropped, o);
-    }
-    bad = __reduce_or_sync(0xffffffffu, bad);
-    if ((threadIdx.x & 31) == 0) {
-        if (bad) atomicOr(out, static_cast<unsigned long long>(bad));
-        if (tot > 0) atomicAdd(out + 1, tot);
-        if (cropped > 0) atomicAdd(out + 2, cropped);
-        if (best > 0) atomicMax(out + 3, static_cast<unsigned long long>(best));
-    }
-}
-
-constexpr unsigned long long kI64Max = (1ull << 63) - 1;
-
 }  // namespace
 
 }  // namespace bsq
@@ -442,23 +423,12 @@ extern "C" int bsq_translate_extent_host(const int64_t *h_offsets, int64_t nseq,
     if (nseq < 0 || (nseq > 0 && h_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
     *total = *crop_total = *max_len = 0;
     if (nseq == 0) return BSQ_OK;
-    if (h_offsets[0] < 0) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
-    __int128 st = 0, sc = 0;
-    int64_t best = 0;
-    for (int64_t i = 0; i < nseq; ++i) {
-        const int64_t len = h_offsets[i + 1] - h_offsets[i];  // (both in [0, INT64_MAX]: no overflow)
-        if (len < 0) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
-        for (int f = 0; f < fs.F; ++f) {
-            const int64_t L = tr_len(len, frame_code(fs.fcode, f)), c = std::min(L, crop_len);
-            st += L;
-            sc += c;
-            best = std::max(best, c);
-        }
-    }
-    if (st > static_cast<__int128>(kI64Max)) return fail(BSQ_ERR_ARG, "the translated batch exceeds INT64_MAX bytes");
-    *total = static_cast<int64_t>(st);
-    *crop_total = static_cast<int64_t>(sc);
-    *max_len = best;
+    Extent e{};
+    if (int rc = reduce_offsets_host(h_offsets, nseq, TranslateMeasure{fs, crop_len}, &e)) return rc;
+    if (e.over) return fail(BSQ_ERR_ARG, "the translated batch exceeds INT64_MAX bytes");
+    *total = e.sum0;
+    *crop_total = e.sum1;
+    *max_len = e.max;
     return BSQ_OK;
 }
 
@@ -473,25 +443,13 @@ extern "C" int bsq_translate_extent_device(int device, void *stream, const int64
     if (nseq < 0 || (nseq > 0 && d_offsets == nullptr)) return fail(BSQ_ERR_ARG, "bad offsets");
     *total = *crop_total = *max_len = 0;
     if (nseq == 0) return BSQ_OK;
-    BSQ_CUDA_TRY(cudaSetDevice(device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    unsigned long long *d_res = nullptr, h_res[4] = {0, 0, 0, 0};
-    BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&d_res), sizeof(h_res), st));
-    BSQ_CUDA_TRY(cudaMemsetAsync(d_res, 0, sizeof(h_res), st));
-    const int blocks = static_cast<int>(std::min<int64_t>((nseq + 255) / 256, static_cast<int64_t>(cur_sms()) * 8));
-    translate_extent_kernel<<<blocks, 256, 0, st>>>(d_offsets, nseq, nbytes, fs, crop_len, d_res);
-    count_launch();
-    BSQ_CUDA_TRY(cudaGetLastError());
-    BSQ_CUDA_TRY(cudaMemcpyAsync(h_res, d_res, sizeof(h_res), cudaMemcpyDeviceToHost, st));
-    BSQ_CUDA_TRY(cudaFreeAsync(d_res, st));
-    BSQ_CUDA_TRY(cudaStreamSynchronize(st));
-    if (h_res[0] & 1u) return fail(BSQ_ERR_ARG, "offsets must be non-decreasing");
-    if (h_res[0] & 2u) return fail(BSQ_ERR_ARG, "offsets must start at or after 0");
-    if (h_res[0] & 4u) return fail(BSQ_ERR_ARG, "offsets run past the end of bytes");
-    if (h_res[1] > kI64Max) return fail(BSQ_ERR_ARG, "the translated batch exceeds INT64_MAX bytes");
-    *total = static_cast<int64_t>(h_res[1]);
-    *crop_total = static_cast<int64_t>(h_res[2]);
-    *max_len = static_cast<int64_t>(h_res[3]);
+    Extent e{};
+    if (int rc = reduce_offsets_device(device, static_cast<cudaStream_t>(stream), d_offsets, nseq, nbytes, TranslateMeasure{fs, crop_len}, &e))
+        return rc;
+    if (e.over) return fail(BSQ_ERR_ARG, "the translated batch exceeds INT64_MAX bytes");
+    *total = e.sum0;
+    *crop_total = e.sum1;
+    *max_len = e.max;
     return BSQ_OK;
 }
 
@@ -501,7 +459,7 @@ extern "C" int bsq_translate(int device, void *stream, const uint8_t *d_bytes, c
     FrameSet fs;
     if (int rc = check_frames(frames, nframes, &fs)) return rc;
     if (int rc = check_code(code64)) return rc;
-    if (nseq < 0 || nseq > static_cast<int64_t>(kI64Max / 6) - 1) return fail(BSQ_ERR_ARG, "bad batch size");
+    if (nseq < 0 || nseq > kI64Max / 6 - 1) return fail(BSQ_ERR_ARG, "bad batch size");
     if (d_out_offsets == nullptr) return fail(BSQ_ERR_ARG, "null output offsets");
     if (nseq > 0 && (d_bytes == nullptr || d_offsets == nullptr || d_out_bytes == nullptr))
         return fail(BSQ_ERR_ARG, "null bytes, offsets or output bytes");
@@ -522,15 +480,7 @@ extern "C" int bsq_translate(int device, void *stream, const uint8_t *d_bytes, c
     std::memcpy(tt.codon, t.codon, sizeof(tt.codon));
     int64_t *S = nullptr;
     BSQ_CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&S), static_cast<size_t>(nseq + 1) * sizeof(int64_t), st));
-    const int64_t nblocks = (nseq + kRowScan - 1) / kRowScan;
-    row_scan_kernel<<<static_cast<unsigned>(nblocks), kRowScan, 0, st>>>(d_offsets, nseq, TranslateCount{fs}, S);
-    count_launch();
-    BSQ_CUDA_TRY(cudaGetLastError());
-    if (nblocks > 1) {
-        row_carry_kernel<<<1, kRowScan, 0, st>>>(S, nseq, nblocks);
-        count_launch();
-        BSQ_CUDA_TRY(cudaGetLastError());
-    }
+    if (int rc = launch_row_scan(st, d_offsets, nseq, TranslateCount{fs}, S)) return rc;
     TrArgs a;
     a.bytes = d_bytes;
     a.offs = d_offsets;
