@@ -5,7 +5,7 @@
 // (g_lo, g_hi, 0, 3), g = seq_index_base + i.  out_offsets is the exclusive scan of len'_i (out_offsets[0] = 0).
 //
 // Three launches, no scratch memory and no state between launches (capturable into a CUDA graph):
-//   row_scan_kernel     one thread per row, kCScan rows per CTA: len'_i (CropCount), the CTA's inclusive scan of them
+//   row_scan_kernel     one thread per row, kRowScan rows per CTA: len'_i (CropCount), the CTA's inclusive scan of them
 //                       (block_exclusive_scan) written to out_offsets[i + 1].  The entry at the end of each CTA's rows
 //                       is then that CTA's total.  (Shared with K11's cu_seqlens, bsq_kernels.cuh.)
 //   row_carry_kernel    one CTA (only when there is more than one scan CTA): scans the CTA totals in place, so every
@@ -29,7 +29,6 @@ namespace bsq {
 
 namespace {
 
-constexpr int kCScan = kRowScan;  // rows per row_scan_kernel CTA
 constexpr int kCThreads = 256;  // crop_gather_kernel: 8 warps, one row each
 
 struct CropParam {
@@ -56,14 +55,12 @@ crop_gather_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict_
     const int64_t s = __ldg(offs + i), len = __ldg(offs + i + 1) - s;
     const int64_t kept = min(len, c.W);
     const int64_t st = crop_start(len, i, c);
-    // the row's end offset: its CTA-local inclusive prefix plus the carry, unless it closes a scan CTA (already final)
-    const int64_t e_idx = i + 1, blk = i / kCScan;
-    const bool final_entry = (e_idx % kCScan) == 0 || e_idx == n;
-    int64_t e = out_offs[e_idx];
-    if (!final_entry && blk > 0) e += out_offs[blk * kCScan];
+    // the row's end offset: its CTA-local inclusive prefix plus the carry it still lacks
+    const int64_t carry = row_scan_carry(out_offs, i + 1, n);
+    const int64_t e = out_offs[i + 1] + carry;
     __syncwarp();
     if (lane == 0) {
-        if (!final_entry) out_offs[e_idx] = e;
+        if (carry != 0) out_offs[i + 1] = e;
         if (starts != nullptr) starts[i] = st;
     }
     if (kept <= 0) return;

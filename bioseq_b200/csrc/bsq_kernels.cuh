@@ -177,21 +177,32 @@ __device__ __forceinline__ uint4 ldg16(uintptr_t addr) {
 
 __device__ __forceinline__ uintptr_t clamp_word(uintptr_t a, uintptr_t lo, uintptr_t hi) { return a < lo ? lo : (a > hi ? hi : a); }
 
-// The 16 bytes at address X (any alignment) as four little-endian words, from the aligned words at X & ~15 and the next
-// one, each clamped to [lo, hi] (16-byte aligned).  The shift may vary from thread to thread, so the words are picked
-// with selects.  Used by K12 (bsq_revcomp.cu) and K13 (bsq_tile.cu).
-__device__ __forceinline__ void fetch16_clamped(uintptr_t X, uintptr_t lo, uintptr_t hi, uint32_t t[4]) {
+// The 4 * kWords bytes at address X (any alignment) as kWords little-endian words (kWords a multiple of 4), from the
+// aligned 16-byte words at X & ~15 and the kWords / 4 after it (the last only when X is not aligned), each clamped to
+// [lo, hi] (16-byte aligned).  The shift may vary from thread to thread, so the words are picked with selects.  K12 and
+// K13a read 16 bytes, K14b 48.
+template <int kWords>
+__device__ __forceinline__ void fetch_clamped(uintptr_t X, uintptr_t lo, uintptr_t hi, uint32_t t[kWords]) {
     const uintptr_t a0 = X & ~uintptr_t(15);
     const uint32_t s = static_cast<uint32_t>(X) & 15u;
-    const uint4 v0 = ldg16(clamp_word(a0, lo, hi));
-    const uint4 v1 = s != 0 ? ldg16(clamp_word(a0 + 16, lo, hi)) : make_uint4(0u, 0u, 0u, 0u);
+    uint32_t w[kWords + 4];
+#pragma unroll
+    for (int k = 0; k <= kWords / 4; ++k) {
+        const uint4 v = k < kWords / 4 || s != 0 ? ldg16(clamp_word(a0 + 16 * k, lo, hi)) : make_uint4(0u, 0u, 0u, 0u);
+        w[4 * k] = v.x;
+        w[4 * k + 1] = v.y;
+        w[4 * k + 2] = v.z;
+        w[4 * k + 3] = v.w;
+    }
     const bool q2 = (s & 8u) != 0, q1 = (s & 4u) != 0;
-    const uint32_t a_0 = q2 ? v0.z : v0.x, a_1 = q2 ? v0.w : v0.y, a_2 = q2 ? v1.x : v0.z, a_3 = q2 ? v1.y : v0.w;
-    const uint32_t a_4 = q2 ? v1.z : v1.x, a_5 = q2 ? v1.w : v1.y;
-    const uint32_t x[5] = {q1 ? a_1 : a_0, q1 ? a_2 : a_1, q1 ? a_3 : a_2, q1 ? a_4 : a_3, q1 ? a_5 : a_4};
+    uint32_t a[kWords + 2], b[kWords + 1];
+#pragma unroll
+    for (int k = 0; k < kWords + 2; ++k) a[k] = q2 ? w[k + 2] : w[k];
+#pragma unroll
+    for (int k = 0; k < kWords + 1; ++k) b[k] = q1 ? a[k + 1] : a[k];
     const uint32_t sh = (s & 3u) * 8u;
 #pragma unroll
-    for (int k = 0; k < 4; ++k) t[k] = __funnelshift_r(x[k], x[k + 1], sh);
+    for (int k = 0; k < kWords; ++k) t[k] = __funnelshift_r(b[k], b[k + 1], sh);
 }
 
 __device__ __forceinline__ void load_lut(uint8_t *lut_smem, const LutParam &p) {
@@ -447,7 +458,7 @@ __device__ __forceinline__ int64_t block_exclusive_scan(int64_t x, int64_t *s_wa
 //                     out[i + 1] (and out[0] = 0), so the entry at the end of each CTA's rows is that CTA's total.
 //   row_carry_kernel  one CTA, only when there is more than one scan CTA: scans the CTA totals in place, so every entry
 //                     at the end of a scan CTA's rows becomes final.
-// The consumer then finishes row i's entry itself (row_scan_final).
+// The consumer then finishes entry e itself by adding row_scan_carry (below).
 constexpr int kRowScan = 1024;  // block_exclusive_scan handles up to 1024 threads
 
 template <typename Count, typename Out>
@@ -493,6 +504,162 @@ int launch_row_scan(cudaStream_t st, const int64_t *d_offs, int64_t n, Count cou
         BSQ_CUDA_TRY(cudaGetLastError());
     }
     return BSQ_OK;
+}
+
+// What entry e of launch_row_scan's n + 1 entries still lacks: the entry that closes the previous scan CTA, or 0 when e
+// lies in the first scan CTA or closes a scan CTA or the batch (those entries are final, and never written by a
+// consumer, so every thread may read them).
+template <typename Out>
+__device__ __forceinline__ int64_t row_scan_carry(const Out *out_offs, int64_t e, int64_t n) {
+    const int64_t blk = (e - 1) / kRowScan;  // the scan CTA of row e - 1
+    if (e % kRowScan == 0 || e == n || blk == 0) return 0;
+    return static_cast<int64_t>(out_offs[blk * kRowScan]);
+}
+
+// ---- row searches over a tile of a packed output (K1v, K12, K13a, K14b) ----------------------------------------------
+
+// The largest r in [lo, hi) with key(r) <= x, for a non-decreasing key with key(lo) <= x: a (kThreads + 1)-ary search,
+// one probe per thread and one __syncthreads_count a round (two rounds up to 66 049 rows at 256 threads, three up to
+// 17 million).  Every thread of the block must call it; all get the answer.
+template <int kThreads, typename Key>
+__device__ __forceinline__ int64_t block_search_le(int64_t lo, int64_t hi, int64_t x, const Key &key) {
+    while (hi - lo > 1) {
+        const int64_t w = hi - lo;
+        const int64_t pr = lo + (static_cast<int64_t>(threadIdx.x) + 1) * w / (kThreads + 1);
+        const int cnt = __syncthreads_count(key(pr) <= x);  // a prefix of the probes
+        const int64_t nlo = cnt > 0 ? lo + static_cast<int64_t>(cnt) * w / (kThreads + 1) : lo;
+        const int64_t nhi = cnt < kThreads ? lo + (static_cast<int64_t>(cnt) + 1) * w / (kThreads + 1) : hi;
+        lo = nlo;
+        hi = nhi;
+    }
+    return lo;
+}
+
+// A tile's row table: stage(j, r) for the rows r = r0 + j <= last, kThreads a round, until a row starts at or after p1.
+// stage writes the caller's shared arrays for entry j and returns row r's start.  Returns the number of rows before
+// that first one (which the table holds as well), or -1 when the kCap entries run out first: an over-full tile.  Every
+// thread of the block must call it.
+template <int kThreads, int kCap, typename Stage>
+__device__ __forceinline__ int block_row_table(int64_t r0, int64_t last, int64_t p1, const Stage &stage) {
+    for (int base = 0; base < kCap; base += kThreads) {
+        const int j = base + static_cast<int>(threadIdx.x);
+        bool past = true;
+        if (r0 + j <= last) past = stage(j, r0 + j) >= p1;
+        const int cnt = __syncthreads_count(past);  // a suffix of the round
+        if (cnt > 0) return base + kThreads - cnt;
+    }
+    return -1;
+}
+
+// ---- the flat map over a packed output's 16-byte vectors (K12, K13a, K14b) -------------------------------------------
+// The output is n rows laid end to end from byte 0: row r covers [start(r), start(r + 1)), start(n) = total, and out may
+// have any alignment.  Its 16-byte aligned vectors are dealt in tiles of kFlatTile to a persistent grid of kFlatMinBlocks
+// CTAs per SM in a static order (no tile counter: a launch is capturable and may run concurrently with itself).  Per tile
+// the CTA
+//   1. finds the row of the tile's first byte with block_search_le over start;
+//   2. stages the tile's row starts, and the kernel's own row data, with block_row_table, up to the first row that starts
+//      at or after the tile's end (row n starts at total, so that entry exists and closes the table).  A tile of more
+//      than kFlatRowCap - 1 rows (rows shorter than 32 bytes on average, or many empty ones) is over-full and reads
+//      everything from global memory instead;
+//   3. per vector of output bytes [q, q + 16): a binary search of the table (or of global memory) for the row of its
+//      first byte, then a walk over the rows it touches up to the first whose end is at or past min(q + 16, total) -- in
+//      the table never past its closing entry.  Each non-empty row adds its bytes with the kernel's piece, merged by
+//      byte mask; a vector inside the output leaves as one st.global.cs.v4, the at most two partial vectors at the ends
+//      as byte stores.
+// The kernel supplies a Map m with
+//   int64_t start(int64_t r)          row r's start, from global memory (r <= n);
+//   void stage(int j, int64_t r)      its own row data of row r into table entry j;
+//   Row row_t(int j), row_g(int64_t r)   that data from entry j, or from global memory;
+//   void piece(q, r, s, e, row, res)  merge16 of row r (output span [s, e), data row) into bytes [q, q + 16) of res.
+constexpr int kFlatThreads = 256;
+constexpr int kFlatVecs = 16;                         // output vectors per thread and tile
+constexpr int kFlatTile = kFlatThreads * kFlatVecs;   // 4096 vectors: 64 KiB of output per tile
+constexpr int kFlatRowCap = 2048;                     // row-table entries: tiles of up to kFlatRowCap - 1 rows use the table
+constexpr int kFlatMinBlocks = 4;                     // CTAs per SM
+
+// Output bytes [k0, k1) of t into res (k0, k1 relative to the vector's first byte, any values)
+__device__ __forceinline__ void merge16(uint32_t res[4], const uint32_t t[4], int64_t k0, int64_t k1) {
+    const int m0 = static_cast<int>(min(max(k0, int64_t(0)), int64_t(16)));
+    const int m1 = static_cast<int>(min(max(k1, int64_t(0)), int64_t(16)));
+#pragma unroll
+    for (int w = 0; w < 4; ++w) {
+        const uint32_t mk = lt_mask(m1, w) & ~lt_mask(m0, w);
+        res[w] = (res[w] & ~mk) | (t[w] & mk);
+    }
+}
+
+// One vector: output bytes [q, q + 16) at dst (16-byte aligned), whose first byte in [0, total) lies in row r
+template <typename Map, typename StartOf, typename RowOf>
+__device__ __forceinline__ void flat_vector(int64_t q, int64_t r, int64_t total, const Map &m, const StartOf &start_of,
+                                            const RowOf &row_of, uint8_t *dst) {
+    uint32_t res[4] = {0u, 0u, 0u, 0u};
+    const int64_t stop = min(q + 16, total);
+    int64_t s = start_of(r);
+    for (;;) {
+        const int64_t e = start_of(r + 1);
+        if (e > s) m.piece(q, r, s, e, row_of(r), res);
+        if (e >= stop) break;
+        ++r;
+        s = e;
+    }
+    if (q >= 0 && q + 16 <= total) {
+        __stcs(reinterpret_cast<uint4 *>(dst), make_uint4(res[0], res[1], res[2], res[3]));
+    } else {
+#pragma unroll
+        for (int k = 0; k < 16; ++k)
+            if (q + k >= 0 && q + k < total) dst[k] = static_cast<uint8_t>(res[k >> 2] >> (8 * (k & 3)));
+    }
+}
+
+// The output's bytes; every thread of the block must call it (blockDim.x = kFlatThreads).
+template <typename Map>
+__device__ __forceinline__ void flat_map(uint8_t *out, int64_t n, int64_t total, const Map &m) {
+    __shared__ int64_t tab[kFlatRowCap];  // starts of rows r0, r0 + 1, ...
+    const int a = static_cast<int>(reinterpret_cast<uintptr_t>(out) & 15u);  // out - a is 16-byte aligned
+    const int64_t nvec = total > 0 ? (total - 1 + a) / 16 + 1 : 0;         // vector v holds bytes [16v - a, 16v - a + 16)
+    const int64_t ntiles = (nvec + kFlatTile - 1) / kFlatTile;
+    auto start_g = [&](int64_t r) { return m.start(r); };
+    auto row_g = [&](int64_t r) { return m.row_g(r); };
+    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        const int64_t v0 = tile * kFlatTile;
+        const int64_t p0 = max(16 * v0 - a, int64_t(0)), p1 = min(16 * (v0 + kFlatTile) - a, total);
+        const int64_t r0 = block_search_le<kFlatThreads>(0, n, p0, start_g);
+        const int nrows = block_row_table<kFlatThreads, kFlatRowCap>(r0, n, p1, [&](int j, int64_t r) {
+            const int64_t s = m.start(r);
+            tab[j] = s;
+            m.stage(j, r);
+            return s;
+        });
+        if (nrows > 0) {
+            for (int k = 0; k < kFlatVecs; ++k) {
+                const int64_t v = v0 + k * kFlatThreads + threadIdx.x;
+                if (v >= nvec) break;
+                const int64_t q = 16 * v - a, x = max(q, int64_t(0));
+                int l = 0, h = nrows;  // the largest j < nrows with tab[j] <= x
+                while (h - l > 1) {
+                    const int mid = (l + h) >> 1;
+                    if (tab[mid] <= x) l = mid;
+                    else h = mid;
+                }
+                flat_vector(q, r0 + l, total, m, [&](int64_t r) { return tab[r - r0]; }, [&](int64_t r) { return m.row_t(r - r0); },
+                            out + q);
+            }
+        } else {
+            for (int k = 0; k < kFlatVecs; ++k) {
+                const int64_t v = v0 + k * kFlatThreads + threadIdx.x;
+                if (v >= nvec) break;
+                const int64_t q = 16 * v - a, x = max(q, int64_t(0));
+                int64_t l = r0, h = n;
+                while (h - l > 1) {
+                    const int64_t mid = (l + h) >> 1;
+                    if (m.start(mid) <= x) l = mid;
+                    else h = mid;
+                }
+                flat_vector(q, l, total, m, start_g, row_g, out + q);
+            }
+        }
+        __syncthreads();  // the table is refilled by the next tile
+    }
 }
 
 // K0: the device offsets reduction.  out = {sum0, sum1, max, what is wrong}: 1 a negative length, 2 offsets[0] < 0,

@@ -163,13 +163,11 @@ kmer_varlen_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict_
     if (i >= n) return;
     const int64_t s0 = __ldg(offs + i), len = __ldg(offs + i + 1) - s0;
     const int64_t ntok = kmer_tokens(len, p.ks);
-    // the row's end entry: its CTA-local inclusive prefix plus the carry, unless it closes a scan CTA (already final)
-    const int64_t e_idx = i + 1, blk = i / kRowScan;
-    const bool final_entry = (e_idx % kRowScan) == 0 || e_idx == n;
-    int64_t e = cu[e_idx];
-    if (!final_entry && blk > 0) e += cu[blk * kRowScan];
+    // the row's end entry: its CTA-local inclusive prefix plus the carry it still lacks
+    const int64_t carry = row_scan_carry(cu, i + 1, n);
+    const int64_t e = cu[i + 1] + carry;
     __syncwarp();
-    if (lane == 0 && !final_entry) cu[e_idx] = static_cast<int32_t>(e);
+    if (lane == 0 && carry != 0) cu[i + 1] = static_cast<int32_t>(e);
     const int64_t f0 = e - ntok;
     if (ntok <= 0) return;
     const int64_t q0 = f0 >> 4, q1 = (e - 1) >> 4;

@@ -10,16 +10,13 @@
 //                       window counts into seq_ptr, then the per-sequence output byte totals (closed form: (m - 1) W +
 //                       len_last for SHORT, m W otherwise) into byte_ptr.  byte_ptr, and seq_ptr when the caller passes
 //                       none, live in stream-ordered scratch (cudaMallocAsync / cudaFreeAsync on the call's stream).
-//   tile_fix_kernel     one thread per sequence adds the carry of its scan CTA to both entries (as K9's gather does).
+//   tile_fix_kernel     one thread per sequence adds the carry of its scan CTA (row_scan_carry) to both entries.
 //   tile_gather_kernel  a grid-stride pass over the windows writes out_offsets, seq_index and starts (a binary search of
-//                       seq_ptr per window), then the bytes: a flat map over the 16-byte aligned output vectors in tiles
-//                       of 64 KiB on a persistent grid.  Per tile the CTA finds the tile's first sequence with K12's
-//                       256-ary search over byte_ptr and stages the tile's byte_ptr entries in shared memory (over-full
-//                       tiles search global memory).  Per vector a binary search of that table gives the sequence, and a
-//                       FastDiv by W the window (every window but a sequence's last is exactly W bytes of output).  Each
-//                       window piece the vector touches is two aligned ld.global.nc loads of its source, realigned with
-//                       funnel shifts and merged in with a byte mask; a vector inside the output leaves as one 16-byte
-//                       store, the at most two partial vectors at the ends of the output (any alignment) as byte stores.
+//                       seq_ptr per window), then the bytes: bsq_kernels.cuh's flat map with the sequences as rows and
+//                       byte_ptr as their starts (no row data of its own).  Its piece of a sequence: a FastDiv by W gives
+//                       the first window the vector touches (every window but a sequence's last is exactly W bytes of
+//                       output), and each window piece is two aligned ld.global.nc loads of its source, realigned with
+//                       funnel shifts and merged in with a byte mask.
 //   With S < W, overlapping windows re-read their shared source bytes; those re-reads hit L2 (a tile's source span is
 //   about 64 KiB * S / W + W bytes).
 //
@@ -87,22 +84,15 @@ struct TileMeasure {
     }
 };
 
-// the scan entries that are not the last of their scan CTA get that CTA's carry (the last ones are final already and are
-// only read here, so no thread reads an entry another thread writes)
+// the scan entries that lack their scan CTA's carry get it (the others are final and only read here, so no thread reads
+// an entry another thread writes)
 __global__ void tile_fix_kernel(int64_t n, int64_t *__restrict__ seq_ptr, int64_t *__restrict__ byte_ptr) {
-    const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const int64_t e = i + 1, blk = i / kRowScan;
-    if ((e % kRowScan) == 0 || e == n || blk == 0) return;
-    seq_ptr[e] += seq_ptr[blk * kRowScan];
-    byte_ptr[e] += byte_ptr[blk * kRowScan];
+    const int64_t e = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x + 1;
+    if (e > n) return;
+    const int64_t cs = row_scan_carry(seq_ptr, e, n), cb = row_scan_carry(byte_ptr, e, n);
+    if (cs != 0) seq_ptr[e] += cs;
+    if (cb != 0) byte_ptr[e] += cb;
 }
-
-constexpr int kTThreads = 256;
-constexpr int kTVecs = 16;                  // output vectors per thread and tile
-constexpr int kTTile = kTThreads * kTVecs;  // 4096 vectors: 64 KiB of output per tile
-constexpr int kTRowCap = 2048;              // sequences a tile's table holds
-constexpr int kTMinBlocks = 4;
 
 struct TileArgs {
     const uint8_t *bytes;
@@ -119,60 +109,41 @@ __device__ __forceinline__ int64_t div_w(int64_t x, const TileArgs &a) {
                                                                    : x / a.t.W;
 }
 
-// Output bytes [q, q + 16) (out + q is 16-byte aligned), whose first byte in [0, total) lies in sequence i.
-// base_of(i) is byte_ptr[i] (from the tile's table or global memory).
-template <typename BASE>
-__device__ __forceinline__ void tile_vector(int64_t q, int64_t i, const TileArgs &a, const BASE &base_of, uint8_t *dst) {
-    uint32_t res[4] = {0u, 0u, 0u, 0u};
-    const uintptr_t src0 = reinterpret_cast<uintptr_t>(a.bytes);
-    int64_t b = base_of(i);
-    const int64_t x = max(q, int64_t(0));
-    for (;;) {
-        const int64_t be = base_of(i + 1);
-        if (be > b) {  // (an empty sequence has no bytes)
-            const int64_t s = __ldg(a.offs + i), len = __ldg(a.offs + i + 1) - s;
-            const int64_t m = tile_count(len, a.t);
-            int64_t j = div_w(max(x, b) - b, a);
-            for (; j < m; ++j) {
-                const int64_t ws = b + j * a.t.W;  // the window's first output byte
-                if (ws >= q + 16) break;
-                const int64_t wl = tile_len(j, len, a.t);
-                const int64_t src = s + tile_start(j, m, len, a.t);  // its first source byte
-                const uintptr_t lo = (src0 + static_cast<uintptr_t>(src)) & ~uintptr_t(15);
-                const uintptr_t hi = (src0 + static_cast<uintptr_t>(src + wl - 1)) & ~uintptr_t(15);
-                uint32_t t[4];
-                fetch16_clamped(src0 + static_cast<uintptr_t>(src + (q - ws)), lo, hi, t);
-                const int k0 = static_cast<int>(min(max(ws - q, int64_t(0)), int64_t(16)));
-                const int k1 = static_cast<int>(min(max(ws + wl - q, int64_t(0)), int64_t(16)));
-#pragma unroll
-                for (int w = 0; w < 4; ++w) {
-                    const uint32_t mk = lt_mask(k1, w) & ~lt_mask(k0, w);
-                    res[w] = (res[w] & ~mk) | (t[w] & mk);
-                }
-            }
-        }
-        if (be >= q + 16 || i + 1 >= a.n) break;
-        ++i;
-        b = be;
-    }
-    if (q >= 0 && q + 16 <= a.total) {
-        __stcs(reinterpret_cast<uint4 *>(dst), make_uint4(res[0], res[1], res[2], res[3]));
-    } else {
-#pragma unroll
-        for (int k = 0; k < 16; ++k)
-            if (q + k >= 0 && q + k < a.total) dst[k] = static_cast<uint8_t>(res[k >> 2] >> (8 * (k & 3)));
-    }
-}
+// K13a's rows for flat_map: the sequences, starting at byte_ptr
+struct TileMap {
+    TileArgs a;
+    struct None {};
 
-__global__ void __launch_bounds__(kTThreads, kTMinBlocks)
+    __device__ __forceinline__ int64_t start(int64_t i) const { return __ldg(a.byte_ptr + i); }
+    __device__ __forceinline__ void stage(int, int64_t) const {}
+    __device__ __forceinline__ None row_t(int) const { return {}; }
+    __device__ __forceinline__ None row_g(int64_t) const { return {}; }
+    // the windows of sequence i (output bytes from b) that output bytes [q, q + 16) touch
+    __device__ __forceinline__ void piece(int64_t q, int64_t i, int64_t b, int64_t, None, uint32_t res[4]) const {
+        const uintptr_t src0 = reinterpret_cast<uintptr_t>(a.bytes);
+        const int64_t s = __ldg(a.offs + i), len = __ldg(a.offs + i + 1) - s;
+        const int64_t m = tile_count(len, a.t);
+        for (int64_t j = div_w(max(q, b) - b, a); j < m; ++j) {
+            const int64_t ws = b + j * a.t.W;  // the window's first output byte
+            if (ws >= q + 16) break;
+            const int64_t wl = tile_len(j, len, a.t);
+            const int64_t src = s + tile_start(j, m, len, a.t);  // its first source byte
+            const uintptr_t lo = (src0 + static_cast<uintptr_t>(src)) & ~uintptr_t(15);
+            const uintptr_t hi = (src0 + static_cast<uintptr_t>(src + wl - 1)) & ~uintptr_t(15);
+            uint32_t t[4];
+            fetch_clamped<4>(src0 + static_cast<uintptr_t>(src + (q - ws)), lo, hi, t);
+            merge16(res, t, ws - q, ws + wl - q);
+        }
+    }
+};
+
+__global__ void __launch_bounds__(kFlatThreads, kFlatMinBlocks)
 tile_gather_kernel(TileArgs a, uint8_t *__restrict__ out, int64_t *__restrict__ out_offs, int64_t *__restrict__ seq_index,
                    int64_t *__restrict__ starts) {
-    __shared__ int64_t tab[kTRowCap];  // byte_ptr of sequences i0, i0 + 1, ...
-    const int tid = threadIdx.x;
     a.total = __ldg(a.byte_ptr + a.n);
     // window table: out_offsets, seq_index, starts
     const int64_t M = __ldg(a.seq_ptr + a.n);
-    for (int64_t w = blockIdx.x * static_cast<int64_t>(kTThreads) + tid; w <= M; w += static_cast<int64_t>(gridDim.x) * kTThreads) {
+    for (int64_t w = blockIdx.x * static_cast<int64_t>(kFlatThreads) + threadIdx.x; w <= M; w += static_cast<int64_t>(gridDim.x) * kFlatThreads) {
         if (w == M) {
             out_offs[M] = a.total;
             break;
@@ -191,67 +162,7 @@ tile_gather_kernel(TileArgs a, uint8_t *__restrict__ out, int64_t *__restrict__ 
             starts[w] = tile_start(j, tile_count(len, a.t), len, a.t);
         }
     }
-    const int al = static_cast<int>(reinterpret_cast<uintptr_t>(out) & 15u);  // out - al is 16-byte aligned
-    const int64_t nvec = a.total > 0 ? (a.total - 1 + al) / 16 + 1 : 0;      // vector v holds bytes [16v - al, 16v - al + 16)
-    const int64_t ntiles = (nvec + kTTile - 1) / kTTile;
-    auto base_g = [&](int64_t i) { return __ldg(a.byte_ptr + i); };
-    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int64_t v0 = tile * kTTile;
-        const int64_t p0 = max(16 * v0 - al, int64_t(0)), p1 = min(16 * (v0 + kTTile) - al, a.total);
-        // 1. first sequence: the largest i in [0, n) with byte_ptr[i] <= p0
-        int64_t lo = 0, hi = a.n;
-        while (hi - lo > 1) {
-            const int64_t w = hi - lo;
-            const int64_t pr = lo + (static_cast<int64_t>(tid) + 1) * w / (kTThreads + 1);
-            const int cnt = __syncthreads_count(base_g(pr) <= p0);
-            const int64_t nlo = cnt > 0 ? lo + static_cast<int64_t>(cnt) * w / (kTThreads + 1) : lo;
-            const int64_t nhi = cnt < kTThreads ? lo + (static_cast<int64_t>(cnt) + 1) * w / (kTThreads + 1) : hi;
-            lo = nlo;
-            hi = nhi;
-        }
-        const int64_t i0 = lo;
-        // 2. table up to the first sequence that starts at or after the tile's end (byte_ptr[n] = total >= p1 closes it)
-        int nrows = -1;
-        for (int base = 0; base < kTRowCap; base += kTThreads) {
-            const int j = base + tid;
-            const int64_t i = i0 + j;
-            bool past = true;
-            if (i <= a.n) {
-                const int64_t s = base_g(i);
-                tab[j] = s;
-                past = s >= p1;
-            }
-            const int cnt = __syncthreads_count(past);
-            if (cnt > 0) {
-                nrows = base + kTThreads - cnt;
-                break;
-            }
-        }
-        for (int k = 0; k < kTVecs; ++k) {
-            const int64_t v = v0 + k * kTThreads + tid;
-            if (v >= nvec) break;
-            const int64_t q = 16 * v - al, x = max(q, int64_t(0));
-            if (nrows > 0) {
-                int l = 0, h = nrows;  // the largest j < nrows with tab[j] <= x
-                while (h - l > 1) {
-                    const int mid = (l + h) >> 1;
-                    if (tab[mid] <= x) l = mid;
-                    else h = mid;
-                }
-                const int64_t r0 = i0;
-                tile_vector(q, i0 + l, a, [&](int64_t i) { return i - r0 <= nrows ? tab[i - r0] : base_g(i); }, out + q);
-            } else {
-                int64_t l = i0, h = a.n;
-                while (h - l > 1) {
-                    const int64_t mid = (l + h) >> 1;
-                    if (base_g(mid) <= x) l = mid;
-                    else h = mid;
-                }
-                tile_vector(q, l, a, base_g, out + q);
-            }
-        }
-        __syncthreads();  // the table is refilled by the next tile
-    }
+    flat_map(out, a.n, a.total, TileMap{a});
 }
 
 // ---- K13b -------------------------------------------------------------------------------------------------------------
@@ -439,7 +350,7 @@ extern "C" int bsq_tile(int device, void *stream, const uint8_t *d_bytes, const 
     a.total = 0;  // (byte_ptr[n]: read by the kernel)
     a.t = t;
     a.wdiv = make_fastdiv(static_cast<uint32_t>(std::min<int64_t>(window, (int64_t(1) << 31) - 1)));
-    tile_gather_kernel<<<cur_sms() * kTMinBlocks, kTThreads, 0, st>>>(a, d_out_bytes, d_out_offsets, d_seq_index, d_starts);
+    tile_gather_kernel<<<cur_sms() * kFlatMinBlocks, kFlatThreads, 0, st>>>(a, d_out_bytes, d_out_offsets, d_seq_index, d_starts);
     count_launch();
     BSQ_CUDA_TRY(cudaGetLastError());
     BSQ_CUDA_TRY(cudaFreeAsync(scratch, st));

@@ -9,20 +9,15 @@
 // tr_len below is the only statement of that length (host extent, device extent and both kernels use it).
 //
 // K14a: row_scan_kernel (+ row_carry_kernel past 1024 sequences, bsq_kernels.cuh) scans the per-sequence output bytes
-//       (the sum of its F frame lengths, TranslateCount) into stream-ordered scratch S[n + 1].  Entries that do not close a
-//       scan CTA lack their CTA's carry; seq_base adds it where it is read, so no fix-up pass runs.
+//       (the sum of its F frame lengths, TranslateCount) into stream-ordered scratch S[n + 1].  seq_base adds the carry
+//       an entry still lacks (row_scan_carry) where it is read, so no fix-up pass runs.
 // K14b: translate_kernel -- a grid-stride pass over the n * F + 1 output offsets (each sequence's base plus the lengths of
-//       its earlier frames), then the bytes: a flat map over the 16-byte aligned output vectors in tiles of 64 KiB on a
-//       persistent grid in static order, the structure K12 and K13a share.  Per tile the CTA finds the tile's first
-//       sequence with a 256-ary search over S and stages the tile's sequence bases and source starts in shared memory
-//       (over-full tiles read global memory).  Per vector a binary search of that table gives the sequence of its first
-//       byte; every (sequence, frame) piece the vector touches then costs
+//       its earlier frames), then the bytes: bsq_kernels.cuh's flat map with the sequences as rows, seq_base as their
+//       starts and their source offsets as row data.  Its piece of a sequence: every frame the vector touches costs
 //         - one 48-byte source span (16 codons) as four clamped aligned 16-byte loads realigned with selects and funnel
 //           shifts; a reverse frame reads the mirrored span and reverses its bytes with PRMT, as K12 does;
 //         - 48 mask look-ups (the complemented mask table for a reverse frame) and 16 codon look-ups in shared memory;
 //         - a merge into the output vector by byte mask.
-//       A vector inside the output leaves as one st.global.cs.v4, the at most two partial vectors at its ends (any
-//       alignment) as byte stores.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -147,12 +142,6 @@ __host__ __device__ __forceinline__ uint8_t bitrev4(uint8_t m) {
     return static_cast<uint8_t>(((m & 1) << 3) | ((m & 2) << 1) | ((m & 4) >> 1) | ((m & 8) >> 3));
 }
 
-constexpr int kTrThreads = 256;
-constexpr int kTrVecs = 16;                     // output vectors per thread and tile
-constexpr int kTrTile = kTrThreads * kTrVecs;   // 4096 vectors: 64 KiB of output per tile
-constexpr int kTrRowCap = 2048;                 // sequences a tile's table holds
-constexpr int kTrMinBlocks = 4;
-
 struct TrTables {
     uint32_t mask[64], cmask[64];  // 256 masks and their complements, 4 per word
     uint32_t codon[1024];          // 4096 letters, 4 per word
@@ -167,41 +156,7 @@ struct TrArgs {
 };
 
 // S[e] with its scan CTA's carry: the global exclusive prefix of the per-sequence output bytes (seq_base(n) = total)
-__device__ __forceinline__ int64_t seq_base(const TrArgs &a, int64_t e) {
-    int64_t v = __ldg(a.S + e);
-    if (e > kRowScan && (e % kRowScan) != 0 && e != a.n) v += __ldg(a.S + ((e - 1) / kRowScan) * kRowScan);
-    return v;
-}
-
-// The 48 bytes at address X (any alignment) as 12 little-endian words, from the aligned words at X & ~15 and the three
-// after it, each clamped to [lo, hi] (16-byte aligned); the shift is picked with selects, as in fetch16_clamped.
-__device__ __forceinline__ void fetch48_clamped(uintptr_t X, uintptr_t lo, uintptr_t hi, uint32_t t[12]) {
-    const uintptr_t a0 = X & ~uintptr_t(15);
-    const uint32_t s = static_cast<uint32_t>(X) & 15u;
-    uint32_t w[16];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-        const uint4 v = ldg16(clamp_word(a0 + 16 * k, lo, hi));
-        w[4 * k] = v.x;
-        w[4 * k + 1] = v.y;
-        w[4 * k + 2] = v.z;
-        w[4 * k + 3] = v.w;
-    }
-    const uint4 v3 = s != 0 ? ldg16(clamp_word(a0 + 48, lo, hi)) : make_uint4(0u, 0u, 0u, 0u);
-    w[12] = v3.x;
-    w[13] = v3.y;
-    w[14] = v3.z;
-    w[15] = v3.w;
-    const bool q2 = (s & 8u) != 0, q1 = (s & 4u) != 0;
-    uint32_t a[14], b[13];
-#pragma unroll
-    for (int k = 0; k < 14; ++k) a[k] = q2 ? w[k + 2] : w[k];
-#pragma unroll
-    for (int k = 0; k < 13; ++k) b[k] = q1 ? a[k + 1] : a[k];
-    const uint32_t sh = (s & 3u) * 8u;
-#pragma unroll
-    for (int k = 0; k < 12; ++k) t[k] = __funnelshift_r(b[k], b[k + 1], sh);
-}
+__device__ __forceinline__ int64_t seq_base(const TrArgs &a, int64_t e) { return __ldg(a.S + e) + row_scan_carry(a.S, e, a.n); }
 
 // The 16 letters of one (sequence, frame) piece for output bytes [q, q + 16): amino acid t0 + j of the frame lands in
 // byte j.  s / len: the sequence's source start and length; fr: the frame's code.
@@ -216,7 +171,7 @@ __device__ __forceinline__ void tr_piece(int64_t q, int64_t ws, int64_t s, int64
     const uintptr_t lo = (src0 + static_cast<uintptr_t>(s)) & ~uintptr_t(15);
     const uintptr_t hi = (src0 + static_cast<uintptr_t>(s + len - 1)) & ~uintptr_t(15);
     uint32_t w[12];
-    fetch48_clamped(src0 + static_cast<uintptr_t>(X), lo, hi, w);
+    fetch_clamped<12>(src0 + static_cast<uintptr_t>(X), lo, hi, w);
     if (rev) {
 #pragma unroll
         for (int k = 0; k < 6; ++k) {
@@ -241,68 +196,53 @@ __device__ __forceinline__ void tr_piece(int64_t q, int64_t ws, int64_t s, int64
     }
 }
 
-struct SeqRow {
-    int64_t base, next, start, end;  // output bases of this sequence and the next; its source offsets
+struct SrcRow {
+    int64_t start, end;  // a sequence's source offsets
 };
 
-// Output bytes [q, q + 16) (out + q is 16-byte aligned), whose first byte in [0, total) lies in sequence i; row_of(i) is
-// its SeqRow (from the tile's table or global memory).
-template <typename ROW>
-__device__ __forceinline__ void tr_vector(int64_t q, int64_t i, const TrArgs &a, const ROW &row_of, const uint8_t *mask,
-                                          const uint8_t *cmask, const uint8_t *codon, uint8_t *dst) {
-    uint32_t res[4] = {0u, 0u, 0u, 0u};
-    const int64_t x = max(q, int64_t(0));
-    for (;;) {
-        const SeqRow r = row_of(i);
-        if (r.next > r.base) {
-            const int64_t len = r.end - r.start;
-            int64_t ws = r.base;
-            for (int f = 0; f < a.fs.F && ws < q + 16; ++f) {
-                const uint32_t fr = frame_code(a.fs.fcode, f);
-                const int64_t L = tr_len(len, fr);
-                if (L > 0 && ws + L > x) {
-                    uint32_t t[4];
-                    tr_piece(q, ws, r.start, len, fr, a, mask, cmask, codon, t);
-                    const int k0 = static_cast<int>(min(max(ws - q, int64_t(0)), int64_t(16)));
-                    const int k1 = static_cast<int>(min(max(ws + L - q, int64_t(0)), int64_t(16)));
-#pragma unroll
-                    for (int w = 0; w < 4; ++w) {
-                        const uint32_t mk = lt_mask(k1, w) & ~lt_mask(k0, w);
-                        res[w] = (res[w] & ~mk) | (t[w] & mk);
-                    }
-                }
-                ws += L;
-            }
-        }
-        if (r.next >= q + 16 || i + 1 >= a.n) break;
-        ++i;
-    }
-    if (q >= 0 && q + 16 <= a.total) {
-        __stcs(reinterpret_cast<uint4 *>(dst), make_uint4(res[0], res[1], res[2], res[3]));
-    } else {
-#pragma unroll
-        for (int k = 0; k < 16; ++k)
-            if (q + k >= 0 && q + k < a.total) dst[k] = static_cast<uint8_t>(res[k >> 2] >> (8 * (k & 3)));
-    }
-}
+// K14b's rows for flat_map: the sequences, starting at seq_base, with their source offsets as row data
+struct TrMap {
+    TrArgs a;
+    const uint8_t *mask, *cmask, *codon;  // tables in shared memory
+    int64_t *src;                         // source starts of the tile's rows, in shared memory
 
-__global__ void __launch_bounds__(kTrThreads, kTrMinBlocks)
+    __device__ __forceinline__ int64_t start(int64_t i) const { return seq_base(a, i); }
+    __device__ __forceinline__ void stage(int j, int64_t i) const { src[j] = __ldg(a.offs + i); }
+    __device__ __forceinline__ SrcRow row_t(int j) const { return {src[j], src[j + 1]}; }
+    __device__ __forceinline__ SrcRow row_g(int64_t i) const { return {__ldg(a.offs + i), __ldg(a.offs + i + 1)}; }
+    // the frames of a sequence (output bytes from b) that output bytes [q, q + 16) touch
+    __device__ __forceinline__ void piece(int64_t q, int64_t, int64_t b, int64_t, SrcRow r, uint32_t res[4]) const {
+        const int64_t len = r.end - r.start;
+        int64_t ws = b;
+        for (int f = 0; f < a.fs.F && ws < q + 16; ++f) {
+            const uint32_t fr = frame_code(a.fs.fcode, f);
+            const int64_t L = tr_len(len, fr);
+            if (L > 0 && ws + L > q) {
+                uint32_t t[4];
+                tr_piece(q, ws, r.start, len, fr, a, mask, cmask, codon, t);
+                merge16(res, t, ws - q, ws + L - q);
+            }
+            ws += L;
+        }
+    }
+};
+
+__global__ void __launch_bounds__(kFlatThreads, kFlatMinBlocks)
 translate_kernel(TrArgs a, const __grid_constant__ TrTables tbl, uint8_t *__restrict__ out, int64_t *__restrict__ out_offs) {
     __shared__ __align__(16) uint8_t s_mask[256];
     __shared__ __align__(16) uint8_t s_cmask[256];
     __shared__ __align__(16) uint8_t s_codon[4096];
-    __shared__ int64_t s_base[kTrRowCap];  // output bases of sequences i0, i0 + 1, ...
-    __shared__ int64_t s_src[kTrRowCap];   // ... and their source starts
+    __shared__ int64_t s_src[kFlatRowCap];
     const int tid = threadIdx.x;
     if (tid < 64) {
         reinterpret_cast<uint32_t *>(s_mask)[tid] = tbl.mask[tid];
         reinterpret_cast<uint32_t *>(s_cmask)[tid] = tbl.cmask[tid];
     }
-    for (int k = tid; k < 1024; k += kTrThreads) reinterpret_cast<uint32_t *>(s_codon)[k] = tbl.codon[k];
+    for (int k = tid; k < 1024; k += kFlatThreads) reinterpret_cast<uint32_t *>(s_codon)[k] = tbl.codon[k];
     a.total = seq_base(a, a.n);
     // output offsets: sequence i's base, then each frame's length
     const int64_t nw = a.n * a.fs.F;
-    for (int64_t w = blockIdx.x * static_cast<int64_t>(kTrThreads) + tid; w <= nw; w += static_cast<int64_t>(gridDim.x) * kTrThreads) {
+    for (int64_t w = blockIdx.x * static_cast<int64_t>(kFlatThreads) + tid; w <= nw; w += static_cast<int64_t>(gridDim.x) * kFlatThreads) {
         if (w == nw) {
             out_offs[nw] = a.total;
             break;
@@ -315,71 +255,7 @@ translate_kernel(TrArgs a, const __grid_constant__ TrTables tbl, uint8_t *__rest
         out_offs[w] = o;
     }
     __syncthreads();  // the tables are in shared memory
-    const int al = static_cast<int>(reinterpret_cast<uintptr_t>(out) & 15u);  // out - al is 16-byte aligned
-    const int64_t nvec = a.total > 0 ? (a.total - 1 + al) / 16 + 1 : 0;      // vector v holds bytes [16v - al, 16v - al + 16)
-    const int64_t ntiles = (nvec + kTrTile - 1) / kTrTile;
-    auto row_g = [&](int64_t i) { return SeqRow{seq_base(a, i), seq_base(a, i + 1), __ldg(a.offs + i), __ldg(a.offs + i + 1)}; };
-    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int64_t v0 = tile * kTrTile;
-        const int64_t p0 = max(16 * v0 - al, int64_t(0)), p1 = min(16 * (v0 + kTrTile) - al, a.total);
-        // 1. first sequence: the largest i in [0, n) with base(i) <= p0
-        int64_t lo = 0, hi = a.n;
-        while (hi - lo > 1) {
-            const int64_t w = hi - lo;
-            const int64_t pr = lo + (static_cast<int64_t>(tid) + 1) * w / (kTrThreads + 1);
-            const int cnt = __syncthreads_count(seq_base(a, pr) <= p0);
-            const int64_t nlo = cnt > 0 ? lo + static_cast<int64_t>(cnt) * w / (kTrThreads + 1) : lo;
-            const int64_t nhi = cnt < kTrThreads ? lo + (static_cast<int64_t>(cnt) + 1) * w / (kTrThreads + 1) : hi;
-            lo = nlo;
-            hi = nhi;
-        }
-        const int64_t i0 = lo;
-        // 2. table up to the first sequence that starts at or after the tile's end (base(n) = total >= p1 closes it)
-        int nrows = -1;
-        for (int b = 0; b < kTrRowCap; b += kTrThreads) {
-            const int j = b + tid;
-            const int64_t i = i0 + j;
-            bool past = true;
-            if (i <= a.n) {
-                const int64_t sb = seq_base(a, i);
-                s_base[j] = sb;
-                s_src[j] = __ldg(a.offs + i);
-                past = sb >= p1;
-            }
-            const int cnt = __syncthreads_count(past);
-            if (cnt > 0) {
-                nrows = b + kTrThreads - cnt;
-                break;
-            }
-        }
-        for (int k = 0; k < kTrVecs; ++k) {
-            const int64_t v = v0 + k * kTrThreads + tid;
-            if (v >= nvec) break;
-            const int64_t q = 16 * v - al, x = max(q, int64_t(0));
-            if (nrows > 0) {
-                int l = 0, h = nrows;  // the largest j < nrows with s_base[j] <= x
-                while (h - l > 1) {
-                    const int mid = (l + h) >> 1;
-                    if (s_base[mid] <= x) l = mid;
-                    else h = mid;
-                }
-                auto row_t = [&](int64_t i) {
-                    const int64_t j = i - i0;
-                    return j < nrows ? SeqRow{s_base[j], s_base[j + 1], s_src[j], s_src[j + 1]} : row_g(i);
-                };
-                tr_vector(q, i0 + l, a, row_t, s_mask, s_cmask, s_codon, out + q);
-            } else {
-                int64_t l = i0, h = a.n;
-                while (h - l > 1) {
-                    const int64_t mid = (l + h) >> 1;
-                    if (seq_base(a, mid) <= x) l = mid;
-                    else h = mid;
-                }
-                tr_vector(q, l, a, row_g, s_mask, s_cmask, s_codon, out + q);
-            }
-        }
-        __syncthreads();  // the table is refilled by the next tile
-    }
+    flat_map(out, a.n, a.total, TrMap{a, s_mask, s_cmask, s_codon, s_src});
 }
 
 }  // namespace
@@ -488,7 +364,7 @@ extern "C" int bsq_translate(int device, void *stream, const uint8_t *d_bytes, c
     a.n = nseq;
     a.total = 0;  // (S's last entry: read by the kernel)
     a.fs = fs;
-    translate_kernel<<<cur_sms() * kTrMinBlocks, kTrThreads, 0, st>>>(a, tt, d_out_bytes, d_out_offsets);
+    translate_kernel<<<cur_sms() * kFlatMinBlocks, kFlatThreads, 0, st>>>(a, tt, d_out_bytes, d_out_offsets);
     count_launch();
     BSQ_CUDA_TRY(cudaGetLastError());
     BSQ_CUDA_TRY(cudaFreeAsync(S, st));

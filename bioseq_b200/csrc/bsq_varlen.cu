@@ -234,35 +234,14 @@ varlen_tile_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict_
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const int64_t f0 = tile * kVTile;
         const int tl = static_cast<int>(min(static_cast<int64_t>(kVTile), total - f0));  // elements of this tile
-        // 1. first row: the largest r with cu[r] <= f0, in [lo, hi)
-        int64_t lo = 0, hi = n;
-        while (hi - lo > 1) {
-            const int64_t w = hi - lo;
-            const int64_t p = lo + (static_cast<int64_t>(tid) + 1) * w / (kVThreads + 1);
-            const int cnt = __syncthreads_count(cu_g(p) <= f0);  // a prefix of the probes (cu is increasing)
-            const int64_t nlo = cnt > 0 ? lo + static_cast<int64_t>(cnt) * w / (kVThreads + 1) : lo;
-            const int64_t nhi = cnt < kVThreads ? lo + (static_cast<int64_t>(cnt) + 1) * w / (kVThreads + 1) : hi;
-            lo = nlo;
-            hi = nhi;
-        }
-        const int64_t r0 = lo;
+        // 1. first row: the largest r with cu[r] <= f0
+        const int64_t r0 = block_search_le<kVThreads>(0, n, f0, cu_g);
         // 2. row table: cu[r0 + j] - f0 up to the first row that starts at or after the tile's end
-        int nrows = -1;
-        for (int base = 0; base < kVRowCap; base += kVThreads) {
-            const int j = base + tid;
-            const int64_t i = r0 + j;
-            bool past = true;
-            if (i <= n) {
-                const int64_t c = cu_g(i) - f0;
-                rowtab[j] = static_cast<int32_t>(c);
-                past = c >= tl;
-            }
-            const int cnt = __syncthreads_count(past);  // a suffix of the chunk
-            if (cnt > 0) {
-                nrows = base + kVThreads - cnt;
-                break;
-            }
-        }
+        int nrows = block_row_table<kVThreads, kVRowCap>(r0, n, tl, [&](int j, int64_t r) {
+            const int64_t c = cu_g(r) - f0;
+            rowtab[j] = static_cast<int32_t>(c);
+            return c;
+        });
         // 3. the residue span, rounded out to 16 bytes, into shared memory
         if (tid == 0) {
             uint32_t copied = 0;

@@ -105,3 +105,14 @@ class Reference:
                 json.dump(rec, f, indent=0, sort_keys=True)
         else:
             assert len(self.got) == len(self.want), f"{self.test}: {len(self.got)} comparisons, {len(self.want)} recorded"
+
+
+def table_cap_lens():
+    """Output bytes per row for the flat map's row-table cap (K12, K13a, K14b): tiles of 2046, 2047 and 2048 rows, 16
+    bytes each but the tile's last.  With the output aligned a 64 KiB tile's row table needs as many rows, misaligned one
+    more (the previous tile's last row), so 2047 rows (the table's cap) and 2048 (the first over-full count) occur at every
+    output alignment."""
+    lens = []
+    for k in (2046, 2047, 2048, 2047, 2046):
+        lens += [16] * (k - 1) + [65536 - 16 * (k - 1)]
+    return lens

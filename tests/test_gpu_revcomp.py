@@ -19,7 +19,7 @@ from bioseq_b200 import batch_tokenize_cropped, batch_tokenize_varlen, batch_tok
 from bioseq_b200 import batch_tokenize_kmer, batch_onehot_encode_bcl, batch_embed  # noqa: E402
 from bioseq_b200.loaders import FlatFileDataset  # noqa: E402
 from oracle.oracle import OracleTokenizer, flatfile_image  # noqa: E402
-from helpers import assert_same_bits, gen  # noqa: E402
+from helpers import assert_same_bits, gen, table_cap_lens  # noqa: E402
 from revcomp_reference import revcomp as reference_revcomp  # noqa: E402
 from crop_reference import crop as reference_crop  # noqa: E402
 
@@ -72,25 +72,31 @@ def test_edge_lengths_every_source_alignment(mode, rc_prob):
         assert torch.equal(b, b0) and torch.equal(o, o0)  # the caller's tensors are unchanged
 
 
+# random rows; the same ending in a run of empty rows (every alignment but one leaves the last vector partial); rows that
+# fill tiles to the row table's cap and one past it
+DEST_LENS = [np.random.default_rng(2).integers(0, 300, size=2000),
+             np.concatenate([np.random.default_rng(2).integers(0, 300, size=500), np.zeros(40, np.int64)]), table_cap_lens()]
+
+
 @pytest.mark.parametrize("mode,rc_prob", MODES)
 def test_every_destination_alignment(mode, rc_prob):
-    lens = np.random.default_rng(2).integers(0, 300, size=2000)
-    buf, offs = batch_of(lens, 3, lead=5)
-    b, o = cuda(buf, offs)
-    wb, wo, wf = reference_revcomp(buf, offs, mode, 0.5 if rc_prob is None else rc_prob, 4, 9)
-    st = torch.cuda.current_stream().cuda_stream
-    for shift in range(16):
-        ob = torch.full((wb.size + 64,), 0xA5, dtype=torch.uint8, device="cuda")
-        oo = torch.empty(wo.size, dtype=torch.int64, device="cuda")
-        of = torch.empty(wf.size, dtype=torch.uint8, device="cuda")
-        mode_i = consumers._RC_MODES[mode]
-        capi.revcomp(0, st, b, o, offs.size - 1, mode_i, rc_prob or 0.0, 4, 9, ob.data_ptr() + shift, oo, of)
-        torch.cuda.synchronize()
-        got = ob.cpu().numpy()
-        assert_same_bits(wb, got[shift:shift + wb.size])
-        assert (got[:shift] == 0xA5).all() and (got[shift + wb.size:] == 0xA5).all()  # nothing written outside
-        assert_same_bits(wo, oo.cpu().numpy())
-        assert_same_bits(wf.astype(np.uint8), of.cpu().numpy())
+    for lens in DEST_LENS:
+        buf, offs = batch_of(lens, 3, lead=5)
+        b, o = cuda(buf, offs)
+        wb, wo, wf = reference_revcomp(buf, offs, mode, 0.5 if rc_prob is None else rc_prob, 4, 9)
+        st = torch.cuda.current_stream().cuda_stream
+        for shift in range(16):
+            ob = torch.full((wb.size + 64,), 0xA5, dtype=torch.uint8, device="cuda")
+            oo = torch.empty(wo.size, dtype=torch.int64, device="cuda")
+            of = torch.empty(wf.size, dtype=torch.uint8, device="cuda")
+            mode_i = consumers._RC_MODES[mode]
+            capi.revcomp(0, st, b, o, offs.size - 1, mode_i, rc_prob or 0.0, 4, 9, ob.data_ptr() + shift, oo, of)
+            torch.cuda.synchronize()
+            got = ob.cpu().numpy()
+            assert_same_bits(wb, got[shift:shift + wb.size])
+            assert (got[:shift] == 0xA5).all() and (got[shift + wb.size:] == 0xA5).all()  # nothing written outside
+            assert_same_bits(wo, oo.cpu().numpy())
+            assert_same_bits(wf.astype(np.uint8), of.cpu().numpy())
 
 
 def test_empty_batches_huge_row_and_overfull_tiles():

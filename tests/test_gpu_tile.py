@@ -19,7 +19,7 @@ from bioseq_b200 import capi, cbioseq, tile_packed, batch_tokenize_tiled, untile
 from bioseq_b200 import batch_tokenize_varlen, batch_tokenize_mlm, batch_tokenize_kmer, revcomp_packed  # noqa: E402
 from bioseq_b200 import VarlenBatch  # noqa: E402
 from oracle.oracle import flatfile_image  # noqa: E402
-from helpers import assert_same_bits  # noqa: E402
+from helpers import assert_same_bits, table_cap_lens  # noqa: E402
 import tile_reference as ref  # noqa: E402
 from revcomp_reference import revcomp as reference_revcomp  # noqa: E402
 
@@ -66,22 +66,28 @@ def test_edge_lengths_every_source_alignment(tail, W, S):
         check(tile_packed(*cuda(buf, offs), W, stride=S, tail=tail), buf, offs, W, S, tail)
 
 
+# (sequence lengths, W, S): mixed lengths; the same ending in a run of empty sequences (every alignment but one leaves the
+# last vector partial); one window per sequence that fills tiles to the row table's cap and one past it
+ALIGN_CASES = [([0, 5, 40, 3, 129, 77, 1, 300], 24, 10), ([0, 5, 40, 3, 129, 77, 1, 300] + [0] * 40, 24, 10),
+               (table_cap_lens(), 65536, 65536)]
+
+
 @pytest.mark.parametrize("tail", ["short", "end", "drop"])
 def test_every_output_alignment_and_null_outputs(tail):
-    buf, offs = batch_of([0, 5, 40, 3, 129, 77, 1, 300], 3)
-    W, S = 24, 10
-    wb, wo, wsp, wsi, wst = ref.tile(buf, offs, W, S, tail)
-    b, o = cuda(buf, offs)
-    st = torch.cuda.current_stream().cuda_stream
-    for a in range(16):
-        out = torch.full((wb.size + 32,), 0xEE, dtype=torch.uint8, device="cuda")
-        oo = torch.empty(wo.size, dtype=torch.int64, device="cuda")
-        capi.tile(0, st, b, o, len(offs) - 1, W, S, TAILS[tail], out[a:].data_ptr(), oo)  # every optional output NULL
-        torch.cuda.synchronize()
-        h = out.cpu().numpy()
-        assert_same_bits(wb, h[a:a + wb.size])
-        assert (h[:a] == 0xEE).all() and (h[a + wb.size:] == 0xEE).all()
-        assert_same_bits(wo, oo.cpu().numpy())
+    for lens, W, S in ALIGN_CASES:
+        buf, offs = batch_of(lens, 3)
+        wb, wo, wsp, wsi, wst = ref.tile(buf, offs, W, S, tail)
+        b, o = cuda(buf, offs)
+        st = torch.cuda.current_stream().cuda_stream
+        for a in range(16):
+            out = torch.full((wb.size + 32,), 0xEE, dtype=torch.uint8, device="cuda")
+            oo = torch.empty(wo.size, dtype=torch.int64, device="cuda")
+            capi.tile(0, st, b, o, len(offs) - 1, W, S, TAILS[tail], out[a:].data_ptr(), oo)  # every optional output NULL
+            torch.cuda.synchronize()
+            h = out.cpu().numpy()
+            assert_same_bits(wb, h[a:a + wb.size])
+            assert (h[:a] == 0xEE).all() and (h[a + wb.size:] == 0xEE).all()
+            assert_same_bits(wo, oo.cpu().numpy())
 
 
 def test_empty_batches_huge_row_and_many_sequences():

@@ -22,7 +22,7 @@ from bioseq_b200 import batch_tokenize_cropped, batch_tokenize_varlen, batch_tok
 from bioseq_b200 import batch_tokenize_kmer, batch_onehot_encode_bcl, batch_embed, VarlenBatch  # noqa: E402
 from bioseq_b200.loaders import FlatFileDataset  # noqa: E402
 from oracle.oracle import flatfile_image  # noqa: E402
-from helpers import assert_same_bits  # noqa: E402
+from helpers import assert_same_bits, table_cap_lens  # noqa: E402
 import translate_reference as ref  # noqa: E402
 
 SIX = (1, 2, 3, -1, -2, -3)
@@ -89,21 +89,28 @@ def test_edge_lengths_every_source_alignment(frames):
         assert torch.equal(b, keep_b) and torch.equal(o, keep_o)  # the caller's tensors are unchanged
 
 
+# (sequence lengths, frames): mixed lengths; the same ending in a run of empty sequences (every alignment but one leaves
+# the last vector partial); sequences whose frame +1 fills tiles to the row table's cap and one past it
+ALIGN_CASES = [([0, 5, 40, 3, 129, 77, 1, 300, 48, 49, 50], SIX), ([0, 5, 40, 3, 129, 77, 1, 300, 48, 49, 50] + [0] * 40, SIX),
+               ([3 * n for n in table_cap_lens()], (1,))]
+
+
 def test_every_output_alignment():
-    buf, offs = batch_of([0, 5, 40, 3, 129, 77, 1, 300, 48, 49, 50], 3)
-    wb, wo = ref.translate(buf, offs, SIX)
-    b, o = cuda(buf, offs)
-    st = torch.cuda.current_stream().cuda_stream
-    code = capi.genetic_code(1)
-    for a in range(16):
-        out = torch.full((wb.size + 32,), 0xEE, dtype=torch.uint8, device="cuda")
-        oo = torch.empty(wo.size, dtype=torch.int64, device="cuda")
-        capi.translate(0, st, b, o, len(offs) - 1, SIX, code, out[a:].data_ptr(), oo)
-        torch.cuda.synchronize()
-        h = out.cpu().numpy()
-        assert_same_bits(wb, h[a:a + wb.size])
-        assert (h[:a] == 0xEE).all() and (h[a + wb.size:] == 0xEE).all()
-        assert_same_bits(wo, oo.cpu().numpy())
+    for lens, frames in ALIGN_CASES:
+        buf, offs = batch_of(lens, 3)
+        wb, wo = ref.translate(buf, offs, frames)
+        b, o = cuda(buf, offs)
+        st = torch.cuda.current_stream().cuda_stream
+        code = capi.genetic_code(1)
+        for a in range(16):
+            out = torch.full((wb.size + 32,), 0xEE, dtype=torch.uint8, device="cuda")
+            oo = torch.empty(wo.size, dtype=torch.int64, device="cuda")
+            capi.translate(0, st, b, o, len(offs) - 1, frames, code, out[a:].data_ptr(), oo)
+            torch.cuda.synchronize()
+            h = out.cpu().numpy()
+            assert_same_bits(wb, h[a:a + wb.size])
+            assert (h[:a] == 0xEE).all() and (h[a + wb.size:] == 0xEE).all()
+            assert_same_bits(wo, oo.cpu().numpy())
 
 
 @pytest.mark.parametrize("code", [1, 2, 4, 5, 6, 11, "custom"])
